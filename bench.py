@@ -2,7 +2,7 @@
 """bench.py -- BP4 CG throughput of the B200-native hot path (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--degree P] [--s S] [--solver merged|plain]
-                  [--mode weak|strong] [--sweep none|default|full]
+                  [--mode weak|strong] [--sweep none|default|full] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the reference algorithm's CPU restatement on host cores
 
 A "step" is one call of the reference's `run_cg_solver` plugin (benchmark.h:193: x0 = 0,
@@ -22,6 +22,12 @@ reference's own `dofs/s/it` column (benchmark.h:222): n_dofs * n_iterations / so
             merged, Q2..Q8 at ~100 M DoFs (merged; plain too with --sweep full)
 Multi-GPU: --mode weak (default) runs s + log2(N) (fixed DoFs per GPU); --mode strong keeps s.
 One JSON line on stdout (rank 0).
+
+  --dump-outputs DIR  after the timed steps, rank 0 writes what the last of them returned to its
+            caller (the end-to-end loop's last run_cg_solver call): DIR/x.npy, the solution of its owned
+            DoFs (float64; above DUMP_MAX_ENTRIES entries a fixed, seeded sample of them), and
+            DIR/iterations.npy.  The inputs depend on the arguments only, so two builds of the
+            project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +47,8 @@ METRIC = "BP4 CG GDoF/s (DoFs x iterations / s)"
 UNIT = "GDoF/s"
 # BASELINE.json configs[3]: Q2..Q8 at ~100 M DoFs (SURVEY 8d)
 DEGREE_SWEEP = [(2, 22), (3, 20), (4, 19), (5, 18), (6, 17), (7, 16), (8, 16)]
+# --dump-outputs: 16 MB of float64 at most for the solution (Q4 s=18 has 51 M DoFs = 407 MB)
+DUMP_MAX_ENTRIES = 1 << 21
 
 
 def n_dofs_of(p, s):
@@ -59,6 +67,17 @@ def cell_kernel_bytes(n_dofs, n_cells, n_private):
     """operator apply 16 B/DoF + 300 B/cell; the in-loop do_cg_update4b/3b add the remaining
     58.67 - 16 B/DoF of the merged iteration on the DoFs they cover"""
     return 16.0 * n_dofs + 300.0 * n_cells + (58.0 + 2.0 / 3.0 - 16.0) * n_private
+
+
+def dump_outputs(out_dir, x, iterations):
+    """--dump-outputs: x.npy (the solution, or the entries at DUMP_MAX_ENTRIES positions drawn with a
+    fixed seed when it is longer) and iterations.npy, both float64"""
+    import numpy as np
+    if x.size > DUMP_MAX_ENTRIES:
+        x = x[np.sort(np.random.default_rng(0).choice(x.size, DUMP_MAX_ENTRIES, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), np.asarray(x, dtype=np.float64))
+    np.save(os.path.join(out_dir, "iterations.npy"), np.array([iterations], dtype=np.float64))
 
 
 def measured_peak():
@@ -160,7 +179,7 @@ def run_reference(args):
     s = min(s_gpu, args.cpu_s)          # the numpy set-up of the oracle needs ~0.2 kB per DoF
     merged = args.solver == "merged"
     arm = CpuArm(args.degree, s, merged)
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     for _ in range(warmup):
         arm.step(min(args.cpu_iters, 3))
     its, sec = 0, 0.0
@@ -253,7 +272,13 @@ def main():
     ap.add_argument("--solver", default="merged", choices=["merged", "plain"])
     ap.add_argument("--sweep", default="default", choices=["none", "default", "full"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the solution and iteration count of the last timed solve to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -351,6 +376,8 @@ def main():
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
     e2e_value = n_dofs * e2e_iters / float(dt.item()) * 1e-9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x_np, it_c.value)
 
     per_rank = None
     if world > 1:   # every rank's share of the iteration (the slowest one sets the pace)

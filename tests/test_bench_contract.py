@@ -1,13 +1,18 @@
-"""CPU checks of bench.py: the size/byte helpers against SURVEY App. C / 8(d), the JSON line of
-the `--impl reference` arm (the CPU restatement on a tiny sample), rank > 0 staying silent, and
-the loud failure of the product arm without a GPU."""
+"""Checks of bench.py: the size/byte helpers against SURVEY App. C / 8(d), the JSON line of the
+`--impl reference` arm (the CPU restatement on a tiny sample), rank > 0 staying silent, the loud
+failure of the product arm without a GPU, and what --dump-outputs writes."""
 import importlib.util
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
+
+from oracle import bp4_oracle as O
+
+from helpers import rel_l2, single
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -68,3 +73,43 @@ def test_product_arm_fails_loudly_without_gpu():
              "--no-cpu-baseline")
     assert r.returncode != 0          # no CPU fallback, no JSON line
     assert not any(ln.startswith("{") for ln in r.stdout.splitlines())
+
+
+def test_dump_outputs_files(tmp_path):
+    """float64 .npy files of 64 MB at most; a long solution is sampled at the same positions on
+    every call, a short one is written whole"""
+    b = _bench_module()
+    x = np.arange(3 * b.DUMP_MAX_ENTRIES, dtype=np.float64)
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), x, 37)
+    xa, xb = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "b" / "x.npy")
+    assert xa.dtype == np.float64 and xa.size == b.DUMP_MAX_ENTRIES and np.array_equal(xa, xb)
+    assert np.all(np.diff(xa) > 0) and 0 <= xa[0] and xa[-1] < x.size     # distinct entries of x
+    it = np.load(tmp_path / "a" / "iterations.npy")
+    assert it.dtype == np.float64 and it.tolist() == [37.0]
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20
+    short = np.random.default_rng(1).standard_normal(1000)
+    b.dump_outputs(str(tmp_path / "c"), short, 5)
+    assert np.array_equal(np.load(tmp_path / "c" / "x.npy"), short)
+
+
+def test_dump_outputs_rejected_for_reference_arm(tmp_path):
+    r = _run(None, "--impl", "reference", "--dump-outputs", str(tmp_path / "d"))
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_solution(tmp_path, c_oracle_lib):
+    """bench.py --dump-outputs on a small mesh: the dumped solution and iteration count are those
+    of the C oracle's merged CG, and --steps sets the number of timed solves"""
+    out = tmp_path / "dump"
+    r = _run(None, "--steps", "2", "--warmup", "1", "--degree", "3", "--s", "6", "--sweep", "none",
+             "--no-cpu-baseline", "--dump-outputs", str(out))
+    assert r.returncode == 0, r.stderr
+    d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    x, it = np.load(out / "x.npy"), np.load(out / "iterations.npy")
+    assert d["steps"] == 2 and abs(d["iterations_per_step"] - int(it[0])) <= 1
+    rd, co = single(3, 6)
+    xo, ito, _ = co.cg(rd.rhs, O.finish_inverse_diagonal(O.inverse_diagonal(rd)), merged=True)
+    assert abs(int(it[0]) - ito) <= 1
+    assert rel_l2(x, xo) <= (1e-8 if ito < 100 else 1e-6)
