@@ -55,16 +55,6 @@ namespace
     }                                                                                         \
   while (0)
 
-// Which form of vmult_with_merged_sums a context starts with when the descriptor carries range
-// tables: true = vector updates inside the cell loop, false = streamed before/after it.  Set from
-// the B200 measurements (DESIGN.md 4.2): the in-loop form wins at Q4 on one rank (2.12 vs 2.14 ms),
-// loses at Q2/Q3 and has no kernel above Q4; on several ranks the loop is three launches with a
-// unit-granular tail each, which has not been measured to pay - bp4_comm_init goes back to the
-// streamed form.  bp4_debug_set_fused / BP4_FUSED override both.
-#ifndef BP4_FUSED_DEFAULT
-#  define BP4_FUSED_DEFAULT(P) ((P) == 4)
-#endif
-
 struct bp4_vec
 {
   double  *buf = nullptr;
@@ -93,10 +83,8 @@ struct bp4_ctx
   double      *d_acc  = nullptr; // [8] reduction scratch
   int         *d_flag = nullptr;
   uint32_t    *d_sched = nullptr; // [4] unit counters of the cell-kernel launches of one loop
-  uint32_t     stagger_ns = 0;    // developer knob BP4_STAGGER_NS
   double      *h_acc  = nullptr; // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
   unsigned long long pub_seq = 0;
-  int          spin_wait = 1;    // BP4_SPIN_WAIT=0: cudaMemcpyAsync + cudaStreamSynchronize instead
   int         *h_flag = nullptr; // pinned
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
@@ -222,30 +210,22 @@ namespace
   {
     if (c->comm)
       NC(ncclAllReduce(c->d_acc, c->d_acc, k, ncclDouble, ncclSum, c->comm, c->stream));
-    if (c->spin_wait)
-      {
-        // the last kernel of the chain writes the values and then a sequence number into mapped
-        // pinned memory; the host polls that word (and the stream, for errors, now and then)
-        volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc + 8);
-        const unsigned long long     seq      = ++c->pub_seq;
-        CU(bp4::launch_publish(c->d_acc, k, c->h_acc, const_cast<unsigned long long *>(seq_word), seq, c->stream));
-        c->launches += 1;
-        int idle = 0;
-        for (unsigned long long spins = 1; *seq_word != seq; ++spins)
-          if ((spins & 0xFFFF) == 0)
-            {
-              const cudaError_t q = cudaStreamQuery(c->stream);
-              if (q != cudaSuccess && q != cudaErrorNotReady)
-                CU(q);
-              if (q == cudaSuccess && ++idle > 8) // stream drained, nothing published: cannot happen
-                return fail(BP4_ERR_CUDA, "reduction result was not published");
-            }
-      }
-    else
-      {
-        CU(cudaMemcpyAsync(c->h_acc, c->d_acc, sizeof(double) * k, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-      }
+    // the last kernel of the chain writes the values and then a sequence number into mapped
+    // pinned memory; the host polls that word (and the stream, for errors, now and then)
+    volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc + 8);
+    const unsigned long long     seq      = ++c->pub_seq;
+    CU(bp4::launch_publish(c->d_acc, k, c->h_acc, const_cast<unsigned long long *>(seq_word), seq, c->stream));
+    c->launches += 1;
+    int idle = 0;
+    for (unsigned long long spins = 1; *seq_word != seq; ++spins)
+      if ((spins & 0xFFFF) == 0)
+        {
+          const cudaError_t q = cudaStreamQuery(c->stream);
+          if (q != cudaSuccess && q != cudaErrorNotReady)
+            CU(q);
+          if (q == cudaSuccess && ++idle > 8) // stream drained, nothing published: cannot happen
+            return fail(BP4_ERR_CUDA, "reduction result was not published");
+        }
     for (int i = 0; i < k; ++i)
       out[i] = c->h_acc[i];
     return 0;
@@ -325,8 +305,6 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   if (c->n_before + c->n_comm > c->n_cells)
     return fail(BP4_ERR_ARG, "cell partitions exceed n_cells");
   CU(cudaDeviceGetAttribute(&c->sms, cudaDevAttrMultiProcessorCount, d->device));
-  if (const char *e = getenv("BP4_STAGGER_NS"))
-    c->stagger_ns = (uint32_t)atoi(e);
   CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   CU(cudaStreamCreateWithFlags(&c->comm_stream, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&c->ev_a, cudaEventDisableTiming));
@@ -381,8 +359,6 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   CU(cudaMalloc(&c->d_sched, sizeof(uint32_t) * 4));
   CU(cudaMallocHost(&c->h_acc, sizeof(double) * 16)); // UVA: the pointer is valid on the device too
   memset(c->h_acc, 0, sizeof(double) * 16);
-  if (const char *e = getenv("BP4_SPIN_WAIT"))
-    c->spin_wait = atoi(e) != 0;
   CU(cudaMallocHost(&c->h_flag, sizeof(int)));
 
   // cell-batch ranges and their private DoF runs -> units and batches of the fused merged loop
@@ -411,9 +387,10 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
           if (rc[rcut[k]] != cut[k])
             return fail(BP4_ERR_ARG, "a cell-batch range straddles a cell partition boundary");
         }
-      const uint32_t cpb = (uint32_t)bp4::cells_per_block(d->degree);
+      bp4::FusedLoopCfg fl;
+      CU(bp4::fused_loop_config(d->degree, fl));
       const uint32_t rsz = rc[1] - rc[0];
-      uint32_t       target = cpb / gcd_u32(cpb, rsz) * rsz; // lcm: whole ranges in whole batches
+      uint32_t       target = fl.cpb / gcd_u32(fl.cpb, rsz) * rsz; // lcm: whole ranges in whole batches
       while (target > 64 && target > rsz)
         target -= rsz;
       std::vector<bp4::BatchDesc> batches;
@@ -421,7 +398,7 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
       for (int k = 0; k < 3; ++k)
         {
           c->unit_part[k] = (uint32_t)unit_batch.size();
-          build_units(rc, rp, rcut[k], rcut[k + 1], cpb, target, batches, unit_batch);
+          build_units(rc, rp, rcut[k], rcut[k + 1], fl.cpb, target, batches, unit_batch);
         }
       c->unit_part[3] = (uint32_t)unit_batch.size();
       unit_batch.push_back((uint32_t)batches.size());
@@ -432,11 +409,10 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
                     cudaMemcpyHostToDevice));
       c->n_private = c->n_coef == 24 ? rp[d->n_ranges] : 0; // in-loop updates: tri-linear kernel only
       // the staged fused loop takes a batch's private run in two jobs of its shared-memory rows
-      const uint32_t limit = bp4::fused_run_limit(d->degree); // 0: no fused kernel at this degree
-      for (const bp4::BatchDesc &b : batches)
-        if (b.pre_end - b.pre_begin > limit || b.post_end - b.post_begin > limit)
+      for (const bp4::BatchDesc &b : batches) // run_limit 0: no fused kernel at this degree
+        if (b.pre_end - b.pre_begin > fl.run_limit || b.post_end - b.post_begin > fl.run_limit)
           c->n_private = 0; // the updates of every DoF are streamed then
-      c->fused     = BP4_FUSED_DEFAULT(d->degree) && c->n_private > 0;
+      c->fused     = fl.is_default && c->n_private > 0;
       if (const char *e = getenv("BP4_FUSED")) // developer knob: 0 = pre kernel + cells + post kernel
         {
           c->fused        = c->n_private > 0 && atoi(e) != 0;
@@ -684,8 +660,6 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
   a.src   = src;
   a.dst   = dst;
   a.sched = c->d_sched + (part < 0 ? 0 : part);
-  a.stagger_ns  = c->stagger_ns;
-  a.claim_depth = 5;
   if (m)
     {
       const uint32_t u0 = part < 0 ? c->unit_part[0] : c->unit_part[part],
@@ -993,8 +967,6 @@ int bp4_dot(bp4_ctx *c, const bp4_vec *a, const bp4_vec *b, double *result)
   if (!c || !a || !b || !result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  if (!c->spin_wait) // the publish kernel leaves the accumulators cleared
-    CU(cudaMemsetAsync(c->d_acc, 0, sizeof(double), c->stream));
   {
     Timed t(c, BP4_K_BLAS1);
     CU(bp4::launch_dot(sweep_len(c, {a, b}), a->p(), b->p(), c->d_acc, c->sms, c->stream));
@@ -1007,8 +979,6 @@ int bp4_add_and_dot(bp4_ctx *c, bp4_vec *g, double a, const bp4_vec *h, const bp
   if (!c || !g || !h || !w || !result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  if (!c->spin_wait) // the publish kernel leaves the accumulators cleared
-    CU(cudaMemsetAsync(c->d_acc, 0, sizeof(double), c->stream));
   {
     Timed t(c, BP4_K_BLAS1);
     CU(bp4::launch_add_and_dot(sweep_len(c, {g, h, w}), g->p(), a, h->p(), w->p(), c->d_acc, c->sms, c->stream));
@@ -1196,7 +1166,7 @@ int bp4_comm_init(bp4_ctx *c, int rank, int n_ranks, const unsigned char id[BP4_
   c->rank    = rank;
   c->n_ranks = n_ranks;
   if (n_ranks > 1 && !c->fused_pinned)
-    c->fused = 0; // see BP4_FUSED_DEFAULT
+    c->fused = 0; // see Cfg<P>::FUSED_DEFAULT
   return p2p_setup(c);
 }
 

@@ -7,32 +7,6 @@
 #include "bp4_launch.h"
 #include "bp4_tables.h"
 
-// degrees >= BP4_FINE_FROM run phases 1 and 3 as fine-grained sweeps (phase1a..c, phase3a..c)
-#ifndef BP4_P2_CALL_FROM
-#  define BP4_P2_CALL_FROM 6 // degrees >= this call phase 2 out of line
-#endif
-#ifndef BP4_PIPE_GATHER
-#  define BP4_PIPE_GATHER(P) ((P) <= 4)
-#endif
-#ifndef BP4_SU
-#  define BP4_SU 6 // scatter unroll
-#endif
-#ifndef BP4_FINE_FROM
-#  define BP4_FINE_FROM 6
-#endif
-#ifndef BP4_DYNAMIC
-// batches / units are claimed from an atomic counter instead of strided.  Measured on B200 (operator
-// apply at ~50-100 M DoFs): Q2 +13 %, Q3 +5 %, Q4 +8 %, Q5 +11 %; Q6 -6 %, Q7 -11 %, Q8 -10 % (the
-// claim bookkeeping makes the register-starved high-degree kernels spill), hence P <= 5.
-#  define BP4_DYNAMIC(P) ((P) <= 5)
-#endif
-#ifndef BP4_PRE_UNROLL
-#  define BP4_PRE_UNROLL 4 // measured: 1 -> 0.496 ms, 2 -> 0.484, 4 -> 0.474 (6.3 TB/s), 6/8 -> 0.48 (Q4 s=18)
-#endif
-#ifndef BP4_POST_UNROLL
-#  define BP4_POST_UNROLL 4 // measured: 1 -> 0.233 ms, 4 -> 0.211 ms (6.45 TB/s), 2 and 8 slower (Q4 s=18)
-#endif
-
 namespace bp4
 {
   // one table per degree in the constant bank: with fully unrolled contractions every
@@ -181,14 +155,12 @@ namespace bp4
   // pre_kernel / post_kernel stream them before / after this kernel.
   // ---------------------------------------------------------------------------------------
   template <int P, int CPB, bool FUSED, bool QUAD>
-  __global__ void __launch_bounds__(Cfg<P>::THREADS, Cfg<P>::BLOCKS) cell_kernel(const CellArgs a)
+  __global__ void __launch_bounds__(kThreads, Cfg<P>::BLOCKS) cell_kernel(const CellArgs a)
   {
     constexpr int NC = Cfg<P, QUAD>::NCOEF;
-    constexpr int kThreads = Cfg<P>::THREADS; // shadows the namespace default inside this kernel
     using G         = Geom<P>;
     constexpr int Q = G::Q;
-    // high degrees: phases 1 and 3 as one sweep per 1-D contraction (see phase1a)
-    constexpr bool kFine = P >= BP4_FINE_FROM;
+    constexpr bool kFine = Cfg<P>::FINE;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     CellSmem<P, CPB, NC> &sm  = *reinterpret_cast<CellSmem<P, CPB, NC> *>(smem_raw);
     const int             tid = threadIdx.x;
@@ -197,7 +169,7 @@ namespace bp4
     BP4_TICK_INIT
     // ---- work list of this block: a unit is one batch (plain) or the batches
     // [unit_batch[u], unit_batch[u+1]) of whole ranges (fused).  Units are claimed dynamically
-    // (BP4_DYNAMIC): the first one is blockIdx.x, the following ones come from an atomic counter,
+    // (Cfg<P>::DYNAMIC): the first one is blockIdx.x, the following ones come from an atomic counter,
     // a few units ahead of their use so that the claim's latency never shows.  The two blocks of
     // an SM run at different speeds (the warp scheduler favours one of them: measured 10.2 vs
     // 14.1 us per batch at Q4), a static split would leave the slower one with a long tail.
@@ -207,10 +179,12 @@ namespace bp4
       bool     valid;
     };
     const uint32_t n_units = FUSED ? a.n_units : (uint32_t)((a.n_cells + CPB - 1) / CPB);
-    const bool     dynamic = BP4_DYNAMIC(P) && a.sched != nullptr;
+    const bool     dynamic = Cfg<P>::DYNAMIC && a.sched != nullptr;
     auto           unit_at = [&](const uint32_t j) {
       return dynamic ? sm.units[j & 7u] : blockIdx.x + j * gridDim.x;
     };
+    // units a block holds claimed (the current one included) in the plain and in the fused loop
+    constexpr uint32_t kClaimDepth = 5, kClaimDepthFused = 2;
     // thread 0 only; visible after the next barrier
     auto claim_ahead = [&](const uint32_t j_from, const uint32_t depth) {
       if (dynamic)
@@ -320,7 +294,7 @@ namespace bp4
     // The fused kernel reads the direction with plain loads, not ld.global.nc: it was written by
     // this block's own do_cg_update4b moments ago (the L1 sees the stores of its own SM, every
     // other DoF the block reads is constant during the kernel).
-    constexpr bool kPipe = BP4_PIPE_GATHER(P);
+    constexpr bool kPipe = Cfg<P>::PIPE_GATHER;
     constexpr int R = (G::DOF + kThreads - 1) / kThreads, S = CPB * R;
     // only the last r can run past the end of the cell
     const bool last_on = tid < G::DOF - (R - 1) * kThreads;
@@ -358,7 +332,7 @@ namespace bp4
     // scatter-add (vector_access_reduced.h:437-521); the cell-interior entity (13) is touched by
     // this cell only -> plain store
     auto scatter = [&](const int bf) {
-      constexpr int SU = BP4_SU;
+      constexpr int SU = 6; // DoFs whose operands are read before their REDs go out
       uint32_t      tt[R];
 #pragma unroll
       for (int r = 0; r < R; ++r)
@@ -419,7 +393,7 @@ namespace bp4
         {
           const int cell = it / G::ITEMS2, r = it % G::ITEMS2;
           const int qz = r / Q, qx = r % Q;
-          if constexpr (P >= BP4_P2_CALL_FROM)
+          if constexpr (Cfg<P>::P2_CALL)
             phase2_call<P, QUAD>((uint32_t)((const unsigned char *)sm.coef[bf][cell] - smem_raw),
                                  (uint32_t)((const unsigned char *)(sm.work + cell * G::WORK) - smem_raw), qx, qz,
                                  sm.xq[qx], sm.xq[qz], sm.wq[qx] * sm.wq[qz]);
@@ -452,14 +426,8 @@ namespace bp4
       {
         sm.units[0]  = blockIdx.x;
         sm.n_claimed = 1;
-        claim_ahead(0, 5);
+        claim_ahead(0, kClaimDepth);
       }
-    // All blocks start together and do the same amount of work per batch, so without help they
-    // reach their memory windows together: HBM sees bursts and idles in between (trace:
-    // 0..294 of 296 blocks in the window at any one time).  A start offset spread over about one
-    // batch period de-phases them once; with equal periods they stay de-phased.
-    if (a.stagger_ns)
-      __nanosleep((unsigned)(((unsigned long long)(blockIdx.x * 2654435761u) * a.stagger_ns) >> 32));
     __syncthreads();
 
     if constexpr (!FUSED)
@@ -507,7 +475,7 @@ namespace bp4
             BP4_TRACE(i, 0)
             BP4_TRACE(i, 4)
             if (tid == 0)
-              claim_ahead(cur_it.j, a.claim_depth);
+              claim_ahead(cur_it.j, kClaimDepth);
             if (nxt_it.valid)
               fetch_meta(nxt.cell0, nxt.nc); // lands during the phases
             phase_1(nc);
@@ -825,7 +793,7 @@ namespace bp4
               job_issue(pb, job_split(pb, pe), true);
             }
             if (tid == 0)
-              claim_ahead(hd.j, 2);
+              claim_ahead(hd.j, kClaimDepthFused);
             if (vm & 1u)
               meta_async(bf ^ 1, dn.cell0, (int)dn.n_cells);
             phase_1(nc);
@@ -970,8 +938,9 @@ namespace bp4
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     const double   c1 = alpha_old != 0. ? alpha + alpha_old / beta_old : 0.;
     const double   c2 = alpha_old != 0. ? alpha_old / beta_old : 0.;
-    // BP4_PRE_UNROLL independent elements per trip: all their loads are in flight together
-    constexpr int U = BP4_PRE_UNROLL;
+    // U independent elements per trip: all their loads are in flight together.  Measured at Q4
+    // s=18: U = 1 -> 0.496 ms, 2 -> 0.484, 4 -> 0.474 (6.3 TB/s), 6/8 -> 0.48
+    constexpr int U = 4;
     for (uint64_t i0 = begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < end; i0 += U * stride)
       {
         double pr[U], ri[U], pi[U], hi[U], xi[U];
@@ -1017,9 +986,9 @@ namespace bp4
   {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     double         s[7]   = {0., 0., 0., 0., 0., 0., 0.};
-#if BP4_POST_UNROLL > 1
-    // BP4_POST_UNROLL independent element groups per trip: all their loads are in flight together
-    constexpr int U = BP4_POST_UNROLL;
+    // U independent element groups per trip: all their loads are in flight together.  Measured at
+    // Q4 s=18: U = 1 -> 0.233 ms, 4 -> 0.211 ms (6.45 TB/s), 2 and 8 slower
+    constexpr int U = 4;
     for (uint64_t i0 = begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < end; i0 += U * stride)
       {
         double rr[U], dd[U], hh[U], pp[U];
@@ -1037,10 +1006,6 @@ namespace bp4
         for (int u = 0; u < U; ++u)
           post_terms(s, rr[u], dd[u], hh[u], pp[u]);
       }
-#else
-    for (uint64_t i = begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < end; i += stride)
-      post_terms(s, r[i], d[i], h[i], prec[i / 3]);
-#endif
     block_accumulate<7>(s, acc);
   }
 
@@ -1337,12 +1302,12 @@ namespace bp4
     if (fused)
       {
         if constexpr (Stage<P>::OK)
-          cell_kernel<P, CPB, true, false><<<grid, Cfg<P>::THREADS, fused_smem<P>(), st>>>(a);
+          cell_kernel<P, CPB, true, false><<<grid, kThreads, fused_smem<P>(), st>>>(a);
       }
     else if (quad)
-      cell_kernel<P, CPBQ, false, true><<<grid, Cfg<P>::THREADS, sizeof(CellSmem<P, CPBQ, 81>), st>>>(a);
+      cell_kernel<P, CPBQ, false, true><<<grid, kThreads, sizeof(CellSmem<P, CPBQ, 81>), st>>>(a);
     else
-      cell_kernel<P, CPB, false, false><<<grid, Cfg<P>::THREADS, sizeof(CellSmem<P, CPB, 24>), st>>>(a);
+      cell_kernel<P, CPB, false, false><<<grid, kThreads, sizeof(CellSmem<P, CPB, 24>), st>>>(a);
 #ifdef BP4_PHASE_TIMING
     if (d_trace)
       {
@@ -1369,7 +1334,7 @@ namespace bp4
           tot += double(h[k]);
         fprintf(stderr, "phase clk share: meta %.1f%% gather %.1f%% barrier %.1f%% P1 %.1f%% P2 %.1f%% P3 %.1f%% scatter %.1f%% post %.1f%% | per-warp total %.0f clk\n",
                 100 * h[0] / tot, 100 * h[1] / tot, 100 * h[2] / tot, 100 * h[3] / tot, 100 * h[4] / tot,
-                100 * h[5] / tot, 100 * h[6] / tot, 100 * h[7] / tot, tot / (grid * (Cfg<P>::THREADS / 32)));
+                100 * h[5] / tot, 100 * h[6] / tot, 100 * h[7] / tot, tot / (grid * (kThreads / 32)));
       }
 #endif
     return cudaGetLastError();
@@ -1402,50 +1367,18 @@ namespace bp4
 #undef CALL
   }
 
-  int cells_per_block(int degree, bool quad)
+  template <int P>
+  static cudaError_t fused_loop_cfg(FusedLoopCfg &out)
   {
-    switch (degree)
-      {
-        case 2: return quad ? Cfg<2, true>::CPB : Cfg<2>::CPB;
-        case 3: return quad ? Cfg<3, true>::CPB : Cfg<3>::CPB;
-        case 4: return quad ? Cfg<4, true>::CPB : Cfg<4>::CPB;
-        case 5: return quad ? Cfg<5, true>::CPB : Cfg<5>::CPB;
-        case 6: return quad ? Cfg<6, true>::CPB : Cfg<6>::CPB;
-        case 7: return quad ? Cfg<7, true>::CPB : Cfg<7>::CPB;
-        case 8: return quad ? Cfg<8, true>::CPB : Cfg<8>::CPB;
-      }
-    return 0;
+    out = {(uint32_t)Cfg<P>::CPB, Stage<P>::OK ? (uint32_t)Stage<P>::LIMIT : 0u, Cfg<P>::FUSED_DEFAULT};
+    return cudaSuccess;
   }
 
-  // longest private run (DoFs) one batch of the fused loop may carry; 0 = the degree has no fused kernel
-  uint32_t fused_run_limit(int degree)
+  cudaError_t fused_loop_config(int degree, FusedLoopCfg &out)
   {
-    switch (degree)
-      {
-        case 2: return Stage<2>::OK ? Stage<2>::LIMIT : 0;
-        case 3: return Stage<3>::OK ? Stage<3>::LIMIT : 0;
-        case 4: return Stage<4>::OK ? Stage<4>::LIMIT : 0;
-        case 5: return Stage<5>::OK ? Stage<5>::LIMIT : 0;
-        case 6: return Stage<6>::OK ? Stage<6>::LIMIT : 0;
-        case 7: return Stage<7>::OK ? Stage<7>::LIMIT : 0;
-        case 8: return Stage<8>::OK ? Stage<8>::LIMIT : 0;
-      }
-    return 0;
-  }
-
-  int blocks_per_sm(int degree)
-  {
-    switch (degree)
-      {
-        case 2: return Cfg<2>::BLOCKS;
-        case 3: return Cfg<3>::BLOCKS;
-        case 4: return Cfg<4>::BLOCKS;
-        case 5: return Cfg<5>::BLOCKS;
-        case 6: return Cfg<6>::BLOCKS;
-        case 7: return Cfg<7>::BLOCKS;
-        case 8: return Cfg<8>::BLOCKS;
-      }
-    return 0;
+#define CALL(P) fused_loop_cfg<P>(out)
+    BP4_DISPATCH(degree, CALL)
+#undef CALL
   }
 
   cudaError_t launch_pre(uint64_t begin, uint64_t end, double *h, double *x, double *r, double *p,

@@ -16,35 +16,43 @@ namespace bp4
   // may use up to 255 registers per thread (phase 2 keeps 9*Q doubles live), and while one
   // block waits on its gather or a barrier the other keeps the FP64 pipe busy.
   constexpr int kThreads     = 128;
-#ifndef BP4_WIDE
-#  define BP4_WIDE(P) false
-#endif
-#ifndef BP4_STAGED
-// degrees with a fused cell kernel (in-loop vector updates staged through shared memory)
-#  define BP4_STAGED(P) ((P) <= 4)
-#endif
   constexpr int kBlocksPerSM = 2;
 
+  // Every per-degree choice of the cell kernel, each one measured on B200 (DESIGN.md 4.1-4.2, 6).
   // QUAD: all 27 geometry coefficients per cell (81 doubles) instead of the 8 tri-linear ones (24)
   template <int P, bool QUAD = false>
   struct Cfg
   {
     using G = Geom<P>;
     static constexpr int NCOEF = QUAD ? 81 : 24;
-    // "wide" configuration: ONE block of 256 threads per SM (255 registers, no spills) whose
-    // batch fills phase 2 exactly (Q6: 4 cells = 256 lines, Q7: 3 cells = 243 lines)
-    static constexpr bool WIDE    = BP4_WIDE(P);
-    static constexpr int  THREADS = WIDE ? 256 : kThreads;
     // resident blocks per SM of the cell kernel: three (<= 168 registers, smaller batches)
     // measured faster at Q2 (+12 %) and Q6 (+13 %), slower or equal elsewhere
-    static constexpr int BLOCKS   = WIDE ? 1 : ((P == 2 || P == 6) ? 3 : kBlocksPerSM);
+    static constexpr int BLOCKS   = (P == 2 || P == 6) ? 3 : kBlocksPerSM;
     static constexpr int budget   = (227 * 1024) / BLOCKS - 512;
     static constexpr int per_cell = (G::WORK + 2 * NCOEF) * 8 + 2 * 28 * 4;
     static constexpr int fit      = (budget - 4 * G::DOF - 16 * G::Q - 256) / per_cell;
-    // phase 2 carries ~2/3 of the FP64 work: prefer Q^2*CPB close to a multiple of the block
-    static constexpr int rounds = WIDE ? 1 : 2;
-    static constexpr int want   = (rounds * THREADS) / (G::Q * G::Q) > 0 ? (rounds * THREADS) / (G::Q * G::Q) : 1;
-    static constexpr int CPB    = fit < 1 ? 1 : (fit < want ? fit : want);
+    // phase 2 carries ~2/3 of the FP64 work: prefer Q^2*CPB close to two rounds of the block
+    static constexpr int want = (2 * kThreads) / (G::Q * G::Q) > 0 ? (2 * kThreads) / (G::Q * G::Q) : 1;
+    static constexpr int CPB  = fit < 1 ? 1 : (fit < want ? fit : want);
+    // phases 1 and 3 as one sweep per 1-D contraction (phase1a..c, phase3a..c): with 3N rows per
+    // cell the high degrees have too few items for 128 threads (29-52 % barrier wait at Q6-Q8)
+    static constexpr bool FINE = P >= 6;
+    // phase 2 called out of line (phase2_call)
+    static constexpr bool P2_CALL = P >= 6;
+    // the gather of batch i+1 is in flight during the scatter of batch i
+    static constexpr bool PIPE_GATHER = P <= 4;
+    // batches / units are claimed from an atomic counter instead of strided.  Measured on B200
+    // (operator apply at ~50-100 M DoFs): Q2 +13 %, Q3 +5 %, Q4 +8 %, Q5 +11 %; Q6 -6 %, Q7 -11 %,
+    // Q8 -10 % (the claim bookkeeping makes the register-starved high-degree kernels spill)
+    static constexpr bool DYNAMIC = P <= 5;
+    // a fused cell kernel (in-loop vector updates staged through shared memory) is built; see Stage
+    static constexpr bool STAGED = P <= 4;
+    // the form of vmult_with_merged_sums a context starts with when it has private DoF runs:
+    // in-loop updates (true) or streamed before/after the cell loop.  The in-loop form wins at Q4
+    // on one rank (2.12 vs 2.14 ms per iteration) and loses at Q2/Q3; on several ranks the loop is
+    // three launches with a unit-granular tail each, which has not been measured to pay, so
+    // bp4_comm_init goes back to the streamed form.  bp4_debug_set_fused / BP4_FUSED override both.
+    static constexpr bool FUSED_DEFAULT = P == 4;
   };
 
   template <int P, int CPB, int NCOEF = 24>
@@ -113,7 +121,7 @@ namespace bp4
     static constexpr long cap   = ((avail / 8 - 11) * 3) / 10;
     static constexpr int  JOB   = cap < 64 ? 0 : (int)(cap & ~1L);
     static constexpr int  LIMIT = 2 * JOB;
-    static constexpr bool OK    = BP4_STAGED(P) && JOB >= 64;
+    static constexpr bool OK    = Cfg<P>::STAGED && JOB >= 64;
   };
 
   struct CellArgs
@@ -125,8 +133,6 @@ namespace bp4
     const double   *src;          // plain: input vector; fused: the search direction d (= p)
     double         *dst;          // plain: output vector; fused: h
     uint32_t       *sched;        // unit counter of this launch (zero at launch), null: strided
-    uint32_t        stagger_ns;   // start offsets of the blocks are spread over [0, stagger_ns)
-    uint32_t        claim_depth;  // plain: units a block holds claimed (the current one included)
     // ---- fused (vmult_with_merged_sums) only ----
     const BatchDesc *batch;       // batches of all units
     const uint32_t  *unit_batch;  // [n_units + 1] first batch of every unit of this launch

@@ -1,6 +1,6 @@
 #!/bin/bash
 # developer tool: build libbp4 with extra nvcc flags into mf_data_locality_b200/variants/libbp4_NAME.so
-# usage: scripts/build_variant.sh NAME [-DBP4_PRE_UNROLL=2 -DBP4_PHASE_TIMING ...]; on the GPU box copy it over libbp4.so to probe it
+# usage: scripts/build_variant.sh NAME [nvcc flags, e.g. -DBP4_PHASE_TIMING]; copy the result over libbp4.so to probe it
 set -e
 name=$1; shift
 root=$(cd "$(dirname "$0")/.." && pwd)
