@@ -15,7 +15,7 @@
  *     host thread (the reference runs one thread per MPI rank, benchmark.h:278).
  *   - calls are asynchronous on the context's stream except those that return host
  *     scalars (bp4_dot, bp4_l2_norm, bp4_add_and_dot, bp4_all_zero, bp4_vmult_merged,
- *     bp4_vec_download), which synchronise.
+ *     bp4_vec_download, bp4_solve_cg, bp4_solve_cg_merged), which synchronise.
  *   - vectors hold n_owned + n_ghost doubles: owned DoFs first (renumbered, three
  *     components interleaved per node), then ghost DoFs sorted by global index --
  *     the layout of LinearAlgebra::distributed::Vector<double>.
@@ -159,6 +159,42 @@ int bp4_add_and_dot(bp4_ctx *ctx, bp4_vec *g, double a, const bp4_vec *h, const 
                     double *result);                                /* g += a h; return g.w */
 int bp4_l2_norm(bp4_ctx *ctx, const bp4_vec *v, double *result);
 int bp4_all_zero(bp4_ctx *ctx, const bp4_vec *v, int *result);
+
+/* ---- whole solves on the device ---------------------------------------------------------
+ * The two CG solvers of the benchmark with the host out of the iteration loop: every scalar
+ * (alpha, beta, the residual, the stopping test) is computed on the device, in the host solver's
+ * arithmetic, and the loop runs as one CUDA graph with a conditional WHILE node.  Step 0 (start
+ * residual g = A x - b, or -b for a zero x, its norm and the first check) runs through the entry
+ * points above; then the graph runs the iterations until the stopping test ends them.
+ *   - stopping test: ReductionControl::check (solver_control.h): step 0 sets
+ *     reduced_tol = |g_0| * reduce; success if value < reduced_tol or value <= tol; failure if
+ *     step >= max_steps or the value is NaN.  reduce = 0 is a plain SolverControl(max_steps, tol).
+ *   - hitting max_steps is not an error: the call returns 0 with state = 2 and x holds the last
+ *     iterate, as the host-driven solvers leave it.
+ *   - one rank only: a context with a ghost-exchange plan (n_peers > 0) or a communicator over
+ *     several ranks gives BP4_ERR_STATE.
+ *   - the merged solve uses the context's in-loop / streamed form (bp4_debug_set_fused), i.e.
+ *     the vector kernels of bp4_vmult_merged.
+ *   - blocking: the call returns when *out is on the host.  The instantiated graph is cached in
+ *     the context per (solver, x, b, prec, in-loop form) together with its temporaries g, d, h;
+ *     a repeated solve re-uses it.
+ *   - measurement: bp4_launch_count adds one per graph launch (plus the step-0 kernels); the
+ *     kernels of the graph are counted once, when it is built.  bp4_profile_* time no kernel
+ *     inside the graph.                                                                      */
+typedef struct bp4_solve_result
+{
+  int      state;         /* 1 = success, 2 = failure (SolverControl::State)   */
+  unsigned last_step;     /* SolverControl::last_step()                        */
+  double   last_value;    /* residual norm checked at last_step                */
+  double   initial_value; /* residual norm at step 0                           */
+} bp4_solve_result;
+/* deal.II SolverCG with DiagonalMatrixBlocked (benchmark_precond/bench.cc:11-16, SURVEY App. B3);
+ * prec holds n_owned/3 inverse-diagonal entries                                               */
+int bp4_solve_cg(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                 double tol, double reduce, bp4_solve_result *out);
+/* SolverCGFullMerge (solver_cg_optimized.h:192-302): x every second iteration, odd/even fix-up */
+int bp4_solve_cg_merged(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
+                        unsigned max_steps, double tol, double reduce, bp4_solve_result *out);
 
 /* ---- multi-GPU (Utilities::MPI::Partitioner / MPI_Allreduce call sites, SURVEY 2a) ------- */
 #define BP4_NCCL_ID_BYTES 128

@@ -75,16 +75,19 @@ def build_cuda(force=False, verbose=False):
 
 
 def build_host(force=False):
-    """the C++ host mirror: one shared library per run_cg_solver plugin + the two CLI executables"""
+    """the C++ host mirror: one shared library per run_cg_solver plugin + the four CLI executables"""
     inc = os.path.join(ROOT, "include")
-    deps = _sources(HOST, (".cc", ".h")) + [os.path.join(inc, "bp4.h"),
-                                            os.path.join(HERE, "benchmark_precond", "bench.cc"),
-                                            os.path.join(HERE, "benchmark_precond_merged", "bench.cc")]
+    plugins = (("plain", [], "benchmark_precond"),
+               ("merged", ["-DBP4_PLUGIN_MERGED"], "benchmark_precond_merged"),
+               ("plain_device", ["-DBP4_PLUGIN_PLAIN_DEVICE"], "benchmark_precond_device"),
+               ("merged_device", ["-DBP4_PLUGIN_MERGED_DEVICE"], "benchmark_precond_merged_device"))
+    deps = _sources(HOST, (".cc", ".h")) + [os.path.join(inc, "bp4.h")] + \
+        [os.path.join(HERE, plug, "bench.cc") for _, _, plug in plugins]
     common = ["/usr/bin/g++", "-O3", "-std=c++17", "-fPIC", "-pthread", "-Wall", "-I", inc]
     link = ["-L", HERE, "-lbp4", "-Wl,-rpath,$ORIGIN"]
     outs = []
     jobs = []
-    for name, macro, plug in (("plain", [], "benchmark_precond"), ("merged", ["-DBP4_PLUGIN_MERGED"], "benchmark_precond_merged")):
+    for name, macro, plug in plugins:
         lib = os.path.join(HERE, f"libbp4_host_{name}.so")
         exe = os.path.join(HERE, plug, "bench")
         outs += [lib, exe]

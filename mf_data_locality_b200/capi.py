@@ -44,7 +44,15 @@ EXPORTS = [
     "bp4_equ", "bp4_add", "bp4_sadd", "bp4_dot", "bp4_add_and_dot", "bp4_l2_norm", "bp4_all_zero",
     "bp4_comm_unique_id", "bp4_comm_init", "bp4_comm_info", "bp4_update_ghost_values", "bp4_compress_add",
     "bp4_profile_enable", "bp4_profile_reset", "bp4_profile_get", "bp4_launch_count",
+    "bp4_solve_cg", "bp4_solve_cg_merged",
 ]
+
+SUCCESS, FAILURE = 1, 2  # SolverControl::State of a device-resident solve
+
+
+class _SolveResult(C.Structure):
+    _fields_ = [("state", C.c_int), ("last_step", C.c_uint), ("last_value", C.c_double),
+                ("initial_value", C.c_double)]
 
 
 def lib():
@@ -66,6 +74,8 @@ def lib():
         _lib.bp4_vec_alloc.argtypes = [vp, C.c_uint64, vp]
         _lib.bp4_vec_upload.argtypes = [vp, vp, vp, C.c_uint64]
         _lib.bp4_vec_download.argtypes = [vp, vp, vp, C.c_uint64]
+        for f in (_lib.bp4_solve_cg, _lib.bp4_solve_cg_merged):
+            f.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp]
     return _lib
 
 
@@ -225,6 +235,16 @@ class Context:
 
     def x_finalize_even(self, x, d, g, prec, c1, c2):
         _chk(lib().bp4_x_finalize_even(self.h, x.h, d.h, g.h, prec.h, c1, c2))
+
+    def solve_cg(self, x, b, prec, merged=True, max_steps=100, tol=1e-15, reduce=1e-8):
+        """CG solve of A x = b with the iteration loop on the device (bp4_solve_cg_merged, or
+        bp4_solve_cg with merged=False) from the start vector in x; prec holds n_owned/3 inverse
+        diagonal entries.  Returns (state, last_step, last_value, initial_value); hitting
+        max_steps is state FAILURE, not an exception."""
+        r = _SolveResult()
+        f = lib().bp4_solve_cg_merged if merged else lib().bp4_solve_cg
+        _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
+        return r.state, r.last_step, r.last_value, r.initial_value
 
     # ---- BLAS-1 -------------------------------------------------------------------
     def equ(self, dst, a, src):

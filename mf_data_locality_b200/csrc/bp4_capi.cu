@@ -68,6 +68,19 @@ struct ProfEvent
   int         id;
 };
 
+// instantiated graph of one device-resident solve (bp4_solve_cg / bp4_solve_cg_merged), keyed by
+// the variant, the caller's x, b and prec buffers and the in-loop form; it owns the temporaries
+// g, d, h so that their addresses, baked into the graph, stay valid
+struct SolveGraph
+{
+  bool            merged = false;
+  int             fused  = 0;
+  const double   *x = nullptr, *b = nullptr, *prec = nullptr;
+  double         *g = nullptr, *d = nullptr, *h = nullptr;
+  cudaGraph_t     graph = nullptr;
+  cudaGraphExec_t exec  = nullptr;
+};
+
 struct bp4_ctx
 {
   int          degree = 0, device = 0, sms = 0;
@@ -86,6 +99,11 @@ struct bp4_ctx
   double      *h_acc  = nullptr; // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
   unsigned long long pub_seq = 0;
   int         *h_flag = nullptr; // pinned
+  // device-resident solves: the solver state, its pinned host images ([0] initial state read by
+  // the graph, [1] final state written by it) and the cached graphs
+  bp4::SolveState        *d_state = nullptr;
+  bp4::SolveState        *h_state = nullptr;
+  std::vector<SolveGraph> solves;
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
   int             fused      = 0;      // 1: do_cg_update4b/3b on private DoFs inside the cell kernel
@@ -133,13 +151,21 @@ struct bp4_ctx
 
 namespace
 {
-  struct Timed // RAII: count a launch, and time it with events when profiling is on
+  bool capturing(cudaStream_t st)
+  {
+    cudaStreamCaptureStatus s = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(st, &s) == cudaSuccess && s != cudaStreamCaptureStatusNone;
+  }
+
+  // RAII: count a launch, and time it with events when profiling is on.  While the stream is
+  // being captured into a graph the launch is counted but not timed (no events inside a graph).
+  struct Timed
   {
     bp4_ctx *c;
     int      id;
     ProfEvent ev{};
     bool      on;
-    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile)
+    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile && !capturing(c_->stream))
     {
       c->launches += n_launches;
       c->prof_cnt[id] += 1;
@@ -360,6 +386,8 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   CU(cudaMallocHost(&c->h_acc, sizeof(double) * 16)); // UVA: the pointer is valid on the device too
   memset(c->h_acc, 0, sizeof(double) * 16);
   CU(cudaMallocHost(&c->h_flag, sizeof(int)));
+  CU(cudaMalloc(&c->d_state, sizeof(bp4::SolveState)));
+  CU(cudaMallocHost(&c->h_state, 2 * sizeof(bp4::SolveState)));
 
   // cell-batch ranges and their private DoF runs -> units and batches of the fused merged loop
   if (d->n_ranges > 0)
@@ -481,6 +509,18 @@ int bp4_ctx_destroy(bp4_ctx *c)
     ncclCommDestroy(c->comm);
   for (auto &kv : c->pool)
     cudaFree(kv.second);
+  for (SolveGraph &sg : c->solves)
+    {
+      if (sg.exec)
+        cudaGraphExecDestroy(sg.exec);
+      if (sg.graph)
+        cudaGraphDestroy(sg.graph);
+      cudaFree(sg.g);
+      cudaFree(sg.d);
+      cudaFree(sg.h);
+    }
+  cudaFree(c->d_state);
+  cudaFreeHost(c->h_state);
   cudaFree(c->d_entity);
   cudaFree(c->d_constrained);
   cudaFree(c->d_walk);
@@ -645,6 +685,7 @@ struct MergedCall
   double *x, *g, *d;
   const double *prec;
   double  alpha, beta, alpha_old, beta_old;
+  const bp4::SolveState *state; // non-null: the scalars come from this solver state instead
 };
 
 // cell loop over the cell partition `part` (0..2, or -1 = all cells): dst += sum_cells A_cell src
@@ -681,6 +722,7 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       a.c1           = a.update_x ? m->alpha + m->alpha_old / m->beta_old : 0.;
       a.c2           = a.update_x ? m->alpha_old / m->beta_old : 0.;
       a.acc          = c->d_acc;
+      a.state        = m->state;
       Timed t(c, BP4_K_MERGED);
       CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream));
     }
@@ -755,6 +797,17 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
   return 0;
 }
 
+// dst = A src on the context's stream (also captured into the plain device solve's loop body)
+static int vmult_on(bp4_ctx *c, double *dst, const double *src)
+{
+  CU(cudaMemsetAsync(dst, 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream));
+  if (int e = cell_loop(c, dst, src, nullptr))
+    return e;
+  Timed t(c, BP4_K_BLAS1);
+  CU(bp4::launch_fixup(c->n_constrained, c->d_constrained, dst, src, c->stream));
+  return 0;
+}
+
 int bp4_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
 {
   if (!c)
@@ -766,14 +819,7 @@ int bp4_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
   if (dst == src)
     return fail(BP4_ERR_ARG, "vmult: dst aliases src");
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(dst->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream));
-  if (int e = cell_loop(c, dst->p(), src->p(), nullptr))
-    return e;
-  {
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_fixup(c->n_constrained, c->d_constrained, dst->p(), src->p(), c->stream));
-  }
-  return 0;
+  return vmult_on(c, dst->p(), src->p());
 }
 
 int bp4_debug_set_fused(bp4_ctx *c, int on)
@@ -802,6 +848,35 @@ int bp4_fused_info(bp4_ctx *c, int *fused, uint64_t *n_private, uint64_t *n_unit
   return 0;
 }
 
+// vmult_with_merged_sums on the context's stream, the seven sums left in d_acc (also captured into
+// the merged device solve's loop body, with the scalars from m.state)
+static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
+{
+  const uint64_t n = c->n_owned;
+  // DoFs private to one cell-batch range get do_cg_update4b / do_cg_update3b inside the cell
+  // kernel; the rest of the vector -- shared between ranges or ranks, Dirichlet -- is streamed
+  // before / after the loop (with the fused path off: everything)
+  const uint64_t tail = c->fused ? c->n_private : 0;
+  {
+    Timed t(c, BP4_K_PRE);
+    if (m.state)
+      CU(bp4::launch_pre_dev(tail, n, h, m.x, m.g, m.d, m.prec, m.state, c->d_acc, c->sms, c->stream));
+    else
+      CU(bp4::launch_pre(tail, n, h, m.x, m.g, m.d, m.prec, m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc,
+                         c->sms, c->stream));
+  }
+  if (c->n_ghost)
+    CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream));
+  if (int e = cell_loop(c, h, m.d, c->fused ? &m : nullptr))
+    return e;
+  if (n > tail)
+    {
+      Timed t(c, BP4_K_POST);
+      CU(bp4::launch_post(tail, n, m.g, m.d, h, m.prec, c->d_acc, c->sms, c->stream));
+    }
+  return 0;
+}
+
 int bp4_vmult_merged(bp4_ctx *c, bp4_vec *x, bp4_vec *g, bp4_vec *d, bp4_vec *h, const bp4_vec *prec,
                      double alpha, double beta, double alpha_old, double beta_old, double out[7])
 {
@@ -814,26 +889,9 @@ int bp4_vmult_merged(bp4_ctx *c, bp4_vec *x, bp4_vec *g, bp4_vec *d, bp4_vec *h,
   if (!prec || prec->n < c->n_owned / 3)
     return fail(BP4_ERR_ARG, "prec needs n_owned/3 entries");
   CU(cudaSetDevice(c->device));
-  const uint64_t n = c->n_owned;
-  // DoFs private to one cell-batch range get do_cg_update4b / do_cg_update3b inside the cell
-  // kernel; the rest of the vector -- shared between ranges or ranks, Dirichlet -- is streamed
-  // before / after the loop (with the fused path off: everything)
-  const uint64_t tail = c->fused ? c->n_private : 0;
-  {
-    Timed t(c, BP4_K_PRE);
-    CU(bp4::launch_pre(tail, n, h->p(), x->p(), g->p(), d->p(), prec->p(), alpha, beta, alpha_old, beta_old,
-                       c->d_acc, c->sms, c->stream));
-  }
-  if (c->n_ghost)
-    CU(cudaMemsetAsync(h->p() + n, 0, sizeof(double) * c->n_ghost, c->stream));
-  MergedCall m{x->p(), g->p(), d->p(), prec->p(), alpha, beta, alpha_old, beta_old};
-  if (int e = cell_loop(c, h->p(), d->p(), c->fused ? &m : nullptr))
+  MergedCall m{x->p(), g->p(), d->p(), prec->p(), alpha, beta, alpha_old, beta_old, nullptr};
+  if (int e = merged_sweep(c, m, h->p()))
     return e;
-  if (n > tail)
-    {
-      Timed t(c, BP4_K_POST);
-      CU(bp4::launch_post(tail, n, g->p(), d->p(), h->p(), prec->p(), c->d_acc, c->sms, c->stream));
-    }
   return reduce_to_host(c, 7, out);
 }
 
@@ -1011,6 +1069,223 @@ int bp4_all_zero(bp4_ctx *c, const bp4_vec *v, int *result)
   CU(cudaStreamSynchronize(c->stream));
   *result = *c->h_flag ? 0 : 1;
   return 0;
+}
+
+// ---- whole solves on the device ----------------------------------------------------------
+// Capture what `launch` enqueues on the context's stream into `graph`, after the nodes `deps`;
+// `leaves` (optional) receives the nodes the next one must follow.  The capture is always ended,
+// also when a launch fails, so that the stream stays usable.
+extern "C++" {
+template <typename F>
+static int capture_into(bp4_ctx *c, cudaGraph_t graph, const cudaGraphNode_t *deps, size_t n_deps, F &&launch,
+                        std::vector<cudaGraphNode_t> *leaves)
+{
+  CU(cudaStreamBeginCaptureToGraph(c->stream, graph, deps, nullptr, n_deps, cudaStreamCaptureModeThreadLocal));
+  int e = launch();
+  if (!e && leaves)
+    {
+      cudaStreamCaptureStatus st;
+      const cudaGraphNode_t  *d = nullptr;
+      size_t                  n = 0;
+      const cudaError_t       q = cudaStreamGetCaptureInfo(c->stream, &st, nullptr, nullptr, &d, &n);
+      if (q == cudaSuccess)
+        leaves->assign(d, d + n);
+      else
+        e = fail(BP4_ERR_CUDA, "cudaStreamGetCaptureInfo: %s", cudaGetErrorString(q));
+    }
+  cudaGraph_t       out = nullptr;
+  const cudaError_t q   = cudaStreamEndCapture(c->stream, &out);
+  if (e)
+    return e;
+  CU(q);
+  return 0;
+}
+} // extern "C++"
+
+// One CUDA graph per solve:  initial state -> prologue -> WHILE { one iteration } -> epilogue ->
+// final state to the host.  The loop body is captured from the launch code of the host-driven
+// path (vmult_on, merged_sweep); the scalar kernels keep alpha, beta, ... in c->d_state and the
+// last one of an iteration sets the loop condition.
+static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
+{
+  const uint64_t n    = c->n_owned;
+  double        *x    = const_cast<double *>(sg.x);
+  const double  *prec = sg.prec;
+  bp4::SolveState *st = c->d_state;
+  double        *acc  = c->d_acc;
+  CU(cudaGraphCreate(&sg.graph, 0));
+  cudaGraphConditionalHandle loop;
+  CU(cudaGraphConditionalHandleCreate(&loop, sg.graph, 1, cudaGraphCondAssignDefault));
+  std::vector<cudaGraphNode_t> leaves;
+  // initial state; plain: h = P g, d = -h, gh = g.h (SolverCG before its loop)
+  auto prologue = [&]() -> int {
+    CU(cudaMemcpyAsync(st, c->h_state, sizeof(bp4::SolveState), cudaMemcpyHostToDevice, c->stream));
+    if (sg.merged)
+      return 0;
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->sms, c->stream));
+    }
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_solve_scalar(bp4::kSolvePlainInit, st, acc, loop, c->stream));
+    }
+    Timed t(c, BP4_K_BLAS1);
+    CU(bp4::launch_sadd(n, sg.d, 0., -1., sg.h, c->sms, c->stream));
+    return 0;
+  };
+  if (int e = capture_into(c, sg.graph, nullptr, 0, prologue, &leaves))
+    return e;
+  cudaGraphNodeParams cp = {};
+  cp.type                = cudaGraphNodeTypeConditional;
+  cp.conditional.handle  = loop;
+  cp.conditional.type    = cudaGraphCondTypeWhile;
+  cp.conditional.size    = 1;
+  cudaGraphNode_t cond;
+  CU(cudaGraphAddNode(&cond, sg.graph, leaves.data(), leaves.size(), &cp));
+  auto body = [&]() -> int {
+    if (sg.merged)
+      {
+        const MergedCall m{x, sg.g, sg.d, prec, 0., 0., 0., 0., st};
+        if (int e = merged_sweep(c, m, sg.h))
+          return e;
+        Timed t(c, BP4_K_BLAS1);
+        CU(bp4::launch_solve_scalar(bp4::kSolveMergedStep, st, acc, loop, c->stream));
+        return 0;
+      }
+    // SolverCG: h = A d; alpha = gh / d.h; x += alpha d; g += alpha h, |g|; check;
+    // h = P g; beta = g.h / gh; d = beta d - h
+    if (int e = vmult_on(c, sg.h, sg.d))
+      return e;
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_dot(n, sg.d, sg.h, acc, c->sms, c->stream));
+    }
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_solve_scalar(bp4::kSolvePlainAlpha, st, acc, loop, c->stream));
+    }
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_cg_xg(n, x, sg.g, sg.d, sg.h, st, acc + 1, c->sms, c->stream));
+    }
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->sms, c->stream));
+    }
+    {
+      Timed t(c, BP4_K_BLAS1);
+      CU(bp4::launch_solve_scalar(bp4::kSolvePlainCheck, st, acc, loop, c->stream));
+    }
+    Timed t(c, BP4_K_BLAS1);
+    CU(bp4::launch_sadd_dev(n, sg.d, &st->beta, -1., sg.h, c->sms, c->stream));
+    return 0;
+  };
+  if (int e = capture_into(c, cp.conditional.phGraph_out[0], nullptr, 0, body, nullptr))
+    return e;
+  // merged: the pending x update; both: the final state to the host
+  auto epilogue = [&]() -> int {
+    if (sg.merged)
+      {
+        Timed t(c, BP4_K_BLAS1);
+        CU(bp4::launch_solve_final(n, x, sg.d, sg.g, prec, st, c->sms, c->stream));
+      }
+    CU(cudaMemcpyAsync(c->h_state + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream));
+    return 0;
+  };
+  if (int e = capture_into(c, sg.graph, &cond, 1, epilogue, nullptr))
+    return e;
+  CU(cudaGraphInstantiate(&sg.exec, sg.graph, 0));
+  return 0;
+}
+
+static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
+                        const unsigned max_steps, const double tol, const double reduce, bp4_solve_result *out)
+{
+  if (!c || !out)
+    return fail(BP4_ERR_ARG, "null argument");
+  if (int e = check_len(c, x, "x"))
+    return e;
+  if (int e = check_len(c, b, "b"))
+    return e;
+  if (!prec || 3 * prec->n < c->n_owned)
+    return fail(BP4_ERR_ARG, "prec needs n_owned/3 entries");
+  if (x == b)
+    return fail(BP4_ERR_ARG, "solve: x aliases b");
+  if (!c->peer.empty() || c->n_ranks > 1)
+    return fail(BP4_ERR_STATE, "the device solve runs on one rank: this context has a ghost-exchange plan or "
+                               "a communicator over several ranks");
+  CU(cudaSetDevice(c->device));
+  SolveGraph *sg = nullptr;
+  for (SolveGraph &e : c->solves)
+    if (e.merged == merged && e.fused == c->fused && e.x == x->p() && e.b == b->p() && e.prec == prec->p())
+      sg = &e;
+  if (!sg)
+    {
+      c->solves.emplace_back();
+      sg         = &c->solves.back();
+      sg->merged = merged, sg->fused = c->fused, sg->x = x->p(), sg->b = b->p(), sg->prec = prec->p();
+      const uint64_t nl = c->n_owned + c->n_ghost;
+      for (double **v : {&sg->g, &sg->d, &sg->h})
+        if (int e = pooled_alloc(c, nl, v, false))
+          return e;
+    }
+  // step 0 on the host, with the entry points the host-driven solvers use: g = A x - b (-b for a
+  // zero start vector), |g|, ReductionControl::check(0)
+  bp4_vec g{sg->g, c->n_owned + c->n_ghost};
+  int     zero = 0;
+  if (int e = bp4_all_zero(c, x, &zero))
+    return e;
+  if (!zero)
+    {
+      if (int e = bp4_vmult(c, &g, x))
+        return e;
+      if (int e = bp4_add(c, &g, -1., b))
+        return e;
+    }
+  else if (int e = bp4_equ(c, &g, -1., b))
+    return e;
+  double res = 0.;
+  if (int e = bp4_l2_norm(c, &g, &res))
+    return e;
+  const double reduced_tol = res * reduce;
+  const int    state0      = (res < reduced_tol || res <= tol) ? 1 : ((max_steps == 0 || std::isnan(res)) ? 2 : 0);
+  *out                     = bp4_solve_result{state0, 0u, res, res};
+  if (state0 != 0)
+    return 0;
+  if (!sg->exec)
+    if (int e = build_solve_graph(c, *sg))
+      {
+        if (sg->graph) // a later call starts over
+          cudaGraphDestroy(sg->graph);
+        sg->graph = nullptr;
+        return e;
+      }
+  bp4::SolveState &init = c->h_state[0];
+  init                  = bp4::SolveState{};
+  init.tol              = tol;
+  init.reduced_tol      = reduced_tol;
+  init.last_value       = res;
+  init.initial_value    = res;
+  init.max_steps        = max_steps;
+  CU(cudaGraphLaunch(sg->exec, c->stream));
+  c->launches += 1;
+  CU(cudaStreamSynchronize(c->stream));
+  const bp4::SolveState &fin = c->h_state[1];
+  *out                       = bp4_solve_result{fin.state, fin.step, fin.last_value, res};
+  return 0;
+}
+
+int bp4_solve_cg(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps, double tol,
+                 double reduce, bp4_solve_result *out)
+{
+  return solve_device(c, false, x, b, prec, max_steps, tol, reduce, out);
+}
+
+int bp4_solve_cg_merged(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                        double tol, double reduce, bp4_solve_result *out)
+{
+  return solve_device(c, true, x, b, prec, max_steps, tol, reduce, out);
 }
 
 // ---- multi-GPU ---------------------------------------------------------------------------

@@ -154,7 +154,9 @@ namespace bp4
   // (and between ranks, and the Dirichlet ones) are the tail [n_private, n_owned) of the vector:
   // pre_kernel / post_kernel stream them before / after this kernel.
   // ---------------------------------------------------------------------------------------
-  template <int P, int CPB, bool FUSED, bool QUAD>
+  // DEV (fused only): the scalars of do_cg_update4b come from the solver state of a device-resident
+  // solve (a.state) instead of the launch arguments
+  template <int P, int CPB, bool FUSED, bool QUAD, bool DEV = false>
   __global__ void __launch_bounds__(kThreads, Cfg<P>::BLOCKS) cell_kernel(const CellArgs a)
   {
     constexpr int NC = Cfg<P, QUAD>::NCOEF;
@@ -613,16 +615,32 @@ namespace bp4
           if (tid == kThreads - 2 && (e & 1u)) // e - 1 is even: never the odd first element
             f(e - 1u);
         };
+        // the scalars of do_cg_update4b (sc.alpha, beta, first, update_x, c1, c2): the launch
+        // arguments, or (DEV) derived from the solver state exactly as cell_range (bp4_capi.cu)
+        // derives them on the host
+        CellArgs dev_args;
+        if constexpr (DEV)
+          {
+            dev_args        = a;
+            const double al = a.state->alpha, ao = a.state->alpha_old, bo = a.state->beta_old;
+            dev_args.alpha    = al;
+            dev_args.beta     = a.state->beta;
+            dev_args.first    = al == 0. ? 1 : 0;
+            dev_args.update_x = (al != 0. && ao != 0.) ? 1 : 0;
+            dev_args.c1       = dev_args.update_x ? __dadd_rn(al, __ddiv_rn(ao, bo)) : 0.;
+            dev_args.c2       = dev_args.update_x ? __ddiv_rn(ao, bo) : 0.;
+          }
+        const CellArgs &sc = DEV ? dev_args : a;
         auto pre_one = [&](const uint32_t i, const double rr, const double pp, const double hh, const double pr) {
-          if (a.first)
+          if (sc.first)
             a.p[i] = -pr * rr;
           else
             {
-              if (a.update_x)
-                atomicAdd(a.x + i, a.c1 * pp + a.c2 * pr * rr);
-              const double rn = rr + a.alpha * hh;
+              if (sc.update_x)
+                atomicAdd(a.x + i, sc.c1 * pp + sc.c2 * pr * rr);
+              const double rn = rr + sc.alpha * hh;
               a.r[i]          = rn;
-              a.p[i]          = a.beta * pp - pr * rn;
+              a.p[i]          = sc.beta * pp - pr * rn;
             }
           a.dst[i] = 0.;
         };
@@ -640,19 +658,19 @@ namespace bp4
             if (w.ok[k])
               {
                 const uint32_t i0 = lo + 2u * (c0 + tid + k * kThreads);
-                if (a.first)
+                if (sc.first)
                   *reinterpret_cast<double2 *>(a.p + i0) = make_double2(-w.d[k].x * w.r[k].x, -w.d[k].y * w.r[k].y);
                 else
                   {
-                    if (a.update_x) // x += ..., fire and forget: x is not read in this kernel
+                    if (sc.update_x) // x += ..., fire and forget: x is not read in this kernel
                       {
-                        atomicAdd(a.x + i0, a.c1 * w.p[k].x + a.c2 * w.d[k].x * w.r[k].x);
-                        atomicAdd(a.x + i0 + 1, a.c1 * w.p[k].y + a.c2 * w.d[k].y * w.r[k].y);
+                        atomicAdd(a.x + i0, sc.c1 * w.p[k].x + sc.c2 * w.d[k].x * w.r[k].x);
+                        atomicAdd(a.x + i0 + 1, sc.c1 * w.p[k].y + sc.c2 * w.d[k].y * w.r[k].y);
                       }
-                    const double r0 = w.r[k].x + a.alpha * w.h[k].x, r1 = w.r[k].y + a.alpha * w.h[k].y;
+                    const double r0 = w.r[k].x + sc.alpha * w.h[k].x, r1 = w.r[k].y + sc.alpha * w.h[k].y;
                     *reinterpret_cast<double2 *>(a.r + i0) = make_double2(r0, r1);
                     *reinterpret_cast<double2 *>(a.p + i0) =
-                      make_double2(a.beta * w.p[k].x - w.d[k].x * r0, a.beta * w.p[k].y - w.d[k].y * r1);
+                      make_double2(sc.beta * w.p[k].x - w.d[k].x * r0, sc.beta * w.p[k].y - w.d[k].y * r1);
                   }
                 *reinterpret_cast<double2 *>(a.dst + i0) = make_double2(0., 0.);
               }
@@ -925,14 +943,23 @@ namespace bp4
   // do_cg_update4b<3,double,true>, solver_cg_optimized.h:65-161, over [begin, end): the DoFs that
   // are not private to one cell-batch range (all of them when the numbering has no such group).
   // Also clears the reduction scratch of this iteration (stream order: before any post).
+  // DEV: the four scalars come from the solver state of a device-resident solve (st).
+  template <bool DEV>
   __global__ void __launch_bounds__(256) pre_kernel(const uint64_t begin, const uint64_t end,
                                                     double *__restrict__ h, double *__restrict__ x,
                                                     double *__restrict__ r, double *__restrict__ p,
                                                     const double *__restrict__ prec,
-                                                    const double alpha, const double beta,
-                                                    const double alpha_old, const double beta_old,
-                                                    double *acc_to_zero)
+                                                    double alpha, double beta,
+                                                    double alpha_old, double beta_old,
+                                                    double *acc_to_zero, const SolveState *st)
   {
+    if constexpr (DEV)
+      {
+        alpha     = st->alpha;
+        beta      = st->beta;
+        alpha_old = st->alpha_old;
+        beta_old  = st->beta_old;
+      }
     if (acc_to_zero && blockIdx.x == 0 && threadIdx.x < 8)
       acc_to_zero[threadIdx.x] = 0.;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -1018,11 +1045,14 @@ namespace bp4
       dst[con[i]] = src[con[i]];
   }
 
-  // dst = s*dst + a*src   (s == 0: dst = a*src without reading dst)
+  // dst = s*dst + a*src   (s == 0: dst = a*src without reading dst); DEV: s = *s_dev
+  template <bool DEV>
   __global__ void __launch_bounds__(256) sadd_kernel(const uint64_t n, double *__restrict__ dst,
-                                                     const double s, const double a,
-                                                     const double *__restrict__ src)
+                                                     double s, const double a,
+                                                     const double *__restrict__ src, const double *s_dev)
   {
+    if constexpr (DEV)
+      s = *s_dev;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
       dst[i] = (s == 0. ? 0. : s * dst[i]) + a * src[i];
@@ -1127,6 +1157,139 @@ namespace bp4
                                                        const double c2)
   {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      x[i] += c1 * d[i] + c2 * prec[i / 3] * g[i];
+  }
+
+  // ---------------------------------------------------------------------------------------
+  // device-resident CG solves (bp4_solve_cg, bp4_solve_cg_merged): the vector sweeps the plain
+  // solve needs beyond the operator, the scalar recurrences of both solvers and the final x update
+  // ---------------------------------------------------------------------------------------
+  // h = P g (diagonal_matrix_blocked.h:21-26) and acc += g.h in one sweep
+  __global__ void __launch_bounds__(256) jacobi_dot_kernel(const uint64_t n, double *__restrict__ h,
+                                                           const double *__restrict__ g,
+                                                           const double *__restrict__ diag, double *acc)
+  {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    double         s[1]   = {0.};
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      {
+        const double gi = g[i], hi = diag[i / 3] * gi;
+        h[i]            = hi;
+        s[0] += gi * hi;
+      }
+    block_accumulate<1>(s, acc);
+  }
+
+  // x += alpha d; g += alpha h; acc += g.g   (SolverCG: x.add, g.add_and_dot), alpha from the state
+  __global__ void __launch_bounds__(256) cg_xg_kernel(const uint64_t n, double *__restrict__ x,
+                                                      double *__restrict__ g, const double *__restrict__ d,
+                                                      const double *__restrict__ h, const SolveState *st,
+                                                      double *acc)
+  {
+    const double   alpha  = st->alpha;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    double         s[1]   = {0.};
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      {
+        x[i] += alpha * d[i];
+        const double gi = g[i] + alpha * h[i];
+        g[i]            = gi;
+        s[0] += gi * gi;
+      }
+    block_accumulate<1>(s, acc);
+  }
+
+  // ReductionControl::check (host/solver_control.h) for a step > 0
+  __device__ int control_check(SolveState &st, const uint32_t step, const double value)
+  {
+    st.step       = step;
+    st.last_value = value;
+    if (value < st.reduced_tol || value <= st.tol)
+      return 1;
+    if (step >= st.max_steps || isnan(value))
+      return 2;
+    return 0;
+  }
+
+  // The scalar work of one iteration on one thread, in the host's association order with
+  // explicitly rounded operations (the host build emits no FMA): for equal sums the scalars are
+  // bit-identical to those of the host-driven solvers.  acc is left zero for the next reduction.
+  //   kMergedStep: SolverCGFullMerge::solve (host/solver_cg_optimized.h) from the seven sums
+  //   kPlainInit : gh = g.h before the first iteration (acc[2])
+  //   kPlainAlpha: alpha = gh / d.h (acc[0])
+  //   kPlainCheck: residual from g.g (acc[1]), the check, beta from the new g.h (acc[2])
+  // kMergedStep and kPlainCheck end the iteration: they set the loop condition.
+  __global__ void solve_scalar_kernel(const int kind, SolveState *stp, double *acc,
+                                      const cudaGraphConditionalHandle loop)
+  {
+    if (threadIdx.x != 0)
+      return;
+    SolveState &st = *stp;
+    if (kind == kSolveMergedStep)
+      {
+        double s[7];
+        for (int k = 0; k < 7; ++k)
+          s[k] = acc[k], acc[k] = 0.;
+        const uint32_t it         = st.step + 1;
+        const double   prev_alpha = st.alpha, prev_beta = st.beta;
+        const double   alpha      = __ddiv_rn(s[6], s[0]);
+        const double   res        = __dsqrt_rn(__dadd_rn(__dadd_rn(s[3], __dmul_rn(__dmul_rn(2., alpha), s[2])),
+                                                         __dmul_rn(__dmul_rn(alpha, alpha), s[1])));
+        const int      state      = control_check(st, it, res);
+        st.alpha    = alpha;
+        st.beta_old = prev_beta;
+        if (state == 0) // the arguments of iteration it + 1: alpha_old only on odd iterations
+          {
+            st.beta      = __ddiv_rn(__dmul_rn(alpha, __dadd_rn(s[4], __dmul_rn(alpha, s[5]))), s[6]);
+            st.alpha_old = ((it + 1) & 1u) ? prev_alpha : 0.;
+          }
+        else // kept for the final x update
+          st.alpha_old = prev_alpha;
+        st.state = state;
+        cudaGraphSetConditional(loop, state == 0 ? 1u : 0u);
+      }
+    else if (kind == kSolvePlainInit)
+      {
+        st.gh  = acc[2];
+        acc[2] = 0.;
+      }
+    else if (kind == kSolvePlainAlpha)
+      {
+        st.alpha = __ddiv_rn(st.gh, acc[0]);
+        acc[0]   = 0.;
+      }
+    else // kSolvePlainCheck
+      {
+        const int state = control_check(st, st.step + 1, __dsqrt_rn(fabs(acc[1])));
+        st.state        = state;
+        // after the stopping check only the temporaries h, d and gh / beta change (the loop
+        // body runs to its end)
+        const double beta_den = st.gh;
+        st.gh                 = acc[2];
+        st.beta               = __ddiv_rn(st.gh, beta_den);
+        acc[1] = acc[2] = 0.;
+        cudaGraphSetConditional(loop, state == 0 ? 1u : 0u);
+      }
+  }
+
+  // the pending x update of SolverCGFullMerge after its last iteration
+  // (solver_cg_optimized.h:256-288): odd step x += alpha d, even step bp4_x_finalize_even's formula
+  __global__ void __launch_bounds__(256) solve_final_kernel(const uint64_t n, double *__restrict__ x,
+                                                            const double *__restrict__ d,
+                                                            const double *__restrict__ g,
+                                                            const double *__restrict__ prec,
+                                                            const SolveState *st)
+  {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    const double   alpha  = st->alpha;
+    if (st->step & 1u)
+      {
+        for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+          x[i] += alpha * d[i];
+        return;
+      }
+    const double c2 = __ddiv_rn(st->alpha_old, st->beta_old), c1 = __dadd_rn(alpha, c2);
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
       x[i] += c1 * d[i] + c2 * prec[i / 3] * g[i];
   }
@@ -1274,8 +1437,14 @@ namespace bp4
     if (e != cudaSuccess)
       return e;
     if constexpr (Stage<P>::OK)
-      e = cudaFuncSetAttribute(cell_kernel<P, CPB, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)fused_smem<P>());
+      {
+        e = cudaFuncSetAttribute(cell_kernel<P, CPB, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)fused_smem<P>());
+        if (e != cudaSuccess)
+          return e;
+        e = cudaFuncSetAttribute(cell_kernel<P, CPB, true, false, true>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fused_smem<P>());
+      }
     return e;
   }
 
@@ -1302,7 +1471,12 @@ namespace bp4
     if (fused)
       {
         if constexpr (Stage<P>::OK)
-          cell_kernel<P, CPB, true, false><<<grid, kThreads, fused_smem<P>(), st>>>(a);
+          {
+            if (a.state)
+              cell_kernel<P, CPB, true, false, true><<<grid, kThreads, fused_smem<P>(), st>>>(a);
+            else
+              cell_kernel<P, CPB, true, false><<<grid, kThreads, fused_smem<P>(), st>>>(a);
+          }
       }
     else if (quad)
       cell_kernel<P, CPBQ, false, true><<<grid, kThreads, sizeof(CellSmem<P, CPBQ, 81>), st>>>(a);
@@ -1385,8 +1559,17 @@ namespace bp4
                          const double *prec, double alpha, double beta, double alpha_old,
                          double beta_old, double *acc_to_zero, int sms, cudaStream_t st)
   {
-    pre_kernel<<<stream_grid(end > begin ? end - begin : 0, sms), 256, 0, st>>>(
-      begin, end, h, x, r, p, prec, alpha, beta, alpha_old, beta_old, acc_to_zero);
+    pre_kernel<false><<<stream_grid(end > begin ? end - begin : 0, sms), 256, 0, st>>>(
+      begin, end, h, x, r, p, prec, alpha, beta, alpha_old, beta_old, acc_to_zero, nullptr);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_pre_dev(uint64_t begin, uint64_t end, double *h, double *x, double *r, double *p,
+                             const double *prec, const SolveState *state, double *acc_to_zero, int sms,
+                             cudaStream_t st)
+  {
+    pre_kernel<true><<<stream_grid(end > begin ? end - begin : 0, sms), 256, 0, st>>>(
+      begin, end, h, x, r, p, prec, 0., 0., 0., 0., acc_to_zero, state);
     return cudaGetLastError();
   }
 
@@ -1413,7 +1596,50 @@ namespace bp4
   {
     if (n == 0)
       return cudaSuccess;
-    sadd_kernel<<<stream_grid(n, sms), 256, 0, st>>>(n, dst, s, a, src);
+    sadd_kernel<false><<<stream_grid(n, sms), 256, 0, st>>>(n, dst, s, a, src, nullptr);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_sadd_dev(uint64_t n, double *dst, const double *s, double a, const double *src, int sms,
+                              cudaStream_t st)
+  {
+    if (n == 0)
+      return cudaSuccess;
+    sadd_kernel<true><<<stream_grid(n, sms), 256, 0, st>>>(n, dst, 0., a, src, s);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_jacobi_dot(uint64_t n, double *h, const double *g, const double *diag, double *acc, int sms,
+                                cudaStream_t st)
+  {
+    if (n == 0)
+      return cudaSuccess;
+    jacobi_dot_kernel<<<stream_grid(n, sms), 256, 0, st>>>(n, h, g, diag, acc);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_cg_xg(uint64_t n, double *x, double *g, const double *d, const double *h,
+                           const SolveState *state, double *acc, int sms, cudaStream_t st)
+  {
+    if (n == 0)
+      return cudaSuccess;
+    cg_xg_kernel<<<stream_grid(n, sms), 256, 0, st>>>(n, x, g, d, h, state, acc);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_solve_scalar(int kind, SolveState *state, double *acc, cudaGraphConditionalHandle loop,
+                                  cudaStream_t st)
+  {
+    solve_scalar_kernel<<<1, 32, 0, st>>>(kind, state, acc, loop);
+    return cudaGetLastError();
+  }
+
+  cudaError_t launch_solve_final(uint64_t n, double *x, const double *d, const double *g, const double *prec,
+                                 const SolveState *state, int sms, cudaStream_t st)
+  {
+    if (n == 0)
+      return cudaSuccess;
+    solve_final_kernel<<<stream_grid(n, sms), 256, 0, st>>>(n, x, d, g, prec, state);
     return cudaGetLastError();
   }
 

@@ -124,6 +124,7 @@ namespace bp4
     static constexpr bool OK    = Cfg<P>::STAGED && JOB >= 64;
   };
 
+  struct SolveState;
   struct CellArgs
   {
     const uint32_t *entity_index; // [n_cells][27]
@@ -143,5 +144,23 @@ namespace bp4
     int              first;       // alpha == 0: p = -P r, h = 0 only
     int              update_x;    // alpha_old != 0
     double          *acc;         // [7]
+    // device-resident solve (cell_kernel<..., DEV = true>): alpha, beta, first, update_x, c1, c2
+    // are derived in-kernel from state->alpha .. beta_old instead of the fields above
+    const SolveState *state;
+  };
+
+  // Solver state of a device-resident CG solve (bp4_solve_cg / bp4_solve_cg_merged), one block
+  // per context.  The scalar kernels write it, the vector kernels of the next sweep read it.
+  struct SolveState
+  {
+    // arguments of the next vmult_with_merged_sums exactly as SolverCGFullMerge passes them
+    // (alpha_old = 0 on even iterations); after the stopping check: alpha, and the true
+    // alpha_old / beta_old of the final x update.  The plain solve keeps alpha and beta here.
+    double   alpha, beta, alpha_old, beta_old;
+    double   gh;                     // plain: g.h of the current iteration
+    double   tol, reduced_tol;       // ReductionControl: absolute and reduced tolerance
+    double   last_value, initial_value;
+    uint32_t max_steps, step;        // step = last checked step
+    int32_t  state, pad;             // SolverControl::State: 0 iterate, 1 success, 2 failure
   };
 } // namespace bp4

@@ -25,12 +25,18 @@ namespace bp4
   cudaError_t launch_pre(uint64_t begin, uint64_t end, double *h, double *x, double *r, double *p,
                          const double *prec, double alpha, double beta, double alpha_old,
                          double beta_old, double *acc_to_zero, int sms, cudaStream_t st);
+  // the same with alpha, beta, alpha_old, beta_old read from a device-resident solve's state
+  cudaError_t launch_pre_dev(uint64_t begin, uint64_t end, double *h, double *x, double *r, double *p,
+                             const double *prec, const SolveState *state, double *acc_to_zero, int sms,
+                             cudaStream_t st);
   cudaError_t launch_post(uint64_t begin, uint64_t end, const double *r, const double *d,
                           const double *h, const double *prec, double *acc, int sms, cudaStream_t st);
   cudaError_t launch_fixup(uint64_t n, const uint32_t *con, double *dst, const double *src,
                            cudaStream_t st);
   cudaError_t launch_sadd(uint64_t n, double *dst, double s, double a, const double *src, int sms,
                           cudaStream_t st);
+  cudaError_t launch_sadd_dev(uint64_t n, double *dst, const double *s, double a, const double *src, int sms,
+                              cudaStream_t st); // s read on the device
   cudaError_t launch_dot(uint64_t n, const double *a, const double *b, double *acc, int sms,
                          cudaStream_t st);
   cudaError_t launch_add_and_dot(uint64_t n, double *g, double a, const double *h, const double *w,
@@ -40,6 +46,22 @@ namespace bp4
                             cudaStream_t st);
   cudaError_t launch_xfinal(uint64_t n, double *x, const double *d, const double *g, const double *prec,
                             double c1, double c2, int sms, cudaStream_t st);
+  // device-resident solves (bp4_solve_cg / bp4_solve_cg_merged)
+  enum SolveScalarKind
+  {
+    kSolveMergedStep = 0,
+    kSolvePlainInit  = 1,
+    kSolvePlainAlpha = 2,
+    kSolvePlainCheck = 3
+  };
+  cudaError_t launch_jacobi_dot(uint64_t n, double *h, const double *g, const double *diag, double *acc, int sms,
+                                cudaStream_t st);
+  cudaError_t launch_cg_xg(uint64_t n, double *x, double *g, const double *d, const double *h,
+                           const SolveState *state, double *acc, int sms, cudaStream_t st);
+  cudaError_t launch_solve_scalar(int kind, SolveState *state, double *acc, cudaGraphConditionalHandle loop,
+                                  cudaStream_t st);
+  cudaError_t launch_solve_final(uint64_t n, double *x, const double *d, const double *g, const double *prec,
+                                 const SolveState *state, int sms, cudaStream_t st);
   cudaError_t launch_diag_assemble(int degree, uint64_t n_cells, const uint32_t *entity_index,
                                    const double *coef, int n_coef, const double *gll, double *diag,
                                    int stride, cudaStream_t st);

@@ -17,7 +17,9 @@ class HostError(RuntimeError):
 
 
 def lib(plugin: str):
-    """plugin: 'plain' (benchmark_precond) or 'merged' (benchmark_precond_merged)"""
+    """plugin: 'plain' (benchmark_precond), 'merged' (benchmark_precond_merged), or the same
+    solvers with the iteration loop on the device, 'plain_device' (benchmark_precond_device) and
+    'merged_device' (benchmark_precond_merged_device; one rank)"""
     if plugin not in _libs:
         path = os.path.join(_HERE, f"libbp4_host_{plugin}.so")
         if not os.path.exists(path):

@@ -1,10 +1,15 @@
 // host_capi.cc -- C entry points over the host-side mirror (benchmark.h + one plugin), so
 // that tests/ and bench.py can drive the SAME C++ path the CLI executables run: problem
 // set-up (mesh, Renumber, LaplaceOperator::initialize), the run_cg_solver plugin and vmult.
-// Built twice, once per plugin: libbp4_host_plain.so / libbp4_host_merged.so.
+// Built once per plugin: libbp4_host_plain.so / libbp4_host_merged.so and the device-resident
+// solves libbp4_host_plain_device.so / libbp4_host_merged_device.so.
 #define BP4_NO_MAIN
-#ifdef BP4_PLUGIN_MERGED
+#if defined(BP4_PLUGIN_MERGED)
 #  include "../benchmark_precond_merged/bench.cc"
+#elif defined(BP4_PLUGIN_PLAIN_DEVICE)
+#  include "../benchmark_precond_device/bench.cc"
+#elif defined(BP4_PLUGIN_MERGED_DEVICE)
+#  include "../benchmark_precond_merged_device/bench.cc"
 #else
 #  include "../benchmark_precond/bench.cc"
 #endif
@@ -75,8 +80,12 @@ extern "C" {
 const char *bp4h_last_error(void) { return g_error.c_str(); }
 const char *bp4h_plugin(void)
 {
-#ifdef BP4_PLUGIN_MERGED
+#if defined(BP4_PLUGIN_MERGED)
   return "benchmark_precond_merged";
+#elif defined(BP4_PLUGIN_PLAIN_DEVICE)
+  return "benchmark_precond_device";
+#elif defined(BP4_PLUGIN_MERGED_DEVICE)
+  return "benchmark_precond_merged_device";
 #else
   return "benchmark_precond";
 #endif

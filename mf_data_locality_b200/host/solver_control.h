@@ -37,6 +37,8 @@ namespace dealii
     double       last_value() const { return lvalue; }
     double       initial_value() const { return initial_val; }
     State        last_check() const { return lcheck; }
+    unsigned int max_steps() const { return maxsteps; }
+    double       tolerance() const { return tol; }
 
   protected:
     unsigned int maxsteps;
@@ -52,7 +54,8 @@ namespace dealii
     ReductionControl(unsigned int n = 100, double tol = 1e-10, double red = 1e-2)
       : SolverControl(n, tol), reduce(red)
     {}
-    State check(const unsigned int step, const double check_value) override
+    double reduction() const { return reduce; }
+    State  check(const unsigned int step, const double check_value) override
     {
       if (step == 0)
         {
