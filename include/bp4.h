@@ -98,6 +98,10 @@ typedef struct bp4_desc
    * use only constant and linear term"); with this field a caller can hand genuinely quadratic
    * cells (the MappingQCache(2) TODO of benchmark.h:75-77).  When given, `vertices` is ignored.  */
   const double *coefficients;
+  /* 1: deterministic mode (see bp4_deterministic_info), 0: default.  The environment variable
+   * BP4_DETERMINISTIC=1 turns it on for every context.  One rank only: with n_peers > 0 it is
+   * BP4_ERR_ARG.                                                                               */
+  int deterministic;
 } bp4_desc;
 
 const char *bp4_last_error(void);
@@ -195,6 +199,26 @@ int bp4_solve_cg(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec
 /* SolverCGFullMerge (solver_cg_optimized.h:192-302): x every second iteration, odd/even fix-up */
 int bp4_solve_cg_merged(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
                         unsigned max_steps, double tol, double reduce, bp4_solve_result *out);
+
+/* ---- deterministic mode -----------------------------------------------------------------
+ * With bp4_desc::deterministic (or BP4_DETERMINISTIC=1) every result of bp4_vmult,
+ * bp4_vmult_merged (vector and sums), bp4_inverse_diagonal / _vector, bp4_dot, bp4_add_and_dot,
+ * bp4_l2_norm, bp4_solve_cg and bp4_solve_cg_merged is a function of the inputs alone: repeated
+ * calls and repeated runs give the same bits, given the same build, the same device model and the
+ * same SM count, on one rank (no ghost-exchange plan; bp4_comm_init over several ranks is
+ * BP4_ERR_STATE).  How:
+ *   - the cells are coloured greedily in the given order (a cell takes the lowest colour that no
+ *     earlier cell sharing one of its valid entities has; at most 64 colours, else BP4_ERR_ARG)
+ *     and the cell loop and the diagonal assembly run one launch per colour: within a colour no
+ *     two cells touch the same DoF, so the additions into every entry happen in colour order;
+ *   - every reduction sums its per-block partials in a fixed order instead of with atomics, and
+ *     the host-driven and device-resident solves use the same reductions, so they give the same
+ *     sums and the same iterates, bit for bit;
+ *   - vmult_with_merged_sums always runs in the streamed form (bp4_debug_set_fused(ctx, 1) is
+ *     BP4_ERR_STATE).
+ * bp4_deterministic_info: *on = 1 in this mode; *n_colors = number of colours (0 when off);
+ * cell_color (optional, [n_cells], the caller's cell order) receives each cell's colour when on. */
+int bp4_deterministic_info(bp4_ctx *ctx, int *on, uint32_t *n_colors, uint32_t *cell_color);
 
 /* ---- multi-GPU (Utilities::MPI::Partitioner / MPI_Allreduce call sites, SURVEY 2a) ------- */
 #define BP4_NCCL_ID_BYTES 128

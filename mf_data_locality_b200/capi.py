@@ -31,7 +31,8 @@ class _Desc(C.Structure):
                 ("export_offset", C.c_void_p), ("export_index", C.c_void_p),
                 ("n_cells_before_comm", C.c_uint64), ("n_cells_comm", C.c_uint64),
                 ("n_ranges", C.c_uint64), ("range_cell_offset", C.c_void_p),
-                ("range_private_offset", C.c_void_p), ("coefficients", C.c_void_p)]
+                ("range_private_offset", C.c_void_p), ("coefficients", C.c_void_p),
+                ("deterministic", C.c_int)]
 
 
 _lib = None
@@ -44,7 +45,7 @@ EXPORTS = [
     "bp4_equ", "bp4_add", "bp4_sadd", "bp4_dot", "bp4_add_and_dot", "bp4_l2_norm", "bp4_all_zero",
     "bp4_comm_unique_id", "bp4_comm_init", "bp4_comm_info", "bp4_update_ghost_values", "bp4_compress_add",
     "bp4_profile_enable", "bp4_profile_reset", "bp4_profile_get", "bp4_launch_count",
-    "bp4_solve_cg", "bp4_solve_cg_merged",
+    "bp4_solve_cg", "bp4_solve_cg_merged", "bp4_deterministic_info",
 ]
 
 SUCCESS, FAILURE = 1, 2  # SolverControl::State of a device-resident solve
@@ -134,10 +135,12 @@ class Context:
     (poisson_operator.h:101-293)."""
 
     def __init__(self, degree, entity_index, vertices, n_owned, n_ghost=0, constrained=None,
-                 device=0, peers=None, ranges=None, partitions=None, coefficients=None):
+                 device=0, peers=None, ranges=None, partitions=None, coefficients=None,
+                 deterministic=False):
         """ranges = (range_cell_offset, range_private_offset): cell-batch ranges of the loop and
         the DoF runs private to them (bp4_desc::n_ranges); partitions = (n_cells_before_comm,
-        n_cells_comm) of the overlapped ghost exchange"""
+        n_cells_comm) of the overlapped ghost exchange; deterministic = bit-reproducible results
+        on one rank (bp4_desc::deterministic, also on with BP4_DETERMINISTIC=1)"""
         ei = np.ascontiguousarray(entity_index, dtype=np.uint32).reshape(-1, 27)
         vt = np.ascontiguousarray(vertices, dtype=np.float64).reshape(-1, 8, 3)
         assert len(ei) == len(vt)
@@ -169,6 +172,7 @@ class Context:
             keep += [cq]
         if partitions is not None:
             d.n_cells_before_comm, d.n_cells_comm = int(partitions[0]), int(partitions[1])
+        d.deterministic = 1 if deterministic else 0
         self.h = C.c_void_p()
         _chk(lib().bp4_ctx_create(C.byref(d), C.byref(self.h)))
         self.degree, self.n_cells = int(degree), len(ei)
@@ -224,6 +228,17 @@ class Context:
         f, npriv, nu = C.c_int(), C.c_uint64(), C.c_uint64()
         _chk(lib().bp4_fused_info(self.h, C.byref(f), C.byref(npriv), C.byref(nu)))
         return bool(f.value), int(npriv.value), int(nu.value)
+
+    def deterministic_info(self):
+        """(on, n_colors, colors): whether the context runs in the deterministic mode, its number of
+        cell colours and the colour of every cell in the caller's order (None when off)"""
+        on, nc = C.c_int(), C.c_uint32()
+        _chk(lib().bp4_deterministic_info(self.h, C.byref(on), C.byref(nc), None))
+        colors = None
+        if on.value:
+            colors = np.zeros(self.n_cells, dtype=np.uint32)
+            _chk(lib().bp4_deterministic_info(self.h, None, None, _ptr(colors)))
+        return bool(on.value), int(nc.value), colors
 
     def inverse_diagonal(self) -> Vector:
         v = Vector(self, self.n_owned // 3)

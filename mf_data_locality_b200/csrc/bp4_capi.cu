@@ -95,7 +95,8 @@ struct bp4_ctx
   double      *d_coef = nullptr, *d_gll = nullptr;
   double      *d_acc  = nullptr; // [8] reduction scratch
   int         *d_flag = nullptr;
-  uint32_t    *d_sched = nullptr; // [4] unit counters of the cell-kernel launches of one loop
+  uint32_t    *d_sched = nullptr; // [n_sched] unit counters of the cell-kernel launches of one loop
+  uint32_t     n_sched = 4;       // 4, or one per colour in the deterministic mode
   double      *h_acc  = nullptr; // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
   unsigned long long pub_seq = 0;
   int         *h_flag = nullptr; // pinned
@@ -112,6 +113,14 @@ struct bp4_ctx
   uint32_t        unit_part[4] = {0, 0, 0, 0}; // first unit of the three cell partitions (+ end)
   bp4::BatchDesc *d_batch      = nullptr;
   uint32_t       *d_unit_batch = nullptr;
+  // deterministic mode (DESIGN.md 4.6): cells stored colour by colour, colour k = stored cells
+  // [color_off[k], color_off[k+1]); cell_color[i] = colour of the caller's cell i; the ordered
+  // reductions' slots and ticket
+  bool                  deterministic = false;
+  uint32_t              n_colors      = 0;
+  std::vector<uint64_t> color_off;
+  std::vector<uint32_t> cell_color;
+  bp4::DetSlots         det;
   // multi-GPU
   ncclComm_t            comm = nullptr;
   int                   rank = 0, n_ranks = 1;
@@ -231,6 +240,19 @@ namespace
     return 0;
   }
 
+  // n rows of `width` elements to the device, in the caller's order or, with `order`, row order[j]
+  // as row j
+  template <typename T>
+  cudaError_t upload_rows(T *dst, const T *src, size_t width, uint64_t n, const std::vector<uint64_t> &order)
+  {
+    if (order.empty())
+      return cudaMemcpy(dst, src, sizeof(T) * width * n, cudaMemcpyHostToDevice);
+    std::vector<T> tmp(width * n);
+    for (uint64_t j = 0; j < n; ++j)
+      std::copy(src + width * order[j], src + width * (order[j] + 1), tmp.data() + width * j);
+    return cudaMemcpy(dst, tmp.data(), sizeof(T) * tmp.size(), cudaMemcpyHostToDevice);
+  }
+
   // sum of acc[0..k) over ranks, returned on the host
   int reduce_to_host(bp4_ctx *c, int k, double *out)
   {
@@ -341,14 +363,58 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   CU(cudaMalloc(&c->d_walk, sizeof(uint32_t) * walk.size()));
   CU(cudaMemcpy(c->d_walk, walk.data(), sizeof(uint32_t) * walk.size(), cudaMemcpyHostToDevice));
 
+  // deterministic mode: colour the cells greedily in the given order -- a cell takes the lowest
+  // colour that no earlier cell sharing one of its valid entities has -- and store them colour by
+  // colour.  Within a colour no two cells touch the same DoF, so a launch per colour adds at most
+  // once to every address.  One 64-bit colour mask per entity, keyed by its first DoF / 3.
+  std::vector<uint64_t> order; // stored cell j = the caller's cell order[j]
+  if (c->deterministic && d->n_cells)
+    {
+      const uint64_t        n_local = d->n_owned + d->n_ghost;
+      std::vector<uint64_t> mask(n_local / 3, 0);
+      c->cell_color.resize(d->n_cells);
+      for (uint64_t i = 0; i < d->n_cells; ++i)
+        {
+          const uint32_t *e    = d->entity_index + 27 * i;
+          uint64_t        used = 0;
+          for (int a = 0; a < 27; ++a)
+            if (e[a] != BP4_INVALID_INDEX)
+              {
+                if (e[a] >= n_local)
+                  return fail(BP4_ERR_ARG, "entity_index[%llu][%d] = %u is not a local DoF", (unsigned long long)i,
+                              a, e[a]);
+                used |= mask[e[a] / 3];
+              }
+          if (~used == 0)
+            return fail(BP4_ERR_ARG, "deterministic mode: cell %llu needs more than 64 colours",
+                        (unsigned long long)i);
+          const uint32_t col = (uint32_t)__builtin_ctzll(~used);
+          for (int a = 0; a < 27; ++a)
+            if (e[a] != BP4_INVALID_INDEX)
+              mask[e[a] / 3] |= 1ull << col;
+          c->cell_color[i] = col;
+          c->n_colors      = std::max(c->n_colors, col + 1);
+        }
+      c->color_off.assign(c->n_colors + 1, 0);
+      for (uint32_t col : c->cell_color)
+        ++c->color_off[col + 1];
+      for (uint32_t k = 0; k < c->n_colors; ++k)
+        c->color_off[k + 1] += c->color_off[k];
+      std::vector<uint64_t> next(c->color_off.begin(), c->color_off.end() - 1);
+      order.resize(d->n_cells);
+      for (uint64_t i = 0; i < d->n_cells; ++i)
+        order[next[c->cell_color[i]]++] = i;
+      c->n_sched = std::max<uint32_t>(c->n_sched, c->n_colors);
+    }
+
   const size_t nc = d->n_cells ? d->n_cells : 1;
   c->n_coef       = d->coefficients ? 81 : 24;
   CU(cudaMalloc(&c->d_entity, sizeof(uint32_t) * 27 * nc));
   CU(cudaMalloc(&c->d_coef, sizeof(double) * c->n_coef * nc));
   if (d->n_cells)
-    CU(cudaMemcpy(c->d_entity, d->entity_index, sizeof(uint32_t) * 27 * d->n_cells, cudaMemcpyHostToDevice));
+    CU(upload_rows(c->d_entity, d->entity_index, 27, d->n_cells, order));
   if (d->n_cells && d->coefficients) // all 27 coefficient vectors of the reference's kernel, as given
-    CU(cudaMemcpy(c->d_coef, d->coefficients, sizeof(double) * 81 * d->n_cells, cudaMemcpyHostToDevice));
+    CU(upload_rows(c->d_coef, d->coefficients, 81, d->n_cells, order));
   else if (d->n_cells)
     {
       // tri-linear coefficients from the 8 vertices, poisson_operator.h:161-178
@@ -369,7 +435,7 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
             o[18 + k] = v6 - v4 - (v2 - v0);
             o[21 + k] = (v7 - v6 - (v5 - v4) - (v3 - v2 - (v1 - v0)));
           }
-      CU(cudaMemcpy(c->d_coef, cf.data(), sizeof(double) * cf.size(), cudaMemcpyHostToDevice));
+      CU(upload_rows(c->d_coef, cf.data(), 24, d->n_cells, order));
     }
   CU(cudaMalloc(&c->d_constrained, sizeof(uint32_t) * (d->n_constrained ? d->n_constrained : 1)));
   if (d->n_constrained)
@@ -382,7 +448,14 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   CU(cudaMalloc(&c->d_acc, sizeof(double) * 8));
   CU(cudaMemset(c->d_acc, 0, sizeof(double) * 8));
   CU(cudaMalloc(&c->d_flag, sizeof(int)));
-  CU(cudaMalloc(&c->d_sched, sizeof(uint32_t) * 4));
+  CU(cudaMalloc(&c->d_sched, sizeof(uint32_t) * c->n_sched));
+  if (c->deterministic)
+    {
+      const size_t n_slot = (size_t)8 * 8 * c->sms; // K <= 7 partials of <= 8 * SMs blocks (stream_grid)
+      CU(cudaMalloc(&c->det.slot, sizeof(double) * n_slot));
+      CU(cudaMalloc(&c->det.ticket, sizeof(uint32_t)));
+      CU(cudaMemset(c->det.ticket, 0, sizeof(uint32_t)));
+    }
   CU(cudaMallocHost(&c->h_acc, sizeof(double) * 16)); // UVA: the pointer is valid on the device too
   memset(c->h_acc, 0, sizeof(double) * 16);
   CU(cudaMallocHost(&c->h_flag, sizeof(int)));
@@ -447,6 +520,8 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
           c->fused_pinned = true;
         }
     }
+  if (c->deterministic) // the in-loop sums are per-block atomics, and ranges do not survive colouring
+    c->fused = 0, c->n_private = 0;
 
   // ghost exchange plan
   if (d->n_peers > 0)
@@ -476,12 +551,17 @@ int bp4_ctx_create(const bp4_desc *d, bp4_ctx **out)
     return fail(BP4_ERR_ARG, "local vector exceeds 32-bit local indices (poisson_operator.h:693)");
   if (d->n_cells && (!d->entity_index || (!d->vertices && !d->coefficients)))
     return fail(BP4_ERR_ARG, "entity_index/vertices missing");
+  const char *det_env       = getenv("BP4_DETERMINISTIC");
+  const bool  deterministic = d->deterministic != 0 || (det_env && atoi(det_env) != 0);
+  if (deterministic && d->n_peers > 0)
+    return fail(BP4_ERR_ARG, "the deterministic mode runs on one rank: the descriptor has a ghost-exchange plan");
   int ndev = 0;
   CU(cudaGetDeviceCount(&ndev));
   if (ndev == 0)
     return fail(BP4_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
   CU(cudaSetDevice(d->device));
-  bp4_ctx *c = new bp4_ctx;
+  bp4_ctx *c       = new bp4_ctx;
+  c->deterministic = deterministic;
   if (int e = ctx_create_impl(d, c))
     {
       const std::string msg = g_err; // bp4_ctx_destroy must not clobber the message
@@ -529,6 +609,8 @@ int bp4_ctx_destroy(bp4_ctx *c)
   cudaFree(c->d_acc);
   cudaFree(c->d_flag);
   cudaFree(c->d_sched);
+  cudaFree(c->det.slot);
+  cudaFree(c->det.ticket);
   cudaFree(c->d_batch);
   cudaFree(c->d_unit_batch);
   cudaFree(c->d_export);
@@ -726,6 +808,19 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       Timed t(c, BP4_K_MERGED);
       CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream));
     }
+  else if (c->deterministic) // one launch per colour (single rank: part = -1), timed as one loop
+    {
+      Timed t(c, BP4_K_VMULT, (int)c->n_colors);
+      for (uint32_t k = 0; k < c->n_colors; ++k)
+        {
+          const uint64_t c0 = c->color_off[k];
+          a.entity_index    = c->d_entity + 27 * c0;
+          a.coef            = c->d_coef + (uint64_t)c->n_coef * c0;
+          a.n_cells         = c->color_off[k + 1] - c0;
+          a.sched           = c->d_sched + k;
+          CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream));
+        }
+    }
   else
     {
       a.entity_index = c->d_entity + 27 * begin;
@@ -751,7 +846,7 @@ static int compress_release(bp4_ctx *c, cudaStream_t st);
 // dst must already be zero where the cells accumulate (owned and ghost slots).
 static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCall *m)
 {
-  CU(cudaMemsetAsync(c->d_sched, 0, sizeof(uint32_t) * 4, c->stream));
+  CU(cudaMemsetAsync(c->d_sched, 0, sizeof(uint32_t) * c->n_sched, c->stream));
   if (c->peer.empty())
     return cell_range(c, dst, src, -1, m);
   if (!c->comm)
@@ -826,6 +921,9 @@ int bp4_debug_set_fused(bp4_ctx *c, int on)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
+  if (on && c->deterministic)
+    return fail(BP4_ERR_STATE, "the deterministic mode runs the streamed form only (the in-loop sums are "
+                               "per-block atomics)");
   if (on && c->n_private == 0)
     return fail(BP4_ERR_STATE, "no private DoF runs: the context was created without range tables, with "
                                "quadratic geometry, at a degree without a fused kernel (> 4), or with runs "
@@ -872,7 +970,7 @@ static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
   if (n > tail)
     {
       Timed t(c, BP4_K_POST);
-      CU(bp4::launch_post(tail, n, m.g, m.d, h, m.prec, c->d_acc, c->sms, c->stream));
+      CU(bp4::launch_post(tail, n, m.g, m.d, h, m.prec, c->d_acc, c->det, c->sms, c->stream));
     }
   return 0;
 }
@@ -895,6 +993,23 @@ int bp4_vmult_merged(bp4_ctx *c, bp4_vec *x, bp4_vec *g, bp4_vec *d, bp4_vec *h,
   return reduce_to_host(c, 7, out);
 }
 
+// the scalar GLL diagonal added into diag[3 * node]: one launch, or one per colour in the
+// deterministic mode (every entry then gets at most one atomic add per launch); the launch count
+// of the record includes the `more` launches of the caller that follow
+static int assemble_diagonal(bp4_ctx *c, double *diag, int more)
+{
+  const uint32_t n_groups = c->deterministic ? c->n_colors : 1;
+  Timed          t(c, BP4_K_BLAS1, (int)n_groups + more);
+  for (uint32_t k = 0; k < n_groups; ++k)
+    {
+      const uint64_t c0 = c->deterministic ? c->color_off[k] : 0,
+                     c1 = c->deterministic ? c->color_off[k + 1] : c->n_cells;
+      CU(bp4::launch_diag_assemble(c->degree, c1 - c0, c->d_entity + 27 * c0, c->d_coef + (uint64_t)c->n_coef * c0,
+                                   c->n_coef, c->d_gll, diag, 3, c->stream));
+    }
+  return 0;
+}
+
 int bp4_inverse_diagonal(bp4_ctx *c, bp4_vec *out)
 {
   if (!c || !out)
@@ -907,11 +1022,8 @@ int bp4_inverse_diagonal(bp4_ctx *c, bp4_vec *out)
   bp4_vec *tmp = nullptr;
   if (int e = bp4_vec_alloc(c, c->n_owned + c->n_ghost, &tmp))
     return e;
-  {
-    Timed t(c, BP4_K_BLAS1, 3);
-    CU(bp4::launch_diag_assemble(c->degree, c->n_cells, c->d_entity, c->d_coef, c->n_coef, c->d_gll, tmp->p(), 3,
-                                 c->stream));
-  }
+  if (int e = assemble_diagonal(c, tmp->p(), 2))
+    return e;
   if (!c->peer.empty())
     if (int e = bp4_compress_add(c, tmp))
       return e;
@@ -930,11 +1042,8 @@ int bp4_inverse_diagonal_vector(bp4_ctx *c, bp4_vec *out)
     return e;
   CU(cudaSetDevice(c->device));
   CU(cudaMemsetAsync(out->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream));
-  {
-    Timed t(c, BP4_K_BLAS1, 2);
-    CU(bp4::launch_diag_assemble(c->degree, c->n_cells, c->d_entity, c->d_coef, c->n_coef, c->d_gll, out->p(), 3,
-                                 c->stream));
-  }
+  if (int e = assemble_diagonal(c, out->p(), 1))
+    return e;
   if (!c->peer.empty())
     if (int e = bp4_compress_add(c, out))
       return e;
@@ -1027,7 +1136,7 @@ int bp4_dot(bp4_ctx *c, const bp4_vec *a, const bp4_vec *b, double *result)
   CU(cudaSetDevice(c->device));
   {
     Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_dot(sweep_len(c, {a, b}), a->p(), b->p(), c->d_acc, c->sms, c->stream));
+    CU(bp4::launch_dot(sweep_len(c, {a, b}), a->p(), b->p(), c->d_acc, c->det, c->sms, c->stream));
   }
   return reduce_to_host(c, 1, result);
 }
@@ -1039,7 +1148,8 @@ int bp4_add_and_dot(bp4_ctx *c, bp4_vec *g, double a, const bp4_vec *h, const bp
   CU(cudaSetDevice(c->device));
   {
     Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_add_and_dot(sweep_len(c, {g, h, w}), g->p(), a, h->p(), w->p(), c->d_acc, c->sms, c->stream));
+    CU(bp4::launch_add_and_dot(sweep_len(c, {g, h, w}), g->p(), a, h->p(), w->p(), c->d_acc, c->det, c->sms,
+                               c->stream));
   }
   return reduce_to_host(c, 1, result);
 }
@@ -1124,7 +1234,7 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
       return 0;
     {
       Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->sms, c->stream));
+      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->det, c->sms, c->stream));
     }
     {
       Timed t(c, BP4_K_BLAS1);
@@ -1159,7 +1269,7 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
       return e;
     {
       Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_dot(n, sg.d, sg.h, acc, c->sms, c->stream));
+      CU(bp4::launch_dot(n, sg.d, sg.h, acc, c->det, c->sms, c->stream));
     }
     {
       Timed t(c, BP4_K_BLAS1);
@@ -1167,11 +1277,11 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
     }
     {
       Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_cg_xg(n, x, sg.g, sg.d, sg.h, st, acc + 1, c->sms, c->stream));
+      CU(bp4::launch_cg_xg(n, x, sg.g, sg.d, sg.h, st, acc + 1, c->det, c->sms, c->stream));
     }
     {
       Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->sms, c->stream));
+      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->det, c->sms, c->stream));
     }
     {
       Timed t(c, BP4_K_BLAS1);
@@ -1188,7 +1298,7 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
     if (sg.merged)
       {
         Timed t(c, BP4_K_BLAS1);
-        CU(bp4::launch_solve_final(n, x, sg.d, sg.g, prec, st, c->sms, c->stream));
+        CU(bp4::launch_solve_final(n, x, sg.d, sg.g, prec, st, c->deterministic, c->sms, c->stream));
       }
     CU(cudaMemcpyAsync(c->h_state + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream));
     return 0;
@@ -1434,6 +1544,8 @@ int bp4_comm_init(bp4_ctx *c, int rank, int n_ranks, const unsigned char id[BP4_
 {
   if (!c || !id)
     return fail(BP4_ERR_ARG, "null argument");
+  if (c->deterministic && n_ranks > 1)
+    return fail(BP4_ERR_STATE, "the deterministic mode runs on one rank");
   CU(cudaSetDevice(c->device));
   ncclUniqueId u;
   memcpy(&u, id, sizeof(u));
@@ -1597,6 +1709,20 @@ int bp4_compress_add(bp4_ctx *c, bp4_vec *v)
   if (int e = compress_release(c, c->stream))
     return e;
   CU(cudaMemsetAsync(v->p() + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream));
+  return 0;
+}
+
+// ---- deterministic mode --------------------------------------------------------------------
+int bp4_deterministic_info(bp4_ctx *c, int *on, uint32_t *n_colors, uint32_t *cell_color)
+{
+  if (!c)
+    return fail(BP4_ERR_ARG, "null ctx");
+  if (on)
+    *on = c->deterministic ? 1 : 0;
+  if (n_colors)
+    *n_colors = c->n_colors;
+  if (cell_color)
+    std::copy(c->cell_color.begin(), c->cell_color.end(), cell_color);
   return 0;
 }
 

@@ -124,6 +124,16 @@ namespace bp4
     static constexpr bool OK    = Cfg<P>::STAGED && JOB >= 64;
   };
 
+  // Scratch of the ordered reductions of the deterministic mode (DESIGN.md 4.6): every block of a
+  // reduction writes its K partial sums to slot[k * gridDim.x + blockIdx.x]; the last block to
+  // take a ticket sums them in a fixed order.  slot = nullptr: the reductions end with one
+  // atomicAdd per block instead (default).
+  struct DetSlots
+  {
+    double   *slot   = nullptr; // [K][grid], grid <= 8 * SMs
+    uint32_t *ticket = nullptr; // zero between launches: the last block re-arms it
+  };
+
   struct SolveState;
   struct CellArgs
   {

@@ -29,18 +29,20 @@ namespace bp4
   cudaError_t launch_pre_dev(uint64_t begin, uint64_t end, double *h, double *x, double *r, double *p,
                              const double *prec, const SolveState *state, double *acc_to_zero, int sms,
                              cudaStream_t st);
+  // the reductions below: det.slot set = ordered cross-block sums (deterministic mode), else atomics
   cudaError_t launch_post(uint64_t begin, uint64_t end, const double *r, const double *d,
-                          const double *h, const double *prec, double *acc, int sms, cudaStream_t st);
+                          const double *h, const double *prec, double *acc, const DetSlots &det, int sms,
+                          cudaStream_t st);
   cudaError_t launch_fixup(uint64_t n, const uint32_t *con, double *dst, const double *src,
                            cudaStream_t st);
   cudaError_t launch_sadd(uint64_t n, double *dst, double s, double a, const double *src, int sms,
                           cudaStream_t st);
   cudaError_t launch_sadd_dev(uint64_t n, double *dst, const double *s, double a, const double *src, int sms,
                               cudaStream_t st); // s read on the device
-  cudaError_t launch_dot(uint64_t n, const double *a, const double *b, double *acc, int sms,
-                         cudaStream_t st);
+  cudaError_t launch_dot(uint64_t n, const double *a, const double *b, double *acc, const DetSlots &det,
+                         int sms, cudaStream_t st);
   cudaError_t launch_add_and_dot(uint64_t n, double *g, double a, const double *h, const double *w,
-                                 double *acc, int sms, cudaStream_t st);
+                                 double *acc, const DetSlots &det, int sms, cudaStream_t st);
   cudaError_t launch_nonzero(uint64_t n, const double *v, int *flag, int sms, cudaStream_t st);
   cudaError_t launch_jacobi(uint64_t n, double *dst, const double *src, const double *diag, int sms,
                             cudaStream_t st);
@@ -54,14 +56,15 @@ namespace bp4
     kSolvePlainAlpha = 2,
     kSolvePlainCheck = 3
   };
-  cudaError_t launch_jacobi_dot(uint64_t n, double *h, const double *g, const double *diag, double *acc, int sms,
-                                cudaStream_t st);
+  cudaError_t launch_jacobi_dot(uint64_t n, double *h, const double *g, const double *diag, double *acc,
+                                const DetSlots &det, int sms, cudaStream_t st);
   cudaError_t launch_cg_xg(uint64_t n, double *x, double *g, const double *d, const double *h,
-                           const SolveState *state, double *acc, int sms, cudaStream_t st);
+                           const SolveState *state, double *acc, const DetSlots &det, int sms, cudaStream_t st);
   cudaError_t launch_solve_scalar(int kind, SolveState *state, double *acc, cudaGraphConditionalHandle loop,
                                   cudaStream_t st);
+  // det: the odd-step update rounded as bp4_add rounds it (deterministic mode)
   cudaError_t launch_solve_final(uint64_t n, double *x, const double *d, const double *g, const double *prec,
-                                 const SolveState *state, int sms, cudaStream_t st);
+                                 const SolveState *state, bool det, int sms, cudaStream_t st);
   cudaError_t launch_diag_assemble(int degree, uint64_t n_cells, const uint32_t *entity_index,
                                    const double *coef, int n_coef, const double *gll, double *diag,
                                    int stride, cudaStream_t st);

@@ -45,13 +45,14 @@ class Problem:
 
     def __init__(self, degree, s, plugin="merged", n_ranks=1, rank=0, device=0, n_lanes=8,
                  batches_per_range=1, renumber=(0, 1, 2), nccl_id: bytes | None = None,
-                 numbering_only=False, mapping_degree=1):
+                 numbering_only=False, mapping_degree=1, deterministic=False):
         """nccl_id: the 128-byte ncclUniqueId shared by all ranks (needed when n_ranks > 1 and a
-        device is used; see capi.unique_id())"""
+        device is used; see capi.unique_id()); deterministic: bit-reproducible operator, reductions
+        and solves on one rank (bp4_desc::deterministic)"""
         self.l = lib(plugin)
         self.plugin = plugin
-        opts = (C.c_int * 10)(n_ranks, rank, device, n_lanes, batches_per_range, *renumber,
-                              1 if numbering_only else 0, mapping_degree)
+        opts = (C.c_int * 11)(n_ranks, rank, device, n_lanes, batches_per_range, *renumber,
+                              1 if numbering_only else 0, mapping_degree, 1 if deterministic else 0)
         idbuf = (C.c_ubyte * 128).from_buffer_copy(nccl_id) if nccl_id else None
         self.h = C.c_void_p()
         self._chk(self.l.bp4h_create(C.c_int(degree), C.c_int(s), opts, idbuf, C.byref(self.h)))

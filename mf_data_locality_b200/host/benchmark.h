@@ -81,6 +81,7 @@ struct BenchmarkOptions
   const unsigned char *nccl_id = nullptr;
   unsigned int mapping_degree = 1; // 2: genuinely quadratic cells (the TODO of benchmark.h:75-77)
   bool numbering_only = false; // stop after Renumber + MatrixFree::reinit (inspection of numberings)
+  bool deterministic  = false; // bit-reproducible results on one rank (bp4_desc::deterministic)
 };
 
 class Timer
@@ -146,7 +147,7 @@ struct BenchmarkProblem
     tick("matrix_free.reinit");
     if (opt.numbering_only)
       return;
-    laplace_operator.initialize(matrix_free, constraints, opt.device);
+    laplace_operator.initialize(matrix_free, constraints, opt.device, opt.deterministic);
     tick("operator.initialize");
     if (opt.device < 0)
       return; // tables only

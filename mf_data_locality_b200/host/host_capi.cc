@@ -92,7 +92,7 @@ const char *bp4h_plugin(void)
 }
 
 // options: [n_ranks, rank, device, n_lanes, batches_per_range, renumber_a, renumber_r, renumber_g,
-//           numbering_only, mapping_degree]
+//           numbering_only, mapping_degree, deterministic]
 int bp4h_create(int degree, int s, const int *options, const unsigned char *nccl_id, void **out)
 {
   return guarded([&] {
@@ -105,6 +105,7 @@ int bp4h_create(int degree, int s, const int *options, const unsigned char *nccl
         opt.renumber_a = options[5], opt.renumber_r = options[6], opt.renumber_g = options[7];
         opt.numbering_only = options[8] != 0;
         opt.mapping_degree = options[9] > 0 ? options[9] : 1;
+        opt.deterministic  = options[10] != 0;
       }
     Timer        t;
     ProblemBase *p = nullptr;

@@ -41,7 +41,7 @@ namespace Poisson
     }
 
     void initialize(std::shared_ptr<const MatrixFree> data_, const AffineConstraints &constraints,
-                    const int device = 0)
+                    const int device = 0, const bool deterministic = false)
     {
       data = data_;
       const DoFHandler &dh = data->get_dof_handler();
@@ -141,6 +141,7 @@ namespace Poisson
       desc.export_index  = part.export_index.data();
       desc.n_cells_before_comm = data->n_cells_before_comm;
       desc.n_cells_comm        = data->n_cells_comm;
+      desc.deterministic       = deterministic ? 1 : 0;
       if (ctx)
         bp4_ctx_destroy(ctx);
       ctx = nullptr;
