@@ -18,6 +18,7 @@
 
 #include "../../include/bp4.h"
 #include "bp4_launch.h"
+#include "bp4_vector_kernels.cuh"
 
 namespace
 {
@@ -222,6 +223,37 @@ namespace
     return 0;
   }
 
+  // The vector kernels (bp4_vector_kernels.cuh) are launched on the context's stream by one helper
+  // per grid rule; nothing is launched for n == 0, a launch error becomes BP4_ERR_CUDA.
+  int stream_grid(uint64_t n, int sms)
+  {
+    const uint64_t blocks = (n + 255) / 256;
+    return (int)std::min<uint64_t>(std::max<uint64_t>(blocks, 1), (uint64_t)sms * 8);
+  }
+
+  // a grid-stride sweep over n elements: stream_grid(n) blocks of 256 threads, one Timed record of `id`
+  template <typename... P, typename... A>
+  int sweep(bp4_ctx *c, int id, uint64_t n, void (*kernel)(P...), A... args)
+  {
+    Timed t(c, id);
+    if (n == 0)
+      return 0;
+    kernel<<<stream_grid(n, c->sms), 256, 0, c->stream>>>(args...);
+    CU(cudaGetLastError());
+    return 0;
+  }
+
+  // one thread per element: ceil(n / B) blocks of B threads, counted in the caller's Timed record
+  template <int B = 256, typename... P, typename... A>
+  int per_element(bp4_ctx *c, uint64_t n, void (*kernel)(P...), A... args)
+  {
+    if (n == 0)
+      return 0;
+    kernel<<<(unsigned)((n + B - 1) / B), B, 0, c->stream>>>(args...);
+    CU(cudaGetLastError());
+    return 0;
+  }
+
   // buffer of n doubles, from the pool when one of that size is cached; zeroed on request only
   // (SolverCGFullMerge takes its temporaries with omit_zeroing_entries = true,
   // solver_cg_optimized.h:215-217)
@@ -262,7 +294,8 @@ namespace
     // pinned memory; the host polls that word (and the stream, for errors, now and then)
     volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc + 8);
     const unsigned long long     seq      = ++c->pub_seq;
-    CU(bp4::launch_publish(c->d_acc, k, c->h_acc, const_cast<unsigned long long *>(seq_word), seq, c->stream));
+    bp4::publish_kernel<<<1, 32, 0, c->stream>>>(c->d_acc, k, c->h_acc, seq_word, seq);
+    CU(cudaGetLastError());
     c->launches += 1;
     int idle = 0;
     for (unsigned long long spins = 1; *seq_word != seq; ++spins)
@@ -834,8 +867,7 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
 
 static int exchange_ghosts_on(bp4_ctx *c, double *v, cudaStream_t st);
 static int exchange_compress_on(bp4_ctx *c, double *v, cudaStream_t st);
-static const double *contrib_buffer(const bp4_ctx *c);
-static int compress_release(bp4_ctx *c, cudaStream_t st);
+static int compress_finish(bp4_ctx *c, double *v);
 
 
 // MatrixFree::cell_loop (poisson_operator.h:310, :339) on one rank: update_ghost_values(src),
@@ -855,7 +887,8 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
   const bool     overlap = c->overlap && c->n_comm > 0;
   {
     Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_pack(ne, c->d_export, src, c->d_sendbuf, c->stream));
+    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export, src, c->d_sendbuf))
+      return e;
   }
   CU(cudaEventRecord(c->ev_a, c->stream));
   CU(cudaStreamWaitEvent(c->comm_stream, c->ev_a, 0));
@@ -882,14 +915,7 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
     if (int e = cell_range(c, dst, src, 2, m))
       return e;
   CU(cudaStreamWaitEvent(c->stream, c->ev_b, 0));
-  {
-    Timed t(c, BP4_K_BLAS1); // one launch for all peers: an owned entry may be exported to several (atomics)
-    CU(bp4::launch_unpack_add(c->export_off.back(), c->d_export, contrib_buffer(c), dst, c->stream));
-  }
-  if (int e = compress_release(c, c->stream))
-    return e;
-  CU(cudaMemsetAsync(dst + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream));
-  return 0;
+  return compress_finish(c, dst);
 }
 
 // dst = A src on the context's stream (also captured into the plain device solve's loop body)
@@ -899,8 +925,7 @@ static int vmult_on(bp4_ctx *c, double *dst, const double *src)
   if (int e = cell_loop(c, dst, src, nullptr))
     return e;
   Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_fixup(c->n_constrained, c->d_constrained, dst, src, c->stream));
-  return 0;
+  return per_element(c, c->n_constrained, bp4::fixup_kernel, c->n_constrained, c->d_constrained, dst, src);
 }
 
 int bp4_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
@@ -955,23 +980,18 @@ static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
   // kernel; the rest of the vector -- shared between ranges or ranks, Dirichlet -- is streamed
   // before / after the loop (with the fused path off: everything)
   const uint64_t tail = c->fused ? c->n_private : 0;
-  {
-    Timed t(c, BP4_K_PRE);
-    if (m.state)
-      CU(bp4::launch_pre_dev(tail, n, h, m.x, m.g, m.d, m.prec, m.state, c->d_acc, c->sms, c->stream));
-    else
-      CU(bp4::launch_pre(tail, n, h, m.x, m.g, m.d, m.prec, m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc,
-                         c->sms, c->stream));
-  }
+  // one block at least: pre_kernel also clears the reduction scratch
+  if (int e = sweep(c, BP4_K_PRE, std::max<uint64_t>(n - tail, 1),
+                    m.state ? bp4::pre_kernel<true> : bp4::pre_kernel<false>, tail, n, h, m.x, m.g, m.d, m.prec,
+                    m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc, m.state))
+    return e;
   if (c->n_ghost)
     CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream));
   if (int e = cell_loop(c, h, m.d, c->fused ? &m : nullptr))
     return e;
   if (n > tail)
-    {
-      Timed t(c, BP4_K_POST);
-      CU(bp4::launch_post(tail, n, m.g, m.d, h, m.prec, c->d_acc, c->det, c->sms, c->stream));
-    }
+    return sweep(c, BP4_K_POST, n - tail, c->deterministic ? bp4::post_kernel<true> : bp4::post_kernel<false>, tail,
+                 n, m.g, m.d, h, m.prec, c->d_acc, c->det);
   return 0;
 }
 
@@ -999,13 +1019,15 @@ int bp4_vmult_merged(bp4_ctx *c, bp4_vec *x, bp4_vec *g, bp4_vec *d, bp4_vec *h,
 static int assemble_diagonal(bp4_ctx *c, double *diag, int more)
 {
   const uint32_t n_groups = c->deterministic ? c->n_colors : 1;
+  const uint64_t n3       = (uint64_t)(c->degree + 1) * (c->degree + 1) * (c->degree + 1);
   Timed          t(c, BP4_K_BLAS1, (int)n_groups + more);
   for (uint32_t k = 0; k < n_groups; ++k)
     {
       const uint64_t c0 = c->deterministic ? c->color_off[k] : 0,
                      c1 = c->deterministic ? c->color_off[k + 1] : c->n_cells;
-      CU(bp4::launch_diag_assemble(c->degree, c1 - c0, c->d_entity + 27 * c0, c->d_coef + (uint64_t)c->n_coef * c0,
-                                   c->n_coef, c->d_gll, diag, 3, c->stream));
+      if (int e = per_element<128>(c, (c1 - c0) * n3, bp4::diag_kernel, c->degree, c1 - c0, c->d_entity + 27 * c0,
+                                   c->d_coef + (uint64_t)c->n_coef * c0, c->n_coef, c->d_gll, diag, 3))
+        return e;
     }
   return 0;
 }
@@ -1027,8 +1049,11 @@ int bp4_inverse_diagonal(bp4_ctx *c, bp4_vec *out)
   if (!c->peer.empty())
     if (int e = bp4_compress_add(c, tmp))
       return e;
-  CU(bp4::launch_stride3(c->n_owned / 3, tmp->p(), out->p(), c->stream));
-  CU(bp4::launch_diag_invert(c->n_owned / 3, out->p(), c->stream));
+  const uint64_t n_nodes = c->n_owned / 3;
+  if (int e = per_element(c, n_nodes, bp4::stride3_kernel, n_nodes, tmp->p(), out->p()))
+    return e;
+  if (int e = per_element(c, n_nodes, bp4::invert_diag_kernel, n_nodes, out->p()))
+    return e;
   return bp4_vec_free(c, tmp);
 }
 
@@ -1047,8 +1072,7 @@ int bp4_inverse_diagonal_vector(bp4_ctx *c, bp4_vec *out)
   if (!c->peer.empty())
     if (int e = bp4_compress_add(c, out))
       return e;
-  CU(bp4::launch_diag_invert(c->n_owned, out->p(), c->stream));
-  return 0;
+  return per_element(c, c->n_owned, bp4::invert_diag_kernel, c->n_owned, out->p());
 }
 
 // dst[i] = src[n_components * i + component]: the extraction loop of benchmark.h:141-147
@@ -1063,8 +1087,7 @@ int bp4_extract_component(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src, int n_co
                 (unsigned long long)dst->n);
   CU(cudaSetDevice(c->device));
   Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_stride3(c->n_owned / 3, src->p() + component, dst->p(), c->stream));
-  return 0;
+  return per_element(c, c->n_owned / 3, bp4::stride3_kernel, c->n_owned / 3, src->p() + component, dst->p());
 }
 
 int bp4_jacobi_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src, const bp4_vec *diag)
@@ -1075,9 +1098,7 @@ int bp4_jacobi_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src, const bp4_vec
     return fail(BP4_ERR_ARG, "Dimension mismatch %llu vs 3 x %llu", (unsigned long long)dst->n,
                 (unsigned long long)diag->n);
   CU(cudaSetDevice(c->device));
-  Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_jacobi(c->n_owned, dst->p(), src->p(), diag->p(), c->sms, c->stream));
-  return 0;
+  return sweep(c, BP4_K_BLAS1, c->n_owned, bp4::jacobi_kernel, c->n_owned, dst->p(), src->p(), diag->p());
 }
 
 int bp4_x_finalize_even(bp4_ctx *c, bp4_vec *x, const bp4_vec *d, const bp4_vec *g, const bp4_vec *prec,
@@ -1094,29 +1115,8 @@ int bp4_x_finalize_even(bp4_ctx *c, bp4_vec *x, const bp4_vec *d, const bp4_vec 
   if (3 * prec->n < c->n_owned)
     return fail(BP4_ERR_ARG, "prec needs n_owned/3 entries");
   CU(cudaSetDevice(c->device));
-  Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_xfinal(c->n_owned, x->p(), d->p(), g->p(), prec->p(), c1, c2, c->sms, c->stream));
-  return 0;
-}
-
-int bp4_equ(bp4_ctx *c, bp4_vec *dst, double a, const bp4_vec *src)
-{
-  if (!c || !dst || !src)
-    return fail(BP4_ERR_ARG, "null argument");
-  CU(cudaSetDevice(c->device));
-  Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_sadd(sweep_len(c, {dst, src}), dst->p(), 0., a, src->p(), c->sms, c->stream));
-  return 0;
-}
-
-int bp4_add(bp4_ctx *c, bp4_vec *dst, double a, const bp4_vec *src)
-{
-  if (!c || !dst || !src)
-    return fail(BP4_ERR_ARG, "null argument");
-  CU(cudaSetDevice(c->device));
-  Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_sadd(sweep_len(c, {dst, src}), dst->p(), 1., a, src->p(), c->sms, c->stream));
-  return 0;
+  return sweep(c, BP4_K_BLAS1, c->n_owned, bp4::xfinal_kernel, c->n_owned, x->p(), d->p(), g->p(), prec->p(), c1,
+               c2);
 }
 
 int bp4_sadd(bp4_ctx *c, bp4_vec *dst, double s, double a, const bp4_vec *src)
@@ -1124,20 +1124,22 @@ int bp4_sadd(bp4_ctx *c, bp4_vec *dst, double s, double a, const bp4_vec *src)
   if (!c || !dst || !src)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  Timed t(c, BP4_K_BLAS1);
-  CU(bp4::launch_sadd(sweep_len(c, {dst, src}), dst->p(), s, a, src->p(), c->sms, c->stream));
-  return 0;
+  const uint64_t n = sweep_len(c, {dst, src});
+  return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<false>, n, dst->p(), s, a, src->p(), nullptr);
 }
+
+int bp4_equ(bp4_ctx *c, bp4_vec *dst, double a, const bp4_vec *src) { return bp4_sadd(c, dst, 0., a, src); }
+int bp4_add(bp4_ctx *c, bp4_vec *dst, double a, const bp4_vec *src) { return bp4_sadd(c, dst, 1., a, src); }
 
 int bp4_dot(bp4_ctx *c, const bp4_vec *a, const bp4_vec *b, double *result)
 {
   if (!c || !a || !b || !result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  {
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_dot(sweep_len(c, {a, b}), a->p(), b->p(), c->d_acc, c->det, c->sms, c->stream));
-  }
+  const uint64_t n = sweep_len(c, {a, b});
+  if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, a->p(),
+                    b->p(), c->d_acc, c->det))
+    return e;
   return reduce_to_host(c, 1, result);
 }
 
@@ -1146,11 +1148,11 @@ int bp4_add_and_dot(bp4_ctx *c, bp4_vec *g, double a, const bp4_vec *h, const bp
   if (!c || !g || !h || !w || !result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  {
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_add_and_dot(sweep_len(c, {g, h, w}), g->p(), a, h->p(), w->p(), c->d_acc, c->det, c->sms,
-                               c->stream));
-  }
+  const uint64_t n = sweep_len(c, {g, h, w});
+  if (int e = sweep(c, BP4_K_BLAS1, n,
+                    c->deterministic ? bp4::add_and_dot_kernel<true> : bp4::add_and_dot_kernel<false>, n, g->p(), a,
+                    h->p(), w->p(), c->d_acc, c->det))
+    return e;
   return reduce_to_host(c, 1, result);
 }
 
@@ -1169,10 +1171,9 @@ int bp4_all_zero(bp4_ctx *c, const bp4_vec *v, int *result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
   CU(cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
-  {
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_nonzero(sweep_len(c, {v}), v->p(), c->d_flag, c->sms, c->stream));
-  }
+  const uint64_t n = sweep_len(c, {v});
+  if (int e = sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, v->p(), c->d_flag))
+    return e;
   if (c->comm)
     NC(ncclAllReduce(c->d_flag, c->d_flag, 1, ncclInt, ncclMax, c->comm, c->stream));
   CU(cudaMemcpyAsync(c->h_flag, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
@@ -1227,22 +1228,26 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   cudaGraphConditionalHandle loop;
   CU(cudaGraphConditionalHandleCreate(&loop, sg.graph, 1, cudaGraphCondAssignDefault));
   std::vector<cudaGraphNode_t> leaves;
+  auto jacobi_dot = [&]() { // h = P g, g.h -> acc[2]
+    return sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::jacobi_dot_kernel<true> : bp4::jacobi_dot_kernel<false>,
+                 n, sg.h, sg.g, prec, acc + 2, c->det);
+  };
+  auto scalar = [&](const int kind) -> int { // solve_scalar_kernel on one thread
+    Timed t(c, BP4_K_BLAS1);
+    bp4::solve_scalar_kernel<<<1, 32, 0, c->stream>>>(kind, st, acc, loop);
+    CU(cudaGetLastError());
+    return 0;
+  };
   // initial state; plain: h = P g, d = -h, gh = g.h (SolverCG before its loop)
   auto prologue = [&]() -> int {
     CU(cudaMemcpyAsync(st, c->h_state, sizeof(bp4::SolveState), cudaMemcpyHostToDevice, c->stream));
     if (sg.merged)
       return 0;
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->det, c->sms, c->stream));
-    }
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_solve_scalar(bp4::kSolvePlainInit, st, acc, loop, c->stream));
-    }
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_sadd(n, sg.d, 0., -1., sg.h, c->sms, c->stream));
-    return 0;
+    if (int e = jacobi_dot())
+      return e;
+    if (int e = scalar(bp4::kSolvePlainInit))
+      return e;
+    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<false>, n, sg.d, 0., -1., sg.h, nullptr);
   };
   if (int e = capture_into(c, sg.graph, nullptr, 0, prologue, &leaves))
     return e;
@@ -1259,47 +1264,35 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
         const MergedCall m{x, sg.g, sg.d, prec, 0., 0., 0., 0., st};
         if (int e = merged_sweep(c, m, sg.h))
           return e;
-        Timed t(c, BP4_K_BLAS1);
-        CU(bp4::launch_solve_scalar(bp4::kSolveMergedStep, st, acc, loop, c->stream));
-        return 0;
+        return scalar(bp4::kSolveMergedStep);
       }
     // SolverCG: h = A d; alpha = gh / d.h; x += alpha d; g += alpha h, |g|; check;
     // h = P g; beta = g.h / gh; d = beta d - h
     if (int e = vmult_on(c, sg.h, sg.d))
       return e;
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_dot(n, sg.d, sg.h, acc, c->det, c->sms, c->stream));
-    }
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_solve_scalar(bp4::kSolvePlainAlpha, st, acc, loop, c->stream));
-    }
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_cg_xg(n, x, sg.g, sg.d, sg.h, st, acc + 1, c->det, c->sms, c->stream));
-    }
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_jacobi_dot(n, sg.h, sg.g, prec, acc + 2, c->det, c->sms, c->stream));
-    }
-    {
-      Timed t(c, BP4_K_BLAS1);
-      CU(bp4::launch_solve_scalar(bp4::kSolvePlainCheck, st, acc, loop, c->stream));
-    }
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_sadd_dev(n, sg.d, &st->beta, -1., sg.h, c->sms, c->stream));
-    return 0;
+    if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, sg.d,
+                      sg.h, acc, c->det))
+      return e;
+    if (int e = scalar(bp4::kSolvePlainAlpha))
+      return e;
+    if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::cg_xg_kernel<true> : bp4::cg_xg_kernel<false>, n, x,
+                      sg.g, sg.d, sg.h, st, acc + 1, c->det))
+      return e;
+    if (int e = jacobi_dot())
+      return e;
+    if (int e = scalar(bp4::kSolvePlainCheck))
+      return e;
+    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, sg.d, 0., -1., sg.h, &st->beta);
   };
   if (int e = capture_into(c, cp.conditional.phGraph_out[0], nullptr, 0, body, nullptr))
     return e;
   // merged: the pending x update; both: the final state to the host
   auto epilogue = [&]() -> int {
     if (sg.merged)
-      {
-        Timed t(c, BP4_K_BLAS1);
-        CU(bp4::launch_solve_final(n, x, sg.d, sg.g, prec, st, c->deterministic, c->sms, c->stream));
-      }
+      if (int e = sweep(c, BP4_K_BLAS1, n,
+                        c->deterministic ? bp4::solve_final_kernel<true> : bp4::solve_final_kernel<false>, n, x, sg.d,
+                        sg.g, prec, st))
+        return e;
     CU(cudaMemcpyAsync(c->h_state + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream));
     return 0;
   };
@@ -1617,7 +1610,7 @@ static int exchange_ghosts_on(bp4_ctx *c, double *v, cudaStream_t st)
 }
 
 // compress(add) on stream st: the ghost slots of v travel to their owners; the owner side ends
-// with the contributions in contrib_buffer(c) ready for unpack_add (compress_release afterwards)
+// with the contributions in contrib_buffer(c) ready for compress_finish
 static int exchange_compress_on(bp4_ctx *c, double *v, cudaStream_t st)
 {
   auto &p = c->p2p;
@@ -1661,15 +1654,25 @@ static const double *contrib_buffer(const bp4_ctx *c)
                    : c->d_recvbuf;
 }
 
-// after unpack_add on stream st: hand this half of contrib_in back to the ghost holders
-static int compress_release(bp4_ctx *c, cudaStream_t st)
+// the end of compress(add) on the context's stream, once exchange_compress_on has delivered the
+// contributions: add them into v, hand this half of contrib_in back to the ghost holders, zero the
+// ghost slots of v
+static int compress_finish(bp4_ctx *c, double *v)
 {
+  {
+    // one launch for all peers: an owned entry may be exported to several (atomics)
+    Timed          t(c, BP4_K_BLAS1);
+    const uint64_t ne = c->export_off.back();
+    if (int e = per_element(c, ne, bp4::unpack_add_kernel, ne, c->d_export, contrib_buffer(c), v))
+      return e;
+  }
   auto &p = c->p2p;
   if (p.on)
     for (size_t k = 0; k < c->peer.size(); ++k)
       if (c->export_off[k + 1] > c->export_off[k])
-        DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k], kFlagAckRev, c->rank), p.epoch_rev,
+        DRV(p.write64((CUstream)c->stream, flag_addr(p.peer_arena[k], kFlagAckRev, c->rank), p.epoch_rev,
                       CU_STREAM_WRITE_VALUE_DEFAULT));
+  CU(cudaMemsetAsync(v + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream));
   return 0;
 }
 
@@ -1684,8 +1687,10 @@ int bp4_update_ghost_values(bp4_ctx *c, bp4_vec *v)
   if (!c->comm)
     return fail(BP4_ERR_STATE, "ghost exchange not initialised (bp4_comm_init)");
   {
-    Timed t(c, BP4_K_BLAS1);
-    CU(bp4::launch_pack(c->export_off.back(), c->d_export, v->p(), c->d_sendbuf, c->stream));
+    Timed          t(c, BP4_K_BLAS1);
+    const uint64_t ne = c->export_off.back();
+    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export, v->p(), c->d_sendbuf))
+      return e;
   }
   return exchange_ghosts_on(c, v->p(), c->stream);
 }
@@ -1702,14 +1707,7 @@ int bp4_compress_add(bp4_ctx *c, bp4_vec *v)
     return fail(BP4_ERR_STATE, "ghost exchange not initialised (bp4_comm_init)");
   if (int e = exchange_compress_on(c, v->p(), c->stream))
     return e;
-  {
-    Timed t(c, BP4_K_BLAS1); // one launch for all peers: an owned entry may be exported to several (atomics)
-    CU(bp4::launch_unpack_add(c->export_off.back(), c->d_export, contrib_buffer(c), v->p(), c->stream));
-  }
-  if (int e = compress_release(c, c->stream))
-    return e;
-  CU(cudaMemsetAsync(v->p() + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream));
-  return 0;
+  return compress_finish(c, v->p());
 }
 
 // ---- deterministic mode --------------------------------------------------------------------

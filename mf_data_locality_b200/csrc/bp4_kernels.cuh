@@ -3,7 +3,8 @@
 //   cell kernel, fused : the same loop with do_cg_update4b run on a cell-batch range's private
 //                        DoFs before its first cell and do_cg_update3b after its last cell
 //                        (poisson_operator.h:339-364)                          (a2/a8/a9)
-//   streaming kernels for the DoFs shared between ranges, the plain-CG BLAS-1 and the Jacobi apply.
+//   streaming kernels for the DoFs shared between ranges, the plain-CG BLAS-1 and the Jacobi apply
+//                        (bp4_vector_kernels.cuh).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -173,4 +174,18 @@ namespace bp4
     uint32_t max_steps, step;        // step = last checked step
     int32_t  state, pad;             // SolverControl::State: 0 iterate, 1 success, 2 failure
   };
+
+  // the seven merged sums of do_cg_update3b (solver_cg_optimized.h:37-44) for one entry
+  __device__ __forceinline__ void post_terms(double (&s)[7], const double ri, const double di,
+                                             const double hi, const double pr)
+  {
+    const double zi = pr * hi;
+    s[0] += di * hi;
+    s[1] += hi * hi;
+    s[2] += ri * hi;
+    s[3] += ri * ri;
+    s[4] += ri * zi;
+    s[5] += hi * zi;
+    s[6] += ri * pr * ri;
+  }
 } // namespace bp4
