@@ -223,6 +223,7 @@ int bp4_deterministic_info(bp4_ctx *ctx, int *on, uint32_t *n_colors, uint32_t *
 /* ---- multi-GPU (Utilities::MPI::Partitioner / MPI_Allreduce call sites, SURVEY 2a) ------- */
 #define BP4_NCCL_ID_BYTES 128
 int bp4_comm_unique_id(unsigned char id[BP4_NCCL_ID_BYTES]);                 /* rank 0 */
+/* once per context: a second call is BP4_ERR_STATE and leaves the first communicator in place  */
 int bp4_comm_init(bp4_ctx *ctx, int rank, int n_ranks, const unsigned char id[BP4_NCCL_ID_BYTES]);
 /* n_ranks of the communicator; peer_copies = 1 when the ghost exchange runs as copy-engine peer
  * copies into IPC-shared buffers with stream-memory-operation flags (no SM involved; the analogue

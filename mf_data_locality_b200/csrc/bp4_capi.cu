@@ -13,7 +13,9 @@
 #include <cstring>
 #include <initializer_list>
 #include <map>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/bp4.h"
@@ -56,11 +58,57 @@ namespace
     }                                                                                         \
   while (0)
 
+// owning handles of CUDA and NCCL resources: std::unique_ptr with the matching release call
+template <auto F>
+struct Release
+{
+  template <typename P>
+  void operator()(P p) const
+  {
+    F(p);
+  }
+};
+template <typename T>
+using dev_ptr = std::unique_ptr<T, Release<cudaFree>>;
+template <typename T>
+using host_ptr   = std::unique_ptr<T, Release<cudaFreeHost>>; // pinned
+using stream_ptr = std::unique_ptr<CUstream_st, Release<cudaStreamDestroy>>;
+using event_ptr  = std::unique_ptr<CUevent_st, Release<cudaEventDestroy>>;
+using graph_ptr  = std::unique_ptr<CUgraph_st, Release<cudaGraphDestroy>>;
+using exec_ptr   = std::unique_ptr<CUgraphExec_st, Release<cudaGraphExecDestroy>>;
+using comm_ptr   = std::unique_ptr<ncclComm, Release<ncclCommDestroy>>;
+using ipc_ptr    = std::unique_ptr<char, Release<cudaIpcCloseMemHandle>>; // a peer's mapped allocation
+
+// n elements, at least one, into p: pinned host memory for a host_ptr, device memory otherwise
+template <typename T, typename D>
+cudaError_t allocate(std::unique_ptr<T, D> &p, size_t n)
+{
+  T           *q     = nullptr;
+  const size_t bytes = sizeof(T) * std::max<size_t>(n, 1);
+  cudaError_t  e;
+  if constexpr (std::is_same_v<D, Release<cudaFreeHost>>)
+    e = cudaMallocHost(&q, bytes);
+  else
+    e = cudaMalloc(&q, bytes);
+  p.reset(q);
+  return e;
+}
+
+// allocate, then copy n elements from the host
+template <typename T>
+cudaError_t upload(dev_ptr<T> &p, const T *src, size_t n)
+{
+  cudaError_t e = allocate(p, n);
+  if (e == cudaSuccess && n)
+    e = cudaMemcpy(p.get(), src, sizeof(T) * n, cudaMemcpyHostToDevice);
+  return e;
+}
+
 struct bp4_vec
 {
-  double  *buf = nullptr;
-  uint64_t n   = 0;
-  double  *p() const { return buf; }
+  dev_ptr<double> buf;
+  uint64_t        n = 0;
+  double         *p() const { return buf.get(); }
 };
 
 struct ProfEvent
@@ -74,61 +122,64 @@ struct ProfEvent
 // g, d, h so that their addresses, baked into the graph, stay valid
 struct SolveGraph
 {
-  bool            merged = false;
-  int             fused  = 0;
-  const double   *x = nullptr, *b = nullptr, *prec = nullptr;
-  double         *g = nullptr, *d = nullptr, *h = nullptr;
-  cudaGraph_t     graph = nullptr;
-  cudaGraphExec_t exec  = nullptr;
+  bool          merged = false;
+  int           fused  = 0;
+  const double *x = nullptr, *b = nullptr, *prec = nullptr;
+  bp4_vec       g, d, h;
+  graph_ptr     graph;
+  exec_ptr      exec;
 };
 
+// Members are released in reverse declaration order, after ~bp4_ctx has synchronised the stream:
+// the streams are declared first so that they are released last.
 struct bp4_ctx
 {
+  stream_ptr   stream, comm_stream;
+  event_ptr    ev_a, ev_b;
   int          degree = 0, device = 0, sms = 0;
   int          n_coef = 24; // geometry coefficients per cell: 24 (tri-linear) or 81 (all 27 vectors)
   uint64_t     n_cells = 0, n_owned = 0, n_ghost = 0, n_constrained = 0;
   uint64_t     n_before = 0, n_comm = 0; // cell partitions for the overlapped exchange
-  cudaStream_t comm_stream = nullptr;
-  cudaEvent_t  ev_a = nullptr, ev_b = nullptr;
   int          overlap = 1;
-  cudaStream_t stream = nullptr;
-  uint32_t    *d_entity = nullptr, *d_constrained = nullptr, *d_walk = nullptr;
-  double      *d_coef = nullptr, *d_gll = nullptr;
-  double      *d_acc  = nullptr; // [8] reduction scratch
-  int         *d_flag = nullptr;
-  uint32_t    *d_sched = nullptr; // [n_sched] unit counters of the cell-kernel launches of one loop
-  uint32_t     n_sched = 4;       // 4, or one per colour in the deterministic mode
-  double      *h_acc  = nullptr; // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
+  dev_ptr<uint32_t> d_entity, d_constrained, d_walk;
+  dev_ptr<double>   d_coef, d_gll;
+  dev_ptr<double>   d_acc; // [8] reduction scratch
+  dev_ptr<int>      d_flag;
+  dev_ptr<uint32_t> d_sched;     // [n_sched] unit counters of the cell-kernel launches of one loop
+  uint32_t          n_sched = 4; // 4, or one per colour in the deterministic mode
+  host_ptr<double>  h_acc;       // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
   unsigned long long pub_seq = 0;
-  int         *h_flag = nullptr; // pinned
+  host_ptr<int>      h_flag;
   // device-resident solves: the solver state, its pinned host images ([0] initial state read by
   // the graph, [1] final state written by it) and the cached graphs
-  bp4::SolveState        *d_state = nullptr;
-  bp4::SolveState        *h_state = nullptr;
-  std::vector<SolveGraph> solves;
+  dev_ptr<bp4::SolveState>  d_state;
+  host_ptr<bp4::SolveState> h_state;
+  std::vector<SolveGraph>   solves;
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
   int             fused      = 0;      // 1: do_cg_update4b/3b on private DoFs inside the cell kernel
   bool            fused_pinned = false; // chosen by BP4_FUSED / bp4_debug_set_fused: comm_init keeps it
   uint64_t        n_private  = 0;      // [0, n_private) are private to one range, the rest is streamed
   uint32_t        unit_part[4] = {0, 0, 0, 0}; // first unit of the three cell partitions (+ end)
-  bp4::BatchDesc *d_batch      = nullptr;
-  uint32_t       *d_unit_batch = nullptr;
+  dev_ptr<bp4::BatchDesc> d_batch;
+  dev_ptr<uint32_t>       d_unit_batch;
   // deterministic mode (DESIGN.md 4.6): cells stored colour by colour, colour k = stored cells
   // [color_off[k], color_off[k+1]); cell_color[i] = colour of the caller's cell i; the ordered
-  // reductions' slots and ticket
+  // reductions' slots and ticket (det views the two buffers)
   bool                  deterministic = false;
   uint32_t              n_colors      = 0;
   std::vector<uint64_t> color_off;
   std::vector<uint32_t> cell_color;
+  dev_ptr<double>       det_slot;
+  dev_ptr<uint32_t>     det_ticket;
   bp4::DetSlots         det;
   // multi-GPU
-  ncclComm_t            comm = nullptr;
+  comm_ptr              comm;
   int                   rank = 0, n_ranks = 1;
   std::vector<int>      peer;
   std::vector<uint64_t> import_off, export_off;
-  uint32_t             *d_export = nullptr;
-  double               *d_sendbuf = nullptr, *d_recvbuf = nullptr;
+  dev_ptr<uint32_t>     d_export;
+  dev_ptr<double>       d_sendbuf, d_recvbuf;
   // Peer exchange without SMs (the USE_SHMEM analogue of benchmark.h:35, :105-108): every rank
   // owns one IPC-shared arena [flags | ghost_in[2] | contrib_in[2]]; owners push their exported
   // values into the peers' ghost_in with copy-engine peer copies, ghost holders push their
@@ -138,9 +189,9 @@ struct bp4_ctx
   struct P2P
   {
     bool                 on = false;
-    char                *arena = nullptr;           // my arena (device)
+    dev_ptr<char>        arena;                     // my arena (device)
     uint64_t             off_ghost[2] = {0, 0}, off_contrib[2] = {0, 0};
-    std::vector<char *>  peer_arena;                // [n_peers] mapped base of peer k's arena
+    std::vector<ipc_ptr> peer_arena;                // [n_peers] mapped base of peer k's arena
     std::vector<uint64_t> peer_off_ghost[2], peer_off_contrib[2]; // [n_peers] byte offsets there
     std::vector<uint64_t> peer_imp_off, peer_exp_off; // [n_peers] where MY data goes (doubles)
     uint64_t             epoch_fwd = 0, epoch_rev = 0;
@@ -149,14 +200,16 @@ struct bp4_ctx
   } p2p;
   // freed vector buffers kept for reuse, keyed by size: plays the role of deal.II's
   // GrowingVectorMemory pool behind SolverCGFullMerge's temporaries (solver_cg_optimized.h:201)
-  std::multimap<uint64_t, double *> pool;
+  std::multimap<uint64_t, dev_ptr<double>> pool;
   // measurement
   bool                   profile = false;
   std::vector<ProfEvent> events;
-  std::vector<cudaEvent_t> event_pool; // recycled timing events (creating one costs microseconds)
+  std::vector<event_ptr> event_pool; // recycled timing events (creating one costs microseconds)
   double                 prof_ms[BP4_K_COUNT]  = {0};
   uint64_t               prof_cnt[BP4_K_COUNT] = {0};
   uint64_t               launches               = 0;
+
+  ~bp4_ctx();
 };
 
 namespace
@@ -175,7 +228,7 @@ namespace
     int      id;
     ProfEvent ev{};
     bool      on;
-    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile && !capturing(c_->stream))
+    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile && !capturing(c_->stream.get()))
     {
       c->launches += n_launches;
       c->prof_cnt[id] += 1;
@@ -186,24 +239,26 @@ namespace
               cudaEventCreate(e);
             else
               {
-                *e = c->event_pool.back();
+                *e = c->event_pool.back().release();
                 c->event_pool.pop_back();
               }
           ev.id = id;
-          cudaEventRecord(ev.a, c->stream);
+          cudaEventRecord(ev.a, c->stream.get());
         }
     }
     ~Timed()
     {
       if (on)
         {
-          cudaEventRecord(ev.b, c->stream);
+          cudaEventRecord(ev.b, c->stream.get());
           c->events.push_back(ev);
         }
     }
   };
 
-  int drain_events(bp4_ctx *c)
+  // collect the times of the recorded event pairs; returns the first error and sets no message, so
+  // that ~bp4_ctx can drain without touching bp4_last_error
+  cudaError_t drain_events(bp4_ctx *c)
   {
     cudaError_t err = cudaSuccess;
     for (auto &ev : c->events) // every event pair is released, also after a failure
@@ -215,12 +270,11 @@ namespace
           err = cudaEventElapsedTime(&ms, ev.a, ev.b);
         if (err == cudaSuccess)
           c->prof_ms[ev.id] += ms;
-        c->event_pool.push_back(ev.a);
-        c->event_pool.push_back(ev.b);
+        c->event_pool.emplace_back(ev.a);
+        c->event_pool.emplace_back(ev.b);
       }
     c->events.clear();
-    CU(err);
-    return 0;
+    return err;
   }
 
   // The vector kernels (bp4_vector_kernels.cuh) are launched on the context's stream by one helper
@@ -238,7 +292,7 @@ namespace
     Timed t(c, id);
     if (n == 0)
       return 0;
-    kernel<<<stream_grid(n, c->sms), 256, 0, c->stream>>>(args...);
+    kernel<<<stream_grid(n, c->sms), 256, 0, c->stream.get()>>>(args...);
     CU(cudaGetLastError());
     return 0;
   }
@@ -249,27 +303,36 @@ namespace
   {
     if (n == 0)
       return 0;
-    kernel<<<(unsigned)((n + B - 1) / B), B, 0, c->stream>>>(args...);
+    kernel<<<(unsigned)((n + B - 1) / B), B, 0, c->stream.get()>>>(args...);
     CU(cudaGetLastError());
     return 0;
   }
 
-  // buffer of n doubles, from the pool when one of that size is cached; zeroed on request only
+  // v = n doubles, from the pool when a buffer of that size is cached; zeroed on request only
   // (SolverCGFullMerge takes its temporaries with omit_zeroing_entries = true,
   // solver_cg_optimized.h:215-217)
-  int pooled_alloc(bp4_ctx *c, uint64_t n, double **out, bool zero)
+  int pooled_alloc(bp4_ctx *c, uint64_t n, bp4_vec &v, bool zero)
   {
+    v.n     = n;
     auto it = c->pool.find(n);
     if (it != c->pool.end())
       {
-        *out = it->second;
+        v.buf = std::move(it->second);
         c->pool.erase(it);
       }
     else
-      CU(cudaMalloc(out, sizeof(double) * (n + 2))); // + 2: the fused loop copies runs in 16-byte pieces, one element past either end
+      CU(allocate(v.buf, n + 2)); // + 2: the fused loop copies runs in 16-byte pieces, one element past either end
     if (zero)
-      CU(cudaMemsetAsync(*out, 0, sizeof(double) * n, c->stream));
+      CU(cudaMemsetAsync(v.p(), 0, sizeof(double) * n, c->stream.get()));
     return 0;
+  }
+
+  // v's buffer back to the pool; stream order makes reuse safe: the next user's work is queued
+  // behind ours
+  void recycle(bp4_ctx *c, bp4_vec &v)
+  {
+    if (v.buf)
+      c->pool.emplace(v.n, std::move(v.buf));
   }
 
   // n rows of `width` elements to the device, in the caller's order or, with `order`, row order[j]
@@ -289,33 +352,39 @@ namespace
   int reduce_to_host(bp4_ctx *c, int k, double *out)
   {
     if (c->comm)
-      NC(ncclAllReduce(c->d_acc, c->d_acc, k, ncclDouble, ncclSum, c->comm, c->stream));
+      NC(ncclAllReduce(c->d_acc.get(), c->d_acc.get(), k, ncclDouble, ncclSum, c->comm.get(), c->stream.get()));
     // the last kernel of the chain writes the values and then a sequence number into mapped
     // pinned memory; the host polls that word (and the stream, for errors, now and then)
-    volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc + 8);
+    volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc.get() + 8);
     const unsigned long long     seq      = ++c->pub_seq;
-    bp4::publish_kernel<<<1, 32, 0, c->stream>>>(c->d_acc, k, c->h_acc, seq_word, seq);
+    bp4::publish_kernel<<<1, 32, 0, c->stream.get()>>>(c->d_acc.get(), k, c->h_acc.get(), seq_word, seq);
     CU(cudaGetLastError());
     c->launches += 1;
     int idle = 0;
     for (unsigned long long spins = 1; *seq_word != seq; ++spins)
       if ((spins & 0xFFFF) == 0)
         {
-          const cudaError_t q = cudaStreamQuery(c->stream);
+          const cudaError_t q = cudaStreamQuery(c->stream.get());
           if (q != cudaSuccess && q != cudaErrorNotReady)
             CU(q);
           if (q == cudaSuccess && ++idle > 8) // stream drained, nothing published: cannot happen
             return fail(BP4_ERR_CUDA, "reduction result was not published");
         }
     for (int i = 0; i < k; ++i)
-      out[i] = c->h_acc[i];
+      out[i] = c->h_acc.get()[i];
     return 0;
   }
 } // namespace
 
-extern "C" {
-static void p2p_teardown(bp4_ctx *c);
+bp4_ctx::~bp4_ctx()
+{
+  cudaSetDevice(device);
+  if (stream)
+    cudaStreamSynchronize(stream.get());
+  drain_events(this);
+}
 
+extern "C" {
 const char *bp4_last_error(void) { return g_err.c_str(); }
 
 int bp4_device_count(int *count)
@@ -386,15 +455,22 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   if (c->n_before + c->n_comm > c->n_cells)
     return fail(BP4_ERR_ARG, "cell partitions exceed n_cells");
   CU(cudaDeviceGetAttribute(&c->sms, cudaDevAttrMultiProcessorCount, d->device));
-  CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
-  CU(cudaStreamCreateWithFlags(&c->comm_stream, cudaStreamNonBlocking));
-  CU(cudaEventCreateWithFlags(&c->ev_a, cudaEventDisableTiming));
-  CU(cudaEventCreateWithFlags(&c->ev_b, cudaEventDisableTiming));
+  for (stream_ptr *s : {&c->stream, &c->comm_stream})
+    {
+      cudaStream_t q;
+      CU(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking));
+      s->reset(q);
+    }
+  for (event_ptr *e : {&c->ev_a, &c->ev_b})
+    {
+      cudaEvent_t q;
+      CU(cudaEventCreateWithFlags(&q, cudaEventDisableTiming));
+      e->reset(q);
+    }
 
   std::vector<uint32_t> walk;
   CU(bp4::launch_init_degree(d->degree, walk));
-  CU(cudaMalloc(&c->d_walk, sizeof(uint32_t) * walk.size()));
-  CU(cudaMemcpy(c->d_walk, walk.data(), sizeof(uint32_t) * walk.size(), cudaMemcpyHostToDevice));
+  CU(upload(c->d_walk, walk.data(), walk.size()));
 
   // deterministic mode: colour the cells greedily in the given order -- a cell takes the lowest
   // colour that no earlier cell sharing one of its valid entities has -- and store them colour by
@@ -440,14 +516,14 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
       c->n_sched = std::max<uint32_t>(c->n_sched, c->n_colors);
     }
 
-  const size_t nc = d->n_cells ? d->n_cells : 1;
-  c->n_coef       = d->coefficients ? 81 : 24;
-  CU(cudaMalloc(&c->d_entity, sizeof(uint32_t) * 27 * nc));
-  CU(cudaMalloc(&c->d_coef, sizeof(double) * c->n_coef * nc));
+  c->n_coef = d->coefficients ? 81 : 24;
+  const uint64_t nc = std::max<uint64_t>(d->n_cells, 1);
+  CU(allocate(c->d_entity, 27 * nc));
+  CU(allocate(c->d_coef, c->n_coef * nc));
   if (d->n_cells)
-    CU(upload_rows(c->d_entity, d->entity_index, 27, d->n_cells, order));
+    CU(upload_rows(c->d_entity.get(), d->entity_index, 27, d->n_cells, order));
   if (d->n_cells && d->coefficients) // all 27 coefficient vectors of the reference's kernel, as given
-    CU(upload_rows(c->d_coef, d->coefficients, 81, d->n_cells, order));
+    CU(upload_rows(c->d_coef.get(), d->coefficients, 81, d->n_cells, order));
   else if (d->n_cells)
     {
       // tri-linear coefficients from the 8 vertices, poisson_operator.h:161-178
@@ -468,32 +544,28 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
             o[18 + k] = v6 - v4 - (v2 - v0);
             o[21 + k] = (v7 - v6 - (v5 - v4) - (v3 - v2 - (v1 - v0)));
           }
-      CU(upload_rows(c->d_coef, cf.data(), 24, d->n_cells, order));
+      CU(upload_rows(c->d_coef.get(), cf.data(), 24, d->n_cells, order));
     }
-  CU(cudaMalloc(&c->d_constrained, sizeof(uint32_t) * (d->n_constrained ? d->n_constrained : 1)));
-  if (d->n_constrained)
-    CU(cudaMemcpy(c->d_constrained, d->constrained, sizeof(uint32_t) * d->n_constrained,
-                  cudaMemcpyHostToDevice));
+  CU(upload(c->d_constrained, d->constrained, d->n_constrained));
   std::vector<double> gll;
   bp4::gll_table(d->degree, gll);
-  CU(cudaMalloc(&c->d_gll, sizeof(double) * gll.size()));
-  CU(cudaMemcpy(c->d_gll, gll.data(), sizeof(double) * gll.size(), cudaMemcpyHostToDevice));
-  CU(cudaMalloc(&c->d_acc, sizeof(double) * 8));
-  CU(cudaMemset(c->d_acc, 0, sizeof(double) * 8));
-  CU(cudaMalloc(&c->d_flag, sizeof(int)));
-  CU(cudaMalloc(&c->d_sched, sizeof(uint32_t) * c->n_sched));
+  CU(upload(c->d_gll, gll.data(), gll.size()));
+  CU(allocate(c->d_acc, 8));
+  CU(cudaMemset(c->d_acc.get(), 0, sizeof(double) * 8));
+  CU(allocate(c->d_flag, 1));
+  CU(allocate(c->d_sched, c->n_sched));
   if (c->deterministic)
     {
-      const size_t n_slot = (size_t)8 * 8 * c->sms; // K <= 7 partials of <= 8 * SMs blocks (stream_grid)
-      CU(cudaMalloc(&c->det.slot, sizeof(double) * n_slot));
-      CU(cudaMalloc(&c->det.ticket, sizeof(uint32_t)));
-      CU(cudaMemset(c->det.ticket, 0, sizeof(uint32_t)));
+      CU(allocate(c->det_slot, (size_t)8 * 8 * c->sms)); // K <= 7 partials of <= 8 * SMs blocks (stream_grid)
+      CU(allocate(c->det_ticket, 1));
+      CU(cudaMemset(c->det_ticket.get(), 0, sizeof(uint32_t)));
+      c->det = {c->det_slot.get(), c->det_ticket.get()};
     }
-  CU(cudaMallocHost(&c->h_acc, sizeof(double) * 16)); // UVA: the pointer is valid on the device too
-  memset(c->h_acc, 0, sizeof(double) * 16);
-  CU(cudaMallocHost(&c->h_flag, sizeof(int)));
-  CU(cudaMalloc(&c->d_state, sizeof(bp4::SolveState)));
-  CU(cudaMallocHost(&c->h_state, 2 * sizeof(bp4::SolveState)));
+  CU(allocate(c->h_acc, 16)); // UVA: the pointer is valid on the device too
+  memset(c->h_acc.get(), 0, sizeof(double) * 16);
+  CU(allocate(c->h_flag, 1));
+  CU(allocate(c->d_state, 1));
+  CU(allocate(c->h_state, 2));
 
   // cell-batch ranges and their private DoF runs -> units and batches of the fused merged loop
   if (d->n_ranges > 0)
@@ -536,11 +608,8 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
         }
       c->unit_part[3] = (uint32_t)unit_batch.size();
       unit_batch.push_back((uint32_t)batches.size());
-      CU(cudaMalloc(&c->d_batch, sizeof(bp4::BatchDesc) * (batches.size() ? batches.size() : 1)));
-      CU(cudaMalloc(&c->d_unit_batch, sizeof(uint32_t) * unit_batch.size()));
-      CU(cudaMemcpy(c->d_batch, batches.data(), sizeof(bp4::BatchDesc) * batches.size(), cudaMemcpyHostToDevice));
-      CU(cudaMemcpy(c->d_unit_batch, unit_batch.data(), sizeof(uint32_t) * unit_batch.size(),
-                    cudaMemcpyHostToDevice));
+      CU(upload(c->d_batch, batches.data(), batches.size()));
+      CU(upload(c->d_unit_batch, unit_batch.data(), unit_batch.size()));
       c->n_private = c->n_coef == 24 ? rp[d->n_ranges] : 0; // in-loop updates: tri-linear kernel only
       // the staged fused loop takes a batch's private run in two jobs of its shared-memory rows
       for (const bp4::BatchDesc &b : batches) // run_limit 0: no fused kernel at this degree
@@ -563,11 +632,9 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
       c->import_off.assign(d->import_offset, d->import_offset + d->n_peers + 1);
       c->export_off.assign(d->export_offset, d->export_offset + d->n_peers + 1);
       const uint64_t ne = c->export_off.back();
-      CU(cudaMalloc(&c->d_export, sizeof(uint32_t) * (ne ? ne : 1)));
-      if (ne)
-        CU(cudaMemcpy(c->d_export, d->export_index, sizeof(uint32_t) * ne, cudaMemcpyHostToDevice));
-      CU(cudaMalloc(&c->d_sendbuf, sizeof(double) * (ne ? ne : 1)));
-      CU(cudaMalloc(&c->d_recvbuf, sizeof(double) * (ne ? ne : 1)));
+      CU(upload(c->d_export, d->export_index, ne));
+      CU(allocate(c->d_sendbuf, ne));
+      CU(allocate(c->d_recvbuf, ne));
     }
   return 0;
 }
@@ -593,72 +660,16 @@ int bp4_ctx_create(const bp4_desc *d, bp4_ctx **out)
   if (ndev == 0)
     return fail(BP4_ERR_CUDA, "no CUDA device: this library has no CPU fallback");
   CU(cudaSetDevice(d->device));
-  bp4_ctx *c       = new bp4_ctx;
+  std::unique_ptr<bp4_ctx> c(new bp4_ctx);
   c->deterministic = deterministic;
-  if (int e = ctx_create_impl(d, c))
-    {
-      const std::string msg = g_err; // bp4_ctx_destroy must not clobber the message
-      bp4_ctx_destroy(c);
-      g_err = msg;
-      return e;
-    }
-  *out = c;
+  if (int e = ctx_create_impl(d, c.get()))
+    return e;
+  *out = c.release();
   return 0;
 }
 
 int bp4_ctx_destroy(bp4_ctx *c)
 {
-  if (!c)
-    return 0;
-  cudaSetDevice(c->device);
-  if (c->stream)
-    cudaStreamSynchronize(c->stream);
-  drain_events(c);
-  for (cudaEvent_t e : c->event_pool)
-    cudaEventDestroy(e);
-  c->event_pool.clear();
-  p2p_teardown(c);
-  if (c->comm)
-    ncclCommDestroy(c->comm);
-  for (auto &kv : c->pool)
-    cudaFree(kv.second);
-  for (SolveGraph &sg : c->solves)
-    {
-      if (sg.exec)
-        cudaGraphExecDestroy(sg.exec);
-      if (sg.graph)
-        cudaGraphDestroy(sg.graph);
-      cudaFree(sg.g);
-      cudaFree(sg.d);
-      cudaFree(sg.h);
-    }
-  cudaFree(c->d_state);
-  cudaFreeHost(c->h_state);
-  cudaFree(c->d_entity);
-  cudaFree(c->d_constrained);
-  cudaFree(c->d_walk);
-  cudaFree(c->d_coef);
-  cudaFree(c->d_gll);
-  cudaFree(c->d_acc);
-  cudaFree(c->d_flag);
-  cudaFree(c->d_sched);
-  cudaFree(c->det.slot);
-  cudaFree(c->det.ticket);
-  cudaFree(c->d_batch);
-  cudaFree(c->d_unit_batch);
-  cudaFree(c->d_export);
-  cudaFree(c->d_sendbuf);
-  cudaFree(c->d_recvbuf);
-  cudaFreeHost(c->h_acc);
-  cudaFreeHost(c->h_flag);
-  if (c->ev_a)
-    cudaEventDestroy(c->ev_a);
-  if (c->ev_b)
-    cudaEventDestroy(c->ev_b);
-  if (c->comm_stream)
-    cudaStreamDestroy(c->comm_stream);
-  if (c->stream)
-    cudaStreamDestroy(c->stream);
   delete c;
   return 0;
 }
@@ -667,7 +678,7 @@ int bp4_ctx_synchronize(bp4_ctx *c)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
-  CU(cudaStreamSynchronize(c->stream));
+  CU(cudaStreamSynchronize(c->stream.get()));
   return 0;
 }
 
@@ -675,7 +686,7 @@ int bp4_ctx_stream(bp4_ctx *c, void **stream)
 {
   if (!c || !stream)
     return fail(BP4_ERR_ARG, "null argument");
-  *stream = (void *)c->stream;
+  *stream = (void *)c->stream.get();
   return 0;
 }
 
@@ -684,14 +695,10 @@ static int vec_alloc(bp4_ctx *c, uint64_t n, bp4_vec **out, bool zero)
   if (!c || !out)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  bp4_vec *v = new bp4_vec;
-  v->n       = n;
-  if (int e = pooled_alloc(c, n, &v->buf, zero))
-    {
-      delete v;
-      return e;
-    }
-  *out = v;
+  std::unique_ptr<bp4_vec> v(new bp4_vec);
+  if (int e = pooled_alloc(c, n, *v, zero))
+    return e;
+  *out = v.release();
   return 0;
 }
 
@@ -700,16 +707,9 @@ int bp4_vec_alloc_uninitialized(bp4_ctx *c, uint64_t n, bp4_vec **out) { return 
 
 int bp4_vec_free(bp4_ctx *c, bp4_vec *v)
 {
-  if (!v)
-    return 0;
-  if (v->buf)
-    {
-      if (c) // stream order makes reuse safe: the next user's work is queued behind ours
-        c->pool.emplace(v->n, v->buf);
-      else
-        cudaFree(v->buf);
-    }
-  delete v;
+  if (c && v)
+    recycle(c, *v);
+  delete v; // without a context the buffer is freed
   return 0;
 }
 
@@ -726,7 +726,7 @@ int bp4_vec_set_zero(bp4_ctx *c, bp4_vec *v)
   if (!c || !v)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(v->p(), 0, sizeof(double) * v->n, c->stream));
+  CU(cudaMemsetAsync(v->p(), 0, sizeof(double) * v->n, c->stream.get()));
   return 0;
 }
 
@@ -738,7 +738,7 @@ int bp4_vec_upload(bp4_ctx *c, bp4_vec *v, const double *host, uint64_t n)
   if (n > v->n)
     return fail(BP4_ERR_ARG, "upload of %llu > vector size %llu", (unsigned long long)n,
                 (unsigned long long)v->n);
-  CU(cudaMemcpyAsync(v->p(), host, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(v->p(), host, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream.get()));
   return 0;
 }
 
@@ -750,8 +750,8 @@ int bp4_vec_download(bp4_ctx *c, const bp4_vec *v, double *host, uint64_t n)
   if (n > v->n)
     return fail(BP4_ERR_ARG, "download of %llu > vector size %llu", (unsigned long long)n,
                 (unsigned long long)v->n);
-  CU(cudaMemcpyAsync(host, v->p(), sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
+  CU(cudaMemcpyAsync(host, v->p(), sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream.get()));
+  CU(cudaStreamSynchronize(c->stream.get()));
   return 0;
 }
 
@@ -812,19 +812,19 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
   if (end <= begin)
     return 0;
   bp4::CellArgs a{};
-  a.dtab  = c->d_walk;
+  a.dtab  = c->d_walk.get();
   a.src   = src;
   a.dst   = dst;
-  a.sched = c->d_sched + (part < 0 ? 0 : part);
+  a.sched = c->d_sched.get() + (part < 0 ? 0 : part);
   if (m)
     {
       const uint32_t u0 = part < 0 ? c->unit_part[0] : c->unit_part[part],
                      u1 = part < 0 ? c->unit_part[3] : c->unit_part[part + 1];
-      a.entity_index = c->d_entity;
-      a.coef         = c->d_coef;
+      a.entity_index = c->d_entity.get();
+      a.coef         = c->d_coef.get();
       a.n_cells      = c->n_cells;
-      a.batch        = c->d_batch;
-      a.unit_batch   = c->d_unit_batch + u0;
+      a.batch        = c->d_batch.get();
+      a.unit_batch   = c->d_unit_batch.get() + u0;
       a.n_units      = u1 - u0;
       a.r            = m->g;
       a.p            = m->d;
@@ -836,10 +836,10 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       a.update_x     = (m->alpha != 0. && m->alpha_old != 0.) ? 1 : 0;
       a.c1           = a.update_x ? m->alpha + m->alpha_old / m->beta_old : 0.;
       a.c2           = a.update_x ? m->alpha_old / m->beta_old : 0.;
-      a.acc          = c->d_acc;
+      a.acc          = c->d_acc.get();
       a.state        = m->state;
       Timed t(c, BP4_K_MERGED);
-      CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream));
+      CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream.get()));
     }
   else if (c->deterministic) // one launch per colour (single rank: part = -1), timed as one loop
     {
@@ -847,20 +847,20 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       for (uint32_t k = 0; k < c->n_colors; ++k)
         {
           const uint64_t c0 = c->color_off[k];
-          a.entity_index    = c->d_entity + 27 * c0;
-          a.coef            = c->d_coef + (uint64_t)c->n_coef * c0;
+          a.entity_index    = c->d_entity.get() + 27 * c0;
+          a.coef            = c->d_coef.get() + (uint64_t)c->n_coef * c0;
           a.n_cells         = c->color_off[k + 1] - c0;
-          a.sched           = c->d_sched + k;
-          CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream));
+          a.sched           = c->d_sched.get() + k;
+          CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream.get()));
         }
     }
   else
     {
-      a.entity_index = c->d_entity + 27 * begin;
-      a.coef         = c->d_coef + (uint64_t)c->n_coef * begin;
+      a.entity_index = c->d_entity.get() + 27 * begin;
+      a.coef         = c->d_coef.get() + (uint64_t)c->n_coef * begin;
       a.n_cells      = end - begin;
       Timed t(c, BP4_K_VMULT);
-      CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream));
+      CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream.get()));
     }
   return 0;
 }
@@ -878,7 +878,7 @@ static int compress_finish(bp4_ctx *c, double *v);
 // dst must already be zero where the cells accumulate (owned and ghost slots).
 static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCall *m)
 {
-  CU(cudaMemsetAsync(c->d_sched, 0, sizeof(uint32_t) * c->n_sched, c->stream));
+  CU(cudaMemsetAsync(c->d_sched.get(), 0, sizeof(uint32_t) * c->n_sched, c->stream.get()));
   if (c->peer.empty())
     return cell_range(c, dst, src, -1, m);
   if (!c->comm)
@@ -887,18 +887,18 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
   const bool     overlap = c->overlap && c->n_comm > 0;
   {
     Timed t(c, BP4_K_BLAS1);
-    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export, src, c->d_sendbuf))
+    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export.get(), src, c->d_sendbuf.get()))
       return e;
   }
-  CU(cudaEventRecord(c->ev_a, c->stream));
-  CU(cudaStreamWaitEvent(c->comm_stream, c->ev_a, 0));
-  if (int e = exchange_ghosts_on(c, const_cast<double *>(src), c->comm_stream))
+  CU(cudaEventRecord(c->ev_a.get(), c->stream.get()));
+  CU(cudaStreamWaitEvent(c->comm_stream.get(), c->ev_a.get(), 0));
+  if (int e = exchange_ghosts_on(c, const_cast<double *>(src), c->comm_stream.get()))
     return e;
-  CU(cudaEventRecord(c->ev_b, c->comm_stream));
+  CU(cudaEventRecord(c->ev_b.get(), c->comm_stream.get()));
   if (overlap)
     if (int e = cell_range(c, dst, src, 0, m))
       return e;
-  CU(cudaStreamWaitEvent(c->stream, c->ev_b, 0));
+  CU(cudaStreamWaitEvent(c->stream.get(), c->ev_b.get(), 0));
   if (overlap)
     {
       if (int e = cell_range(c, dst, src, 1, m))
@@ -906,26 +906,26 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
     }
   else if (int e = cell_range(c, dst, src, -1, m))
     return e;
-  CU(cudaEventRecord(c->ev_a, c->stream));
-  CU(cudaStreamWaitEvent(c->comm_stream, c->ev_a, 0));
-  if (int e = exchange_compress_on(c, dst, c->comm_stream))
+  CU(cudaEventRecord(c->ev_a.get(), c->stream.get()));
+  CU(cudaStreamWaitEvent(c->comm_stream.get(), c->ev_a.get(), 0));
+  if (int e = exchange_compress_on(c, dst, c->comm_stream.get()))
     return e;
-  CU(cudaEventRecord(c->ev_b, c->comm_stream));
+  CU(cudaEventRecord(c->ev_b.get(), c->comm_stream.get()));
   if (overlap)
     if (int e = cell_range(c, dst, src, 2, m))
       return e;
-  CU(cudaStreamWaitEvent(c->stream, c->ev_b, 0));
+  CU(cudaStreamWaitEvent(c->stream.get(), c->ev_b.get(), 0));
   return compress_finish(c, dst);
 }
 
 // dst = A src on the context's stream (also captured into the plain device solve's loop body)
 static int vmult_on(bp4_ctx *c, double *dst, const double *src)
 {
-  CU(cudaMemsetAsync(dst, 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream));
+  CU(cudaMemsetAsync(dst, 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream.get()));
   if (int e = cell_loop(c, dst, src, nullptr))
     return e;
   Timed t(c, BP4_K_BLAS1);
-  return per_element(c, c->n_constrained, bp4::fixup_kernel, c->n_constrained, c->d_constrained, dst, src);
+  return per_element(c, c->n_constrained, bp4::fixup_kernel, c->n_constrained, c->d_constrained.get(), dst, src);
 }
 
 int bp4_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
@@ -983,15 +983,15 @@ static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
   // one block at least: pre_kernel also clears the reduction scratch
   if (int e = sweep(c, BP4_K_PRE, std::max<uint64_t>(n - tail, 1),
                     m.state ? bp4::pre_kernel<true> : bp4::pre_kernel<false>, tail, n, h, m.x, m.g, m.d, m.prec,
-                    m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc, m.state))
+                    m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc.get(), m.state))
     return e;
   if (c->n_ghost)
-    CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream));
+    CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream.get()));
   if (int e = cell_loop(c, h, m.d, c->fused ? &m : nullptr))
     return e;
   if (n > tail)
     return sweep(c, BP4_K_POST, n - tail, c->deterministic ? bp4::post_kernel<true> : bp4::post_kernel<false>, tail,
-                 n, m.g, m.d, h, m.prec, c->d_acc, c->det);
+                 n, m.g, m.d, h, m.prec, c->d_acc.get(), c->det);
   return 0;
 }
 
@@ -1025,8 +1025,8 @@ static int assemble_diagonal(bp4_ctx *c, double *diag, int more)
     {
       const uint64_t c0 = c->deterministic ? c->color_off[k] : 0,
                      c1 = c->deterministic ? c->color_off[k + 1] : c->n_cells;
-      if (int e = per_element<128>(c, (c1 - c0) * n3, bp4::diag_kernel, c->degree, c1 - c0, c->d_entity + 27 * c0,
-                                   c->d_coef + (uint64_t)c->n_coef * c0, c->n_coef, c->d_gll, diag, 3))
+      if (int e = per_element<128>(c, (c1 - c0) * n3, bp4::diag_kernel, c->degree, c1 - c0, c->d_entity.get() + 27 * c0,
+                                   c->d_coef.get() + (uint64_t)c->n_coef * c0, c->n_coef, c->d_gll.get(), diag, 3))
         return e;
     }
   return 0;
@@ -1041,20 +1041,22 @@ int bp4_inverse_diagonal(bp4_ctx *c, bp4_vec *out)
     return fail(BP4_ERR_ARG, "diagonal vector needs n_owned/3 entries");
   // assemble DoF-wise into slot 3*node of a local vector so that the ordinary ghost
   // compress(add) (poisson_operator.h:419) can be reused, then keep one entry per owned node
-  bp4_vec *tmp = nullptr;
-  if (int e = bp4_vec_alloc(c, c->n_owned + c->n_ghost, &tmp))
+  // (the temporary goes back to the pool on success and is freed on an error return)
+  bp4_vec tmp;
+  if (int e = pooled_alloc(c, c->n_owned + c->n_ghost, tmp, true))
     return e;
-  if (int e = assemble_diagonal(c, tmp->p(), 2))
+  if (int e = assemble_diagonal(c, tmp.p(), 2))
     return e;
   if (!c->peer.empty())
-    if (int e = bp4_compress_add(c, tmp))
+    if (int e = bp4_compress_add(c, &tmp))
       return e;
   const uint64_t n_nodes = c->n_owned / 3;
-  if (int e = per_element(c, n_nodes, bp4::stride3_kernel, n_nodes, tmp->p(), out->p()))
+  if (int e = per_element(c, n_nodes, bp4::stride3_kernel, n_nodes, tmp.p(), out->p()))
     return e;
   if (int e = per_element(c, n_nodes, bp4::invert_diag_kernel, n_nodes, out->p()))
     return e;
-  return bp4_vec_free(c, tmp);
+  recycle(c, tmp);
+  return 0;
 }
 
 // the reference's own layout of the result (poisson_operator.h:392-426): a DoF vector whose
@@ -1066,7 +1068,7 @@ int bp4_inverse_diagonal_vector(bp4_ctx *c, bp4_vec *out)
   if (int e = check_len(c, out, "out"))
     return e;
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(out->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream));
+  CU(cudaMemsetAsync(out->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream.get()));
   if (int e = assemble_diagonal(c, out->p(), 1))
     return e;
   if (!c->peer.empty())
@@ -1138,7 +1140,7 @@ int bp4_dot(bp4_ctx *c, const bp4_vec *a, const bp4_vec *b, double *result)
   CU(cudaSetDevice(c->device));
   const uint64_t n = sweep_len(c, {a, b});
   if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, a->p(),
-                    b->p(), c->d_acc, c->det))
+                    b->p(), c->d_acc.get(), c->det))
     return e;
   return reduce_to_host(c, 1, result);
 }
@@ -1151,7 +1153,7 @@ int bp4_add_and_dot(bp4_ctx *c, bp4_vec *g, double a, const bp4_vec *h, const bp
   const uint64_t n = sweep_len(c, {g, h, w});
   if (int e = sweep(c, BP4_K_BLAS1, n,
                     c->deterministic ? bp4::add_and_dot_kernel<true> : bp4::add_and_dot_kernel<false>, n, g->p(), a,
-                    h->p(), w->p(), c->d_acc, c->det))
+                    h->p(), w->p(), c->d_acc.get(), c->det))
     return e;
   return reduce_to_host(c, 1, result);
 }
@@ -1170,14 +1172,14 @@ int bp4_all_zero(bp4_ctx *c, const bp4_vec *v, int *result)
   if (!c || !v || !result)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(c->d_flag, 0, sizeof(int), c->stream));
+  CU(cudaMemsetAsync(c->d_flag.get(), 0, sizeof(int), c->stream.get()));
   const uint64_t n = sweep_len(c, {v});
-  if (int e = sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, v->p(), c->d_flag))
+  if (int e = sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, v->p(), c->d_flag.get()))
     return e;
   if (c->comm)
-    NC(ncclAllReduce(c->d_flag, c->d_flag, 1, ncclInt, ncclMax, c->comm, c->stream));
-  CU(cudaMemcpyAsync(c->h_flag, c->d_flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
+    NC(ncclAllReduce(c->d_flag.get(), c->d_flag.get(), 1, ncclInt, ncclMax, c->comm.get(), c->stream.get()));
+  CU(cudaMemcpyAsync(c->h_flag.get(), c->d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, c->stream.get()));
+  CU(cudaStreamSynchronize(c->stream.get()));
   *result = *c->h_flag ? 0 : 1;
   return 0;
 }
@@ -1191,21 +1193,21 @@ template <typename F>
 static int capture_into(bp4_ctx *c, cudaGraph_t graph, const cudaGraphNode_t *deps, size_t n_deps, F &&launch,
                         std::vector<cudaGraphNode_t> *leaves)
 {
-  CU(cudaStreamBeginCaptureToGraph(c->stream, graph, deps, nullptr, n_deps, cudaStreamCaptureModeThreadLocal));
+  CU(cudaStreamBeginCaptureToGraph(c->stream.get(), graph, deps, nullptr, n_deps, cudaStreamCaptureModeThreadLocal));
   int e = launch();
   if (!e && leaves)
     {
       cudaStreamCaptureStatus st;
       const cudaGraphNode_t  *d = nullptr;
       size_t                  n = 0;
-      const cudaError_t       q = cudaStreamGetCaptureInfo(c->stream, &st, nullptr, nullptr, &d, &n);
+      const cudaError_t       q = cudaStreamGetCaptureInfo(c->stream.get(), &st, nullptr, nullptr, &d, &n);
       if (q == cudaSuccess)
         leaves->assign(d, d + n);
       else
         e = fail(BP4_ERR_CUDA, "cudaStreamGetCaptureInfo: %s", cudaGetErrorString(q));
     }
   cudaGraph_t       out = nullptr;
-  const cudaError_t q   = cudaStreamEndCapture(c->stream, &out);
+  const cudaError_t q   = cudaStreamEndCapture(c->stream.get(), &out);
   if (e)
     return e;
   CU(q);
@@ -1222,34 +1224,37 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   const uint64_t n    = c->n_owned;
   double        *x    = const_cast<double *>(sg.x);
   const double  *prec = sg.prec;
-  bp4::SolveState *st = c->d_state;
-  double        *acc  = c->d_acc;
-  CU(cudaGraphCreate(&sg.graph, 0));
+  bp4::SolveState *st = c->d_state.get();
+  double        *acc  = c->d_acc.get();
+  double        *g = sg.g.p(), *d = sg.d.p(), *h = sg.h.p();
+  cudaGraph_t    graph;
+  CU(cudaGraphCreate(&graph, 0));
+  sg.graph.reset(graph);
   cudaGraphConditionalHandle loop;
-  CU(cudaGraphConditionalHandleCreate(&loop, sg.graph, 1, cudaGraphCondAssignDefault));
+  CU(cudaGraphConditionalHandleCreate(&loop, graph, 1, cudaGraphCondAssignDefault));
   std::vector<cudaGraphNode_t> leaves;
   auto jacobi_dot = [&]() { // h = P g, g.h -> acc[2]
     return sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::jacobi_dot_kernel<true> : bp4::jacobi_dot_kernel<false>,
-                 n, sg.h, sg.g, prec, acc + 2, c->det);
+                 n, h, g, prec, acc + 2, c->det);
   };
   auto scalar = [&](const int kind) -> int { // solve_scalar_kernel on one thread
     Timed t(c, BP4_K_BLAS1);
-    bp4::solve_scalar_kernel<<<1, 32, 0, c->stream>>>(kind, st, acc, loop);
+    bp4::solve_scalar_kernel<<<1, 32, 0, c->stream.get()>>>(kind, st, acc, loop);
     CU(cudaGetLastError());
     return 0;
   };
   // initial state; plain: h = P g, d = -h, gh = g.h (SolverCG before its loop)
   auto prologue = [&]() -> int {
-    CU(cudaMemcpyAsync(st, c->h_state, sizeof(bp4::SolveState), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(st, c->h_state.get(), sizeof(bp4::SolveState), cudaMemcpyHostToDevice, c->stream.get()));
     if (sg.merged)
       return 0;
     if (int e = jacobi_dot())
       return e;
     if (int e = scalar(bp4::kSolvePlainInit))
       return e;
-    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<false>, n, sg.d, 0., -1., sg.h, nullptr);
+    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<false>, n, d, 0., -1., h, nullptr);
   };
-  if (int e = capture_into(c, sg.graph, nullptr, 0, prologue, &leaves))
+  if (int e = capture_into(c, graph, nullptr, 0, prologue, &leaves))
     return e;
   cudaGraphNodeParams cp = {};
   cp.type                = cudaGraphNodeTypeConditional;
@@ -1257,32 +1262,32 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   cp.conditional.type    = cudaGraphCondTypeWhile;
   cp.conditional.size    = 1;
   cudaGraphNode_t cond;
-  CU(cudaGraphAddNode(&cond, sg.graph, leaves.data(), leaves.size(), &cp));
+  CU(cudaGraphAddNode(&cond, graph, leaves.data(), leaves.size(), &cp));
   auto body = [&]() -> int {
     if (sg.merged)
       {
-        const MergedCall m{x, sg.g, sg.d, prec, 0., 0., 0., 0., st};
-        if (int e = merged_sweep(c, m, sg.h))
+        const MergedCall m{x, g, d, prec, 0., 0., 0., 0., st};
+        if (int e = merged_sweep(c, m, h))
           return e;
         return scalar(bp4::kSolveMergedStep);
       }
     // SolverCG: h = A d; alpha = gh / d.h; x += alpha d; g += alpha h, |g|; check;
     // h = P g; beta = g.h / gh; d = beta d - h
-    if (int e = vmult_on(c, sg.h, sg.d))
+    if (int e = vmult_on(c, h, d))
       return e;
-    if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, sg.d,
-                      sg.h, acc, c->det))
+    if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, d,
+                      h, acc, c->det))
       return e;
     if (int e = scalar(bp4::kSolvePlainAlpha))
       return e;
     if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::cg_xg_kernel<true> : bp4::cg_xg_kernel<false>, n, x,
-                      sg.g, sg.d, sg.h, st, acc + 1, c->det))
+                      g, d, h, st, acc + 1, c->det))
       return e;
     if (int e = jacobi_dot())
       return e;
     if (int e = scalar(bp4::kSolvePlainCheck))
       return e;
-    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, sg.d, 0., -1., sg.h, &st->beta);
+    return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, d, 0., -1., h, &st->beta);
   };
   if (int e = capture_into(c, cp.conditional.phGraph_out[0], nullptr, 0, body, nullptr))
     return e;
@@ -1290,15 +1295,17 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   auto epilogue = [&]() -> int {
     if (sg.merged)
       if (int e = sweep(c, BP4_K_BLAS1, n,
-                        c->deterministic ? bp4::solve_final_kernel<true> : bp4::solve_final_kernel<false>, n, x, sg.d,
-                        sg.g, prec, st))
+                        c->deterministic ? bp4::solve_final_kernel<true> : bp4::solve_final_kernel<false>, n, x, d,
+                        g, prec, st))
         return e;
-    CU(cudaMemcpyAsync(c->h_state + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(c->h_state.get() + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream.get()));
     return 0;
   };
-  if (int e = capture_into(c, sg.graph, &cond, 1, epilogue, nullptr))
+  if (int e = capture_into(c, graph, &cond, 1, epilogue, nullptr))
     return e;
-  CU(cudaGraphInstantiate(&sg.exec, sg.graph, 0));
+  cudaGraphExec_t exec;
+  CU(cudaGraphInstantiate(&exec, graph, 0));
+  sg.exec.reset(exec);
   return 0;
 }
 
@@ -1323,33 +1330,32 @@ static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec
   for (SolveGraph &e : c->solves)
     if (e.merged == merged && e.fused == c->fused && e.x == x->p() && e.b == b->p() && e.prec == prec->p())
       sg = &e;
-  if (!sg)
+  if (!sg) // the entry goes into the cache once its temporaries are allocated
     {
-      c->solves.emplace_back();
-      sg         = &c->solves.back();
-      sg->merged = merged, sg->fused = c->fused, sg->x = x->p(), sg->b = b->p(), sg->prec = prec->p();
-      const uint64_t nl = c->n_owned + c->n_ghost;
-      for (double **v : {&sg->g, &sg->d, &sg->h})
-        if (int e = pooled_alloc(c, nl, v, false))
+      SolveGraph ns;
+      ns.merged = merged, ns.fused = c->fused, ns.x = x->p(), ns.b = b->p(), ns.prec = prec->p();
+      for (bp4_vec *v : {&ns.g, &ns.d, &ns.h})
+        if (int e = pooled_alloc(c, c->n_owned + c->n_ghost, *v, false))
           return e;
+      c->solves.push_back(std::move(ns));
+      sg = &c->solves.back();
     }
   // step 0 on the host, with the entry points the host-driven solvers use: g = A x - b (-b for a
   // zero start vector), |g|, ReductionControl::check(0)
-  bp4_vec g{sg->g, c->n_owned + c->n_ghost};
-  int     zero = 0;
+  int zero = 0;
   if (int e = bp4_all_zero(c, x, &zero))
     return e;
   if (!zero)
     {
-      if (int e = bp4_vmult(c, &g, x))
+      if (int e = bp4_vmult(c, &sg->g, x))
         return e;
-      if (int e = bp4_add(c, &g, -1., b))
+      if (int e = bp4_add(c, &sg->g, -1., b))
         return e;
     }
-  else if (int e = bp4_equ(c, &g, -1., b))
+  else if (int e = bp4_equ(c, &sg->g, -1., b))
     return e;
   double res = 0.;
-  if (int e = bp4_l2_norm(c, &g, &res))
+  if (int e = bp4_l2_norm(c, &sg->g, &res))
     return e;
   const double reduced_tol = res * reduce;
   const int    state0      = (res < reduced_tol || res <= tol) ? 1 : ((max_steps == 0 || std::isnan(res)) ? 2 : 0);
@@ -1359,22 +1365,20 @@ static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec
   if (!sg->exec)
     if (int e = build_solve_graph(c, *sg))
       {
-        if (sg->graph) // a later call starts over
-          cudaGraphDestroy(sg->graph);
-        sg->graph = nullptr;
+        sg->graph.reset(); // a later call starts over
         return e;
       }
-  bp4::SolveState &init = c->h_state[0];
+  bp4::SolveState &init = *c->h_state;
   init                  = bp4::SolveState{};
   init.tol              = tol;
   init.reduced_tol      = reduced_tol;
   init.last_value       = res;
   init.initial_value    = res;
   init.max_steps        = max_steps;
-  CU(cudaGraphLaunch(sg->exec, c->stream));
+  CU(cudaGraphLaunch(sg->exec.get(), c->stream.get()));
   c->launches += 1;
-  CU(cudaStreamSynchronize(c->stream));
-  const bp4::SolveState &fin = c->h_state[1];
+  CU(cudaStreamSynchronize(c->stream.get()));
+  const bp4::SolveState &fin = c->h_state.get()[1];
   *out                       = bp4_solve_result{fin.state, fin.step, fin.last_value, res};
   return 0;
 }
@@ -1466,9 +1470,9 @@ static int p2p_setup(bp4_ctx *c)
       mine.off_contrib[k] = off;
       off += up(sizeof(double) * (ne ? ne : 1));
     }
-  CU(cudaMalloc(&p.arena, off));
-  CU(cudaMemset(p.arena, 0, off));
-  CU(cudaIpcGetMemHandle(&mine.handle, p.arena));
+  CU(allocate(p.arena, off));
+  CU(cudaMemset(p.arena.get(), 0, off));
+  CU(cudaIpcGetMemHandle(&mine.handle, p.arena.get()));
   for (int r = 0; r < kP2PMaxRanks; ++r)
     mine.imp_off_for[r] = mine.exp_off_for[r] = -1;
   for (size_t k = 0; k < c->peer.size(); ++k)
@@ -1479,16 +1483,13 @@ static int p2p_setup(bp4_ctx *c)
   for (int k = 0; k < 2; ++k)
     p.off_ghost[k] = mine.off_ghost[k], p.off_contrib[k] = mine.off_contrib[k];
   // all-gather the cards through NCCL (device staging buffers)
-  P2PCard *d_mine = nullptr, *d_all = nullptr;
-  CU(cudaMalloc(&d_mine, sizeof(P2PCard)));
-  CU(cudaMalloc(&d_all, sizeof(P2PCard) * c->n_ranks));
-  CU(cudaMemcpy(d_mine, &mine, sizeof(P2PCard), cudaMemcpyHostToDevice));
-  NC(ncclAllGather(d_mine, d_all, sizeof(P2PCard), ncclChar, c->comm, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
+  dev_ptr<P2PCard> d_mine, d_all;
+  CU(upload(d_mine, &mine, 1));
+  CU(allocate(d_all, c->n_ranks));
+  NC(ncclAllGather(d_mine.get(), d_all.get(), sizeof(P2PCard), ncclChar, c->comm.get(), c->stream.get()));
+  CU(cudaStreamSynchronize(c->stream.get()));
   std::vector<P2PCard> all(c->n_ranks);
-  CU(cudaMemcpy(all.data(), d_all, sizeof(P2PCard) * c->n_ranks, cudaMemcpyDeviceToHost));
-  CU(cudaFree(d_mine));
-  CU(cudaFree(d_all));
+  CU(cudaMemcpy(all.data(), d_all.get(), sizeof(P2PCard) * c->n_ranks, cudaMemcpyDeviceToHost));
   bool ok = true;
   for (size_t k = 0; k < c->peer.size() && ok; ++k)
     {
@@ -1500,7 +1501,7 @@ static int p2p_setup(bp4_ctx *c)
           ok = false;
           break;
         }
-      p.peer_arena.push_back((char *)base);
+      p.peer_arena.emplace_back((char *)base);
       for (int b = 0; b < 2; ++b)
         {
           p.peer_off_ghost[b].push_back(q.off_ghost[b]);
@@ -1512,25 +1513,14 @@ static int p2p_setup(bp4_ctx *c)
       p.peer_exp_off.push_back((uint64_t)std::max<int64_t>(q.exp_off_for[c->rank], 0));
     }
   // every rank must take the same path: agree on the outcome
-  int *d_ok = nullptr, h_ok = ok ? 1 : 0;
-  CU(cudaMalloc(&d_ok, sizeof(int)));
-  CU(cudaMemcpy(d_ok, &h_ok, sizeof(int), cudaMemcpyHostToDevice));
-  NC(ncclAllReduce(d_ok, d_ok, 1, ncclInt, ncclMin, c->comm, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  CU(cudaMemcpy(&h_ok, d_ok, sizeof(int), cudaMemcpyDeviceToHost));
-  CU(cudaFree(d_ok));
+  int          h_ok = ok ? 1 : 0;
+  dev_ptr<int> d_ok;
+  CU(upload(d_ok, &h_ok, 1));
+  NC(ncclAllReduce(d_ok.get(), d_ok.get(), 1, ncclInt, ncclMin, c->comm.get(), c->stream.get()));
+  CU(cudaStreamSynchronize(c->stream.get()));
+  CU(cudaMemcpy(&h_ok, d_ok.get(), sizeof(int), cudaMemcpyDeviceToHost));
   p.on = h_ok == 1;
   return 0;
-}
-
-static void p2p_teardown(bp4_ctx *c)
-{
-  for (char *b : c->p2p.peer_arena)
-    cudaIpcCloseMemHandle(b);
-  c->p2p.peer_arena.clear();
-  cudaFree(c->p2p.arena);
-  c->p2p.arena = nullptr;
-  c->p2p.on    = false;
 }
 
 int bp4_comm_init(bp4_ctx *c, int rank, int n_ranks, const unsigned char id[BP4_NCCL_ID_BYTES])
@@ -1539,10 +1529,15 @@ int bp4_comm_init(bp4_ctx *c, int rank, int n_ranks, const unsigned char id[BP4_
     return fail(BP4_ERR_ARG, "null argument");
   if (c->deterministic && n_ranks > 1)
     return fail(BP4_ERR_STATE, "the deterministic mode runs on one rank");
+  if (c->comm)
+    return fail(BP4_ERR_STATE, "the communicator is already initialised (rank %d of %d): bp4_comm_init may be "
+                               "called once per context", c->rank, c->n_ranks);
   CU(cudaSetDevice(c->device));
   ncclUniqueId u;
   memcpy(&u, id, sizeof(u));
-  NC(ncclCommInitRank(&c->comm, n_ranks, u, rank));
+  ncclComm_t comm;
+  NC(ncclCommInitRank(&comm, n_ranks, u, rank));
+  c->comm.reset(comm);
   c->rank    = rank;
   c->n_ranks = n_ranks;
   if (n_ranks > 1 && !c->fused_pinned)
@@ -1578,21 +1573,21 @@ static int exchange_ghosts_on(bp4_ctx *c, double *v, cudaStream_t st)
           if (!ns)
             continue;
           if (e > 2) // the peer has emptied this half of its ghost_in (exchange e - 2)
-            DRV(p.wait64((CUstream)st, flag_addr(p.arena, kFlagAckFwd, c->peer[k]), e - 2, CU_STREAM_WAIT_VALUE_GEQ));
-          CU(cudaMemcpyAsync(p.peer_arena[k] + p.peer_off_ghost[b][k] + sizeof(double) * p.peer_imp_off[k],
-                             c->d_sendbuf + c->export_off[k], sizeof(double) * ns, cudaMemcpyDeviceToDevice, st));
-          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k], kFlagDataFwd, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
+            DRV(p.wait64((CUstream)st, flag_addr(p.arena.get(), kFlagAckFwd, c->peer[k]), e - 2, CU_STREAM_WAIT_VALUE_GEQ));
+          CU(cudaMemcpyAsync(p.peer_arena[k].get() + p.peer_off_ghost[b][k] + sizeof(double) * p.peer_imp_off[k],
+                             c->d_sendbuf.get() + c->export_off[k], sizeof(double) * ns, cudaMemcpyDeviceToDevice, st));
+          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k].get(), kFlagDataFwd, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
         }
       for (size_t k = 0; k < c->peer.size(); ++k)
         {
           const uint64_t nr = c->import_off[k + 1] - c->import_off[k];
           if (!nr)
             continue;
-          DRV(p.wait64((CUstream)st, flag_addr(p.arena, kFlagDataFwd, c->peer[k]), e, CU_STREAM_WAIT_VALUE_GEQ));
+          DRV(p.wait64((CUstream)st, flag_addr(p.arena.get(), kFlagDataFwd, c->peer[k]), e, CU_STREAM_WAIT_VALUE_GEQ));
           CU(cudaMemcpyAsync(v + c->n_owned + c->import_off[k],
-                             p.arena + p.off_ghost[b] + sizeof(double) * c->import_off[k], sizeof(double) * nr,
+                             p.arena.get() + p.off_ghost[b] + sizeof(double) * c->import_off[k], sizeof(double) * nr,
                              cudaMemcpyDeviceToDevice, st));
-          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k], kFlagAckFwd, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
+          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k].get(), kFlagAckFwd, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
         }
       return 0;
     }
@@ -1601,9 +1596,9 @@ static int exchange_ghosts_on(bp4_ctx *c, double *v, cudaStream_t st)
     {
       const uint64_t ns = c->export_off[k + 1] - c->export_off[k], nr = c->import_off[k + 1] - c->import_off[k];
       if (ns)
-        NC(ncclSend(c->d_sendbuf + c->export_off[k], ns, ncclDouble, c->peer[k], c->comm, st));
+        NC(ncclSend(c->d_sendbuf.get() + c->export_off[k], ns, ncclDouble, c->peer[k], c->comm.get(), st));
       if (nr)
-        NC(ncclRecv(v + c->n_owned + c->import_off[k], nr, ncclDouble, c->peer[k], c->comm, st));
+        NC(ncclRecv(v + c->n_owned + c->import_off[k], nr, ncclDouble, c->peer[k], c->comm.get(), st));
     }
   NC(ncclGroupEnd());
   return 0;
@@ -1624,14 +1619,14 @@ static int exchange_compress_on(bp4_ctx *c, double *v, cudaStream_t st)
           if (!ns)
             continue;
           if (e > 2)
-            DRV(p.wait64((CUstream)st, flag_addr(p.arena, kFlagAckRev, c->peer[k]), e - 2, CU_STREAM_WAIT_VALUE_GEQ));
-          CU(cudaMemcpyAsync(p.peer_arena[k] + p.peer_off_contrib[b][k] + sizeof(double) * p.peer_exp_off[k],
+            DRV(p.wait64((CUstream)st, flag_addr(p.arena.get(), kFlagAckRev, c->peer[k]), e - 2, CU_STREAM_WAIT_VALUE_GEQ));
+          CU(cudaMemcpyAsync(p.peer_arena[k].get() + p.peer_off_contrib[b][k] + sizeof(double) * p.peer_exp_off[k],
                              v + c->n_owned + c->import_off[k], sizeof(double) * ns, cudaMemcpyDeviceToDevice, st));
-          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k], kFlagDataRev, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
+          DRV(p.write64((CUstream)st, flag_addr(p.peer_arena[k].get(), kFlagDataRev, c->rank), e, CU_STREAM_WRITE_VALUE_DEFAULT));
         }
       for (size_t k = 0; k < c->peer.size(); ++k)
         if (c->export_off[k + 1] > c->export_off[k])
-          DRV(p.wait64((CUstream)st, flag_addr(p.arena, kFlagDataRev, c->peer[k]), e, CU_STREAM_WAIT_VALUE_GEQ));
+          DRV(p.wait64((CUstream)st, flag_addr(p.arena.get(), kFlagDataRev, c->peer[k]), e, CU_STREAM_WAIT_VALUE_GEQ));
       return 0;
     }
   NC(ncclGroupStart());
@@ -1639,9 +1634,9 @@ static int exchange_compress_on(bp4_ctx *c, double *v, cudaStream_t st)
     {
       const uint64_t nr = c->export_off[k + 1] - c->export_off[k], ns = c->import_off[k + 1] - c->import_off[k];
       if (ns)
-        NC(ncclSend(v + c->n_owned + c->import_off[k], ns, ncclDouble, c->peer[k], c->comm, st));
+        NC(ncclSend(v + c->n_owned + c->import_off[k], ns, ncclDouble, c->peer[k], c->comm.get(), st));
       if (nr)
-        NC(ncclRecv(c->d_recvbuf + c->export_off[k], nr, ncclDouble, c->peer[k], c->comm, st));
+        NC(ncclRecv(c->d_recvbuf.get() + c->export_off[k], nr, ncclDouble, c->peer[k], c->comm.get(), st));
     }
   NC(ncclGroupEnd());
   return 0;
@@ -1650,8 +1645,8 @@ static int exchange_compress_on(bp4_ctx *c, double *v, cudaStream_t st)
 // where the contributions of the last compress exchange wait for unpack_add
 static const double *contrib_buffer(const bp4_ctx *c)
 {
-  return c->p2p.on ? reinterpret_cast<const double *>(c->p2p.arena + c->p2p.off_contrib[c->p2p.epoch_rev & 1])
-                   : c->d_recvbuf;
+  return c->p2p.on ? reinterpret_cast<const double *>(c->p2p.arena.get() + c->p2p.off_contrib[c->p2p.epoch_rev & 1])
+                   : c->d_recvbuf.get();
 }
 
 // the end of compress(add) on the context's stream, once exchange_compress_on has delivered the
@@ -1663,16 +1658,16 @@ static int compress_finish(bp4_ctx *c, double *v)
     // one launch for all peers: an owned entry may be exported to several (atomics)
     Timed          t(c, BP4_K_BLAS1);
     const uint64_t ne = c->export_off.back();
-    if (int e = per_element(c, ne, bp4::unpack_add_kernel, ne, c->d_export, contrib_buffer(c), v))
+    if (int e = per_element(c, ne, bp4::unpack_add_kernel, ne, c->d_export.get(), contrib_buffer(c), v))
       return e;
   }
   auto &p = c->p2p;
   if (p.on)
     for (size_t k = 0; k < c->peer.size(); ++k)
       if (c->export_off[k + 1] > c->export_off[k])
-        DRV(p.write64((CUstream)c->stream, flag_addr(p.peer_arena[k], kFlagAckRev, c->rank), p.epoch_rev,
+        DRV(p.write64((CUstream)c->stream.get(), flag_addr(p.peer_arena[k].get(), kFlagAckRev, c->rank), p.epoch_rev,
                       CU_STREAM_WRITE_VALUE_DEFAULT));
-  CU(cudaMemsetAsync(v + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream));
+  CU(cudaMemsetAsync(v + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream.get()));
   return 0;
 }
 
@@ -1689,10 +1684,10 @@ int bp4_update_ghost_values(bp4_ctx *c, bp4_vec *v)
   {
     Timed          t(c, BP4_K_BLAS1);
     const uint64_t ne = c->export_off.back();
-    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export, v->p(), c->d_sendbuf))
+    if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export.get(), v->p(), c->d_sendbuf.get()))
       return e;
   }
-  return exchange_ghosts_on(c, v->p(), c->stream);
+  return exchange_ghosts_on(c, v->p(), c->stream.get());
 }
 
 // ghost contributions -> owners, added (compress(VectorOperation::add)); ghost slots are zeroed
@@ -1705,7 +1700,7 @@ int bp4_compress_add(bp4_ctx *c, bp4_vec *v)
     return 0;
   if (!c->comm)
     return fail(BP4_ERR_STATE, "ghost exchange not initialised (bp4_comm_init)");
-  if (int e = exchange_compress_on(c, v->p(), c->stream))
+  if (int e = exchange_compress_on(c, v->p(), c->stream.get()))
     return e;
   return compress_finish(c, v->p());
 }
@@ -1730,8 +1725,7 @@ int bp4_profile_enable(bp4_ctx *c, int on)
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
   if (!on)
-    if (int e = drain_events(c))
-      return e;
+    CU(drain_events(c));
   c->profile = on != 0;
   return 0;
 }
@@ -1740,8 +1734,7 @@ int bp4_profile_reset(bp4_ctx *c)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
-  if (int e = drain_events(c))
-    return e;
+  CU(drain_events(c));
   for (int i = 0; i < BP4_K_COUNT; ++i)
     {
       c->prof_ms[i]  = 0;
@@ -1755,8 +1748,7 @@ int bp4_profile_get(bp4_ctx *c, int id, double *total_ms, uint64_t *launches)
 {
   if (!c || id < 0 || id >= BP4_K_COUNT)
     return fail(BP4_ERR_ARG, "bad kernel id");
-  if (int e = drain_events(c))
-    return e;
+  CU(drain_events(c));
   if (total_ms)
     *total_ms = c->prof_ms[id];
   if (launches)
