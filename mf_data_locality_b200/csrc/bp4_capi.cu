@@ -144,6 +144,7 @@ struct bp4_ctx
   dev_ptr<uint32_t> d_entity, d_constrained, d_walk;
   dev_ptr<double>   d_coef, d_gll;
   dev_ptr<double>   d_acc; // [8] reduction scratch
+  dev_ptr<bp4::Update4b> d_update4b; // the scalars pre_kernel derives for the fused cell kernel
   dev_ptr<int>      d_flag;
   dev_ptr<uint32_t> d_sched;     // [n_sched] unit counters of the cell-kernel launches of one loop
   uint32_t          n_sched = 4; // 4, or one per colour in the deterministic mode
@@ -552,6 +553,7 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   CU(upload(c->d_gll, gll.data(), gll.size()));
   CU(allocate(c->d_acc, 8));
   CU(cudaMemset(c->d_acc.get(), 0, sizeof(double) * 8));
+  CU(allocate(c->d_update4b, 1));
   CU(allocate(c->d_flag, 1));
   CU(allocate(c->d_sched, c->n_sched));
   if (c->deterministic)
@@ -794,7 +796,8 @@ static uint64_t sweep_len(const bp4_ctx *c, std::initializer_list<const bp4_vec 
   return n;
 }
 
-// scalars and vectors of one vmult_with_merged_sums call, for the fused cell loop
+// vectors and scalars of one vmult_with_merged_sums call; the scalars go to pre_kernel, which
+// derives those of do_cg_update4b for the streamed and the in-loop DoFs
 struct MergedCall
 {
   double *x, *g, *d;
@@ -830,14 +833,8 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       a.p            = m->d;
       a.x            = m->x;
       a.prec         = m->prec;
-      a.alpha        = m->alpha;
-      a.beta         = m->beta;
-      a.first        = m->alpha == 0. ? 1 : 0;
-      a.update_x     = (m->alpha != 0. && m->alpha_old != 0.) ? 1 : 0;
-      a.c1           = a.update_x ? m->alpha + m->alpha_old / m->beta_old : 0.;
-      a.c2           = a.update_x ? m->alpha_old / m->beta_old : 0.;
+      a.scalars      = c->d_update4b.get();
       a.acc          = c->d_acc.get();
-      a.state        = m->state;
       Timed t(c, BP4_K_MERGED);
       CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream.get()));
     }
@@ -980,10 +977,11 @@ static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
   // kernel; the rest of the vector -- shared between ranges or ranks, Dirichlet -- is streamed
   // before / after the loop (with the fused path off: everything)
   const uint64_t tail = c->fused ? c->n_private : 0;
-  // one block at least: pre_kernel also clears the reduction scratch
+  // one block at least: pre_kernel also clears the reduction scratch and publishes the scalars
+  // the fused cell kernel reads
   if (int e = sweep(c, BP4_K_PRE, std::max<uint64_t>(n - tail, 1),
                     m.state ? bp4::pre_kernel<true> : bp4::pre_kernel<false>, tail, n, h, m.x, m.g, m.d, m.prec,
-                    m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc.get(), m.state))
+                    m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc.get(), c->d_update4b.get(), m.state))
     return e;
   if (c->n_ghost)
     CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream.get()));

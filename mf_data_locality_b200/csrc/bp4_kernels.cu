@@ -131,11 +131,11 @@ namespace bp4
   //   do_cg_update3b on the run while h, r, p are still in L2; 7 sums -> warp -> block -> acc.
   // No counters, no ping-pong buffers, no inter-block ordering.  The DoFs shared between ranges
   // (and between ranks, and the Dirichlet ones) are the tail [n_private, n_owned) of the vector:
-  // pre_kernel / post_kernel stream them before / after this kernel.
+  // pre_kernel / post_kernel stream them before / after this kernel.  The scalars of
+  // do_cg_update4b are the ones pre_kernel derived and left in *a.scalars, from the caller's
+  // arguments or from the solver state of a device-resident solve.
   // ---------------------------------------------------------------------------------------
-  // DEV (fused only): the scalars of do_cg_update4b come from the solver state of a device-resident
-  // solve (a.state) instead of the launch arguments
-  template <int P, int CPB, bool FUSED, bool QUAD, bool DEV = false>
+  template <int P, int CPB, bool FUSED, bool QUAD>
   __global__ void __launch_bounds__(kThreads, Cfg<P>::BLOCKS) cell_kernel(const CellArgs a)
   {
     constexpr int NC = Cfg<P, QUAD>::NCOEF;
@@ -594,23 +594,8 @@ namespace bp4
           if (tid == kThreads - 2 && (e & 1u)) // e - 1 is even: never the odd first element
             f(e - 1u);
         };
-        // the scalars of do_cg_update4b (sc.alpha, beta, first, update_x, c1, c2): the launch
-        // arguments, or (DEV) derived from the solver state exactly as cell_range (bp4_capi.cu)
-        // derives them on the host
-        CellArgs dev_args;
-        if constexpr (DEV)
-          {
-            dev_args        = a;
-            const double al = a.state->alpha, ao = a.state->alpha_old, bo = a.state->beta_old;
-            dev_args.alpha    = al;
-            dev_args.beta     = a.state->beta;
-            dev_args.first    = al == 0. ? 1 : 0;
-            dev_args.update_x = (al != 0. && ao != 0.) ? 1 : 0;
-            dev_args.c1       = dev_args.update_x ? __dadd_rn(al, __ddiv_rn(ao, bo)) : 0.;
-            dev_args.c2       = dev_args.update_x ? __ddiv_rn(ao, bo) : 0.;
-          }
-        const CellArgs &sc = DEV ? dev_args : a;
-        auto pre_one = [&](const uint32_t i, const double rr, const double pp, const double hh, const double pr) {
+        auto pre_one = [&](const Update4b &sc, const uint32_t i, const double rr, const double pp, const double hh,
+                           const double pr) {
           if (sc.first)
             a.p[i] = -pr * rr;
           else
@@ -629,6 +614,9 @@ namespace bp4
             job_wait(ts);
           if (e <= b)
             return;
+          // the scalars as pre_kernel derived them, read per job: held over the compute phases they
+          // would take registers that phase 2 needs (Q4 spilled 80/40 instead of 52/32 bytes)
+          const Update4b sc = *a.scalars;
           Pairs w;
           job_load(w, b, e);
           const uint32_t lo = b & ~1u, c0 = b & 1u, q0 = div3(b) & ~1u;
@@ -654,7 +642,7 @@ namespace bp4
                 *reinterpret_cast<double2 *>(a.dst + i0) = make_double2(0., 0.);
               }
           job_edges(b, e, [&](const uint32_t i) {
-            pre_one(i, js.row[0][i - lo], js.row[1][i - lo], js.row[2][i - lo], js.prec[div3(i) - q0]);
+            pre_one(sc, i, js.row[0][i - lo], js.row[1][i - lo], js.row[2][i - lo], js.prec[div3(i) - q0]);
           });
         };
         // do_cg_update3b<3,double> (solver_cg_optimized.h:12-61) on [b, e): the seven sums of a
@@ -891,12 +879,24 @@ namespace bp4
   // ---------------------------------------------------------------------------------------
   // launchers
   // ---------------------------------------------------------------------------------------
-  // dynamic shared memory of the fused instantiation: the staging rows follow the cell rows
-  template <int P>
-  constexpr size_t fused_smem()
+  // One instance of the cell kernel and its dynamic shared memory.  A degree has three: plain
+  // tri-linear, plain quadratic, and fused tri-linear if Stage<P>::OK (its staging rows follow the
+  // cell rows).
+  template <int P, bool FUSED, bool QUAD>
+  struct CellInstance
   {
-    return sizeof(CellSmem<P, Cfg<P>::CPB, 24>) + sizeof(JobSmem<(Stage<P>::OK ? Stage<P>::JOB : 2)>);
-  }
+    static constexpr int CPB  = Cfg<P, QUAD>::CPB;
+    static constexpr int SMEM = (int)(sizeof(CellSmem<P, CPB, Cfg<P, QUAD>::NCOEF>) +
+                                      (FUSED ? sizeof(JobSmem<Stage<P>::JOB>) : 0));
+    static cudaError_t init()
+    {
+      return cudaFuncSetAttribute(cell_kernel<P, CPB, FUSED, QUAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+    }
+    static void launch(const int grid, const CellArgs &a, cudaStream_t st)
+    {
+      cell_kernel<P, CPB, FUSED, QUAD><<<grid, kThreads, SMEM, st>>>(a);
+    }
+  };
 
   template <int P>
   static cudaError_t init_degree(std::vector<uint32_t> &walk)
@@ -906,26 +906,13 @@ namespace bp4
     walk.resize(Geom<P>::DOF);
     build_dof_table<P>(walk.data());
     cudaError_t e = cudaMemcpyToSymbol(c_tab<P>, &tb, sizeof(tb));
-    if (e != cudaSuccess)
-      return e;
-    constexpr int CPB = Cfg<P>::CPB, CPBQ = Cfg<P, true>::CPB;
-    e = cudaFuncSetAttribute(cell_kernel<P, CPB, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)sizeof(CellSmem<P, CPB, 24>));
-    if (e != cudaSuccess)
-      return e;
-    e = cudaFuncSetAttribute(cell_kernel<P, CPBQ, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)sizeof(CellSmem<P, CPBQ, 81>));
-    if (e != cudaSuccess)
-      return e;
+    if (e == cudaSuccess)
+      e = CellInstance<P, false, false>::init();
+    if (e == cudaSuccess)
+      e = CellInstance<P, false, true>::init();
     if constexpr (Stage<P>::OK)
-      {
-        e = cudaFuncSetAttribute(cell_kernel<P, CPB, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)fused_smem<P>());
-        if (e != cudaSuccess)
-          return e;
-        e = cudaFuncSetAttribute(cell_kernel<P, CPB, true, false, true>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fused_smem<P>());
-      }
+      if (e == cudaSuccess)
+        e = CellInstance<P, true, false>::init();
     return e;
   }
 
@@ -952,17 +939,12 @@ namespace bp4
     if (fused)
       {
         if constexpr (Stage<P>::OK)
-          {
-            if (a.state)
-              cell_kernel<P, CPB, true, false, true><<<grid, kThreads, fused_smem<P>(), st>>>(a);
-            else
-              cell_kernel<P, CPB, true, false><<<grid, kThreads, fused_smem<P>(), st>>>(a);
-          }
+          CellInstance<P, true, false>::launch(grid, a, st);
       }
     else if (quad)
-      cell_kernel<P, CPBQ, false, true><<<grid, kThreads, sizeof(CellSmem<P, CPBQ, 81>), st>>>(a);
+      CellInstance<P, false, true>::launch(grid, a, st);
     else
-      cell_kernel<P, CPB, false, false><<<grid, kThreads, sizeof(CellSmem<P, CPB, 24>), st>>>(a);
+      CellInstance<P, false, false>::launch(grid, a, st);
 #ifdef BP4_PHASE_TIMING
     if (d_trace)
       {

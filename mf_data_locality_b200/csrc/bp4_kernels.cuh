@@ -135,7 +135,30 @@ namespace bp4
     uint32_t *ticket = nullptr; // zero between launches: the last block re-arms it
   };
 
-  struct SolveState;
+  // The scalars of do_cg_update4b (solver_cg_optimized.h:65-161) for one vmult_with_merged_sums call.
+  // pre_kernel derives them (update4b) and publishes them for the fused cell kernel, so the streamed
+  // and the in-loop DoFs are updated with the same values.
+  struct Update4b
+  {
+    double alpha, beta, c1, c2; // c1 = alpha + alpha_old/beta_old, c2 = alpha_old/beta_old
+    int    first;               // alpha == 0: p = -P r, h = 0 only
+    int    update_x;            // alpha != 0 and alpha_old != 0
+  };
+
+  // IEEE divide, then add: the same bits as the host's alpha + alpha_old / beta_old
+  __device__ __forceinline__ Update4b update4b(const double alpha, const double beta, const double alpha_old,
+                                               const double beta_old)
+  {
+    Update4b u;
+    u.alpha    = alpha;
+    u.beta     = beta;
+    u.first    = alpha == 0. ? 1 : 0;
+    u.update_x = (alpha != 0. && alpha_old != 0.) ? 1 : 0;
+    u.c2       = u.update_x ? __ddiv_rn(alpha_old, beta_old) : 0.;
+    u.c1       = u.update_x ? __dadd_rn(alpha, u.c2) : 0.;
+    return u;
+  }
+
   struct CellArgs
   {
     const uint32_t *entity_index; // [n_cells][27]
@@ -151,13 +174,8 @@ namespace bp4
     uint32_t         n_units;
     double          *r, *p, *x;   // g, d, x of SolverCGFullMerge; p == src
     const double    *prec;        // [n_owned / 3]
-    double           alpha, beta, c1, c2; // c1 = alpha + alpha_old/beta_old, c2 = alpha_old/beta_old
-    int              first;       // alpha == 0: p = -P r, h = 0 only
-    int              update_x;    // alpha_old != 0
+    const Update4b  *scalars;     // written by the pre_kernel launched before this kernel
     double          *acc;         // [7]
-    // device-resident solve (cell_kernel<..., DEV = true>): alpha, beta, first, update_x, c1, c2
-    // are derived in-kernel from state->alpha .. beta_old instead of the fields above
-    const SolveState *state;
   };
 
   // Solver state of a device-resident CG solve (bp4_solve_cg / bp4_solve_cg_merged), one block

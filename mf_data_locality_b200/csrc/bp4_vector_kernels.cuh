@@ -124,29 +124,26 @@ namespace bp4
   // ---------------------------------------------------------------------------------------
   // do_cg_update4b<3,double,true>, solver_cg_optimized.h:65-161, over [begin, end): the DoFs that
   // are not private to one cell-batch range (all of them when the numbering has no such group).
-  // Also clears the reduction scratch of this iteration (stream order: before any post).
+  // Also clears the reduction scratch of this iteration (stream order: before any post) and leaves
+  // its scalars in *scalars for the fused cell kernel that follows.
   // DEV: the four scalars come from the solver state of a device-resident solve (st).
   template <bool DEV>
   __global__ void __launch_bounds__(256) pre_kernel(const uint64_t begin, const uint64_t end,
                                                     double *__restrict__ h, double *__restrict__ x,
                                                     double *__restrict__ r, double *__restrict__ p,
                                                     const double *__restrict__ prec,
-                                                    double alpha, double beta,
-                                                    double alpha_old, double beta_old,
-                                                    double *acc_to_zero, const SolveState *st)
+                                                    const double alpha, const double beta,
+                                                    const double alpha_old, const double beta_old,
+                                                    double *acc_to_zero, Update4b *scalars,
+                                                    const SolveState *st)
   {
-    if constexpr (DEV)
-      {
-        alpha     = st->alpha;
-        beta      = st->beta;
-        alpha_old = st->alpha_old;
-        beta_old  = st->beta_old;
-      }
+    const Update4b sc = DEV ? update4b(st->alpha, st->beta, st->alpha_old, st->beta_old)
+                            : update4b(alpha, beta, alpha_old, beta_old);
     if (acc_to_zero && blockIdx.x == 0 && threadIdx.x < 8)
       acc_to_zero[threadIdx.x] = 0.;
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+      *scalars = sc;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    const double   c1 = alpha_old != 0. ? alpha + alpha_old / beta_old : 0.;
-    const double   c2 = alpha_old != 0. ? alpha_old / beta_old : 0.;
     // U independent elements per trip: all their loads are in flight together.  Measured at Q4
     // s=18: U = 1 -> 0.496 ms, 2 -> 0.484, 4 -> 0.474 (6.3 TB/s), 6/8 -> 0.48
     constexpr int U = 4;
@@ -160,9 +157,9 @@ namespace bp4
             const bool     ok = i < end;
             pr[u] = ok ? prec[i / 3] : 0.;
             ri[u] = ok ? r[i] : 0.;
-            pi[u] = ok && alpha != 0. ? p[i] : 0.;
-            hi[u] = ok && alpha != 0. ? h[i] : 0.;
-            xi[u] = ok && alpha_old != 0. ? x[i] : 0.;
+            pi[u] = ok && !sc.first ? p[i] : 0.;
+            hi[u] = ok && !sc.first ? h[i] : 0.;
+            xi[u] = ok && sc.update_x ? x[i] : 0.;
           }
 #pragma unroll
         for (int u = 0; u < U; ++u)
@@ -170,15 +167,15 @@ namespace bp4
             const uint64_t i = i0 + u * stride;
             if (i < end)
               {
-                if (alpha == 0.)
+                if (sc.first)
                   p[i] = -pr[u] * ri[u];
                 else
                   {
-                    if (alpha_old != 0.)
-                      x[i] = xi[u] + (c1 * pi[u] + c2 * pr[u] * ri[u]);
-                    const double rn = ri[u] + alpha * hi[u];
+                    if (sc.update_x)
+                      x[i] = xi[u] + (sc.c1 * pi[u] + sc.c2 * pr[u] * ri[u]);
+                    const double rn = ri[u] + sc.alpha * hi[u];
                     r[i] = rn;
-                    p[i] = beta * pi[u] - pr[u] * rn;
+                    p[i] = sc.beta * pi[u] - pr[u] * rn;
                   }
                 h[i] = 0.;
               }
