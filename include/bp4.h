@@ -124,6 +124,22 @@ int bp4_vec_set_zero(bp4_ctx *ctx, bp4_vec *v);                            /* v 
 int bp4_vec_upload(bp4_ctx *ctx, bp4_vec *v, const double *host, uint64_t n);
 int bp4_vec_download(bp4_ctx *ctx, const bp4_vec *v, double *host, uint64_t n);
 int bp4_vec_device_ptr(bp4_ctx *ctx, bp4_vec *v, double **dev);            /* current buffer */
+/* v views n doubles of caller-owned device memory at dev: no copy, no allocation.  Every entry
+ * point that takes a bp4_vec accepts it, with the usual length checks (n_owned + n_ghost for
+ * operator operands, n_owned/3 for prec).
+ *   - dev must be device memory (cudaMalloc, a caching allocator's block) of the context's device,
+ *     16-byte aligned; n > 0.  A host pointer, managed memory, another GPU's memory, a null or
+ *     misaligned pointer is BP4_ERR_ARG and nothing is launched.
+ *   - lifetime: the memory must stay valid until bp4_vec_free and until the context's queued work
+ *     on it has run.  bp4_vec_free releases the handle only; the memory stays the caller's and
+ *     never enters the context's buffer pool.
+ *   - stream order is the caller's: the context reads and writes the memory on its own stream
+ *     (bp4_ctx_stream).  Make that stream wait for the work that produced the data and make the
+ *     consumer wait for the context's stream, e.g. with cudaEventRecord + cudaStreamWaitEvent.
+ *   - device-resident solves cache their graph and three temporaries per (x, b, prec) address;
+ *     bp4_vec_free of a wrapped vector drops the entries that name its memory, so wrapping a
+ *     fresh x for every solve keeps one entry.                                                   */
+int bp4_vec_wrap(bp4_ctx *ctx, double *dev, uint64_t n, bp4_vec **v);
 
 /* ---- operator ------------------------------------------------------------------------- */
 /* dst = A src, identity on constrained rows: LaplaceOperator::vmult, poisson_operator.h:307 */
@@ -181,7 +197,8 @@ int bp4_all_zero(bp4_ctx *ctx, const bp4_vec *v, int *result);
  *     the vector kernels of bp4_vmult_merged.
  *   - blocking: the call returns when *out is on the host.  The instantiated graph is cached in
  *     the context per (solver, x, b, prec, in-loop form) together with its temporaries g, d, h;
- *     a repeated solve re-uses it.
+ *     a repeated solve re-uses it; bp4_vec_free of a wrapped x, b or prec drops the entries that
+ *     name it and returns their temporaries to the context's pool.
  *   - measurement: bp4_launch_count adds one per graph launch (plus the step-0 kernels); the
  *     kernels of the graph are counted once, when it is built.  bp4_profile_* time no kernel
  *     inside the graph.                                                                      */

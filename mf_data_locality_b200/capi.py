@@ -45,7 +45,7 @@ EXPORTS = [
     "bp4_equ", "bp4_add", "bp4_sadd", "bp4_dot", "bp4_add_and_dot", "bp4_l2_norm", "bp4_all_zero",
     "bp4_comm_unique_id", "bp4_comm_init", "bp4_comm_info", "bp4_update_ghost_values", "bp4_compress_add",
     "bp4_profile_enable", "bp4_profile_reset", "bp4_profile_get", "bp4_launch_count",
-    "bp4_solve_cg", "bp4_solve_cg_merged", "bp4_deterministic_info",
+    "bp4_solve_cg", "bp4_solve_cg_merged", "bp4_deterministic_info", "bp4_vec_wrap",
 ]
 
 SUCCESS, FAILURE = 1, 2  # SolverControl::State of a device-resident solve
@@ -75,6 +75,7 @@ def lib():
         _lib.bp4_vec_alloc.argtypes = [vp, C.c_uint64, vp]
         _lib.bp4_vec_upload.argtypes = [vp, vp, vp, C.c_uint64]
         _lib.bp4_vec_download.argtypes = [vp, vp, vp, C.c_uint64]
+        _lib.bp4_vec_wrap.argtypes = [vp, vp, C.c_uint64, vp]
         for f in (_lib.bp4_solve_cg, _lib.bp4_solve_cg_merged):
             f.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp]
     return _lib
@@ -102,32 +103,94 @@ def _ptr(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None and a.size else None
 
 
+def check_tensor(t, device: int):
+    """Raise TypeError / ValueError unless `t` can be wrapped by a context on CUDA device `device`:
+    a contiguous, non-empty float64 CUDA tensor on that device whose data starts on a 16-byte
+    boundary (the in-loop vector updates move 16-byte pieces from even indices)."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"expected a torch.Tensor, got {type(t).__name__}")
+    if t.device.type != "cuda" or t.device.index != device:
+        raise ValueError(f"tensor is on {t.device}, the context runs on cuda:{device}")
+    if t.dtype != torch.float64:
+        raise ValueError(f"tensor has dtype {t.dtype}, need torch.float64")
+    if not t.is_contiguous():
+        raise ValueError("tensor is not contiguous")
+    if t.numel() == 0:
+        raise ValueError("tensor is empty")
+    if t.data_ptr() % 16:
+        raise ValueError(f"tensor data at {t.data_ptr():#x} is not 16-byte aligned (a view at an odd offset?)")
+
+
 class Vector:
+    tensor = None  # the torch tensor a wrapped vector views (Context.wrap); None for owned memory
+
     def __init__(self, ctx: "Context", n: int):
         self.ctx, self.n = ctx, int(n)
         self.h = C.c_void_p()
         _chk(lib().bp4_vec_alloc(ctx.h, C.c_uint64(self.n), C.byref(self.h)))
 
+    @classmethod
+    def _view(cls, ctx: "Context", t):
+        self = cls.__new__(cls)
+        self.ctx, self.n, self.tensor = ctx, t.numel(), t
+        self.h = C.c_void_p()
+        _chk(lib().bp4_vec_wrap(ctx.h, C.c_void_p(t.data_ptr()), C.c_uint64(self.n), C.byref(self.h)))
+        return self
+
     def upload(self, a):
         a = np.ascontiguousarray(a, dtype=np.float64)
-        _chk(lib().bp4_vec_upload(self.ctx.h, self.h, _ptr(a), C.c_uint64(a.size)))
+        with _Ordered(self.ctx, (self,)):
+            _chk(lib().bp4_vec_upload(self.ctx.h, self.h, _ptr(a), C.c_uint64(a.size)))
         self.ctx.synchronize()      # `a` may be a temporary
         return self
 
     def download(self, n=None):
         n = self.n if n is None else int(n)
         out = np.empty(n)
-        _chk(lib().bp4_vec_download(self.ctx.h, self.h, _ptr(out), C.c_uint64(n)))
+        with _Ordered(self.ctx, (self,)):
+            _chk(lib().bp4_vec_download(self.ctx.h, self.h, _ptr(out), C.c_uint64(n)))
         return out
 
     def zero(self):
-        _chk(lib().bp4_vec_set_zero(self.ctx.h, self.h))
+        with _Ordered(self.ctx, (self,)):
+            _chk(lib().bp4_vec_set_zero(self.ctx.h, self.h))
         return self
 
     def free(self):
+        """release the handle; a wrapped vector's tensor stays the caller's, with its contents"""
         if self.h:
             lib().bp4_vec_free(self.ctx.h, self.h)
             self.h = C.c_void_p()
+        self.tensor = None
+
+
+class _Ordered:
+    """Orders a context call on wrapped vectors with PyTorch's current stream, without a host
+    synchronisation: the context's stream waits for the work queued so far on the current stream,
+    and the current stream waits for the call.  Every wrapped tensor is then recorded on the
+    current stream, which now runs behind the call, so the caching allocator does not hand its
+    memory out while the call is queued.  (Not on the context's stream itself: the allocator
+    records an event on each recorded stream when the tensor is freed, and close() destroys that
+    stream while the tensor may live on.)  A call on owned vectors only does nothing here."""
+    __slots__ = ("ctx", "ts", "cur")
+
+    def __init__(self, ctx: "Context", vecs):
+        self.ctx = ctx
+        self.ts = [v.tensor for v in vecs if v is not None and v.tensor is not None]
+
+    def __enter__(self):
+        if self.ts:
+            import torch
+            self.cur = torch.cuda.current_stream(self.ctx.device)
+            self.ctx.torch_stream().wait_stream(self.cur)
+
+    def __exit__(self, *exc):
+        if self.ts:
+            self.cur.wait_stream(self.ctx.torch_stream())
+            for t in self.ts:
+                t.record_stream(self.cur)
+        return False
 
 
 class Context:
@@ -178,12 +241,14 @@ class Context:
         self.degree, self.n_cells = int(degree), len(ei)
         self.n_owned, self.n_ghost = int(n_owned), int(n_ghost)
         self.n_local = self.n_owned + self.n_ghost
+        self.device = int(device)
 
     @classmethod
-    def from_handle(cls, handle, degree, n_cells, n_owned, n_ghost=0):
+    def from_handle(cls, handle, degree, n_cells, n_owned, n_ghost=0, device=0):
         """view of a context owned by someone else (the C++ host's LaplaceOperator); close() is a no-op"""
         self = cls.__new__(cls)
         self.h = C.c_void_p(handle)
+        self.device = int(device)
         self.degree, self.n_cells = int(degree), int(n_cells)
         self.n_owned, self.n_ghost = int(n_owned), int(n_ghost)
         self.n_local = self.n_owned + self.n_ghost
@@ -195,6 +260,7 @@ class Context:
         if self.h and not getattr(self, "borrowed", False):
             lib().bp4_ctx_destroy(self.h)
         self.h = C.c_void_p()
+        self._torch_stream = None
 
     def synchronize(self):
         _chk(lib().bp4_ctx_synchronize(self.h))
@@ -204,20 +270,38 @@ class Context:
         _chk(lib().bp4_ctx_stream(self.h, C.byref(s)))
         return s.value or 0
 
+    def torch_stream(self):
+        """the context's stream as a torch.cuda.ExternalStream"""
+        if getattr(self, "_torch_stream", None) is None:
+            import torch
+            self._torch_stream = torch.cuda.ExternalStream(self.stream(), device=torch.device("cuda", self.device))
+        return self._torch_stream
+
     def vector(self, n=None, data=None) -> Vector:
         v = Vector(self, self.n_local if n is None else n)
         if data is not None:
             v.upload(data)
         return v
 
+    def wrap(self, t) -> Vector:
+        """A Vector that views the CUDA tensor t in place (bp4_vec_wrap): no copy.  t must be a
+        contiguous float64 tensor on the context's device starting on a 16-byte boundary
+        (check_tensor); anything else raises before any device call.  The Vector keeps t alive;
+        its free() releases the handle only.  Calls on wrapped vectors are ordered with PyTorch's
+        current stream, so t can be filled and read by torch ops without a synchronisation."""
+        check_tensor(t, self.device)
+        return Vector._view(self, t)
+
     # ---- operator -----------------------------------------------------------------
     def vmult(self, dst: Vector, src: Vector):
-        _chk(lib().bp4_vmult(self.h, dst.h, src.h))
+        with _Ordered(self, (dst, src)):
+            _chk(lib().bp4_vmult(self.h, dst.h, src.h))
 
     def vmult_merged(self, x, g, d, h, prec, alpha, beta, alpha_old, beta_old):
         out = (C.c_double * 7)()
-        _chk(lib().bp4_vmult_merged(self.h, x.h, g.h, d.h, h.h, prec.h, alpha, beta, alpha_old,
-                                    beta_old, out))
+        with _Ordered(self, (x, g, d, h, prec)):
+            _chk(lib().bp4_vmult_merged(self.h, x.h, g.h, d.h, h.h, prec.h, alpha, beta, alpha_old,
+                                        beta_old, out))
         return np.array(out[:])
 
     def set_fused(self, on: bool):
@@ -240,16 +324,20 @@ class Context:
             _chk(lib().bp4_deterministic_info(self.h, None, None, _ptr(colors)))
         return bool(on.value), int(nc.value), colors
 
-    def inverse_diagonal(self) -> Vector:
-        v = Vector(self, self.n_owned // 3)
-        _chk(lib().bp4_inverse_diagonal(self.h, v.h))
+    def inverse_diagonal(self, out=None) -> Vector:
+        """1/diag per node (n_owned/3 entries) into `out`, or into a new vector"""
+        v = Vector(self, self.n_owned // 3) if out is None else out
+        with _Ordered(self, (v,)):
+            _chk(lib().bp4_inverse_diagonal(self.h, v.h))
         return v
 
     def jacobi_vmult(self, dst, src, diag):
-        _chk(lib().bp4_jacobi_vmult(self.h, dst.h, src.h, diag.h))
+        with _Ordered(self, (dst, src, diag)):
+            _chk(lib().bp4_jacobi_vmult(self.h, dst.h, src.h, diag.h))
 
     def x_finalize_even(self, x, d, g, prec, c1, c2):
-        _chk(lib().bp4_x_finalize_even(self.h, x.h, d.h, g.h, prec.h, c1, c2))
+        with _Ordered(self, (x, d, g, prec)):
+            _chk(lib().bp4_x_finalize_even(self.h, x.h, d.h, g.h, prec.h, c1, c2))
 
     def solve_cg(self, x, b, prec, merged=True, max_steps=100, tol=1e-15, reduce=1e-8):
         """CG solve of A x = b with the iteration loop on the device (bp4_solve_cg_merged, or
@@ -258,37 +346,45 @@ class Context:
         max_steps is state FAILURE, not an exception."""
         r = _SolveResult()
         f = lib().bp4_solve_cg_merged if merged else lib().bp4_solve_cg
-        _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
+        with _Ordered(self, (x, b, prec)):
+            _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
         return r.state, r.last_step, r.last_value, r.initial_value
 
     # ---- BLAS-1 -------------------------------------------------------------------
     def equ(self, dst, a, src):
-        _chk(lib().bp4_equ(self.h, dst.h, a, src.h))
+        with _Ordered(self, (dst, src)):
+            _chk(lib().bp4_equ(self.h, dst.h, a, src.h))
 
     def add(self, dst, a, src):
-        _chk(lib().bp4_add(self.h, dst.h, a, src.h))
+        with _Ordered(self, (dst, src)):
+            _chk(lib().bp4_add(self.h, dst.h, a, src.h))
 
     def sadd(self, dst, s, a, src):
-        _chk(lib().bp4_sadd(self.h, dst.h, s, a, src.h))
+        with _Ordered(self, (dst, src)):
+            _chk(lib().bp4_sadd(self.h, dst.h, s, a, src.h))
 
     def dot(self, a, b) -> float:
         r = C.c_double()
-        _chk(lib().bp4_dot(self.h, a.h, b.h, C.byref(r)))
+        with _Ordered(self, (a, b)):
+            _chk(lib().bp4_dot(self.h, a.h, b.h, C.byref(r)))
         return r.value
 
     def add_and_dot(self, g, a, h, w) -> float:
         r = C.c_double()
-        _chk(lib().bp4_add_and_dot(self.h, g.h, a, h.h, w.h, C.byref(r)))
+        with _Ordered(self, (g, h, w)):
+            _chk(lib().bp4_add_and_dot(self.h, g.h, a, h.h, w.h, C.byref(r)))
         return r.value
 
     def l2_norm(self, v) -> float:
         r = C.c_double()
-        _chk(lib().bp4_l2_norm(self.h, v.h, C.byref(r)))
+        with _Ordered(self, (v,)):
+            _chk(lib().bp4_l2_norm(self.h, v.h, C.byref(r)))
         return r.value
 
     def all_zero(self, v) -> bool:
         r = C.c_int()
-        _chk(lib().bp4_all_zero(self.h, v.h, C.byref(r)))
+        with _Ordered(self, (v,)):
+            _chk(lib().bp4_all_zero(self.h, v.h, C.byref(r)))
         return bool(r.value)
 
     # ---- measurement --------------------------------------------------------------

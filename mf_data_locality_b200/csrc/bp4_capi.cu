@@ -12,6 +12,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <initializer_list>
+#include <list>
 #include <map>
 #include <memory>
 #include <string>
@@ -104,11 +105,21 @@ cudaError_t upload(dev_ptr<T> &p, const T *src, size_t n)
   return e;
 }
 
+// A vector owns its buffer (bp4_vec_alloc: n + 2 doubles, recycled through the context's pool)
+// or views caller-owned memory (bp4_vec_wrap: exactly n doubles, never freed or pooled here).
 struct bp4_vec
 {
   dev_ptr<double> buf;
-  uint64_t        n = 0;
+  bool            owned = true;
+  uint64_t        n     = 0;
   double         *p() const { return buf.get(); }
+  bp4_vec() = default;
+  bp4_vec(bp4_vec &&) = default; // no move assignment: it would free a wrapped target's memory
+  ~bp4_vec()
+  {
+    if (!owned)
+      (void)buf.release();
+  }
 };
 
 struct ProfEvent
@@ -119,7 +130,8 @@ struct ProfEvent
 
 // instantiated graph of one device-resident solve (bp4_solve_cg / bp4_solve_cg_merged), keyed by
 // the variant, the caller's x, b and prec buffers and the in-loop form; it owns the temporaries
-// g, d, h so that their addresses, baked into the graph, stay valid
+// g, d, h so that their addresses, baked into the graph, stay valid.  Freeing a wrapped vector
+// drops the entries that name its buffer (drop_solves_on).
 struct SolveGraph
 {
   bool          merged = false;
@@ -155,7 +167,7 @@ struct bp4_ctx
   // the graph, [1] final state written by it) and the cached graphs
   dev_ptr<bp4::SolveState>  d_state;
   host_ptr<bp4::SolveState> h_state;
-  std::vector<SolveGraph>   solves;
+  std::list<SolveGraph>     solves; // a list: erasing an entry moves no other (bp4_vec has no move assignment)
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
   int             fused      = 0;      // 1: do_cg_update4b/3b on private DoFs inside the cell kernel
@@ -329,10 +341,10 @@ namespace
   }
 
   // v's buffer back to the pool; stream order makes reuse safe: the next user's work is queued
-  // behind ours
+  // behind ours.  A wrapped buffer is the caller's and stays out of the pool.
   void recycle(bp4_ctx *c, bp4_vec &v)
   {
-    if (v.buf)
+    if (v.buf && v.owned)
       c->pool.emplace(v.n, std::move(v.buf));
   }
 
@@ -617,6 +629,11 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
       for (const bp4::BatchDesc &b : batches) // run_limit 0: no fused kernel at this degree
         if (b.pre_end - b.pre_begin > fl.run_limit || b.post_end - b.post_begin > fl.run_limit)
           c->n_private = 0; // the updates of every DoF are streamed then
+      // a job copies whole 16-byte pieces: a run ending at n_owned reads the element past the last
+      // DoF (odd end) and the prec entry past the last node, which a wrapped vector does not have
+      // (DESIGN.md 3).  Runs that end earlier stop at least one node before the end.
+      if (rp[d->n_ranges] == d->n_owned)
+        c->n_private = 0;
       c->fused     = fl.is_default && c->n_private > 0;
       if (const char *e = getenv("BP4_FUSED")) // developer knob: 0 = pre kernel + cells + post kernel
         {
@@ -707,11 +724,59 @@ static int vec_alloc(bp4_ctx *c, uint64_t n, bp4_vec **out, bool zero)
 int bp4_vec_alloc(bp4_ctx *c, uint64_t n, bp4_vec **out) { return vec_alloc(c, n, out, true); }
 int bp4_vec_alloc_uninitialized(bp4_ctx *c, uint64_t n, bp4_vec **out) { return vec_alloc(c, n, out, false); }
 
+int bp4_vec_wrap(bp4_ctx *c, double *dev, uint64_t n, bp4_vec **out)
+{
+  if (!c || !out)
+    return fail(BP4_ERR_ARG, "null argument");
+  if (!dev || n == 0)
+    return fail(BP4_ERR_ARG, "wrap: null pointer or empty vector");
+  if (reinterpret_cast<uintptr_t>(dev) % 16)
+    return fail(BP4_ERR_ARG, "wrap: %p is not 16-byte aligned", (void *)dev);
+  CU(cudaSetDevice(c->device));
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, dev) != cudaSuccess)
+    {
+      cudaGetLastError();
+      return fail(BP4_ERR_ARG, "wrap: %p is not device memory of device %d", (void *)dev, c->device);
+    }
+  if (at.type != cudaMemoryTypeDevice || at.device != c->device) // host, managed or another GPU's
+    return fail(BP4_ERR_ARG, "wrap: %p is not device memory of device %d (memory type %d, device %d)", (void *)dev,
+                c->device, (int)at.type, at.device);
+  std::unique_ptr<bp4_vec> v(new bp4_vec);
+  v->owned = false;
+  v->n     = n;
+  v->buf.reset(dev);
+  *out = v.release();
+  return 0;
+}
+
+// drop the cached solve graphs that name buf; their temporaries go back to the pool
+static void drop_solves_on(bp4_ctx *c, const double *buf)
+{
+  for (auto it = c->solves.begin(); it != c->solves.end();)
+    if (it->x == buf || it->b == buf || it->prec == buf)
+      {
+        for (bp4_vec *t : {&it->g, &it->d, &it->h})
+          recycle(c, *t);
+        it = c->solves.erase(it);
+      }
+    else
+      ++it;
+}
+
 int bp4_vec_free(bp4_ctx *c, bp4_vec *v)
 {
   if (c && v)
-    recycle(c, *v);
-  delete v; // without a context the buffer is freed
+    {
+      if (v->owned)
+        recycle(c, *v);
+      else // the caller's next buffer has another address: without this the cache grew per solve
+        {
+          cudaSetDevice(c->device);
+          drop_solves_on(c, v->p());
+        }
+    }
+  delete v; // without a context an owned buffer is freed
   return 0;
 }
 
