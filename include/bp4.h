@@ -12,10 +12,11 @@
  *   - every function returns 0 on success, a negative bp4_status otherwise;
  *     bp4_last_error() returns a thread-local message for the last failure.
  *   - a context is bound to one CUDA device and one stream and must be driven by one
- *     host thread (the reference runs one thread per MPI rank, benchmark.h:278).
- *   - calls are asynchronous on the context's stream except those that return host
- *     scalars (bp4_dot, bp4_l2_norm, bp4_add_and_dot, bp4_all_zero, bp4_vmult_merged,
- *     bp4_vec_download, bp4_solve_cg, bp4_solve_cg_merged), which synchronise.
+ *     host thread (the reference runs one thread per MPI rank, benchmark.h:278).  The stream
+ *     is the context's own, or the caller's after bp4_ctx_set_stream.
+ *   - calls are asynchronous on that stream except those that return host scalars (bp4_dot,
+ *     bp4_l2_norm, bp4_add_and_dot, bp4_all_zero, bp4_vmult_merged, bp4_vec_download,
+ *     bp4_solve_cg, bp4_solve_cg_merged), which synchronise it.
  *   - vectors hold n_owned + n_ghost doubles: owned DoFs first (renumbered, three
  *     components interleaved per node), then ghost DoFs sorted by global index --
  *     the layout of LinearAlgebra::distributed::Vector<double>.
@@ -111,8 +112,31 @@ int         bp4_device_count(int *count);
 int bp4_ctx_create(const bp4_desc *desc, bp4_ctx **ctx);
 int bp4_ctx_destroy(bp4_ctx *ctx);
 int bp4_ctx_synchronize(bp4_ctx *ctx);
-/* cudaStream_t of the context as an opaque pointer (for event timing by the caller) */
+/* cudaStream_t the context currently queues its work on, as an opaque pointer: its own stream,
+ * or the one bp4_ctx_set_stream bound */
 int bp4_ctx_stream(bp4_ctx *ctx, void **stream);
+/* From now on every piece of work of the context goes on `stream` (a cudaStream_t), as with the
+ * stream argument of cuBLAS or NCCL: kernels, copies, memsets, solve-graph launches, NCCL calls
+ * and the timing events of bp4_profile_*.  The ghost exchange still forks onto a second stream of
+ * the context and joins back.  stream = NULL returns the context to its own stream; the legacy
+ * default stream is accepted as cudaStreamLegacy (and cudaStreamPerThread as itself), since NULL
+ * means "the context's own".
+ *   - switching is safe: the new stream waits, through an event, for everything the context
+ *     queued on the old one (pooled vectors, solve temporaries and the reduction scratch may still
+ *     be in use there); the host does not wait.
+ *   - a stream of another device, or not a stream, is BP4_ERR_ARG; switching while the old or
+ *     the new stream is being captured into a graph is BP4_ERR_STATE.  Nothing is queued then.
+ *   - the stream must stay valid while it is bound: until the next bp4_ctx_set_stream or
+ *     bp4_ctx_destroy.  bp4_ctx_destroy never destroys or drains it; it waits for an event
+ *     recorded there after the context's last call.
+ *   - while the bound stream is being captured into a caller's graph, asynchronous calls
+ *     (bp4_vmult, the BLAS-1 updates, ...) are captured with it; calls that synchronise, allocate
+ *     or launch a solve graph (the host-scalar calls above, bp4_vec_alloc*, bp4_vec_upload,
+ *     bp4_inverse_diagonal, the solves, bp4_ctx_synchronize, bp4_profile_*, bp4_comm_init) are
+ *     BP4_ERR_STATE before anything is queued.
+ *   - multi-rank: nothing here is rank-specific (the exchange and the all-reduce run on the bound
+ *     stream), but only one rank is tested.                                                      */
+int bp4_ctx_set_stream(bp4_ctx *ctx, void *stream);
 
 /* ---- vectors: initialize_dof_vector (poisson_operator.h:298-302), reinit/operator= ------- */
 int bp4_vec_alloc(bp4_ctx *ctx, uint64_t n, bp4_vec **v); /* zero-initialised, n doubles */
@@ -133,9 +157,10 @@ int bp4_vec_device_ptr(bp4_ctx *ctx, bp4_vec *v, double **dev);            /* cu
  *   - lifetime: the memory must stay valid until bp4_vec_free and until the context's queued work
  *     on it has run.  bp4_vec_free releases the handle only; the memory stays the caller's and
  *     never enters the context's buffer pool.
- *   - stream order is the caller's: the context reads and writes the memory on its own stream
- *     (bp4_ctx_stream).  Make that stream wait for the work that produced the data and make the
- *     consumer wait for the context's stream, e.g. with cudaEventRecord + cudaStreamWaitEvent.
+ *   - stream order is the caller's: the context reads and writes the memory on its stream
+ *     (bp4_ctx_stream).  Bind the stream that produces and consumes the data (bp4_ctx_set_stream),
+ *     or make the context's stream wait for the producer and the consumer wait for the context's
+ *     stream, e.g. with cudaEventRecord + cudaStreamWaitEvent.
  *   - device-resident solves cache their graph and three temporaries per (x, b, prec) address;
  *     bp4_vec_free of a wrapped vector drops the entries that name its memory, so wrapping a
  *     fresh x for every solve keeps one entry.                                                   */
@@ -183,9 +208,10 @@ int bp4_all_zero(bp4_ctx *ctx, const bp4_vec *v, int *result);
 /* ---- whole solves on the device ---------------------------------------------------------
  * The two CG solvers of the benchmark with the host out of the iteration loop: every scalar
  * (alpha, beta, the residual, the stopping test) is computed on the device, in the host solver's
- * arithmetic, and the loop runs as one CUDA graph with a conditional WHILE node.  Step 0 (start
- * residual g = A x - b, or -b for a zero x, its norm and the first check) runs through the entry
- * points above; then the graph runs the iterations until the stopping test ends them.
+ * arithmetic, and the whole solve runs as one CUDA graph: step 0 (start residual g = A x - b, or
+ * -b for a zero x, chosen on the device by an IF node, its norm and the first check) with the
+ * kernels of the entry points above, then a conditional WHILE node runs the iterations until the
+ * stopping test ends them.  A solve that ends at step 0 runs no iteration and leaves x untouched.
  *   - stopping test: ReductionControl::check (solver_control.h): step 0 sets
  *     reduced_tol = |g_0| * reduce; success if value < reduced_tol or value <= tol; failure if
  *     step >= max_steps or the value is NaN.  reduce = 0 is a plain SolverControl(max_steps, tol).
@@ -195,13 +221,16 @@ int bp4_all_zero(bp4_ctx *ctx, const bp4_vec *v, int *result);
  *     several ranks gives BP4_ERR_STATE.
  *   - the merged solve uses the context's in-loop / streamed form (bp4_debug_set_fused), i.e.
  *     the vector kernels of bp4_vmult_merged.
- *   - blocking: the call returns when *out is on the host.  The instantiated graph is cached in
- *     the context per (solver, x, b, prec, in-loop form) together with its temporaries g, d, h;
- *     a repeated solve re-uses it; bp4_vec_free of a wrapped x, b or prec drops the entries that
- *     name it and returns their temporaries to the context's pool.
- *   - measurement: bp4_launch_count adds one per graph launch (plus the step-0 kernels); the
- *     kernels of the graph are counted once, when it is built.  bp4_profile_* time no kernel
- *     inside the graph.                                                                      */
+ *   - bp4_solve_cg / bp4_solve_cg_merged block: they are the _async call, a synchronisation of
+ *     the stream and a copy of the result into *out.  The instantiated graph is cached in the
+ *     context per (solver, x, b, prec, in-loop form) together with its temporaries g, d, h; a
+ *     repeated solve re-uses it, whatever its max_steps, tolerances, result and history: those are
+ *     kernel parameters of the graph's first node, replaced per launch without a new graph.
+ *     bp4_vec_free of a wrapped x, b or prec drops the entries that name it and returns their
+ *     temporaries to the context's pool.
+ *   - measurement: bp4_launch_count adds one per graph launch; the kernels of the graph, step 0
+ *     included, are counted once, when it is built.  bp4_profile_* time no kernel inside the
+ *     graph.                                                                                  */
 typedef struct bp4_solve_result
 {
   int      state;         /* 1 = success, 2 = failure (SolverControl::State)   */
@@ -216,6 +245,24 @@ int bp4_solve_cg(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec
 /* SolverCGFullMerge (solver_cg_optimized.h:192-302): x every second iteration, odd/even fix-up */
 int bp4_solve_cg_merged(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
                         unsigned max_steps, double tol, double reduce, bp4_solve_result *out);
+/* The same solves, queued on the context's stream without any host synchronisation: the call
+ * returns once the graph launch is queued, and the stream writes *result when the solve ends, so
+ * that a caller can queue solve k + 1, or the work that reads x, behind solve k.
+ *   - result: device memory of the context's device or mapped pinned host memory
+ *     (cudaHostAlloc / cudaMallocHost, cudaHostRegister with cudaHostRegisterMapped), 8-byte
+ *     aligned; anything else is BP4_ERR_ARG and nothing is queued.  Read it after the stream
+ *     (or an event recorded behind the call) has completed.
+ *   - history (optional, NULL for none): the same kinds of memory, room for max_steps + 1
+ *     doubles (the ABI cannot check the size: a plain pointer carries none).  It receives the
+ *     residual norm checked at steps 0 .. last_step, the values deal.II's SolverControl records
+ *     with enable_history_data(); the entries after last_step are left untouched.
+ *   - x, b, prec and the memory behind result and history must stay valid until the solve has
+ *     run.  Several solves may be queued back to back; each keeps its own arguments.        */
+int bp4_solve_cg_async(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                       double tol, double reduce, bp4_solve_result *result, double *history);
+int bp4_solve_cg_merged_async(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
+                              unsigned max_steps, double tol, double reduce, bp4_solve_result *result,
+                              double *history);
 
 /* ---- deterministic mode -----------------------------------------------------------------
  * With bp4_desc::deterministic (or BP4_DETERMINISTIC=1) every result of bp4_vmult,

@@ -46,9 +46,11 @@ EXPORTS = [
     "bp4_comm_unique_id", "bp4_comm_init", "bp4_comm_info", "bp4_update_ghost_values", "bp4_compress_add",
     "bp4_profile_enable", "bp4_profile_reset", "bp4_profile_get", "bp4_launch_count",
     "bp4_solve_cg", "bp4_solve_cg_merged", "bp4_deterministic_info", "bp4_vec_wrap",
+    "bp4_ctx_set_stream", "bp4_solve_cg_async", "bp4_solve_cg_merged_async",
 ]
 
 SUCCESS, FAILURE = 1, 2  # SolverControl::State of a device-resident solve
+CUDA_STREAM_LEGACY = 1   # cudaStreamLegacy: the legacy default stream (a null stream means "the context's own")
 
 
 class _SolveResult(C.Structure):
@@ -78,6 +80,9 @@ def lib():
         _lib.bp4_vec_wrap.argtypes = [vp, vp, C.c_uint64, vp]
         for f in (_lib.bp4_solve_cg, _lib.bp4_solve_cg_merged):
             f.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp]
+        for f in (_lib.bp4_solve_cg_async, _lib.bp4_solve_cg_merged_async):
+            f.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp, vp]
+        _lib.bp4_ctx_set_stream.argtypes = [vp, vp]
     return _lib
 
 
@@ -166,36 +171,68 @@ class Vector:
 
 
 class _Ordered:
-    """Orders a context call on wrapped vectors with PyTorch's current stream, without a host
-    synchronisation: the context's stream waits for the work queued so far on the current stream,
-    and the current stream waits for the call.  Every wrapped tensor is then recorded on the
-    current stream, which now runs behind the call, so the caching allocator does not hand its
-    memory out while the call is queued.  (Not on the context's stream itself: the allocator
-    records an event on each recorded stream when the tensor is freed, and close() destroys that
-    stream while the tensor may live on.)  A call on owned vectors only does nothing here."""
-    __slots__ = ("ctx", "ts", "cur")
+    """Orders a context call on wrapped vectors (and the extra tensors `ts`) with PyTorch's current
+    stream, without a host synchronisation: the context's stream waits for the work queued so far
+    on the current stream, and the current stream waits for the call.  When the context runs on
+    the current stream itself (Context.use_stream) stream order does that, and no event is needed.
+    Every tensor is then recorded on the current stream, which runs behind the call, so the
+    caching allocator does not hand its memory out while the call is queued.  (Not on the
+    context's own stream: the allocator records an event on each recorded stream when the tensor
+    is freed, and close() destroys that stream while the tensor may live on.)  A call on owned
+    vectors only does nothing here."""
+    __slots__ = ("ctx", "ts", "cur", "same")
 
-    def __init__(self, ctx: "Context", vecs):
+    def __init__(self, ctx: "Context", vecs, ts=()):
         self.ctx = ctx
-        self.ts = [v.tensor for v in vecs if v is not None and v.tensor is not None]
+        self.ts = [v.tensor for v in vecs if v is not None and v.tensor is not None] + list(ts)
 
     def __enter__(self):
         if self.ts:
             import torch
             self.cur = torch.cuda.current_stream(self.ctx.device)
-            self.ctx.torch_stream().wait_stream(self.cur)
+            bound = self.ctx._bound
+            self.same = bound is not None and bound.cuda_stream == self.cur.cuda_stream
+            if not self.same:
+                self.ctx.torch_stream().wait_stream(self.cur)
 
     def __exit__(self, *exc):
         if self.ts:
-            self.cur.wait_stream(self.ctx.torch_stream())
+            if not self.same:
+                self.cur.wait_stream(self.ctx.torch_stream())
             for t in self.ts:
                 t.record_stream(self.cur)
         return False
 
 
+class SolveHandle:
+    """A device-resident solve queued by Context.solve_cg(blocking=False).  `result_tensor` (three
+    float64 on the device, one bp4_solve_result) and `history` (None, or max_steps + 1 float64:
+    the residual checked at steps 0 .. last_step, NaN after it) are written by the stream when
+    the solve ends; reading them on the stream the solve was queued on, or after result(), needs
+    no other synchronisation."""
+
+    def __init__(self, result_tensor, history, event):
+        self.result_tensor, self.history, self._event = result_tensor, history, event
+
+    def done(self) -> bool:
+        return self._event.query()
+
+    def result(self):
+        """wait for the solve; (state, last_step, last_value, initial_value) as the blocking call"""
+        import struct
+        self._event.synchronize()
+        return struct.unpack("<iIdd", self.result_tensor.cpu().numpy().tobytes())
+
+    def history_values(self):
+        """the residuals of steps 0 .. last_step as a numpy array (waits for the solve)"""
+        last = self.result()[1]
+        return self.history[:last + 1].cpu().numpy()
+
+
 class Context:
     """Device-side operator: mirrors what LaplaceOperator::initialize holds
     (poisson_operator.h:101-293)."""
+    _bound = None  # the torch.cuda.Stream bound with use_stream, None: the context's own stream
 
     def __init__(self, degree, entity_index, vertices, n_owned, n_ghost=0, constrained=None,
                  device=0, peers=None, ranges=None, partitions=None, coefficients=None,
@@ -261,6 +298,7 @@ class Context:
             lib().bp4_ctx_destroy(self.h)
         self.h = C.c_void_p()
         self._torch_stream = None
+        self._bound = None
 
     def synchronize(self):
         _chk(lib().bp4_ctx_synchronize(self.h))
@@ -270,8 +308,21 @@ class Context:
         _chk(lib().bp4_ctx_stream(self.h, C.byref(s)))
         return s.value or 0
 
+    def use_stream(self, stream):
+        """Queue every call of the context on `stream`, a torch.cuda.Stream of its device (PyTorch's
+        default stream included), or on the context's own stream again with None
+        (bp4_ctx_set_stream).  The new stream first waits, on the device, for what the context
+        queued on the old one.  While the context runs on PyTorch's current stream, calls on
+        wrapped tensors need no event pair to be ordered with torch's work."""
+        handle = None if stream is None else (stream.cuda_stream or CUDA_STREAM_LEGACY)
+        _chk(lib().bp4_ctx_set_stream(self.h, C.c_void_p(handle)))
+        self._bound = stream
+        self._torch_stream = None
+
     def torch_stream(self):
-        """the context's stream as a torch.cuda.ExternalStream"""
+        """the context's current stream as a torch.cuda stream object"""
+        if self._bound is not None:
+            return self._bound
         if getattr(self, "_torch_stream", None) is None:
             import torch
             self._torch_stream = torch.cuda.ExternalStream(self.stream(), device=torch.device("cuda", self.device))
@@ -339,16 +390,41 @@ class Context:
         with _Ordered(self, (x, d, g, prec)):
             _chk(lib().bp4_x_finalize_even(self.h, x.h, d.h, g.h, prec.h, c1, c2))
 
-    def solve_cg(self, x, b, prec, merged=True, max_steps=100, tol=1e-15, reduce=1e-8):
+    def solve_cg(self, x, b, prec, merged=True, max_steps=100, tol=1e-15, reduce=1e-8, blocking=True,
+                 history=False):
         """CG solve of A x = b with the iteration loop on the device (bp4_solve_cg_merged, or
         bp4_solve_cg with merged=False) from the start vector in x; prec holds n_owned/3 inverse
         diagonal entries.  Returns (state, last_step, last_value, initial_value); hitting
-        max_steps is state FAILURE, not an exception."""
-        r = _SolveResult()
-        f = lib().bp4_solve_cg_merged if merged else lib().bp4_solve_cg
-        with _Ordered(self, (x, b, prec)):
-            _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
-        return r.state, r.last_step, r.last_value, r.initial_value
+        max_steps is state FAILURE, not an exception.
+        blocking=False queues the solve without a host synchronisation (bp4_solve_cg*_async) and
+        returns a SolveHandle; history=True (or a float64 CUDA tensor of at least max_steps + 1
+        entries) also collects the residual of every checked step there."""
+        if blocking:
+            if history is not False:
+                raise ValueError("history needs blocking=False")
+            r = _SolveResult()
+            f = lib().bp4_solve_cg_merged if merged else lib().bp4_solve_cg
+            with _Ordered(self, (x, b, prec)):
+                _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
+            return r.state, r.last_step, r.last_value, r.initial_value
+        import torch
+        dev = torch.device("cuda", self.device)
+        res = torch.empty(3, dtype=torch.float64, device=dev)
+        hist = None
+        if history is True:
+            hist = torch.full((max_steps + 1,), float("nan"), dtype=torch.float64, device=dev)
+        elif history is not False:
+            hist = history
+            check_tensor(hist, self.device)
+            if hist.numel() < max_steps + 1:
+                raise ValueError(f"history has {hist.numel()} entries, the solve needs max_steps + 1 = {max_steps + 1}")
+        f = lib().bp4_solve_cg_merged_async if merged else lib().bp4_solve_cg_async
+        with _Ordered(self, (x, b, prec), [res] + ([hist] if hist is not None else [])):
+            _chk(f(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.c_void_p(res.data_ptr()),
+                   C.c_void_p(hist.data_ptr()) if hist is not None else None))
+            ev = torch.cuda.Event()
+            ev.record(self.torch_stream())
+        return SolveHandle(res, hist, ev)
 
     # ---- BLAS-1 -------------------------------------------------------------------
     def equ(self, dst, a, src):

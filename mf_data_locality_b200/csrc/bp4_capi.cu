@@ -128,7 +128,7 @@ struct ProfEvent
   int         id;
 };
 
-// instantiated graph of one device-resident solve (bp4_solve_cg / bp4_solve_cg_merged), keyed by
+// instantiated graph of one device-resident solve (bp4_solve_cg*, bp4_solve_cg*_async), keyed by
 // the variant, the caller's x, b and prec buffers and the in-loop form; it owns the temporaries
 // g, d, h so that their addresses, baked into the graph, stay valid.  Freeing a wrapped vector
 // drops the entries that name its buffer (drop_solves_on).
@@ -140,13 +140,17 @@ struct SolveGraph
   bp4_vec       g, d, h;
   graph_ptr     graph;
   exec_ptr      exec;
+  cudaGraphNode_t            begin = nullptr; // the solve_begin_kernel node: per-launch arguments
+  cudaGraphConditionalHandle apply = 0;       // its IF node: g = A x for a non-zero x
 };
 
-// Members are released in reverse declaration order, after ~bp4_ctx has synchronised the stream:
-// the streams are declared first so that they are released last.
+// Members are released in reverse declaration order, after ~bp4_ctx has waited for the context's
+// work: the streams are declared first so that they are released last.
 struct bp4_ctx
 {
   stream_ptr   stream, comm_stream;
+  cudaStream_t cur = nullptr; // the caller's stream (bp4_ctx_set_stream), null: the own `stream`
+  cudaStream_t st() const { return cur ? cur : stream.get(); } // where all work of the context goes
   event_ptr    ev_a, ev_b;
   int          degree = 0, device = 0, sms = 0;
   int          n_coef = 24; // geometry coefficients per cell: 24 (tri-linear) or 81 (all 27 vectors)
@@ -163,10 +167,10 @@ struct bp4_ctx
   host_ptr<double>  h_acc;       // pinned [8] + sequence word (h_acc[8] reinterpreted), device-mapped
   unsigned long long pub_seq = 0;
   host_ptr<int>      h_flag;
-  // device-resident solves: the solver state, its pinned host images ([0] initial state read by
-  // the graph, [1] final state written by it) and the cached graphs
-  dev_ptr<bp4::SolveState>  d_state;
-  host_ptr<bp4::SolveState> h_state;
+  // device-resident solves: the solver state, the pinned (device-mapped) result of the blocking
+  // calls and the cached graphs
+  dev_ptr<bp4::SolveState>   d_state;
+  host_ptr<bp4_solve_result> h_result;
   std::list<SolveGraph>     solves; // a list: erasing an entry moves no other (bp4_vec has no move assignment)
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
@@ -233,6 +237,16 @@ namespace
     return cudaStreamIsCapturing(st, &s) == cudaSuccess && s != cudaStreamCaptureStatusNone;
   }
 
+  // A call that waits on the host, allocates or builds a graph cannot run while the caller is
+  // capturing the stream into a graph of its own: refuse it before anything is queued.
+  int refuse_capture(const bp4_ctx *c, const char *call)
+  {
+    if (capturing(c->st()))
+      return fail(BP4_ERR_STATE, "%s synchronises the stream or allocates, and the stream is being captured into a "
+                                 "graph: call it before the capture begins or after it ends", call);
+    return 0;
+  }
+
   // RAII: count a launch, and time it with events when profiling is on.  While the stream is
   // being captured into a graph the launch is counted but not timed (no events inside a graph).
   struct Timed
@@ -241,7 +255,7 @@ namespace
     int      id;
     ProfEvent ev{};
     bool      on;
-    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile && !capturing(c_->stream.get()))
+    Timed(bp4_ctx *c_, int id_, int n_launches = 1) : c(c_), id(id_), on(c_->profile && !capturing(c_->st()))
     {
       c->launches += n_launches;
       c->prof_cnt[id] += 1;
@@ -256,14 +270,14 @@ namespace
                 c->event_pool.pop_back();
               }
           ev.id = id;
-          cudaEventRecord(ev.a, c->stream.get());
+          cudaEventRecord(ev.a, c->st());
         }
     }
     ~Timed()
     {
       if (on)
         {
-          cudaEventRecord(ev.b, c->stream.get());
+          cudaEventRecord(ev.b, c->st());
           c->events.push_back(ev);
         }
     }
@@ -305,7 +319,7 @@ namespace
     Timed t(c, id);
     if (n == 0)
       return 0;
-    kernel<<<stream_grid(n, c->sms), 256, 0, c->stream.get()>>>(args...);
+    kernel<<<stream_grid(n, c->sms), 256, 0, c->st()>>>(args...);
     CU(cudaGetLastError());
     return 0;
   }
@@ -316,7 +330,7 @@ namespace
   {
     if (n == 0)
       return 0;
-    kernel<<<(unsigned)((n + B - 1) / B), B, 0, c->stream.get()>>>(args...);
+    kernel<<<(unsigned)((n + B - 1) / B), B, 0, c->st()>>>(args...);
     CU(cudaGetLastError());
     return 0;
   }
@@ -336,7 +350,7 @@ namespace
     else
       CU(allocate(v.buf, n + 2)); // + 2: the fused loop copies runs in 16-byte pieces, one element past either end
     if (zero)
-      CU(cudaMemsetAsync(v.p(), 0, sizeof(double) * n, c->stream.get()));
+      CU(cudaMemsetAsync(v.p(), 0, sizeof(double) * n, c->st()));
     return 0;
   }
 
@@ -365,19 +379,19 @@ namespace
   int reduce_to_host(bp4_ctx *c, int k, double *out)
   {
     if (c->comm)
-      NC(ncclAllReduce(c->d_acc.get(), c->d_acc.get(), k, ncclDouble, ncclSum, c->comm.get(), c->stream.get()));
+      NC(ncclAllReduce(c->d_acc.get(), c->d_acc.get(), k, ncclDouble, ncclSum, c->comm.get(), c->st()));
     // the last kernel of the chain writes the values and then a sequence number into mapped
     // pinned memory; the host polls that word (and the stream, for errors, now and then)
     volatile unsigned long long *seq_word = reinterpret_cast<volatile unsigned long long *>(c->h_acc.get() + 8);
     const unsigned long long     seq      = ++c->pub_seq;
-    bp4::publish_kernel<<<1, 32, 0, c->stream.get()>>>(c->d_acc.get(), k, c->h_acc.get(), seq_word, seq);
+    bp4::publish_kernel<<<1, 32, 0, c->st()>>>(c->d_acc.get(), k, c->h_acc.get(), seq_word, seq);
     CU(cudaGetLastError());
     c->launches += 1;
     int idle = 0;
     for (unsigned long long spins = 1; *seq_word != seq; ++spins)
       if ((spins & 0xFFFF) == 0)
         {
-          const cudaError_t q = cudaStreamQuery(c->stream.get());
+          const cudaError_t q = cudaStreamQuery(c->st());
           if (q != cudaSuccess && q != cudaErrorNotReady)
             CU(q);
           if (q == cudaSuccess && ++idle > 8) // stream drained, nothing published: cannot happen
@@ -389,9 +403,13 @@ namespace
   }
 } // namespace
 
+// The caller's stream is not the context's to destroy or drain: an event recorded on it after the
+// context's last call marks where the context's work ends there.
 bp4_ctx::~bp4_ctx()
 {
   cudaSetDevice(device);
+  if (cur && ev_a && cudaEventRecord(ev_a.get(), cur) == cudaSuccess)
+    cudaEventSynchronize(ev_a.get());
   if (stream)
     cudaStreamSynchronize(stream.get());
   drain_events(this);
@@ -579,7 +597,7 @@ static int ctx_create_impl(const bp4_desc *d, bp4_ctx *c)
   memset(c->h_acc.get(), 0, sizeof(double) * 16);
   CU(allocate(c->h_flag, 1));
   CU(allocate(c->d_state, 1));
-  CU(allocate(c->h_state, 2));
+  CU(allocate(c->h_result, 1));
 
   // cell-batch ranges and their private DoF runs -> units and batches of the fused merged loop
   if (d->n_ranges > 0)
@@ -697,7 +715,9 @@ int bp4_ctx_synchronize(bp4_ctx *c)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
-  CU(cudaStreamSynchronize(c->stream.get()));
+  if (int e = refuse_capture(c, "bp4_ctx_synchronize"))
+    return e;
+  CU(cudaStreamSynchronize(c->st()));
   return 0;
 }
 
@@ -705,7 +725,40 @@ int bp4_ctx_stream(bp4_ctx *c, void **stream)
 {
   if (!c || !stream)
     return fail(BP4_ERR_ARG, "null argument");
-  *stream = (void *)c->stream.get();
+  *stream = (void *)c->st();
+  return 0;
+}
+
+// The new stream waits for everything queued so far on the old one (an event, no host wait):
+// pooled buffers, solve temporaries and the reduction scratch may still be in use there.
+int bp4_ctx_set_stream(bp4_ctx *c, void *stream)
+{
+  if (!c)
+    return fail(BP4_ERR_ARG, "null ctx");
+  CU(cudaSetDevice(c->device));
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (s)
+    {
+      int dev = -1;
+      if (cudaStreamGetDevice(s, &dev) != cudaSuccess)
+        {
+          cudaGetLastError();
+          return fail(BP4_ERR_ARG, "set_stream: %p is not a stream", stream);
+        }
+      if (dev != c->device)
+        return fail(BP4_ERR_ARG, "set_stream: stream %p belongs to device %d, the context runs on device %d", stream,
+                    dev, c->device);
+    }
+  const cudaStream_t next = s ? s : c->stream.get();
+  if (capturing(c->st()) || capturing(next))
+    return fail(BP4_ERR_STATE, "set_stream: the old or the new stream is being captured into a graph: switch "
+                               "streams outside a capture");
+  if (next != c->st())
+    {
+      CU(cudaEventRecord(c->ev_a.get(), c->st()));
+      CU(cudaStreamWaitEvent(next, c->ev_a.get(), 0));
+    }
+  c->cur = s;
   return 0;
 }
 
@@ -713,6 +766,8 @@ static int vec_alloc(bp4_ctx *c, uint64_t n, bp4_vec **out, bool zero)
 {
   if (!c || !out)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_vec_alloc"))
+    return e;
   CU(cudaSetDevice(c->device));
   std::unique_ptr<bp4_vec> v(new bp4_vec);
   if (int e = pooled_alloc(c, n, *v, zero))
@@ -793,7 +848,7 @@ int bp4_vec_set_zero(bp4_ctx *c, bp4_vec *v)
   if (!c || !v)
     return fail(BP4_ERR_ARG, "null argument");
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(v->p(), 0, sizeof(double) * v->n, c->stream.get()));
+  CU(cudaMemsetAsync(v->p(), 0, sizeof(double) * v->n, c->st()));
   return 0;
 }
 
@@ -801,11 +856,13 @@ int bp4_vec_upload(bp4_ctx *c, bp4_vec *v, const double *host, uint64_t n)
 {
   if (!c || !v || (!host && n))
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_vec_upload"))
+    return e;
   CU(cudaSetDevice(c->device));
   if (n > v->n)
     return fail(BP4_ERR_ARG, "upload of %llu > vector size %llu", (unsigned long long)n,
                 (unsigned long long)v->n);
-  CU(cudaMemcpyAsync(v->p(), host, sizeof(double) * n, cudaMemcpyHostToDevice, c->stream.get()));
+  CU(cudaMemcpyAsync(v->p(), host, sizeof(double) * n, cudaMemcpyHostToDevice, c->st()));
   return 0;
 }
 
@@ -813,12 +870,14 @@ int bp4_vec_download(bp4_ctx *c, const bp4_vec *v, double *host, uint64_t n)
 {
   if (!c || !v || (!host && n))
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_vec_download"))
+    return e;
   CU(cudaSetDevice(c->device));
   if (n > v->n)
     return fail(BP4_ERR_ARG, "download of %llu > vector size %llu", (unsigned long long)n,
                 (unsigned long long)v->n);
-  CU(cudaMemcpyAsync(host, v->p(), sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream.get()));
-  CU(cudaStreamSynchronize(c->stream.get()));
+  CU(cudaMemcpyAsync(host, v->p(), sizeof(double) * n, cudaMemcpyDeviceToHost, c->st()));
+  CU(cudaStreamSynchronize(c->st()));
   return 0;
 }
 
@@ -901,7 +960,7 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       a.scalars      = c->d_update4b.get();
       a.acc          = c->d_acc.get();
       Timed t(c, BP4_K_MERGED);
-      CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->stream.get()));
+      CU(bp4::launch_cell(c->degree, true, false, a, c->sms, c->st()));
     }
   else if (c->deterministic) // one launch per colour (single rank: part = -1), timed as one loop
     {
@@ -913,7 +972,7 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
           a.coef            = c->d_coef.get() + (uint64_t)c->n_coef * c0;
           a.n_cells         = c->color_off[k + 1] - c0;
           a.sched           = c->d_sched.get() + k;
-          CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream.get()));
+          CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->st()));
         }
     }
   else
@@ -922,7 +981,7 @@ static int cell_range(bp4_ctx *c, double *dst, const double *src, int part, cons
       a.coef         = c->d_coef.get() + (uint64_t)c->n_coef * begin;
       a.n_cells      = end - begin;
       Timed t(c, BP4_K_VMULT);
-      CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->stream.get()));
+      CU(bp4::launch_cell(c->degree, false, c->n_coef == 81, a, c->sms, c->st()));
     }
   return 0;
 }
@@ -940,7 +999,7 @@ static int compress_finish(bp4_ctx *c, double *v);
 // dst must already be zero where the cells accumulate (owned and ghost slots).
 static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCall *m)
 {
-  CU(cudaMemsetAsync(c->d_sched.get(), 0, sizeof(uint32_t) * c->n_sched, c->stream.get()));
+  CU(cudaMemsetAsync(c->d_sched.get(), 0, sizeof(uint32_t) * c->n_sched, c->st()));
   if (c->peer.empty())
     return cell_range(c, dst, src, -1, m);
   if (!c->comm)
@@ -952,7 +1011,7 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
     if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export.get(), src, c->d_sendbuf.get()))
       return e;
   }
-  CU(cudaEventRecord(c->ev_a.get(), c->stream.get()));
+  CU(cudaEventRecord(c->ev_a.get(), c->st()));
   CU(cudaStreamWaitEvent(c->comm_stream.get(), c->ev_a.get(), 0));
   if (int e = exchange_ghosts_on(c, const_cast<double *>(src), c->comm_stream.get()))
     return e;
@@ -960,7 +1019,7 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
   if (overlap)
     if (int e = cell_range(c, dst, src, 0, m))
       return e;
-  CU(cudaStreamWaitEvent(c->stream.get(), c->ev_b.get(), 0));
+  CU(cudaStreamWaitEvent(c->st(), c->ev_b.get(), 0));
   if (overlap)
     {
       if (int e = cell_range(c, dst, src, 1, m))
@@ -968,7 +1027,7 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
     }
   else if (int e = cell_range(c, dst, src, -1, m))
     return e;
-  CU(cudaEventRecord(c->ev_a.get(), c->stream.get()));
+  CU(cudaEventRecord(c->ev_a.get(), c->st()));
   CU(cudaStreamWaitEvent(c->comm_stream.get(), c->ev_a.get(), 0));
   if (int e = exchange_compress_on(c, dst, c->comm_stream.get()))
     return e;
@@ -976,14 +1035,14 @@ static int cell_loop(bp4_ctx *c, double *dst, const double *src, const MergedCal
   if (overlap)
     if (int e = cell_range(c, dst, src, 2, m))
       return e;
-  CU(cudaStreamWaitEvent(c->stream.get(), c->ev_b.get(), 0));
+  CU(cudaStreamWaitEvent(c->st(), c->ev_b.get(), 0));
   return compress_finish(c, dst);
 }
 
 // dst = A src on the context's stream (also captured into the plain device solve's loop body)
 static int vmult_on(bp4_ctx *c, double *dst, const double *src)
 {
-  CU(cudaMemsetAsync(dst, 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream.get()));
+  CU(cudaMemsetAsync(dst, 0, sizeof(double) * (c->n_owned + c->n_ghost), c->st()));
   if (int e = cell_loop(c, dst, src, nullptr))
     return e;
   Timed t(c, BP4_K_BLAS1);
@@ -1049,7 +1108,7 @@ static int merged_sweep(bp4_ctx *c, const MergedCall &m, double *h)
                     m.alpha, m.beta, m.alpha_old, m.beta_old, c->d_acc.get(), c->d_update4b.get(), m.state))
     return e;
   if (c->n_ghost)
-    CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->stream.get()));
+    CU(cudaMemsetAsync(h + n, 0, sizeof(double) * c->n_ghost, c->st()));
   if (int e = cell_loop(c, h, m.d, c->fused ? &m : nullptr))
     return e;
   if (n > tail)
@@ -1069,6 +1128,8 @@ int bp4_vmult_merged(bp4_ctx *c, bp4_vec *x, bp4_vec *g, bp4_vec *d, bp4_vec *h,
       return e;
   if (!prec || prec->n < c->n_owned / 3)
     return fail(BP4_ERR_ARG, "prec needs n_owned/3 entries");
+  if (int e = refuse_capture(c, "bp4_vmult_merged"))
+    return e;
   CU(cudaSetDevice(c->device));
   MergedCall m{x->p(), g->p(), d->p(), prec->p(), alpha, beta, alpha_old, beta_old, nullptr};
   if (int e = merged_sweep(c, m, h->p()))
@@ -1099,6 +1160,8 @@ int bp4_inverse_diagonal(bp4_ctx *c, bp4_vec *out)
 {
   if (!c || !out)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_inverse_diagonal"))
+    return e;
   CU(cudaSetDevice(c->device));
   if (out->n < c->n_owned / 3)
     return fail(BP4_ERR_ARG, "diagonal vector needs n_owned/3 entries");
@@ -1131,7 +1194,7 @@ int bp4_inverse_diagonal_vector(bp4_ctx *c, bp4_vec *out)
   if (int e = check_len(c, out, "out"))
     return e;
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(out->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->stream.get()));
+  CU(cudaMemsetAsync(out->p(), 0, sizeof(double) * (c->n_owned + c->n_ghost), c->st()));
   if (int e = assemble_diagonal(c, out->p(), 1))
     return e;
   if (!c->peer.empty())
@@ -1200,6 +1263,8 @@ int bp4_dot(bp4_ctx *c, const bp4_vec *a, const bp4_vec *b, double *result)
 {
   if (!c || !a || !b || !result)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_dot"))
+    return e;
   CU(cudaSetDevice(c->device));
   const uint64_t n = sweep_len(c, {a, b});
   if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n, a->p(),
@@ -1212,6 +1277,8 @@ int bp4_add_and_dot(bp4_ctx *c, bp4_vec *g, double a, const bp4_vec *h, const bp
 {
   if (!c || !g || !h || !w || !result)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_add_and_dot"))
+    return e;
   CU(cudaSetDevice(c->device));
   const uint64_t n = sweep_len(c, {g, h, w});
   if (int e = sweep(c, BP4_K_BLAS1, n,
@@ -1234,43 +1301,49 @@ int bp4_all_zero(bp4_ctx *c, const bp4_vec *v, int *result)
 {
   if (!c || !v || !result)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_all_zero"))
+    return e;
   CU(cudaSetDevice(c->device));
-  CU(cudaMemsetAsync(c->d_flag.get(), 0, sizeof(int), c->stream.get()));
+  CU(cudaMemsetAsync(c->d_flag.get(), 0, sizeof(int), c->st()));
   const uint64_t n = sweep_len(c, {v});
   if (int e = sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, v->p(), c->d_flag.get()))
     return e;
   if (c->comm)
-    NC(ncclAllReduce(c->d_flag.get(), c->d_flag.get(), 1, ncclInt, ncclMax, c->comm.get(), c->stream.get()));
-  CU(cudaMemcpyAsync(c->h_flag.get(), c->d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, c->stream.get()));
-  CU(cudaStreamSynchronize(c->stream.get()));
+    NC(ncclAllReduce(c->d_flag.get(), c->d_flag.get(), 1, ncclInt, ncclMax, c->comm.get(), c->st()));
+  CU(cudaMemcpyAsync(c->h_flag.get(), c->d_flag.get(), sizeof(int), cudaMemcpyDeviceToHost, c->st()));
+  CU(cudaStreamSynchronize(c->st()));
   *result = *c->h_flag ? 0 : 1;
   return 0;
 }
 
 // ---- whole solves on the device ----------------------------------------------------------
-// Capture what `launch` enqueues on the context's stream into `graph`, after the nodes `deps`;
-// `leaves` (optional) receives the nodes the next one must follow.  The capture is always ended,
-// also when a launch fails, so that the stream stays usable.
+// Capture what `launch` enqueues into `graph`, after the nodes `deps`; `leaves` (optional)
+// receives the nodes the next one must follow.  The capture runs on the context's own stream
+// whichever stream is current (a caller's stream may be the legacy default stream, which cannot be
+// captured) and is always ended, also when a launch fails, so that the stream stays usable.
 extern "C++" {
 template <typename F>
 static int capture_into(bp4_ctx *c, cudaGraph_t graph, const cudaGraphNode_t *deps, size_t n_deps, F &&launch,
                         std::vector<cudaGraphNode_t> *leaves)
 {
-  CU(cudaStreamBeginCaptureToGraph(c->stream.get(), graph, deps, nullptr, n_deps, cudaStreamCaptureModeThreadLocal));
-  int e = launch();
+  const cudaStream_t cur = c->cur, own = c->stream.get();
+  CU(cudaStreamBeginCaptureToGraph(own, graph, deps, nullptr, n_deps, cudaStreamCaptureModeThreadLocal));
+  c->cur = nullptr;
+  int e  = launch();
+  c->cur = cur;
   if (!e && leaves)
     {
       cudaStreamCaptureStatus st;
       const cudaGraphNode_t  *d = nullptr;
       size_t                  n = 0;
-      const cudaError_t       q = cudaStreamGetCaptureInfo(c->stream.get(), &st, nullptr, nullptr, &d, &n);
+      const cudaError_t       q = cudaStreamGetCaptureInfo(own, &st, nullptr, nullptr, &d, &n);
       if (q == cudaSuccess)
         leaves->assign(d, d + n);
       else
         e = fail(BP4_ERR_CUDA, "cudaStreamGetCaptureInfo: %s", cudaGetErrorString(q));
     }
   cudaGraph_t       out = nullptr;
-  const cudaError_t q   = cudaStreamEndCapture(c->stream.get(), &out);
+  const cudaError_t q   = cudaStreamEndCapture(own, &out);
   if (e)
     return e;
   CU(q);
@@ -1278,10 +1351,54 @@ static int capture_into(bp4_ctx *c, cudaGraph_t graph, const cudaGraphNode_t *de
 }
 } // extern "C++"
 
-// One CUDA graph per solve:  initial state -> prologue -> WHILE { one iteration } -> epilogue ->
-// final state to the host.  The loop body is captured from the launch code of the host-driven
-// path (vmult_on, merged_sweep); the scalar kernels keep alpha, beta, ... in c->d_state and the
-// last one of an iteration sets the loop condition.
+// a conditional node (IF or WHILE on handle h) after `deps`; *body receives the graph it runs
+static int add_conditional(cudaGraph_t graph, const std::vector<cudaGraphNode_t> &deps, cudaGraphConditionalHandle h,
+                           cudaGraphConditionalNodeType type, cudaGraphNode_t *node, cudaGraph_t *body)
+{
+  cudaGraphNodeParams cp = {};
+  cp.type                = cudaGraphNodeTypeConditional;
+  cp.conditional.handle  = h;
+  cp.conditional.type    = type;
+  cp.conditional.size    = 1;
+  CU(cudaGraphAddNode(node, graph, deps.data(), deps.size(), &cp));
+  *body = cp.conditional.phGraph_out[0];
+  return 0;
+}
+
+// the per-call arguments of a solve, as the parameters of its solve_begin_kernel node
+struct SolveArgs
+{
+  bp4::SolveState           *st;
+  const int                 *nonzero;
+  uint32_t                   max_steps;
+  double                     tol, reduce;
+  double                    *history;
+  void                      *result;
+  cudaGraphConditionalHandle apply;
+  void                      *ptr[8] = {&st, &nonzero, &max_steps, &tol, &reduce, &history, &result, &apply};
+  SolveArgs(const SolveArgs &) = delete; // ptr points into this object
+  SolveArgs(bp4::SolveState *st_, const int *nz, uint32_t ms, double t, double r, double *hi, void *re,
+            cudaGraphConditionalHandle ap)
+    : st(st_), nonzero(nz), max_steps(ms), tol(t), reduce(r), history(hi), result(re), apply(ap)
+  {}
+  cudaKernelNodeParams params()
+  {
+    cudaKernelNodeParams kp = {};
+    kp.func                 = reinterpret_cast<void *>(bp4::solve_begin_kernel);
+    kp.gridDim              = dim3(1);
+    kp.blockDim             = dim3(32);
+    kp.kernelParams         = ptr;
+    return kp;
+  }
+};
+
+// One CUDA graph per solve, every step of it on the device:
+//   x != 0?  -> solve_begin (per-call arguments) -> IF x != 0 { g = A x } -> g = g_scale g - b,
+//   |g|, check(0) -> [plain: h = P g, d = -h, gh] -> WHILE { one iteration }
+//   -> [merged: IF iterated { pending x update }] -> result to the caller.
+// The start residual and the loop body are captured from the launch code of the host-driven path
+// (bp4_all_zero, vmult_on, bp4_add / bp4_equ, bp4_dot, merged_sweep); the scalar kernels keep
+// alpha, beta, ... in c->d_state and set the loop condition.
 static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
 {
   const uint64_t n    = c->n_owned;
@@ -1293,8 +1410,14 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   cudaGraph_t    graph;
   CU(cudaGraphCreate(&graph, 0));
   sg.graph.reset(graph);
-  cudaGraphConditionalHandle loop;
-  CU(cudaGraphConditionalHandleCreate(&loop, graph, 1, cudaGraphCondAssignDefault));
+  // every handle needs its conditional node: the plain solve has no final x update, and its
+  // step-0 kernel sets `loop` twice
+  cudaGraphConditionalHandle loop, iterated;
+  CU(cudaGraphConditionalHandleCreate(&sg.apply, graph, 0, cudaGraphCondAssignDefault));
+  CU(cudaGraphConditionalHandleCreate(&loop, graph, 0, cudaGraphCondAssignDefault));
+  iterated = loop;
+  if (sg.merged)
+    CU(cudaGraphConditionalHandleCreate(&iterated, graph, 0, cudaGraphCondAssignDefault));
   std::vector<cudaGraphNode_t> leaves;
   auto jacobi_dot = [&]() { // h = P g, g.h -> acc[2]
     return sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::jacobi_dot_kernel<true> : bp4::jacobi_dot_kernel<false>,
@@ -1302,13 +1425,39 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   };
   auto scalar = [&](const int kind) -> int { // solve_scalar_kernel on one thread
     Timed t(c, BP4_K_BLAS1);
-    bp4::solve_scalar_kernel<<<1, 32, 0, c->stream.get()>>>(kind, st, acc, loop);
+    bp4::solve_scalar_kernel<<<1, 32, 0, c->st()>>>(kind, st, acc, loop);
     CU(cudaGetLastError());
     return 0;
   };
-  // initial state; plain: h = P g, d = -h, gh = g.h (SolverCG before its loop)
-  auto prologue = [&]() -> int {
-    CU(cudaMemcpyAsync(st, c->h_state.get(), sizeof(bp4::SolveState), cudaMemcpyHostToDevice, c->stream.get()));
+  auto nonzero = [&]() -> int { // bp4_all_zero without the host round trip
+    CU(cudaMemsetAsync(c->d_flag.get(), 0, sizeof(int), c->st()));
+    return sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, (const double *)x, c->d_flag.get());
+  };
+  if (int e = capture_into(c, graph, nullptr, 0, nonzero, &leaves))
+    return e;
+  SolveArgs             a(st, c->d_flag.get(), 0u, 0., 0., nullptr, nullptr, sg.apply);
+  cudaKernelNodeParams  kp = a.params();
+  CU(cudaGraphAddKernelNode(&sg.begin, graph, leaves.data(), leaves.size(), &kp));
+  c->launches += 1;
+  cudaGraphNode_t apply_node;
+  cudaGraph_t     apply_body;
+  if (int e = add_conditional(graph, {sg.begin}, sg.apply, cudaGraphCondTypeIf, &apply_node, &apply_body))
+    return e;
+  if (int e = capture_into(c, apply_body, nullptr, 0, [&]() { return vmult_on(c, g, x); }, nullptr))
+    return e;
+  // g = 1 g - b or -b (bp4_add / bp4_equ), |g|^2 (bp4_dot), check(0); plain: h = P g, d = -h,
+  // gh = g.h (SolverCG before its loop)
+  auto step0 = [&]() -> int {
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, g, 0., -1., sg.b, &st->g_scale))
+      return e;
+    if (int e = sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::dot_kernel<true> : bp4::dot_kernel<false>, n,
+                      (const double *)g, (const double *)g, acc, c->det))
+      return e;
+    {
+      Timed t(c, BP4_K_BLAS1);
+      bp4::solve_step0_kernel<<<1, 32, 0, c->st()>>>(st, acc, loop, iterated);
+      CU(cudaGetLastError());
+    }
     if (sg.merged)
       return 0;
     if (int e = jacobi_dot())
@@ -1317,15 +1466,12 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
       return e;
     return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<false>, n, d, 0., -1., h, nullptr);
   };
-  if (int e = capture_into(c, graph, nullptr, 0, prologue, &leaves))
+  if (int e = capture_into(c, graph, &apply_node, 1, step0, &leaves))
     return e;
-  cudaGraphNodeParams cp = {};
-  cp.type                = cudaGraphNodeTypeConditional;
-  cp.conditional.handle  = loop;
-  cp.conditional.type    = cudaGraphCondTypeWhile;
-  cp.conditional.size    = 1;
   cudaGraphNode_t cond;
-  CU(cudaGraphAddNode(&cond, graph, leaves.data(), leaves.size(), &cp));
+  cudaGraph_t     loop_body;
+  if (int e = add_conditional(graph, leaves, loop, cudaGraphCondTypeWhile, &cond, &loop_body))
+    return e;
   auto body = [&]() -> int {
     if (sg.merged)
       {
@@ -1352,19 +1498,29 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
       return e;
     return sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, d, 0., -1., h, &st->beta);
   };
-  if (int e = capture_into(c, cp.conditional.phGraph_out[0], nullptr, 0, body, nullptr))
+  if (int e = capture_into(c, loop_body, nullptr, 0, body, nullptr))
     return e;
-  // merged: the pending x update; both: the final state to the host
-  auto epilogue = [&]() -> int {
-    if (sg.merged)
-      if (int e = sweep(c, BP4_K_BLAS1, n,
-                        c->deterministic ? bp4::solve_final_kernel<true> : bp4::solve_final_kernel<false>, n, x, d,
-                        g, prec, st))
+  // merged: the pending x update, after at least one iteration
+  cudaGraphNode_t last = cond;
+  if (sg.merged)
+    {
+      cudaGraph_t fin_body;
+      if (int e = add_conditional(graph, {cond}, iterated, cudaGraphCondTypeIf, &last, &fin_body))
         return e;
-    CU(cudaMemcpyAsync(c->h_state.get() + 1, st, sizeof(bp4::SolveState), cudaMemcpyDeviceToHost, c->stream.get()));
+      auto fin = [&]() {
+        return sweep(c, BP4_K_BLAS1, n, c->deterministic ? bp4::solve_final_kernel<true> : bp4::solve_final_kernel<false>,
+                     n, x, d, g, prec, st);
+      };
+      if (int e = capture_into(c, fin_body, nullptr, 0, fin, nullptr))
+        return e;
+    }
+  auto result = [&]() -> int {
+    Timed t(c, BP4_K_BLAS1);
+    bp4::solve_result_kernel<<<1, 32, 0, c->st()>>>(st);
+    CU(cudaGetLastError());
     return 0;
   };
-  if (int e = capture_into(c, graph, &cond, 1, epilogue, nullptr))
+  if (int e = capture_into(c, graph, &last, 1, result, nullptr))
     return e;
   cudaGraphExec_t exec;
   CU(cudaGraphInstantiate(&exec, graph, 0));
@@ -1372,10 +1528,33 @@ static int build_solve_graph(bp4_ctx *c, SolveGraph &sg)
   return 0;
 }
 
-static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
-                        const unsigned max_steps, const double tol, const double reduce, bp4_solve_result *out)
+// p must be readable and writable by the context's kernels: device memory of its device, or
+// mapped pinned host memory (*dev receives its device address); 8-byte aligned
+static int device_visible(const bp4_ctx *c, void *p, const char *name, void **dev)
 {
-  if (!c || !out)
+  if (reinterpret_cast<uintptr_t>(p) % 8)
+    return fail(BP4_ERR_ARG, "%s: %p is not 8-byte aligned", name, p);
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess)
+    {
+      cudaGetLastError();
+      at.type = cudaMemoryTypeUnregistered;
+    }
+  if (at.type == cudaMemoryTypeDevice && at.device == c->device)
+    *dev = p;
+  else if (at.type == cudaMemoryTypeHost && at.devicePointer)
+    *dev = at.devicePointer;
+  else
+    return fail(BP4_ERR_ARG, "%s: %p is neither device memory of device %d nor mapped pinned host memory (memory "
+                             "type %d, device %d)", name, p, c->device, (int)at.type, at.device);
+  return 0;
+}
+
+static int solve_async(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
+                       const unsigned max_steps, const double tol, const double reduce, bp4_solve_result *result,
+                       double *history)
+{
+  if (!c || !result)
     return fail(BP4_ERR_ARG, "null argument");
   if (int e = check_len(c, x, "x"))
     return e;
@@ -1389,6 +1568,14 @@ static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec
     return fail(BP4_ERR_STATE, "the device solve runs on one rank: this context has a ghost-exchange plan or "
                                "a communicator over several ranks");
   CU(cudaSetDevice(c->device));
+  if (int e = refuse_capture(c, merged ? "bp4_solve_cg_merged" : "bp4_solve_cg"))
+    return e;
+  void *res_dev = nullptr, *hist_dev = nullptr;
+  if (int e = device_visible(c, result, "result", &res_dev))
+    return e;
+  if (history)
+    if (int e = device_visible(c, history, "history", &hist_dev))
+      return e;
   SolveGraph *sg = nullptr;
   for (SolveGraph &e : c->solves)
     if (e.merged == merged && e.fused == c->fused && e.x == x->p() && e.b == b->p() && e.prec == prec->p())
@@ -1403,59 +1590,57 @@ static int solve_device(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec
       c->solves.push_back(std::move(ns));
       sg = &c->solves.back();
     }
-  // step 0 on the host, with the entry points the host-driven solvers use: g = A x - b (-b for a
-  // zero start vector), |g|, ReductionControl::check(0)
-  int zero = 0;
-  if (int e = bp4_all_zero(c, x, &zero))
-    return e;
-  if (!zero)
-    {
-      if (int e = bp4_vmult(c, &sg->g, x))
-        return e;
-      if (int e = bp4_add(c, &sg->g, -1., b))
-        return e;
-    }
-  else if (int e = bp4_equ(c, &sg->g, -1., b))
-    return e;
-  double res = 0.;
-  if (int e = bp4_l2_norm(c, &sg->g, &res))
-    return e;
-  const double reduced_tol = res * reduce;
-  const int    state0      = (res < reduced_tol || res <= tol) ? 1 : ((max_steps == 0 || std::isnan(res)) ? 2 : 0);
-  *out                     = bp4_solve_result{state0, 0u, res, res};
-  if (state0 != 0)
-    return 0;
   if (!sg->exec)
     if (int e = build_solve_graph(c, *sg))
       {
         sg->graph.reset(); // a later call starts over
         return e;
       }
-  bp4::SolveState &init = *c->h_state;
-  init                  = bp4::SolveState{};
-  init.tol              = tol;
-  init.reduced_tol      = reduced_tol;
-  init.last_value       = res;
-  init.initial_value    = res;
-  init.max_steps        = max_steps;
-  CU(cudaGraphLaunch(sg->exec.get(), c->stream.get()));
+  // this launch's arguments; launches queued before keep theirs
+  SolveArgs            a(c->d_state.get(), c->d_flag.get(), max_steps, tol, reduce, static_cast<double *>(hist_dev),
+                         res_dev, sg->apply);
+  cudaKernelNodeParams kp = a.params();
+  CU(cudaGraphExecKernelNodeSetParams(sg->exec.get(), sg->begin, &kp));
+  CU(cudaGraphLaunch(sg->exec.get(), c->st()));
   c->launches += 1;
-  CU(cudaStreamSynchronize(c->stream.get()));
-  const bp4::SolveState &fin = c->h_state.get()[1];
-  *out                       = bp4_solve_result{fin.state, fin.step, fin.last_value, res};
+  return 0;
+}
+
+// the enqueued solve, then a wait for its result in the context's pinned result block
+static int solve_blocking(bp4_ctx *c, const bool merged, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec,
+                          const unsigned max_steps, const double tol, const double reduce, bp4_solve_result *out)
+{
+  if (!c || !out)
+    return fail(BP4_ERR_ARG, "null argument");
+  if (int e = solve_async(c, merged, x, b, prec, max_steps, tol, reduce, c->h_result.get(), nullptr))
+    return e;
+  CU(cudaStreamSynchronize(c->st()));
+  *out = *c->h_result;
   return 0;
 }
 
 int bp4_solve_cg(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps, double tol,
                  double reduce, bp4_solve_result *out)
 {
-  return solve_device(c, false, x, b, prec, max_steps, tol, reduce, out);
+  return solve_blocking(c, false, x, b, prec, max_steps, tol, reduce, out);
 }
 
 int bp4_solve_cg_merged(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
                         double tol, double reduce, bp4_solve_result *out)
 {
-  return solve_device(c, true, x, b, prec, max_steps, tol, reduce, out);
+  return solve_blocking(c, true, x, b, prec, max_steps, tol, reduce, out);
+}
+
+int bp4_solve_cg_async(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps, double tol,
+                       double reduce, bp4_solve_result *result, double *history)
+{
+  return solve_async(c, false, x, b, prec, max_steps, tol, reduce, result, history);
+}
+
+int bp4_solve_cg_merged_async(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                              double tol, double reduce, bp4_solve_result *result, double *history)
+{
+  return solve_async(c, true, x, b, prec, max_steps, tol, reduce, result, history);
 }
 
 // ---- multi-GPU ---------------------------------------------------------------------------
@@ -1549,8 +1734,8 @@ static int p2p_setup(bp4_ctx *c)
   dev_ptr<P2PCard> d_mine, d_all;
   CU(upload(d_mine, &mine, 1));
   CU(allocate(d_all, c->n_ranks));
-  NC(ncclAllGather(d_mine.get(), d_all.get(), sizeof(P2PCard), ncclChar, c->comm.get(), c->stream.get()));
-  CU(cudaStreamSynchronize(c->stream.get()));
+  NC(ncclAllGather(d_mine.get(), d_all.get(), sizeof(P2PCard), ncclChar, c->comm.get(), c->st()));
+  CU(cudaStreamSynchronize(c->st()));
   std::vector<P2PCard> all(c->n_ranks);
   CU(cudaMemcpy(all.data(), d_all.get(), sizeof(P2PCard) * c->n_ranks, cudaMemcpyDeviceToHost));
   bool ok = true;
@@ -1579,8 +1764,8 @@ static int p2p_setup(bp4_ctx *c)
   int          h_ok = ok ? 1 : 0;
   dev_ptr<int> d_ok;
   CU(upload(d_ok, &h_ok, 1));
-  NC(ncclAllReduce(d_ok.get(), d_ok.get(), 1, ncclInt, ncclMin, c->comm.get(), c->stream.get()));
-  CU(cudaStreamSynchronize(c->stream.get()));
+  NC(ncclAllReduce(d_ok.get(), d_ok.get(), 1, ncclInt, ncclMin, c->comm.get(), c->st()));
+  CU(cudaStreamSynchronize(c->st()));
   CU(cudaMemcpy(&h_ok, d_ok.get(), sizeof(int), cudaMemcpyDeviceToHost));
   p.on = h_ok == 1;
   return 0;
@@ -1590,6 +1775,8 @@ int bp4_comm_init(bp4_ctx *c, int rank, int n_ranks, const unsigned char id[BP4_
 {
   if (!c || !id)
     return fail(BP4_ERR_ARG, "null argument");
+  if (int e = refuse_capture(c, "bp4_comm_init"))
+    return e;
   if (c->deterministic && n_ranks > 1)
     return fail(BP4_ERR_STATE, "the deterministic mode runs on one rank");
   if (c->comm)
@@ -1728,9 +1915,9 @@ static int compress_finish(bp4_ctx *c, double *v)
   if (p.on)
     for (size_t k = 0; k < c->peer.size(); ++k)
       if (c->export_off[k + 1] > c->export_off[k])
-        DRV(p.write64((CUstream)c->stream.get(), flag_addr(p.peer_arena[k].get(), kFlagAckRev, c->rank), p.epoch_rev,
+        DRV(p.write64((CUstream)c->st(), flag_addr(p.peer_arena[k].get(), kFlagAckRev, c->rank), p.epoch_rev,
                       CU_STREAM_WRITE_VALUE_DEFAULT));
-  CU(cudaMemsetAsync(v + c->n_owned, 0, sizeof(double) * c->n_ghost, c->stream.get()));
+  CU(cudaMemsetAsync(v + c->n_owned, 0, sizeof(double) * c->n_ghost, c->st()));
   return 0;
 }
 
@@ -1750,7 +1937,7 @@ int bp4_update_ghost_values(bp4_ctx *c, bp4_vec *v)
     if (int e = per_element(c, ne, bp4::pack_kernel, ne, c->d_export.get(), v->p(), c->d_sendbuf.get()))
       return e;
   }
-  return exchange_ghosts_on(c, v->p(), c->stream.get());
+  return exchange_ghosts_on(c, v->p(), c->st());
 }
 
 // ghost contributions -> owners, added (compress(VectorOperation::add)); ghost slots are zeroed
@@ -1763,7 +1950,7 @@ int bp4_compress_add(bp4_ctx *c, bp4_vec *v)
     return 0;
   if (!c->comm)
     return fail(BP4_ERR_STATE, "ghost exchange not initialised (bp4_comm_init)");
-  if (int e = exchange_compress_on(c, v->p(), c->stream.get()))
+  if (int e = exchange_compress_on(c, v->p(), c->st()))
     return e;
   return compress_finish(c, v->p());
 }
@@ -1787,6 +1974,8 @@ int bp4_profile_enable(bp4_ctx *c, int on)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
+  if (int e = refuse_capture(c, "bp4_profile_enable"))
+    return e;
   if (!on)
     CU(drain_events(c));
   c->profile = on != 0;
@@ -1797,6 +1986,8 @@ int bp4_profile_reset(bp4_ctx *c)
 {
   if (!c)
     return fail(BP4_ERR_ARG, "null ctx");
+  if (int e = refuse_capture(c, "bp4_profile_reset"))
+    return e;
   CU(drain_events(c));
   for (int i = 0; i < BP4_K_COUNT; ++i)
     {
@@ -1811,6 +2002,8 @@ int bp4_profile_get(bp4_ctx *c, int id, double *total_ms, uint64_t *launches)
 {
   if (!c || id < 0 || id >= BP4_K_COUNT)
     return fail(BP4_ERR_ARG, "bad kernel id");
+  if (int e = refuse_capture(c, "bp4_profile_get"))
+    return e;
   CU(drain_events(c));
   if (total_ms)
     *total_ms = c->prof_ms[id];

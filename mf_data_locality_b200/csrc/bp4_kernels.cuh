@@ -191,6 +191,12 @@ namespace bp4
     double   last_value, initial_value;
     uint32_t max_steps, step;        // step = last checked step
     int32_t  state, pad;             // SolverControl::State: 0 iterate, 1 success, 2 failure
+    // set per launch by solve_begin_kernel: ReductionControl's factor, 1 (x != 0: g = A x - b) or
+    // 0 (g = -b), where the residual of every checked step goes (optional) and where the
+    // bp4_solve_result goes when the solve ends
+    double   reduce, g_scale;
+    double  *history;
+    void    *result;
   };
 
   // the seven merged sums of do_cg_update3b (solver_cg_optimized.h:37-44) for one entry

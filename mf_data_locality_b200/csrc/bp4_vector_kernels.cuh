@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/bp4.h"
 #include "bp4_kernels.cuh"
 
 namespace bp4
@@ -392,11 +393,67 @@ namespace bp4
     accumulate<DET>(s, acc, ds);
   }
 
-  // ReductionControl::check (host/solver_control.h) for a step > 0
+  // Step 0 of a device-resident solve, first node of its graph.  The per-call arguments are this
+  // kernel's parameters, replaced per launch in the instantiated graph (cudaGraphExecKernelNodeSetParams),
+  // so that solves queued back to back share no host buffer.  Starts a fresh solver state and
+  // reads the flag nonzero_kernel left: x != 0 runs the IF node `apply` (g = A x) and makes the
+  // sadd_kernel<true> that follows g = 1 g - b, x == 0 skips it and makes that sadd g = -b
+  // (bp4_add / bp4_equ of the host-driven solvers).
+  __global__ void solve_begin_kernel(SolveState *stp, const int *nonzero, const uint32_t max_steps, const double tol,
+                                     const double reduce, double *history, void *result,
+                                     const cudaGraphConditionalHandle apply)
+  {
+    if (threadIdx.x != 0)
+      return;
+    SolveState st{};
+    st.max_steps = max_steps;
+    st.tol       = tol;
+    st.reduce    = reduce;
+    st.history   = history;
+    st.result    = result;
+    st.g_scale   = *nonzero ? 1. : 0.;
+    *stp         = st;
+    cudaGraphSetConditional(apply, *nonzero ? 1u : 0u);
+  }
+
+  // ReductionControl::check(0, |g|) from g.g in acc[0] (sqrt rounded as std::sqrt rounds it):
+  // reduced_tol = |g| reduce; success below either tolerance, failure for max_steps = 0 or NaN.
+  // `loop` (the WHILE node) and `iterated` (the IF node of the final x update) stay 0 when the
+  // solve ends here, so that x is not touched.
+  __global__ void solve_step0_kernel(SolveState *stp, double *acc, const cudaGraphConditionalHandle loop,
+                                     const cudaGraphConditionalHandle iterated)
+  {
+    if (threadIdx.x != 0)
+      return;
+    SolveState  &st  = *stp;
+    const double res = __dsqrt_rn(acc[0]);
+    acc[0]           = 0.;
+    st.reduced_tol   = __dmul_rn(res, st.reduce);
+    st.initial_value = st.last_value = res;
+    st.step                          = 0;
+    if (st.history)
+      st.history[0] = res;
+    st.state = (res < st.reduced_tol || res <= st.tol) ? 1 : ((st.max_steps == 0 || isnan(res)) ? 2 : 0);
+    cudaGraphSetConditional(loop, st.state == 0 ? 1u : 0u);
+    cudaGraphSetConditional(iterated, st.state == 0 ? 1u : 0u);
+  }
+
+  // last node of a device-resident solve: the outcome to the caller's bp4_solve_result
+  __global__ void solve_result_kernel(const SolveState *st)
+  {
+    if (threadIdx.x == 0)
+      *static_cast<bp4_solve_result *>(st->result) =
+        bp4_solve_result{st->state, st->step, st->last_value, st->initial_value};
+  }
+
+  // ReductionControl::check (host/solver_control.h) for a step > 0; the value also goes to the
+  // caller's history
   __device__ int control_check(SolveState &st, const uint32_t step, const double value)
   {
     st.step       = step;
     st.last_value = value;
+    if (st.history)
+      st.history[step] = value;
     if (value < st.reduced_tol || value <= st.tol)
       return 1;
     if (step >= st.max_steps || isnan(value))

@@ -150,6 +150,15 @@ class Problem:
         self._chk(self.l.bp4h_run_cg_solver(self.h, _p(b), _p(x), C.byref(it)))
         return x, it.value
 
+    def solver_history(self):
+        """the residual norms the last run_cg_solver checked at steps 0 .. last_step (the
+        plugin's ReductionControl with its history data enabled)"""
+        n = C.c_uint()
+        self._chk(self.l.bp4h_solver_history(None, C.byref(n)))
+        out = np.empty(n.value)
+        self._chk(self.l.bp4h_solver_history(_p(out), C.byref(n)))
+        return out
+
     def vmult(self, src=None, want_dst=True):
         if src is not None:
             src = np.ascontiguousarray(src, dtype=np.float64)

@@ -16,6 +16,7 @@
 #include <iomanip>
 #include <iostream>
 #include <memory>
+#include <vector>
 
 #include "curved_manifold.h"
 #include "device_vector.h"
@@ -52,6 +53,13 @@ inline SolverSettings &solver_settings()
   return s;
 }
 
+// the residuals the last solve checked, step by step (bp4h_solver_history)
+inline std::vector<double> &last_solve_history()
+{
+  static std::vector<double> h;
+  return h;
+}
+
 // shared body of the two plugins: build the solver on the benchmark's stopping rule, solve, and
 // report the iteration count -- hitting the iteration cap is a normal outcome here, not an error
 // (the reference swallows NoConvergence the same way, bench.cc:19-24)
@@ -60,6 +68,7 @@ unsigned int solve_and_count(const Operator &A, VectorType &x, const VectorType 
 {
   const SolverSettings &st = solver_settings();
   ReductionControl      control(st.max_steps, st.abs_tol, st.rel_tol);
+  control.enable_history_data();
   SolverType            solver(control);
   try
     {
@@ -67,6 +76,7 @@ unsigned int solve_and_count(const Operator &A, VectorType &x, const VectorType 
     }
   catch (const SolverControl::NoConvergence &)
     {}
+  last_solve_history() = control.get_history_data();
   return control.last_step();
 }
 

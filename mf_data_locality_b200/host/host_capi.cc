@@ -266,6 +266,17 @@ int bp4h_run_cg_solver(void *h, const double *b_host, double *x_host, unsigned i
   });
 }
 
+// the residuals the last bp4h_run_cg_solver checked, steps 0 .. last_step: *n = their number;
+// out (may be null) receives them
+int bp4h_solver_history(double *out, unsigned int *n)
+{
+  const std::vector<double> &hist = last_solve_history();
+  *n                              = (unsigned int)hist.size();
+  if (out)
+    std::copy(hist.begin(), hist.end(), out);
+  return 0;
+}
+
 int bp4h_vmult(void *h, const double *src_host, double *dst_host)
 {
   return guarded([&] {

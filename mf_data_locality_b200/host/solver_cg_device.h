@@ -1,7 +1,10 @@
 // solver_cg_device.h -- SolverCG and SolverCGFullMerge with the whole iteration loop on the
-// device (bp4_solve_cg / bp4_solve_cg_merged): same constructor and solve() as the host-driven
+// device (bp4_solve_cg_async / bp4_solve_cg_merged_async): same constructor and solve() as the host-driven
 // classes, same algorithm and stopping test, but no host round trip per iteration.  One rank only.
 #pragma once
+#include <cstring>
+#include <vector>
+
 #include "device_vector.h"
 #include "solver_control.h"
 
@@ -20,16 +23,32 @@ namespace dealii
       // a plain SolverControl is a ReductionControl that never reduces
       const auto      *rc     = dynamic_cast<const ReductionControl *>(&control);
       const double     reduce = rc ? rc->reduction() : 0.;
-      bp4_solve_result r{};
-      bp4_check((merged ? bp4_solve_cg_merged : bp4_solve_cg)(x.context(), x.handle(), b.handle(),
-                                                               preconditioner.get_vector().handle(),
-                                                               control.max_steps(), control.tolerance(),
-                                                               reduce, &r));
-      // replay the checks so that last_step(), last_value() and last_check() read as the
-      // host-driven solver leaves them
-      SolverControl::State conv = control.check(0, r.initial_value);
-      if (r.last_step > 0)
-        conv = control.check(r.last_step, r.last_value);
+      // queued on the context's stream with the residual of every checked step; the result and
+      // the history share one vector [bp4_solve_result (3 doubles) | history (max_steps + 1)],
+      // read back with one download
+      static_assert(sizeof(bp4_solve_result) == 3 * sizeof(double), "result = three doubles");
+      bp4_ctx       *ctx = x.context();
+      const unsigned max_steps = control.max_steps();
+      std::vector<double> out(3 + max_steps + 1);
+      bp4_vec       *buf = nullptr;
+      double        *dev = nullptr;
+      bp4_check(bp4_vec_alloc_uninitialized(ctx, out.size(), &buf));
+      int err = bp4_vec_device_ptr(ctx, buf, &dev);
+      if (!err)
+        err = (merged ? bp4_solve_cg_merged_async : bp4_solve_cg_async)(
+          ctx, x.handle(), b.handle(), preconditioner.get_vector().handle(), max_steps, control.tolerance(), reduce,
+          reinterpret_cast<bp4_solve_result *>(dev), dev + 3);
+      if (!err)
+        err = bp4_vec_download(ctx, buf, out.data(), out.size());
+      bp4_vec_free(ctx, buf);
+      bp4_check(err);
+      bp4_solve_result r;
+      std::memcpy(&r, out.data(), sizeof(r));
+      // replay every check, so that last_step(), last_value(), last_check() and the history data
+      // read as the host-driven solver leaves them
+      SolverControl::State conv = SolverControl::iterate;
+      for (unsigned int k = 0; k <= r.last_step; ++k)
+        conv = control.check(k, out[3 + k]);
       if (conv != SolverControl::success)
         throw SolverControl::NoConvergence(r.last_step, r.last_value);
     }

@@ -6,6 +6,7 @@
 #include <cmath>
 #include <limits>
 #include <stdexcept>
+#include <vector>
 
 namespace dealii
 {
@@ -27,6 +28,8 @@ namespace dealii
         initial_val = check_value;
       lstep  = step;
       lvalue = check_value;
+      if (history_data_enabled)
+        history_data.push_back(check_value);
       if (check_value <= tol)
         return lcheck = success;
       if (step >= maxsteps || std::isnan(check_value))
@@ -39,8 +42,13 @@ namespace dealii
     State        last_check() const { return lcheck; }
     unsigned int max_steps() const { return maxsteps; }
     double       tolerance() const { return tol; }
+    // every checked value, in check order (deal.II's enable_history_data / get_history_data)
+    void                       enable_history_data() { history_data_enabled = true; }
+    const std::vector<double> &get_history_data() const { return history_data; }
 
   protected:
+    bool                history_data_enabled = false;
+    std::vector<double> history_data;
     unsigned int maxsteps;
     double       tol, lvalue = 0, initial_val = 0;
     unsigned int lstep  = 0;
@@ -66,6 +74,8 @@ namespace dealii
         {
           lstep  = step;
           lvalue = check_value;
+          if (history_data_enabled)
+            history_data.push_back(check_value);
           return lcheck = success;
         }
       return SolverControl::check(step, check_value);
