@@ -264,6 +264,44 @@ int bp4_solve_cg_merged_async(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const 
                               unsigned max_steps, double tol, double reduce, bp4_solve_result *result,
                               double *history);
 
+/* ---- mixed-precision solve --------------------------------------------------------------
+ * CG to an FP64-accurate answer with most of the operator work in FP32 (DESIGN.md 4.7): iterative
+ * refinement whose outer loop computes the true residual b - A x with the FP64 operator and tests
+ * it, and whose inner loop solves for the correction with merged CG (SolverCGFullMerge's
+ * recurrences, streamed form) on an FP32 cell kernel and FP32 vectors.  One CUDA graph, one rank.
+ *   - stopping test: tol, reduce and the NaN rule are ReductionControl::check on the FP64 true
+ *     residual |b - A x|; initial_value is that residual at the given x (step 0), last_value the
+ *     one at the last refinement step.
+ *   - max_steps caps the total number of inner FP32 iterations over all refinement steps.
+ *   - every refinement step starts the inner solve from zero on the residual scaled to norm 1 and
+ *     stops it at a fixed relative reduction (1e-3, chosen by measurement: DESIGN.md 4.7) or when the
+ *     remaining step budget runs out; x += the correction scaled back.
+ *   - history (optional): room for max_steps + 1 doubles; it receives the FP64 true residual of
+ *     every refinement step 0 .. refinements.
+ *   - state 1: success.  state 2 when the step budget is used up, when a refinement step does not
+ *     reduce the true residual (stagnation: FP32 cannot resolve a smaller correction) or when the
+ *     residual is NaN; x then holds the last iterate.  A solve that ends at step 0 (a zero right-
+ *     hand side, an x that already passes, max_steps = 0) leaves x untouched.
+ *   - refused like the solves above: BP4_ERR_STATE on a context with a ghost-exchange plan or a
+ *     communicator over several ranks, BP4_ERR_ARG for result / history memory the device cannot
+ *     use; also BP4_ERR_STATE in the deterministic mode (FP32 ordered reductions are not built).
+ *   - the graph is cached per (x, b, prec) with its temporaries: an FP64 A x and the FP32 residual,
+ *     direction, product, correction and preconditioner (4.33 floats per DoF); bp4_vec_free of a
+ *     wrapped x, b or prec drops it.  The _async form queues the solve like bp4_solve_cg_async;
+ *     bp4_solve_cg_mixed is the async call, a synchronisation and a copy into *out.            */
+typedef struct bp4_mixed_result
+{
+  int      state;         /* 1 = success, 2 = failure                                  */
+  unsigned refinements;   /* last refinement step checked                              */
+  unsigned inner_steps;   /* FP32 iterations over all refinement steps                 */
+  double   last_value;    /* FP64 true residual at the last refinement step            */
+  double   initial_value; /* FP64 true residual at step 0                              */
+} bp4_mixed_result;
+int bp4_solve_cg_mixed_async(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                             double tol, double reduce, bp4_mixed_result *result, double *history);
+int bp4_solve_cg_mixed(bp4_ctx *ctx, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                       double tol, double reduce, bp4_mixed_result *out);
+
 /* ---- deterministic mode -----------------------------------------------------------------
  * With bp4_desc::deterministic (or BP4_DETERMINISTIC=1) every result of bp4_vmult,
  * bp4_vmult_merged (vector and sums), bp4_inverse_diagonal / _vector, bp4_dot, bp4_add_and_dot,
@@ -305,6 +343,10 @@ int bp4_compress_add(bp4_ctx *ctx, bp4_vec *v);          /* ghost contributions 
  * variable BP4_FUSED=0/1 or this call pin it.  Same sums up to summation order.             */
 int bp4_debug_set_fused(bp4_ctx *ctx, int on);
 int bp4_fused_info(bp4_ctx *ctx, int *fused, uint64_t *n_private, uint64_t *n_units);
+/* dst = A src with the FP32 cell kernel of the mixed solve: src rounded to float, the result
+ * widened to double; constrained rows are the identity as in bp4_vmult.  One rank, not in the
+ * deterministic mode (BP4_ERR_STATE).                                                        */
+int bp4_debug_vmult_f32(bp4_ctx *ctx, bp4_vec *dst, const bp4_vec *src);
 typedef enum bp4_kernel_id
 {
   BP4_K_VMULT  = 0, /* cell kernel, plain                                   */

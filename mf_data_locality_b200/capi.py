@@ -47,6 +47,7 @@ EXPORTS = [
     "bp4_profile_enable", "bp4_profile_reset", "bp4_profile_get", "bp4_launch_count",
     "bp4_solve_cg", "bp4_solve_cg_merged", "bp4_deterministic_info", "bp4_vec_wrap",
     "bp4_ctx_set_stream", "bp4_solve_cg_async", "bp4_solve_cg_merged_async",
+    "bp4_solve_cg_mixed", "bp4_solve_cg_mixed_async", "bp4_debug_vmult_f32",
 ]
 
 SUCCESS, FAILURE = 1, 2  # SolverControl::State of a device-resident solve
@@ -56,6 +57,11 @@ CUDA_STREAM_LEGACY = 1   # cudaStreamLegacy: the legacy default stream (a null s
 class _SolveResult(C.Structure):
     _fields_ = [("state", C.c_int), ("last_step", C.c_uint), ("last_value", C.c_double),
                 ("initial_value", C.c_double)]
+
+
+class _MixedResult(C.Structure):
+    _fields_ = [("state", C.c_int), ("refinements", C.c_uint), ("inner_steps", C.c_uint),
+                ("last_value", C.c_double), ("initial_value", C.c_double)]
 
 
 def lib():
@@ -83,6 +89,9 @@ def lib():
         for f in (_lib.bp4_solve_cg_async, _lib.bp4_solve_cg_merged_async):
             f.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp, vp]
         _lib.bp4_ctx_set_stream.argtypes = [vp, vp]
+        _lib.bp4_solve_cg_mixed.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp]
+        _lib.bp4_solve_cg_mixed_async.argtypes = [vp, vp, vp, vp, C.c_uint, d, d, vp, vp]
+        _lib.bp4_debug_vmult_f32.argtypes = [vp, vp, vp]
     return _lib
 
 
@@ -229,6 +238,18 @@ class SolveHandle:
         return self.history[:last + 1].cpu().numpy()
 
 
+class MixedSolveHandle(SolveHandle):
+    """A mixed-precision solve queued by Context.solve_cg_mixed(blocking=False): `result_tensor`
+    (four float64 on the device) holds one bp4_mixed_result, `history` the FP64 true residual of
+    refinement steps 0 .. refinements."""
+
+    def result(self):
+        """wait for the solve; (state, refinements, inner_steps, last_value, initial_value)"""
+        import struct
+        self._event.synchronize()
+        return struct.unpack("<iII4xdd", self.result_tensor.cpu().numpy().tobytes())
+
+
 class Context:
     """Device-side operator: mirrors what LaplaceOperator::initialize holds
     (poisson_operator.h:101-293)."""
@@ -355,6 +376,12 @@ class Context:
                                         beta_old, out))
         return np.array(out[:])
 
+    def vmult_f32(self, dst: Vector, src: Vector):
+        """developer hook: dst = A src with the FP32 cell kernel (src rounded to float, the result
+        widened; bp4_debug_vmult_f32)"""
+        with _Ordered(self, (dst, src)):
+            _chk(lib().bp4_debug_vmult_f32(self.h, dst.h, src.h))
+
     def set_fused(self, on: bool):
         """developer hook: in-loop vector updates on (default with range tables) / off"""
         _chk(lib().bp4_debug_set_fused(self.h, C.c_int(1 if on else 0)))
@@ -425,6 +452,39 @@ class Context:
             ev = torch.cuda.Event()
             ev.record(self.torch_stream())
         return SolveHandle(res, hist, ev)
+
+    def solve_cg_mixed(self, x, b, prec, max_steps=1000, tol=1e-15, reduce=1e-8, blocking=True,
+                       history=False):
+        """Mixed-precision CG (bp4_solve_cg_mixed): FP64 refinement steps around an inner FP32
+        merged CG, stopped by ReductionControl(max_steps, tol, reduce) on the FP64 true residual;
+        max_steps caps the inner FP32 iterations.  Returns (state, refinements, inner_steps,
+        last_value, initial_value).  blocking=False and history as in solve_cg; the history holds
+        the true residual of refinement steps 0 .. refinements."""
+        if blocking:
+            if history is not False:
+                raise ValueError("history needs blocking=False")
+            r = _MixedResult()
+            with _Ordered(self, (x, b, prec)):
+                _chk(lib().bp4_solve_cg_mixed(self.h, x.h, b.h, prec.h, max_steps, tol, reduce, C.byref(r)))
+            return r.state, r.refinements, r.inner_steps, r.last_value, r.initial_value
+        import torch
+        dev = torch.device("cuda", self.device)
+        res = torch.empty(4, dtype=torch.float64, device=dev)
+        hist = None
+        if history is True:
+            hist = torch.full((max_steps + 1,), float("nan"), dtype=torch.float64, device=dev)
+        elif history is not False:
+            hist = history
+            check_tensor(hist, self.device)
+            if hist.numel() < max_steps + 1:
+                raise ValueError(f"history has {hist.numel()} entries, the solve needs max_steps + 1 = {max_steps + 1}")
+        with _Ordered(self, (x, b, prec), [res] + ([hist] if hist is not None else [])):
+            _chk(lib().bp4_solve_cg_mixed_async(self.h, x.h, b.h, prec.h, max_steps, tol, reduce,
+                                                C.c_void_p(res.data_ptr()),
+                                                C.c_void_p(hist.data_ptr()) if hist is not None else None))
+            ev = torch.cuda.Event()
+            ev.record(self.torch_stream())
+        return MixedSolveHandle(res, hist, ev)
 
     # ---- BLAS-1 -------------------------------------------------------------------
     def equ(self, dst, a, src):

@@ -144,6 +144,20 @@ struct SolveGraph
   cudaGraphConditionalHandle apply = 0;       // its IF node: g = A x for a non-zero x
 };
 
+// instantiated graph of one mixed-precision solve (bp4_solve_cg_mixed*), keyed by x, b and prec like
+// SolveGraph; it owns the FP64 temporary g (= A x, then A x - b) and the FP32 residual, direction,
+// product, correction and preconditioner of the inner solve
+struct MixedGraph
+{
+  const double  *x = nullptr, *b = nullptr, *prec = nullptr;
+  bp4_vec        g;
+  dev_ptr<float> r32, d32, h32, e32, prec32;
+  graph_ptr      graph;
+  exec_ptr       exec;
+  cudaGraphNode_t            begin = nullptr; // the mixed_begin_kernel node: per-launch arguments
+  cudaGraphConditionalHandle apply = 0;       // its IF node: g = A x for a non-zero x
+};
+
 // Members are released in reverse declaration order, after ~bp4_ctx has waited for the context's
 // work: the streams are declared first so that they are released last.
 struct bp4_ctx
@@ -172,6 +186,12 @@ struct bp4_ctx
   dev_ptr<bp4::SolveState>   d_state;
   host_ptr<bp4_solve_result> h_result;
   std::list<SolveGraph>     solves; // a list: erasing an entry moves no other (bp4_vec has no move assignment)
+  // mixed-precision solves (allocated on first use): the float copy of the geometry coefficients
+  // for the FP32 cell kernel, the solver state, the pinned result of the blocking call, the graphs
+  dev_ptr<float>             d_coef32;
+  dev_ptr<bp4::MixedState>   d_mixed;
+  host_ptr<bp4_mixed_result> h_mixed;
+  std::list<MixedGraph>      mixed;
   // fused merged loop (vmult_with_merged_sums): units of whole cell-batch ranges, their batches
   // and the private DoF runs the vector updates are hooked to (bp4_kernels.cuh, BatchDesc)
   int             fused      = 0;      // 1: do_cg_update4b/3b on private DoFs inside the cell kernel
@@ -817,6 +837,14 @@ static void drop_solves_on(bp4_ctx *c, const double *buf)
       }
     else
       ++it;
+  for (auto it = c->mixed.begin(); it != c->mixed.end();)
+    if (it->x == buf || it->b == buf || it->prec == buf)
+      {
+        recycle(c, it->g);
+        it = c->mixed.erase(it);
+      }
+    else
+      ++it;
 }
 
 int bp4_vec_free(bp4_ctx *c, bp4_vec *v)
@@ -1046,7 +1074,8 @@ static int vmult_on(bp4_ctx *c, double *dst, const double *src)
   if (int e = cell_loop(c, dst, src, nullptr))
     return e;
   Timed t(c, BP4_K_BLAS1);
-  return per_element(c, c->n_constrained, bp4::fixup_kernel, c->n_constrained, c->d_constrained.get(), dst, src);
+  return per_element(c, c->n_constrained, bp4::fixup_kernel<double>, c->n_constrained, c->d_constrained.get(), dst,
+                     src);
 }
 
 int bp4_vmult(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
@@ -1641,6 +1670,321 @@ int bp4_solve_cg_merged_async(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp
                               double tol, double reduce, bp4_solve_result *result, double *history)
 {
   return solve_async(c, true, x, b, prec, max_steps, tol, reduce, result, history);
+}
+
+// ---- mixed-precision solve ---------------------------------------------------------------
+// The FP32 paths run on one rank outside the deterministic mode (no ghost exchange of float
+// vectors, no ordered FP32 reductions)
+static int refuse_f32(const bp4_ctx *c, const char *call)
+{
+  if (!c->peer.empty() || c->n_ranks > 1)
+    return fail(BP4_ERR_STATE, "%s runs on one rank: this context has a ghost-exchange plan or a communicator over "
+                               "several ranks", call);
+  if (c->deterministic)
+    return fail(BP4_ERR_STATE, "%s: the deterministic mode has no FP32 path (its ordered reductions are FP64 only)",
+                call);
+  return 0;
+}
+
+// the float copy of the geometry coefficients, made on first use
+static int ensure_coef32(bp4_ctx *c)
+{
+  if (c->d_coef32)
+    return 0;
+  const uint64_t n = (uint64_t)c->n_coef * std::max<uint64_t>(c->n_cells, 1);
+  CU(allocate(c->d_coef32, n));
+  return sweep(c, BP4_K_BLAS1, n, bp4::narrow_kernel, n, (const double *)c->d_coef.get(), c->d_coef32.get());
+}
+
+// dst += sum_cells A_cell src with the FP32 cell kernel, all cells (one rank)
+static int cell_loop_f32(bp4_ctx *c, float *dst, const float *src)
+{
+  CU(cudaMemsetAsync(c->d_sched.get(), 0, sizeof(uint32_t) * c->n_sched, c->st()));
+  if (c->n_cells == 0)
+    return 0;
+  bp4::CellArgsT<float> a{};
+  a.entity_index = c->d_entity.get();
+  a.coef         = c->d_coef32.get();
+  a.dtab         = c->d_walk.get();
+  a.n_cells      = c->n_cells;
+  a.src          = src;
+  a.dst          = dst;
+  a.sched        = c->d_sched.get();
+  Timed t(c, BP4_K_VMULT);
+  CU(bp4::launch_cell_f32(c->degree, c->n_coef == 81, a, c->sms, c->st()));
+  return 0;
+}
+
+int bp4_debug_vmult_f32(bp4_ctx *c, bp4_vec *dst, const bp4_vec *src)
+{
+  if (!c)
+    return fail(BP4_ERR_ARG, "null ctx");
+  if (int e = check_len(c, dst, "dst"))
+    return e;
+  if (int e = check_len(c, src, "src"))
+    return e;
+  if (dst == src)
+    return fail(BP4_ERR_ARG, "vmult: dst aliases src");
+  if (int e = refuse_f32(c, "bp4_debug_vmult_f32"))
+    return e;
+  if (int e = refuse_capture(c, "bp4_debug_vmult_f32"))
+    return e;
+  CU(cudaSetDevice(c->device));
+  if (int e = ensure_coef32(c))
+    return e;
+  const uint64_t n = c->n_owned + c->n_ghost;
+  dev_ptr<float> s32, d32;
+  CU(allocate(s32, n));
+  CU(allocate(d32, n));
+  if (int e = sweep(c, BP4_K_BLAS1, n, bp4::narrow_kernel, n, (const double *)src->p(), s32.get()))
+    return e;
+  CU(cudaMemsetAsync(d32.get(), 0, sizeof(float) * n, c->st()));
+  if (int e = cell_loop_f32(c, d32.get(), s32.get()))
+    return e;
+  {
+    Timed t(c, BP4_K_BLAS1);
+    if (int e = per_element(c, c->n_constrained, bp4::fixup_kernel<float>, c->n_constrained, c->d_constrained.get(),
+                            d32.get(), (const float *)s32.get()))
+      return e;
+  }
+  if (int e = sweep(c, BP4_K_BLAS1, n, bp4::widen_kernel, n, (const float *)d32.get(), dst->p()))
+    return e;
+  CU(cudaStreamSynchronize(c->st())); // the float temporaries are freed on return
+  return 0;
+}
+
+// the per-call arguments of a mixed solve, as the parameters of its mixed_begin_kernel node
+struct MixedArgs
+{
+  bp4::MixedState           *st;
+  const int                 *nonzero;
+  uint32_t                   max_steps;
+  double                     tol, reduce;
+  double                    *history;
+  void                      *result;
+  cudaGraphConditionalHandle apply;
+  void                      *ptr[8] = {&st, &nonzero, &max_steps, &tol, &reduce, &history, &result, &apply};
+  MixedArgs(const MixedArgs &) = delete; // ptr points into this object
+  MixedArgs(bp4::MixedState *st_, const int *nz, uint32_t ms, double t, double r, double *hi, void *re,
+            cudaGraphConditionalHandle ap)
+    : st(st_), nonzero(nz), max_steps(ms), tol(t), reduce(r), history(hi), result(re), apply(ap)
+  {}
+  cudaKernelNodeParams params()
+  {
+    cudaKernelNodeParams kp = {};
+    kp.func                 = reinterpret_cast<void *>(bp4::mixed_begin_kernel);
+    kp.gridDim              = dim3(1);
+    kp.blockDim             = dim3(32);
+    kp.kernelParams         = ptr;
+    return kp;
+  }
+};
+
+// One CUDA graph per mixed solve (conditional nodes nest: CUDA 12.4 and later allow conditional
+// nodes in conditional bodies, and every handle is created on the top-level graph, the graph "or one
+// of its children" that holds its node):
+//   x != 0? -> mixed_begin -> IF apply { g = A x } -> prec32 = (float) prec
+//   -> WHILE loop { g = g_scale g - b, |g|, check
+//                   IF go { r32 = s g, e = 0, WHILE inner { FP32 merged iteration }, final e update,
+//                           x += e / s, g = A x } }
+//   -> result to the caller.
+// The FP64 pieces are the kernels of the device-resident solves; the inner iteration is merged_sweep's
+// streamed form on float vectors with the FP32 cell kernel, driven by solve_scalar_kernel on ms.inner.
+static int build_mixed_graph(bp4_ctx *c, MixedGraph &mg)
+{
+  const uint64_t   n   = c->n_owned, nl = c->n_owned + c->n_ghost;
+  double          *x   = const_cast<double *>(mg.x), *g = mg.g.p();
+  bp4::MixedState *ms  = c->d_mixed.get();
+  double          *acc = c->d_acc.get();
+  float *r32 = mg.r32.get(), *d32 = mg.d32.get(), *h32 = mg.h32.get(), *e32 = mg.e32.get(), *p32 = mg.prec32.get();
+  cudaGraph_t graph;
+  CU(cudaGraphCreate(&graph, 0));
+  mg.graph.reset(graph);
+  cudaGraphConditionalHandle loop, go, inner;
+  CU(cudaGraphConditionalHandleCreate(&mg.apply, graph, 0, cudaGraphCondAssignDefault));
+  CU(cudaGraphConditionalHandleCreate(&loop, graph, 1, cudaGraphCondAssignDefault));
+  CU(cudaGraphConditionalHandleCreate(&go, graph, 0, cudaGraphCondAssignDefault));
+  CU(cudaGraphConditionalHandleCreate(&inner, graph, 0, cudaGraphCondAssignDefault));
+  std::vector<cudaGraphNode_t> leaves;
+  auto nonzero = [&]() -> int {
+    CU(cudaMemsetAsync(c->d_flag.get(), 0, sizeof(int), c->st()));
+    return sweep(c, BP4_K_BLAS1, n, bp4::nonzero_kernel, n, (const double *)x, c->d_flag.get());
+  };
+  if (int e = capture_into(c, graph, nullptr, 0, nonzero, &leaves))
+    return e;
+  MixedArgs            a(ms, c->d_flag.get(), 0u, 0., 0., nullptr, nullptr, mg.apply);
+  cudaKernelNodeParams kp = a.params();
+  CU(cudaGraphAddKernelNode(&mg.begin, graph, leaves.data(), leaves.size(), &kp));
+  c->launches += 1;
+  cudaGraphNode_t apply_node;
+  cudaGraph_t     apply_body;
+  if (int e = add_conditional(graph, {mg.begin}, mg.apply, cudaGraphCondTypeIf, &apply_node, &apply_body))
+    return e;
+  if (int e = capture_into(c, apply_body, nullptr, 0, [&]() { return vmult_on(c, g, x); }, nullptr))
+    return e;
+  auto narrow_prec = [&]() {
+    return sweep(c, BP4_K_BLAS1, n / 3, bp4::narrow_kernel, n / 3, mg.prec, p32);
+  };
+  if (int e = capture_into(c, graph, &apply_node, 1, narrow_prec, &leaves))
+    return e;
+  cudaGraphNode_t loop_node;
+  cudaGraph_t     loop_body;
+  if (int e = add_conditional(graph, leaves, loop, cudaGraphCondTypeWhile, &loop_node, &loop_body))
+    return e;
+  // refinement step: the FP64 true residual and its check
+  auto check = [&]() -> int {
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::sadd_kernel<true>, n, g, 0., -1., mg.b, &ms->outer.g_scale))
+      return e;
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::dot_kernel<false>, n, (const double *)g, (const double *)g, acc, c->det))
+      return e;
+    Timed t(c, BP4_K_BLAS1);
+    bp4::mixed_check_kernel<<<1, 32, 0, c->st()>>>(ms, acc, loop, go);
+    CU(cudaGetLastError());
+    return 0;
+  };
+  if (int e = capture_into(c, loop_body, nullptr, 0, check, &leaves))
+    return e;
+  cudaGraphNode_t go_node;
+  cudaGraph_t     go_body;
+  if (int e = add_conditional(loop_body, leaves, go, cudaGraphCondTypeIf, &go_node, &go_body))
+    return e;
+  auto start = [&]() -> int { // r32 = s (A x - b), e = 0; sets `inner`
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::mixed_residual_kernel, n, r32, (const double *)g,
+                      (const bp4::MixedState *)ms, inner))
+      return e;
+    CU(cudaMemsetAsync(e32, 0, sizeof(float) * nl, c->st()));
+    return 0;
+  };
+  if (int e = capture_into(c, go_body, nullptr, 0, start, &leaves))
+    return e;
+  cudaGraphNode_t inner_node;
+  cudaGraph_t     inner_body;
+  if (int e = add_conditional(go_body, leaves, inner, cudaGraphCondTypeWhile, &inner_node, &inner_body))
+    return e;
+  // one FP32 merged iteration: merged_sweep's streamed form (pre, cells, post) and the scalar step
+  auto iteration = [&]() -> int {
+    bp4::SolveState *in = &ms->inner;
+    if (int e = sweep(c, BP4_K_PRE, std::max<uint64_t>(n, 1), bp4::pre_kernel<true, float>, (uint64_t)0, n, h32, e32,
+                      r32, d32, (const float *)p32, 0., 0., 0., 0., acc, c->d_update4b.get(), (const bp4::SolveState *)in))
+      return e;
+    if (c->n_ghost)
+      CU(cudaMemsetAsync(h32 + n, 0, sizeof(float) * c->n_ghost, c->st()));
+    if (int e = cell_loop_f32(c, h32, d32))
+      return e;
+    if (n)
+      if (int e = sweep(c, BP4_K_POST, n, bp4::post_kernel<false, float>, (uint64_t)0, n, (const float *)r32,
+                        (const float *)d32, (const float *)h32, (const float *)p32, acc, c->det))
+        return e;
+    Timed t(c, BP4_K_BLAS1);
+    bp4::solve_scalar_kernel<<<1, 32, 0, c->st()>>>(bp4::kSolveMergedStep, in, acc, inner);
+    CU(cudaGetLastError());
+    return 0;
+  };
+  if (int e = capture_into(c, inner_body, nullptr, 0, iteration, nullptr))
+    return e;
+  // the inner solve's pending e update, x += e / s, and A x for the next refinement step
+  auto finish = [&]() -> int {
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::solve_final_kernel<false, float>, n, e32, (const float *)d32,
+                      (const float *)r32, (const float *)p32, (const bp4::SolveState *)&ms->inner))
+      return e;
+    if (int e = sweep(c, BP4_K_BLAS1, n, bp4::mixed_update_kernel, n, x, (const float *)e32,
+                      (const bp4::MixedState *)ms))
+      return e;
+    return vmult_on(c, g, x);
+  };
+  if (int e = capture_into(c, go_body, &inner_node, 1, finish, nullptr))
+    return e;
+  auto result = [&]() -> int {
+    Timed t(c, BP4_K_BLAS1);
+    bp4::mixed_result_kernel<<<1, 32, 0, c->st()>>>(ms);
+    CU(cudaGetLastError());
+    return 0;
+  };
+  if (int e = capture_into(c, graph, &loop_node, 1, result, nullptr))
+    return e;
+  cudaGraphExec_t exec;
+  CU(cudaGraphInstantiate(&exec, graph, 0));
+  mg.exec.reset(exec);
+  return 0;
+}
+
+int bp4_solve_cg_mixed_async(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps,
+                             double tol, double reduce, bp4_mixed_result *result, double *history)
+{
+  if (!c || !result)
+    return fail(BP4_ERR_ARG, "null argument");
+  if (int e = check_len(c, x, "x"))
+    return e;
+  if (int e = check_len(c, b, "b"))
+    return e;
+  if (!prec || 3 * prec->n < c->n_owned)
+    return fail(BP4_ERR_ARG, "prec needs n_owned/3 entries");
+  if (x == b)
+    return fail(BP4_ERR_ARG, "solve: x aliases b");
+  if (int e = refuse_f32(c, "bp4_solve_cg_mixed"))
+    return e;
+  CU(cudaSetDevice(c->device));
+  if (int e = refuse_capture(c, "bp4_solve_cg_mixed"))
+    return e;
+  void *res_dev = nullptr, *hist_dev = nullptr;
+  if (int e = device_visible(c, result, "result", &res_dev))
+    return e;
+  if (history)
+    if (int e = device_visible(c, history, "history", &hist_dev))
+      return e;
+  if (!c->d_mixed)
+    CU(allocate(c->d_mixed, 1));
+  if (int e = ensure_coef32(c))
+    return e;
+  MixedGraph *mg = nullptr;
+  for (MixedGraph &e : c->mixed)
+    if (e.x == x->p() && e.b == b->p() && e.prec == prec->p())
+      mg = &e;
+  if (!mg) // the entry goes into the cache once its temporaries are allocated
+    {
+      const uint64_t nl = c->n_owned + c->n_ghost;
+      MixedGraph     ns;
+      ns.x = x->p(), ns.b = b->p(), ns.prec = prec->p();
+      if (int e = pooled_alloc(c, nl, ns.g, false))
+        return e;
+      for (dev_ptr<float> *v : {&ns.r32, &ns.d32, &ns.h32, &ns.e32})
+        CU(allocate(*v, nl));
+      CU(allocate(ns.prec32, c->n_owned / 3));
+      c->mixed.push_back(std::move(ns));
+      mg = &c->mixed.back();
+    }
+  if (!mg->exec)
+    if (int e = build_mixed_graph(c, *mg))
+      {
+        mg->graph.reset(); // a later call starts over
+        return e;
+      }
+  MixedArgs            a(c->d_mixed.get(), c->d_flag.get(), max_steps, tol, reduce, static_cast<double *>(hist_dev),
+                         res_dev, mg->apply);
+  cudaKernelNodeParams kp = a.params();
+  CU(cudaGraphExecKernelNodeSetParams(mg->exec.get(), mg->begin, &kp));
+  CU(cudaGraphLaunch(mg->exec.get(), c->st()));
+  c->launches += 1;
+  return 0;
+}
+
+int bp4_solve_cg_mixed(bp4_ctx *c, bp4_vec *x, const bp4_vec *b, const bp4_vec *prec, unsigned max_steps, double tol,
+                       double reduce, bp4_mixed_result *out)
+{
+  if (!c || !out)
+    return fail(BP4_ERR_ARG, "null argument");
+  if (!c->h_mixed)
+    {
+      if (int e = refuse_capture(c, "bp4_solve_cg_mixed"))
+        return e;
+      CU(cudaSetDevice(c->device));
+      CU(allocate(c->h_mixed, 1));
+    }
+  if (int e = bp4_solve_cg_mixed_async(c, x, b, prec, max_steps, tol, reduce, c->h_mixed.get(), nullptr))
+    return e;
+  CU(cudaStreamSynchronize(c->st()));
+  *out = *c->h_mixed;
+  return 0;
 }
 
 // ---- multi-GPU ---------------------------------------------------------------------------

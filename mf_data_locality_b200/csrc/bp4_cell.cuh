@@ -53,25 +53,38 @@ namespace bp4
     return 1.0 / x;
 #endif
   }
+  // the FP32 form: MUFU.RCP seed (~23 bits with .ftz) + one Newton step
+  BP4_HD float rcp_nobranch(const float x)
+  {
+#ifdef __CUDA_ARCH__
+    float r;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    const float e = fmaf(-x, r, 1.0f);
+    return fmaf(r, e, r);
+#else
+    return 1.0f / x;
+#endif
+  }
 
-  template <int P>
+  // T = float: the same tables rounded to float, for the FP32 cell kernel
+  template <int P, typename T = double>
   struct Tab
   {
     static constexpr int N = P + 1; // nodes per direction (GLL)
     static constexpr int Q = P + 2; // Gauss points per direction
-    double S[N][Q];                 // S[i][q]  = l_i^GLL(x_q)            (shape_values)
-    double Dn[N][Q];                // Dn[i][q] = d/dx l_i^GLL(x_q)       (= S * D)
-    double D[Q][Q];                 // D[i][q]  = d/dx l_i^Gauss(x_q)     (collocation gradient)
-    double xq[Q];                   // Gauss points on [0,1]
-    double wq[Q];                   // Gauss weights
+    T S[N][Q];                      // S[i][q]  = l_i^GLL(x_q)            (shape_values)
+    T Dn[N][Q];                     // Dn[i][q] = d/dx l_i^GLL(x_q)       (= S * D)
+    T D[Q][Q];                      // D[i][q]  = d/dx l_i^Gauss(x_q)     (collocation gradient)
+    T xq[Q];                        // Gauss points on [0,1]
+    T wq[Q];                        // Gauss weights
     // even-odd halves (the role of deal.II's shape_values_eo / shape_gradients_collocation_eo,
     // poisson_operator.h:461-463): S[i][q] = S[N-1-i][Q-1-q], D and Dn change sign under the
     // same reflection.  Xf* pair the FIRST index (used when it is contracted), Xs* the SECOND:
     //   Xfp[i][q] = (X[i][q] + X[n-1-i][q]) / 2,  Xfm[i][q] = (X[i][q] - X[n-1-i][q]) / 2
     //   Xsp[i][q] = (X[i][q] + X[i][m-1-q]) / 2,  Xsm[i][q] = (X[i][q] - X[i][m-1-q]) / 2
-    double Sfp[N][Q], Sfm[N][Q], Ssp[N][Q], Ssm[N][Q];
-    double Dnfp[N][Q], Dnfm[N][Q], Dnsp[N][Q], Dnsm[N][Q];
-    double Dfp[Q][Q], Dfm[Q][Q], Dsp[Q][Q], Dsm[Q][Q];
+    T Sfp[N][Q], Sfm[N][Q], Ssp[N][Q], Ssm[N][Q];
+    T Dnfp[N][Q], Dnfm[N][Q], Dnsp[N][Q], Dnsm[N][Q];
+    T Dfp[Q][Q], Dfm[Q][Q], Dsp[Q][Q], Dsm[Q][Q];
   };
 
   // ---------------------------------------------------------------------------------------
@@ -81,12 +94,12 @@ namespace bp4
   // mirrored outputs are E + O and SG (E - O).
   // ---------------------------------------------------------------------------------------
   // out[q] = sum_i M[i][q] in[i]   (first index contracted; Mp/Mm = M's "f" halves)
-  template <int NI, int NO, int SG>
-  BP4_HD void eo_first(const double (&Mp)[NI][NO], const double (&Mm)[NI][NO], const double (&M)[NI][NO],
-                       const double (&in)[NI], double (&out)[NO])
+  template <int NI, int NO, int SG, typename T>
+  BP4_HD void eo_first(const T (&Mp)[NI][NO], const T (&Mm)[NI][NO], const T (&M)[NI][NO], const T (&in)[NI],
+                       T (&out)[NO])
   {
     constexpr int HI = NI / 2, HO = NO / 2;
-    double        e[HI > 0 ? HI : 1], o[HI > 0 ? HI : 1];
+    T        e[HI > 0 ? HI : 1], o[HI > 0 ? HI : 1];
     BP4_UNROLL
     for (int i = 0; i < HI; ++i)
       {
@@ -96,7 +109,7 @@ namespace bp4
     BP4_UNROLL
     for (int q = 0; q < HO; ++q)
       {
-        double E = Mp[0][q] * e[0], O = Mm[0][q] * o[0];
+        T E = Mp[0][q] * e[0], O = Mm[0][q] * o[0];
         BP4_UNROLL
         for (int i = 1; i < HI; ++i)
           {
@@ -110,7 +123,7 @@ namespace bp4
       }
     if (NO % 2) // the middle output is its own mirror image: only one half contributes
       {
-        double s;
+        T s;
         if (SG > 0)
           {
             s = Mp[0][HO] * e[0];
@@ -132,12 +145,12 @@ namespace bp4
   }
 
   // out[i] = sum_q M[i][q] in[q]   (second index contracted; Mp/Mm = M's "s" halves)
-  template <int NI, int NO, int SG>
-  BP4_HD void eo_second(const double (&Mp)[NI][NO], const double (&Mm)[NI][NO], const double (&M)[NI][NO],
-                        const double (&in)[NO], double (&out)[NI])
+  template <int NI, int NO, int SG, typename T>
+  BP4_HD void eo_second(const T (&Mp)[NI][NO], const T (&Mm)[NI][NO], const T (&M)[NI][NO], const T (&in)[NO],
+                        T (&out)[NI])
   {
     constexpr int HI = NI / 2, HO = NO / 2;
-    double        e[HO > 0 ? HO : 1], o[HO > 0 ? HO : 1];
+    T        e[HO > 0 ? HO : 1], o[HO > 0 ? HO : 1];
     BP4_UNROLL
     for (int q = 0; q < HO; ++q)
       {
@@ -147,7 +160,7 @@ namespace bp4
     BP4_UNROLL
     for (int i = 0; i < HI; ++i)
       {
-        double E = Mp[i][0] * e[0], O = Mm[i][0] * o[0];
+        T E = Mp[i][0] * e[0], O = Mm[i][0] * o[0];
         BP4_UNROLL
         for (int q = 1; q < HO; ++q)
           {
@@ -161,7 +174,7 @@ namespace bp4
       }
     if (NI % 2)
       {
-        double s;
+        T s;
         if (SG > 0)
           {
             s = Mp[HI][0] * e[0];
@@ -284,26 +297,28 @@ namespace bp4
   // ---------------------------------------------------------------------------------------
   // phase 1: item = row (c, j).  dofs_row[k][i] -> work_row[{0,1,2}][qz][qx]
   // ---------------------------------------------------------------------------------------
+  template <typename T>
   struct RowIn // staged DoFs of one row, dofs_row[k*N + i]
   {
-    const double *p;
-    BP4_HD double operator()(const int kk) const { return p[kk]; }
+    const T *p;
+    BP4_HD T operator()(const int kk) const { return p[kk]; }
   };
+  template <typename T>
   struct RowOut
   {
-    double *p;
-    BP4_HD void operator()(const int kk, const double v) const { p[kk] = v; }
+    T *p;
+    BP4_HD void operator()(const int kk, const T v) const { p[kk] = v; }
   };
-  template <int P, typename In>
-  BP4_HD void phase1_io(const Tab<P> &tb, const In in, double *out)
+  template <int P, typename In, typename T>
+  BP4_HD void phase1_io(const Tab<P, T> &tb, const In in, T *out)
   {
     using G         = Geom<P>;
     constexpr int N = G::N, Q = G::Q, HN = N / 2, HQ = Q / 2;
-    double        t[N][Q];
+    T        t[N][Q];
     BP4_UNROLL
     for (int k = 0; k < N; ++k)
       {
-        double r[N];
+        T r[N];
         BP4_UNROLL
         for (int i = 0; i < N; ++i)
           r[i] = in(k * N + i);
@@ -316,7 +331,7 @@ namespace bp4
       BP4_UNROLL
     for (int q = 0; q < Q; ++q)
       {
-        const double e = t[k][q] + t[N - 1 - k][q], o = t[k][q] - t[N - 1 - k][q];
+        const T e = t[k][q] + t[N - 1 - k][q], o = t[k][q] - t[N - 1 - k][q];
         t[k][q]         = e;
         t[N - 1 - k][q] = o;
       }
@@ -324,12 +339,12 @@ namespace bp4
     for (int qz = 0; qz < (Q + 1) / 2; ++qz)
       {
         const bool mid = (Q % 2) && qz == HQ; // the middle layer is its own mirror image
-        double     uA[Q], uB[Q], zA[Q], zB[Q], sA[Q], sB[Q];
+        T     uA[Q], uB[Q], zA[Q], zB[Q], sA[Q], sB[Q];
         BP4_UNROLL
         for (int q = 0; q < Q; ++q)
           {
-            double Eu = tb.Sfp[0][qz] * t[0][q], Ou = tb.Sfm[0][qz] * t[N - 1][q];
-            double Ez = tb.Dnfp[0][qz] * t[0][q], Oz = tb.Dnfm[0][qz] * t[N - 1][q];
+            T Eu = tb.Sfp[0][qz] * t[0][q], Ou = tb.Sfm[0][qz] * t[N - 1][q];
+            T Ez = tb.Dnfp[0][qz] * t[0][q], Oz = tb.Dnfm[0][qz] * t[N - 1][q];
             BP4_UNROLL
             for (int k = 1; k < HN; ++k)
               {
@@ -392,30 +407,30 @@ namespace bp4
   // Same FMAs as phase1/phase3, (N + Q) registers of data per item, Q or N independent chains.
   // The matrix entries stay compile-time constant-bank operands: the line index only selects data.
   // ---------------------------------------------------------------------------------------
-  template <int P>
-  BP4_HD void phase1a(const Tab<P> &tb, double *row, const int k)
+  template <int P, typename T>
+  BP4_HD void phase1a(const Tab<P, T> &tb, T *row, const int k)
   {
     constexpr int N = Geom<P>::N, Q = Geom<P>::Q;
-    double        r[N];
+    T        r[N];
     BP4_UNROLL
     for (int i = 0; i < N; ++i)
       r[i] = row[k * N + i];
-    double o[Q];
+    T o[Q];
     eo_first<N, Q, 1>(tb.Sfp, tb.Sfm, tb.S, r, o);
     BP4_UNROLL
     for (int q = 0; q < Q; ++q)
       row[2 * Q * Q + k * Q + q] = o[q];
   }
 
-  template <int P>
-  BP4_HD void phase1b(const Tab<P> &tb, double *row, const int qx)
+  template <int P, typename T>
+  BP4_HD void phase1b(const Tab<P, T> &tb, T *row, const int qx)
   {
     constexpr int N = Geom<P>::N, Q = Geom<P>::Q;
-    double        t[N];
+    T        t[N];
     BP4_UNROLL
     for (int k = 0; k < N; ++k)
       t[k] = row[2 * Q * Q + k * Q + qx];
-    double su[Q], sz[Q];
+    T su[Q], sz[Q];
     eo_first<N, Q, 1>(tb.Sfp, tb.Sfm, tb.S, t, su);
     eo_first<N, Q, -1>(tb.Dnfp, tb.Dnfm, tb.Dn, t, sz);
     BP4_UNROLL
@@ -426,48 +441,48 @@ namespace bp4
       }
   }
 
-  template <int P>
-  BP4_HD void phase1c(const Tab<P> &tb, double *row, const int qz)
+  template <int P, typename T>
+  BP4_HD void phase1c(const Tab<P, T> &tb, T *row, const int qz)
   {
     constexpr int Q = Geom<P>::Q;
-    double        u[Q];
+    T        u[Q];
     BP4_UNROLL
     for (int i = 0; i < Q; ++i)
       u[i] = row[qz * Q + i];
-    double sx[Q];
+    T sx[Q];
     eo_first<Q, Q, -1>(tb.Dfp, tb.Dfm, tb.D, u, sx);
     BP4_UNROLL
     for (int q = 0; q < Q; ++q)
       row[1 * Q * Q + qz * Q + q] = sx[q];
   }
 
-  template <int P>
-  BP4_HD void phase3a(const Tab<P> &tb, double *row, const int qz)
+  template <int P, typename T>
+  BP4_HD void phase3a(const Tab<P, T> &tb, T *row, const int qz)
   {
     constexpr int Q = Geom<P>::Q;
-    double        fx[Q];
+    T        fx[Q];
     BP4_UNROLL
     for (int q = 0; q < Q; ++q)
       fx[q] = row[1 * Q * Q + qz * Q + q];
-    double d[Q];
+    T d[Q];
     eo_second<Q, Q, -1>(tb.Dsp, tb.Dsm, tb.D, fx, d);
     BP4_UNROLL
     for (int i = 0; i < Q; ++i)
       row[qz * Q + i] += d[i];
   }
 
-  template <int P>
-  BP4_HD void phase3b(const Tab<P> &tb, double *row, const int qx)
+  template <int P, typename T>
+  BP4_HD void phase3b(const Tab<P, T> &tb, T *row, const int qx)
   {
     constexpr int N = Geom<P>::N, Q = Geom<P>::Q;
-    double        v[Q], fz[Q];
+    T        v[Q], fz[Q];
     BP4_UNROLL
     for (int qz = 0; qz < Q; ++qz)
       {
         v[qz]  = row[0 * Q * Q + qz * Q + qx];
         fz[qz] = row[2 * Q * Q + qz * Q + qx];
       }
-    double sv[N], sf[N];
+    T sv[N], sf[N];
     eo_second<N, Q, 1>(tb.Ssp, tb.Ssm, tb.S, v, sv);
     eo_second<N, Q, -1>(tb.Dnsp, tb.Dnsm, tb.Dn, fz, sf);
     BP4_UNROLL
@@ -475,15 +490,15 @@ namespace bp4
       row[2 * Q * Q + k * Q + qx] = sv[k] + sf[k];
   }
 
-  template <int P>
-  BP4_HD void phase3c(const Tab<P> &tb, double *row, const int k)
+  template <int P, typename T>
+  BP4_HD void phase3c(const Tab<P, T> &tb, T *row, const int k)
   {
     constexpr int N = Geom<P>::N, Q = Geom<P>::Q;
-    double        t[Q];
+    T        t[Q];
     BP4_UNROLL
     for (int q = 0; q < Q; ++q)
       t[q] = row[2 * Q * Q + k * Q + q];
-    double o[N];
+    T o[N];
     eo_second<N, Q, 1>(tb.Ssp, tb.Ssm, tb.S, t, o);
     BP4_UNROLL
     for (int i = 0; i < N; ++i)
@@ -498,9 +513,9 @@ namespace bp4
   // form local_apply evaluates (poisson_operator.h:577-602).
   // x = xq[qx], z = xq[qz], wxz = wq[qx]*wq[qz].
   // ---------------------------------------------------------------------------------------
-  template <int P, bool QUAD = false>
-  BP4_HD void phase2(const Tab<P> &tb, const double *cf, double *work, const int qx, const int qz,
-                     const double x, const double z, const double wxz)
+  template <int P, bool QUAD = false, typename T = double>
+  BP4_HD void phase2(const Tab<P, T> &tb, const T *cf, T *work, const int qx, const int qz,
+                     const T x, const T z, const T wxz)
   {
     using G         = Geom<P>;
     constexpr int N = G::N, Q = G::Q;
@@ -512,27 +527,27 @@ namespace bp4
     //               r2 = dX/dzeta = (v9 + x v10) + y (v12 + x v13)
     //   quadratic : r0, r2 quadratic and r1 linear in y (same collapse order as the reference:
     //               xi_i = v_i + z (v_{9+i} + z v_{18+i}), di_i = v_{9+i} + 2 z v_{18+i})
-    double g00[Q], g01[Q], g02[Q], g11[Q], g12[Q], g22[Q];
+    T g00[Q], g01[Q], g02[Q], g11[Q], g12[Q], g22[Q];
     {
       constexpr int NB = QUAD ? 3 : 2; // coefficients in y of r0 and r2
-      double        A[NB][3], Cc[NB][3], R1[2][3];
+      T        A[NB][3], Cc[NB][3], R1[2][3];
       BP4_UNROLL
       for (int d = 0; d < 3; ++d)
         {
           if constexpr (!QUAD)
             {
-              const double v1 = cf[3 + d], v3 = cf[6 + d], v4 = cf[9 + d], v9 = cf[12 + d],
+              const T v1 = cf[3 + d], v3 = cf[6 + d], v4 = cf[9 + d], v9 = cf[12 + d],
                            v10 = cf[15 + d], v12 = cf[18 + d], v13 = cf[21 + d];
               A[0][d]  = v1 + z * v10;
               A[1][d]  = v4 + z * v13;
               R1[0][d] = (v3 + z * v12) + x * A[1][d];
-              R1[1][d] = 0.;
+              R1[1][d] = T(0);
               Cc[0][d] = v9 + x * v10;
               Cc[1][d] = v12 + x * v13;
             }
           else
             {
-              double xi[9], di[9];
+              T xi[9], di[9];
               BP4_UNROLL
               for (int i = 0; i < 9; ++i)
                 {
@@ -552,8 +567,8 @@ namespace bp4
       BP4_UNROLL
       for (int q = 0; q < Q; ++q)
         {
-          const double y = tb.xq[q];
-          double       r0[3], r1[3], r2[3];
+          const T y = tb.xq[q];
+          T       r0[3], r1[3], r2[3];
           BP4_UNROLL
           for (int d = 0; d < 3; ++d)
             {
@@ -572,7 +587,7 @@ namespace bp4
             }
           // columns of adj: k0 = r1 x r2, k1 = r2 x r0, k2 = r0 x r1;  det = r0 . k0
           // (the cofactor inverse of poisson_operator.h:41-63 without the division)
-          double k0[3], k1[3], k2[3];
+          T k0[3], k1[3], k2[3];
           k0[0] = r1[1] * r2[2] - r1[2] * r2[1];
           k0[1] = r1[2] * r2[0] - r1[0] * r2[2];
           k0[2] = r1[0] * r2[1] - r1[1] * r2[0];
@@ -582,9 +597,9 @@ namespace bp4
           k2[0] = r0[1] * r1[2] - r0[2] * r1[1];
           k2[1] = r0[2] * r1[0] - r0[0] * r1[2];
           k2[2] = r0[0] * r1[1] - r0[1] * r1[0];
-          const double det = r0[0] * k0[0] + r0[1] * k0[1] + r0[2] * k0[2];
+          const T det = r0[0] * k0[0] + r0[1] * k0[1] + r0[2] * k0[2];
           // == det * w * J^-1 J^-T  (poisson_operator.h:604-625)
-          const double sc = (wxz * tb.wq[q]) * rcp_nobranch(det);
+          const T sc = (wxz * tb.wq[q]) * rcp_nobranch(det);
           g00[q]          = sc * (k0[0] * k0[0] + k0[1] * k0[1] + k0[2] * k0[2]);
           g01[q]          = sc * (k0[0] * k1[0] + k0[1] * k1[1] + k0[2] * k1[2]);
           g02[q]          = sc * (k0[0] * k2[0] + k0[1] * k2[1] + k0[2] * k2[2]);
@@ -601,8 +616,8 @@ namespace bp4
 #endif
     for (int c = 0; c < 3; ++c)
       {
-        double *base = work + (c * N) * G::RW + qz * Q + qx; // rows (c, j), j = 0..N-1
-        double  gx[Q], gy[Q], gz[Q], v[Q], a0[N], a1[N], a2[N];
+        T *base = work + (c * N) * G::RW + qz * Q + qx; // rows (c, j), j = 0..N-1
+        T  gx[Q], gy[Q], gz[Q], v[Q], a0[N], a1[N], a2[N];
         BP4_UNROLL
         for (int j = 0; j < N; ++j)
           {
@@ -619,7 +634,7 @@ namespace bp4
         BP4_UNROLL
         for (int q = 0; q < Q; ++q)
           {
-            const double a = gx[q], b = gy[q], e = gz[q];
+            const T a = gx[q], b = gy[q], e = gz[q];
             gx[q] = g00[q] * a + g01[q] * b + g02[q] * e;
             gy[q] = g01[q] * a + g11[q] * b + g12[q] * e;
             gz[q] = g02[q] * a + g12[q] * b + g22[q] * e;
@@ -642,25 +657,25 @@ namespace bp4
   // ---------------------------------------------------------------------------------------
   // phase 3: item = row (c, j).  work_row[{0,1,2}][qz][qx] -> dofs_row[k][i]
   // ---------------------------------------------------------------------------------------
-  template <int P>
-  BP4_HD void phase1(const Tab<P> &tb, const double *in, double *out)
+  template <int P, typename T>
+  BP4_HD void phase1(const Tab<P, T> &tb, const T *in, T *out)
   {
-    phase1_io<P>(tb, RowIn{in}, out);
+    phase1_io<P>(tb, RowIn<T>{in}, out);
   }
 
-  template <int P, typename Out>
-  BP4_HD void phase3_io(const Tab<P> &tb, const double *in, const Out out)
+  template <int P, typename Out, typename T>
+  BP4_HD void phase3_io(const Tab<P, T> &tb, const T *in, const Out out)
   {
     using G         = Geom<P>;
     constexpr int N = G::N, Q = G::Q, HN = N / 2, HQ = Q / 2;
     // X = (even part of S^T v) + (odd part of Dn^T fz), Y = (odd of S^T v) + (even of Dn^T fz):
     // t[k] = X[k] + Y[k], t[N-1-k] = X[k] - Y[k]
-    double X[(N + 1) / 2][Q], Y[HN > 0 ? HN : 1][Q];
+    T X[(N + 1) / 2][Q], Y[HN > 0 ? HN : 1][Q];
     BP4_UNROLL
     for (int qz = 0; qz < (Q + 1) / 2; ++qz)
       {
         const bool mid = (Q % 2) && qz == HQ;
-        double     vA[Q], fA[Q], zA[Q], vB[Q], fB[Q], zB[Q], d[Q];
+        T     vA[Q], fA[Q], zA[Q], vB[Q], fB[Q], zB[Q], d[Q];
         BP4_UNROLL
         for (int q = 0; q < Q; ++q)
           {
@@ -685,18 +700,18 @@ namespace bp4
             BP4_UNROLL
             for (int q = 0; q < Q; ++q)
               {
-                const double vb = vB[q] + d[q];
-                const double ev = vA[q] + vb, ov = vA[q] - vb, ef = zA[q] + zB[q], of = zA[q] - zB[q];
+                const T vb = vB[q] + d[q];
+                const T ev = vA[q] + vb, ov = vA[q] - vb, ef = zA[q] + zB[q], of = zA[q] - zB[q];
                 BP4_UNROLL
                 for (int k = 0; k < (N + 1) / 2; ++k)
                   {
-                    const double x = tb.Ssp[k][qz] * ev + tb.Dnsm[k][qz] * of;
+                    const T x = tb.Ssp[k][qz] * ev + tb.Dnsm[k][qz] * of;
                     X[k][q]        = qz == 0 ? x : X[k][q] + x;
                   }
                 BP4_UNROLL
                 for (int k = 0; k < HN; ++k)
                   {
-                    const double y = tb.Ssm[k][qz] * ov + tb.Dnsp[k][qz] * ef;
+                    const T y = tb.Ssm[k][qz] * ov + tb.Dnsp[k][qz] * ef;
                     Y[k][q]        = qz == 0 ? y : Y[k][q] + y;
                   }
               }
@@ -718,12 +733,12 @@ namespace bp4
     BP4_UNROLL
     for (int k = 0; k < (N + 1) / 2; ++k)
       {
-        double tA[Q], tB[Q], o[N];
+        T tA[Q], tB[Q], o[N];
         BP4_UNROLL
         for (int q = 0; q < Q; ++q)
           {
             tA[q] = k < HN ? X[k][q] + Y[k < HN ? k : 0][q] : X[k][q];
-            tB[q] = k < HN ? X[k][q] - Y[k < HN ? k : 0][q] : 0.;
+            tB[q] = k < HN ? X[k][q] - Y[k < HN ? k : 0][q] : T(0);
           }
         eo_second<N, Q, 1>(tb.Ssp, tb.Ssm, tb.S, tA, o);
         BP4_UNROLL
@@ -739,9 +754,9 @@ namespace bp4
       }
   }
 
-  template <int P>
-  BP4_HD void phase3(const Tab<P> &tb, const double *in, double *out)
+  template <int P, typename T>
+  BP4_HD void phase3(const Tab<P, T> &tb, const T *in, T *out)
   {
-    phase3_io<P>(tb, in, RowOut{out});
+    phase3_io<P>(tb, in, RowOut<T>{out});
   }
 } // namespace bp4

@@ -14,16 +14,37 @@ namespace bp4
   // matrix entry becomes a c[bank][offset] operand of a DFMA, no load instruction
   template <int P>
   __constant__ Tab<P> c_tab;
+  // instantiated here, ahead of the float tables, so that the FP64 tables keep their constant-bank
+  // offsets (and the FP64 kernels their code) whatever the FP32 kernel adds
+  template __constant__ Tab<2> c_tab<2>;
+  template __constant__ Tab<3> c_tab<3>;
+  template __constant__ Tab<4> c_tab<4>;
+  template __constant__ Tab<5> c_tab<5>;
+  template __constant__ Tab<6> c_tab<6>;
+  template __constant__ Tab<7> c_tab<7>;
+  template __constant__ Tab<8> c_tab<8>;
+  // the same tables rounded to float, for the FP32 kernel (a second constant bank)
+  template <int P>
+  __constant__ Tab<P, float> c_tab32;
 
-  template <int P, int CPB, int NC>
-  __device__ __forceinline__ void load_tables(CellSmem<P, CPB, NC> &sm, const uint32_t *dtab)
+  template <int P, typename T>
+  __device__ __forceinline__ const Tab<P, T> &ctab()
+  {
+    if constexpr (sizeof(T) == 4)
+      return c_tab32<P>;
+    else
+      return c_tab<P>;
+  }
+
+  template <int P, int CPB, int NC, typename T>
+  __device__ __forceinline__ void load_tables(CellSmem<P, CPB, NC, T> &sm, const uint32_t *dtab)
   {
     for (int i = threadIdx.x; i < Geom<P>::DOF; i += blockDim.x)
       sm.dtab[i] = dtab[i];
     if (threadIdx.x < Geom<P>::Q)
       {
-        sm.xq[threadIdx.x] = c_tab<P>.xq[threadIdx.x];
-        sm.wq[threadIdx.x] = c_tab<P>.wq[threadIdx.x];
+        sm.xq[threadIdx.x] = ctab<P, T>().xq[threadIdx.x];
+        sm.wq[threadIdx.x] = ctab<P, T>().wq[threadIdx.x];
       }
     if (threadIdx.x < 8)
       sm.red[threadIdx.x] = 0.;
@@ -68,13 +89,13 @@ namespace bp4
   // Phase 2 as a real call for the high degrees: its ~100 live doubles get a register allocation
   // of their own instead of competing with whatever the gather/scatter code around it keeps
   // alive (the inlined form spilled 2.6x more after an unrelated change to the gather).
-  template <int P, bool QUAD>
+  template <int P, bool QUAD, typename T>
   __device__ __noinline__ void phase2_call(const uint32_t cf_off, const uint32_t work_off, const int qx,
-                                           const int qz, const double x, const double z, const double wxz)
+                                           const int qz, const T x, const T z, const T wxz)
   {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    phase2<P, QUAD>(c_tab<P>, reinterpret_cast<const double *>(smem_raw + cf_off),
-              reinterpret_cast<double *>(smem_raw + work_off), qx, qz, x, z, wxz);
+    phase2<P, QUAD>(ctab<P, T>(), reinterpret_cast<const T *>(smem_raw + cf_off),
+              reinterpret_cast<T *>(smem_raw + work_off), qx, qz, x, z, wxz);
   }
 
   // i / 3 for 32-bit i without an integer division
@@ -134,19 +155,22 @@ namespace bp4
   // pre_kernel / post_kernel stream them before / after this kernel.  The scalars of
   // do_cg_update4b are the ones pre_kernel derived and left in *a.scalars, from the caller's
   // arguments or from the solver state of a device-resident solve.
+  //
+  // T = float: the FP32 plain kernel of the mixed-precision solve -- the same code with float work
+  // rows, coefficients, tables and phase-2 arithmetic, and float REDs in the scatter.
   // ---------------------------------------------------------------------------------------
-  template <int P, int CPB, bool FUSED, bool QUAD>
-  __global__ void __launch_bounds__(kThreads, Cfg<P>::BLOCKS) cell_kernel(const CellArgs a)
+  template <int P, int CPB, bool FUSED, bool QUAD, typename T = double>
+  __global__ void __launch_bounds__(kThreads, Cfg<P, QUAD, T>::BLOCKS) cell_kernel(const CellArgsT<T> a)
   {
     constexpr int NC = Cfg<P, QUAD>::NCOEF;
     using G         = Geom<P>;
     constexpr int Q = G::Q;
     constexpr bool kFine = Cfg<P>::FINE;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    CellSmem<P, CPB, NC> &sm  = *reinterpret_cast<CellSmem<P, CPB, NC> *>(smem_raw);
-    const int             tid = threadIdx.x;
-    const Tab<P>         &tb  = c_tab<P>;
-    load_tables<P, CPB, NC>(sm, a.dtab);
+    CellSmem<P, CPB, NC, T> &sm  = *reinterpret_cast<CellSmem<P, CPB, NC, T> *>(smem_raw);
+    const int                tid = threadIdx.x;
+    const Tab<P, T>         &tb  = ctab<P, T>();
+    load_tables<P, CPB, NC, T>(sm, a.dtab);
     BP4_TICK_INIT
     // ---- work list of this block: a unit is one batch (plain) or the batches
     // [unit_batch[u], unit_batch[u+1]) of whole ranges (fused).  Units are claimed dynamically
@@ -160,7 +184,7 @@ namespace bp4
       bool     valid;
     };
     const uint32_t n_units = FUSED ? a.n_units : (uint32_t)((a.n_cells + CPB - 1) / CPB);
-    const bool     dynamic = Cfg<P>::DYNAMIC && a.sched != nullptr;
+    const bool     dynamic = Cfg<P, QUAD, T>::DYNAMIC && a.sched != nullptr;
     auto           unit_at = [&](const uint32_t j) {
       return dynamic ? sm.units[j & 7u] : blockIdx.x + j * gridDim.x;
     };
@@ -212,7 +236,7 @@ namespace bp4
     // metadata items of a batch handled by this thread: at most ME indices and MC coefficients
     constexpr int ME = (CPB * 27 + kThreads - 1) / kThreads, MC = (CPB * NC + kThreads - 1) / kThreads;
     uint32_t      me[ME];
-    double        mc[MC];
+    T             mc[MC];
     auto          fetch_meta = [&](const uint32_t cell0, const int nc) {
 #pragma unroll
       for (int u = 0; u < ME; ++u)
@@ -224,7 +248,7 @@ namespace bp4
       for (int u = 0; u < MC; ++u)
         {
           const int k = tid + u * kThreads;
-          mc[u]       = k < nc * NC ? __ldg(a.coef + (uint64_t)cell0 * NC + k) : 0.;
+          mc[u]       = k < nc * NC ? __ldg(a.coef + (uint64_t)cell0 * NC + k) : T(0);
         }
     };
     auto park_meta = [&](const int bf) {
@@ -275,12 +299,12 @@ namespace bp4
     // The fused kernel reads the direction with plain loads, not ld.global.nc: it was written by
     // this block's own do_cg_update4b moments ago (the L1 sees the stores of its own SM, every
     // other DoF the block reads is constant during the kernel).
-    constexpr bool kPipe = Cfg<P>::PIPE_GATHER;
+    constexpr bool kPipe = Cfg<P, QUAD, T>::PIPE_GATHER;
     constexpr int R = (G::DOF + kThreads - 1) / kThreads, S = CPB * R;
     // only the last r can run past the end of the cell
     const bool last_on = tid < G::DOF - (R - 1) * kThreads;
     auto       on      = [&](const int r) { return r < R - 1 || last_on; };
-    double     gv[S];
+    T          gv[S];
     auto       gather_issue = [&](const int bf) {
       uint32_t tt[R], idx[S];
 #pragma unroll
@@ -295,7 +319,7 @@ namespace bp4
         }
 #pragma unroll
       for (int s1 = 0; s1 < S; ++s1)
-        gv[s1] = idx[s1] != 0xFFFFFFFFu ? (FUSED ? a.src[idx[s1]] : __ldg(a.src + idx[s1])) : 0.;
+        gv[s1] = idx[s1] != 0xFFFFFFFFu ? (FUSED ? a.src[idx[s1]] : __ldg(a.src + idx[s1])) : T(0);
     };
     auto gather_store = [&]() {
       uint32_t tt[R];
@@ -321,7 +345,7 @@ namespace bp4
 #pragma unroll
       for (int s0 = 0; s0 < S; s0 += SU)
         {
-          double   v[SU];
+          T        v[SU];
           uint32_t adr[SU];
 #pragma unroll
           for (int u = 0; u < SU; ++u)
@@ -375,7 +399,7 @@ namespace bp4
           const int cell = it / G::ITEMS2, r = it % G::ITEMS2;
           const int qz = r / Q, qx = r % Q;
           if constexpr (Cfg<P>::P2_CALL)
-            phase2_call<P, QUAD>((uint32_t)((const unsigned char *)sm.coef[bf][cell] - smem_raw),
+            phase2_call<P, QUAD, T>((uint32_t)((const unsigned char *)sm.coef[bf][cell] - smem_raw),
                                  (uint32_t)((const unsigned char *)(sm.work + cell * G::WORK) - smem_raw), qx, qz,
                                  sm.xq[qx], sm.xq[qz], sm.wq[qx] * sm.wq[qz]);
           else
@@ -879,22 +903,23 @@ namespace bp4
   // ---------------------------------------------------------------------------------------
   // launchers
   // ---------------------------------------------------------------------------------------
-  // One instance of the cell kernel and its dynamic shared memory.  A degree has three: plain
-  // tri-linear, plain quadratic, and fused tri-linear if Stage<P>::OK (its staging rows follow the
-  // cell rows).
-  template <int P, bool FUSED, bool QUAD>
+  // One instance of the cell kernel and its dynamic shared memory.  A degree has five: plain
+  // tri-linear, plain quadratic, fused tri-linear if Stage<P>::OK (its staging rows follow the
+  // cell rows), and the FP32 plain tri-linear and quadratic ones.
+  template <int P, bool FUSED, bool QUAD, typename T = double>
   struct CellInstance
   {
-    static constexpr int CPB  = Cfg<P, QUAD>::CPB;
-    static constexpr int SMEM = (int)(sizeof(CellSmem<P, CPB, Cfg<P, QUAD>::NCOEF>) +
+    static constexpr int CPB  = Cfg<P, QUAD, T>::CPB;
+    static constexpr int SMEM = (int)(sizeof(CellSmem<P, CPB, Cfg<P, QUAD>::NCOEF, T>) +
                                       (FUSED ? sizeof(JobSmem<Stage<P>::JOB>) : 0));
     static cudaError_t init()
     {
-      return cudaFuncSetAttribute(cell_kernel<P, CPB, FUSED, QUAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+      return cudaFuncSetAttribute(cell_kernel<P, CPB, FUSED, QUAD, T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  SMEM);
     }
-    static void launch(const int grid, const CellArgs &a, cudaStream_t st)
+    static void launch(const int grid, const CellArgsT<T> &a, cudaStream_t st)
     {
-      cell_kernel<P, CPB, FUSED, QUAD><<<grid, kThreads, SMEM, st>>>(a);
+      cell_kernel<P, CPB, FUSED, QUAD, T><<<grid, kThreads, SMEM, st>>>(a);
     }
   };
 
@@ -905,25 +930,39 @@ namespace bp4
     fill_tab<P>(tb);
     walk.resize(Geom<P>::DOF);
     build_dof_table<P>(walk.data());
+    // the FP32 tables: every entry of the FP64 ones rounded to float
+    Tab<P, float> tb32;
+    const double *from = &tb.S[0][0];
+    float        *to   = &tb32.S[0][0];
+    static_assert(sizeof(tb) == 2 * sizeof(tb32), "Tab<P> is an array of doubles");
+    for (size_t i = 0; i < sizeof(tb32) / sizeof(float); ++i)
+      to[i] = (float)from[i];
     cudaError_t e = cudaMemcpyToSymbol(c_tab<P>, &tb, sizeof(tb));
+    if (e == cudaSuccess)
+      e = cudaMemcpyToSymbol(c_tab32<P>, &tb32, sizeof(tb32));
     if (e == cudaSuccess)
       e = CellInstance<P, false, false>::init();
     if (e == cudaSuccess)
       e = CellInstance<P, false, true>::init();
+    if (e == cudaSuccess)
+      e = CellInstance<P, false, false, float>::init();
+    if (e == cudaSuccess)
+      e = CellInstance<P, false, true, float>::init();
     if constexpr (Stage<P>::OK)
       if (e == cudaSuccess)
         e = CellInstance<P, true, false>::init();
     return e;
   }
 
-  template <int P>
-  static cudaError_t run_cell(const bool fused, const bool quad, const CellArgs &a, int sms, cudaStream_t st)
+  template <int P, typename T>
+  static cudaError_t run_cell(const bool fused, const bool quad, const CellArgsT<T> &a, int sms, cudaStream_t st)
   {
-    constexpr int  CPB = Cfg<P>::CPB, CPBQ = Cfg<P, true>::CPB;
-    if (fused && (quad || !Stage<P>::OK))
+    constexpr bool F64 = sizeof(T) == 8;
+    constexpr int  CPB = Cfg<P, false, T>::CPB, CPBQ = Cfg<P, true, T>::CPB;
+    if (fused && (quad || !Stage<P>::OK || !F64))
       return cudaErrorInvalidValue;
     const uint64_t units = fused ? a.n_units : (a.n_cells + (quad ? CPBQ : CPB) - 1) / (quad ? CPBQ : CPB);
-    const int      grid  = (int)std::min<uint64_t>(units, (uint64_t)sms * Cfg<P>::BLOCKS);
+    const int      grid  = (int)std::min<uint64_t>(units, (uint64_t)sms * Cfg<P, false, T>::BLOCKS);
     if (grid == 0)
       return cudaSuccess;
 #ifdef BP4_PHASE_TIMING
@@ -938,13 +977,13 @@ namespace bp4
 #endif
     if (fused)
       {
-        if constexpr (Stage<P>::OK)
+        if constexpr (Stage<P>::OK && F64)
           CellInstance<P, true, false>::launch(grid, a, st);
       }
     else if (quad)
-      CellInstance<P, false, true>::launch(grid, a, st);
+      CellInstance<P, false, true, T>::launch(grid, a, st);
     else
-      CellInstance<P, false, false>::launch(grid, a, st);
+      CellInstance<P, false, false, T>::launch(grid, a, st);
 #ifdef BP4_PHASE_TIMING
     if (d_trace)
       {
@@ -1000,6 +1039,13 @@ namespace bp4
   cudaError_t launch_cell(int degree, bool fused, bool quad, const CellArgs &a, int sms, cudaStream_t st)
   {
 #define CALL(P) run_cell<P>(fused, quad, a, sms, st)
+    BP4_DISPATCH(degree, CALL)
+#undef CALL
+  }
+
+  cudaError_t launch_cell_f32(int degree, bool quad, const CellArgsT<float> &a, int sms, cudaStream_t st)
+  {
+#define CALL(P) run_cell<P>(false, quad, a, sms, st)
     BP4_DISPATCH(degree, CALL)
 #undef CALL
   }

@@ -20,18 +20,22 @@ namespace bp4
   constexpr int kBlocksPerSM = 2;
 
   // Every per-degree choice of the cell kernel, each one measured on B200 (DESIGN.md 4.1-4.2, 6).
-  // QUAD: all 27 geometry coefficients per cell (81 doubles) instead of the 8 tri-linear ones (24)
-  template <int P, bool QUAD = false>
+  // QUAD: all 27 geometry coefficients per cell (81 values) instead of the 8 tri-linear ones (24)
+  // T: the scalar type of the work rows, coefficients, tables and scatter (float: the FP32 kernel of
+  // the mixed-precision solve, DESIGN.md 4.7; plain instances only)
+  template <int P, bool QUAD = false, typename T = double>
   struct Cfg
   {
     using G = Geom<P>;
     static constexpr int NCOEF = QUAD ? 81 : 24;
     // resident blocks per SM of the cell kernel: three (<= 168 registers, smaller batches)
-    // measured faster at Q2 (+12 %) and Q6 (+13 %), slower or equal elsewhere
-    static constexpr int BLOCKS   = (P == 2 || P == 6) ? 3 : kBlocksPerSM;
+    // measured faster at Q2 (+12 %) and Q6 (+13 %), slower or equal elsewhere.  FP32: three at every
+    // degree (121-168 registers, no spills): 15-18 % faster than two at Q3-Q5 and Q8, 2.6 % at Q7;
+    // two is 24 % / 20 % slower at Q2 / Q6 (DESIGN.md 4.7)
+    static constexpr int BLOCKS   = (P == 2 || P == 6 || sizeof(T) == 4) ? 3 : kBlocksPerSM;
     static constexpr int budget   = (227 * 1024) / BLOCKS - 512;
-    static constexpr int per_cell = (G::WORK + 2 * NCOEF) * 8 + 2 * 28 * 4;
-    static constexpr int fit      = (budget - 4 * G::DOF - 16 * G::Q - 256) / per_cell;
+    static constexpr int per_cell = (G::WORK + 2 * NCOEF) * (int)sizeof(T) + 2 * 28 * 4;
+    static constexpr int fit      = (budget - 4 * G::DOF - 2 * (int)sizeof(T) * G::Q - 256) / per_cell;
     // phase 2 carries ~2/3 of the FP64 work: prefer Q^2*CPB close to two rounds of the block
     static constexpr int want = (2 * kThreads) / (G::Q * G::Q) > 0 ? (2 * kThreads) / (G::Q * G::Q) : 1;
     static constexpr int CPB  = fit < 1 ? 1 : (fit < want ? fit : want);
@@ -41,11 +45,14 @@ namespace bp4
     // phase 2 called out of line (phase2_call)
     static constexpr bool P2_CALL = P >= 6;
     // the gather of batch i+1 is in flight during the scatter of batch i
-    static constexpr bool PIPE_GATHER = P <= 4;
+    // FP32 (three blocks): also at Q5 and Q6 (-1.7 / -1.3 %), not at Q7 / Q8 (+0.5 / +2.4 %)
+    static constexpr bool PIPE_GATHER = P <= 4 || (sizeof(T) == 4 && P <= 6);
     // batches / units are claimed from an atomic counter instead of strided.  Measured on B200
     // (operator apply at ~50-100 M DoFs): Q2 +13 %, Q3 +5 %, Q4 +8 %, Q5 +11 %; Q6 -6 %, Q7 -11 %,
-    // Q8 -10 % (the claim bookkeeping makes the register-starved high-degree kernels spill)
-    static constexpr bool DYNAMIC = P <= 5;
+    // Q8 -10 % (the claim bookkeeping makes the register-starved high-degree kernels spill).
+    // FP32, which does not spill, with three blocks: claimed units are faster at Q8 (-3.6 %) and slower
+    // at Q6 / Q7 (+0.3 / +9.8 %)
+    static constexpr bool DYNAMIC = P <= 5 || (sizeof(T) == 4 && P == 8);
     // a fused cell kernel (in-loop vector updates staged through shared memory) is built; see Stage
     static constexpr bool STAGED = P <= 4;
     // the form of vmult_with_merged_sums a context starts with when it has private DoF runs:
@@ -56,16 +63,16 @@ namespace bp4
     static constexpr bool FUSED_DEFAULT = P == 4;
   };
 
-  template <int P, int CPB, int NCOEF = 24>
+  template <int P, int CPB, int NCOEF = 24, typename T = double>
   struct alignas(16) CellSmem
   {
     using G = Geom<P>;
     // the gathered DoFs, the three phases and the result all live in the work rows: gather
     // fills the first N*N slots of each row, phases 1 and 3 run in place
-    double   work[CPB * G::WORK];
-    double   coef[2][CPB][NCOEF]; // double-buffered: the next batch's metadata is prefetched
-    double   xq[G::Q];
-    double   wq[G::Q];
+    T        work[CPB * G::WORK];
+    T        coef[2][CPB][NCOEF]; // double-buffered: the next batch's metadata is prefetched
+    T        xq[G::Q];
+    T        wq[G::Q];
     double   red[8];           // (spare)
     uint32_t units[8];         // ring of the units this block has claimed
     uint32_t n_claimed;
@@ -159,14 +166,16 @@ namespace bp4
     return u;
   }
 
-  struct CellArgs
+  // T = float: the FP32 plain kernel (src, dst and the coefficients in float; no fused fields)
+  template <typename T>
+  struct CellArgsT
   {
     const uint32_t *entity_index; // [n_cells][27]
-    const double   *coef;         // [n_cells][24] tri-linear or [n_cells][81] quadratic coefficients
+    const T        *coef;         // [n_cells][24] tri-linear or [n_cells][81] quadratic coefficients
     const uint32_t *dtab;         // [3 N^3] gather/scatter table (build_dof_table)
     uint64_t        n_cells;      // plain: cells of this launch, batches are cut on the fly
-    const double   *src;          // plain: input vector; fused: the search direction d (= p)
-    double         *dst;          // plain: output vector; fused: h
+    const T        *src;          // plain: input vector; fused: the search direction d (= p)
+    T              *dst;          // plain: output vector; fused: h
     uint32_t       *sched;        // unit counter of this launch (zero at launch), null: strided
     // ---- fused (vmult_with_merged_sums) only ----
     const BatchDesc *batch;       // batches of all units
@@ -177,6 +186,7 @@ namespace bp4
     const Update4b  *scalars;     // written by the pre_kernel launched before this kernel
     double          *acc;         // [7]
   };
+  using CellArgs = CellArgsT<double>;
 
   // Solver state of a device-resident CG solve (bp4_solve_cg / bp4_solve_cg_merged), one block
   // per context.  The scalar kernels write it, the vector kernels of the next sweep read it.

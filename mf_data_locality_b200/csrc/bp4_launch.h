@@ -21,5 +21,7 @@ namespace bp4
   // plain: a.n_cells cells from a.entity_index on; fused: a.n_units units of a.unit_batch;
   // quad: a.coef holds all 27 coefficients per cell (plain kernel only)
   cudaError_t launch_cell(int degree, bool fused, bool quad, const CellArgs &a, int sms, cudaStream_t st);
+  // the FP32 plain kernel: a.src, a.dst and a.coef in float (the float copy of the coefficients)
+  cudaError_t launch_cell_f32(int degree, bool quad, const CellArgsT<float> &a, int sms, cudaStream_t st);
   void        gll_table(int degree, std::vector<double> &out);
 } // namespace bp4

@@ -128,11 +128,12 @@ namespace bp4
   // Also clears the reduction scratch of this iteration (stream order: before any post) and leaves
   // its scalars in *scalars for the fused cell kernel that follows.
   // DEV: the four scalars come from the solver state of a device-resident solve (st).
-  template <bool DEV>
+  // T = float: the vectors of the inner FP32 solve of bp4_solve_cg_mixed (the scalars stay double)
+  template <bool DEV, typename T = double>
   __global__ void __launch_bounds__(256) pre_kernel(const uint64_t begin, const uint64_t end,
-                                                    double *__restrict__ h, double *__restrict__ x,
-                                                    double *__restrict__ r, double *__restrict__ p,
-                                                    const double *__restrict__ prec,
+                                                    T *__restrict__ h, T *__restrict__ x,
+                                                    T *__restrict__ r, T *__restrict__ p,
+                                                    const T *__restrict__ prec,
                                                     const double alpha, const double beta,
                                                     const double alpha_old, const double beta_old,
                                                     double *acc_to_zero, Update4b *scalars,
@@ -150,17 +151,17 @@ namespace bp4
     constexpr int U = 4;
     for (uint64_t i0 = begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < end; i0 += U * stride)
       {
-        double pr[U], ri[U], pi[U], hi[U], xi[U];
+        T pr[U], ri[U], pi[U], hi[U], xi[U];
 #pragma unroll
         for (int u = 0; u < U; ++u)
           {
             const uint64_t i  = i0 + u * stride;
             const bool     ok = i < end;
-            pr[u] = ok ? prec[i / 3] : 0.;
-            ri[u] = ok ? r[i] : 0.;
-            pi[u] = ok && !sc.first ? p[i] : 0.;
-            hi[u] = ok && !sc.first ? h[i] : 0.;
-            xi[u] = ok && sc.update_x ? x[i] : 0.;
+            pr[u] = ok ? prec[i / 3] : T(0);
+            ri[u] = ok ? r[i] : T(0);
+            pi[u] = ok && !sc.first ? p[i] : T(0);
+            hi[u] = ok && !sc.first ? h[i] : T(0);
+            xi[u] = ok && sc.update_x ? x[i] : T(0);
           }
 #pragma unroll
         for (int u = 0; u < U; ++u)
@@ -178,20 +179,21 @@ namespace bp4
                     r[i] = rn;
                     p[i] = sc.beta * pi[u] - pr[u] * rn;
                   }
-                h[i] = 0.;
+                h[i] = T(0);
               }
           }
       }
   }
 
   // do_cg_update3b<3,double>, solver_cg_optimized.h:12-61, over [begin, end) -> acc[7]
-  // DET: ordered cross-block sum (block_accumulate_ordered) instead of atomics
-  template <bool DET>
+  // DET: ordered cross-block sum (block_accumulate_ordered) instead of atomics.  T = float: FP32
+  // vectors, the sums still accumulated in double
+  template <bool DET, typename T = double>
   __global__ void __launch_bounds__(256) post_kernel(const uint64_t begin, const uint64_t end,
-                                                     const double *__restrict__ r,
-                                                     const double *__restrict__ d,
-                                                     const double *__restrict__ h,
-                                                     const double *__restrict__ prec, double *acc,
+                                                     const T *__restrict__ r,
+                                                     const T *__restrict__ d,
+                                                     const T *__restrict__ h,
+                                                     const T *__restrict__ prec, double *acc,
                                                      const DetSlots ds)
   {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -201,16 +203,16 @@ namespace bp4
     constexpr int U = 4;
     for (uint64_t i0 = begin + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < end; i0 += U * stride)
       {
-        double rr[U], dd[U], hh[U], pp[U];
+        T rr[U], dd[U], hh[U], pp[U];
 #pragma unroll
         for (int u = 0; u < U; ++u)
           {
             const uint64_t i  = i0 + u * stride;
             const bool     ok = i < end;
-            rr[u] = ok ? r[i] : 0.;
-            dd[u] = ok ? d[i] : 0.;
-            hh[u] = ok ? h[i] : 0.;
-            pp[u] = ok ? prec[i / 3] : 0.;
+            rr[u] = ok ? r[i] : T(0);
+            dd[u] = ok ? d[i] : T(0);
+            hh[u] = ok ? h[i] : T(0);
+            pp[u] = ok ? prec[i / 3] : T(0);
           }
 #pragma unroll
         for (int u = 0; u < U; ++u)
@@ -219,9 +221,9 @@ namespace bp4
     accumulate<DET>(s, acc, ds);
   }
 
+  template <typename T>
   __global__ void __launch_bounds__(256) fixup_kernel(const uint64_t n, const uint32_t *__restrict__ con,
-                                                      double *__restrict__ dst,
-                                                      const double *__restrict__ src)
+                                                      T *__restrict__ dst, const T *__restrict__ src)
   {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n)
@@ -527,12 +529,13 @@ namespace bp4
 
   // the pending x update of SolverCGFullMerge after its last iteration
   // (solver_cg_optimized.h:256-288): odd step x += alpha d, even step bp4_x_finalize_even's formula.
-  // DET: the odd step rounded as bp4_add rounds it (see cg_xg_kernel)
-  template <bool DET>
-  __global__ void __launch_bounds__(256) solve_final_kernel(const uint64_t n, double *__restrict__ x,
-                                                            const double *__restrict__ d,
-                                                            const double *__restrict__ g,
-                                                            const double *__restrict__ prec,
+  // DET: the odd step rounded as bp4_add rounds it (see cg_xg_kernel).  T = float: the inner FP32
+  // solve of bp4_solve_cg_mixed
+  template <bool DET, typename T = double>
+  __global__ void __launch_bounds__(256) solve_final_kernel(const uint64_t n, T *__restrict__ x,
+                                                            const T *__restrict__ d,
+                                                            const T *__restrict__ g,
+                                                            const T *__restrict__ prec,
                                                             const SolveState *st)
   {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -549,6 +552,144 @@ namespace bp4
     const double c2 = __ddiv_rn(st->alpha_old, st->beta_old), c1 = __dadd_rn(alpha, c2);
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
       x[i] += c1 * d[i] + c2 * prec[i / 3] * g[i];
+  }
+
+  // ---------------------------------------------------------------------------------------
+  // mixed-precision solve (bp4_solve_cg_mixed): FP64 refinement around an inner FP32 merged CG
+  // ---------------------------------------------------------------------------------------
+  // The inner FP32 solve stops at this relative reduction of its residual (DESIGN.md 4.7)
+  constexpr double kMixedInnerReduce = 1e-3;
+
+  // Solver state of a mixed solve, one block per context.  `outer` is the FP64 ReductionControl on
+  // the true residual |b - A x| (step = refinement step); `inner` the state of the FP32 merged CG,
+  // which the scalar kernels of the device-resident merged solve drive unchanged.
+  struct MixedState
+  {
+    SolveState outer, inner;
+    double     scale;       // 1 / |b - A x| of the current refinement step
+    uint32_t   inner_steps; // inner iterations of the finished refinement steps
+    int32_t    checked;     // step 0 has been checked
+  };
+
+  // first node of a mixed solve: the per-call arguments (replaced per launch, as solve_begin_kernel's)
+  __global__ void mixed_begin_kernel(MixedState *msp, const int *nonzero, const uint32_t max_steps, const double tol,
+                                     const double reduce, double *history, void *result,
+                                     const cudaGraphConditionalHandle apply)
+  {
+    if (threadIdx.x != 0)
+      return;
+    MixedState ms{};
+    ms.outer.max_steps = max_steps;
+    ms.outer.tol       = tol;
+    ms.outer.reduce    = reduce;
+    ms.outer.history   = history;
+    ms.outer.result    = result;
+    ms.outer.g_scale   = *nonzero ? 1. : 0.;
+    *msp               = ms;
+    cudaGraphSetConditional(apply, *nonzero ? 1u : 0u);
+  }
+
+  // ReductionControl::check on the FP64 true residual (|g|^2 in acc[0], g = A x - b), once per
+  // refinement step, plus the two rules of the refinement: a step that does not reduce the residual
+  // (stagnation) and a used-up inner step budget end the solve with state 2.  Continuing: the inner
+  // solve gets a fresh state (zero start, the remaining budget, the fixed relative reduction of a
+  // right-hand side of norm 1) and `go` runs the refinement body; `loop` is the outer WHILE.
+  __global__ void mixed_check_kernel(MixedState *msp, double *acc, const cudaGraphConditionalHandle loop,
+                                     const cudaGraphConditionalHandle go)
+  {
+    if (threadIdx.x != 0)
+      return;
+    MixedState  &ms  = *msp;
+    SolveState  &st  = ms.outer;
+    const double res = __dsqrt_rn(acc[0]);
+    acc[0]           = 0.;
+    uint32_t step    = 0;
+    int      state;
+    if (!ms.checked)
+      {
+        ms.checked       = 1;
+        st.reduced_tol   = __dmul_rn(res, st.reduce);
+        st.initial_value = res;
+      }
+    else
+      {
+        step = st.step + 1;
+        ms.inner_steps += ms.inner.step;
+      }
+    const double prev = st.last_value;
+    st.step           = step;
+    st.last_value     = res;
+    if (st.history)
+      st.history[step] = res;
+    if (res < st.reduced_tol || res <= st.tol)
+      state = 1;
+    else if (isnan(res) || ms.inner_steps >= st.max_steps || (step > 0 && !(res < prev)))
+      state = 2;
+    else
+      state = 0;
+    st.state = state;
+    if (state == 0)
+      {
+        ms.scale   = __drcp_rn(res);
+        st.g_scale = 1.; // the refinement body leaves A x in g
+        SolveState in{};
+        in.max_steps   = st.max_steps - ms.inner_steps;
+        in.reduced_tol = kMixedInnerReduce;
+        ms.inner       = in;
+      }
+    cudaGraphSetConditional(loop, state == 0 ? 1u : 0u);
+    cudaGraphSetConditional(go, state == 0 ? 1u : 0u);
+  }
+
+  // r32 = (float)(s (A x - b)) = the inner solve's starting residual (the merged CG's g = A e - rhs at
+  // e = 0 for rhs = s (b - A x)), s = 1 / |b - A x|: O(1) at every refinement step.  Sets `inner`
+  // (the WHILE node that follows it in the same body) to run.
+  __global__ void __launch_bounds__(256) mixed_residual_kernel(const uint64_t n, float *__restrict__ r32,
+                                                               const double *__restrict__ g, const MixedState *ms,
+                                                               const cudaGraphConditionalHandle inner)
+  {
+    const double   s      = ms->scale;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      r32[i] = (float)(s * g[i]);
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+      cudaGraphSetConditional(inner, 1u);
+  }
+
+  // x += (double) e32 / s: the inner correction scaled back (1 / s = the residual it was made for)
+  __global__ void __launch_bounds__(256) mixed_update_kernel(const uint64_t n, double *__restrict__ x,
+                                                             const float *__restrict__ e32, const MixedState *ms)
+  {
+    const double   res    = ms->outer.last_value;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      x[i] += (double)e32[i] * res;
+  }
+
+  // last node of a mixed solve: the outcome to the caller's bp4_mixed_result
+  __global__ void mixed_result_kernel(const MixedState *ms)
+  {
+    if (threadIdx.x == 0)
+      *static_cast<bp4_mixed_result *>(ms->outer.result) = bp4_mixed_result{
+        ms->outer.state, ms->outer.step, ms->inner_steps, ms->outer.last_value, ms->outer.initial_value};
+  }
+
+  // out = (float) in: the preconditioner of the inner solve, and the FP32 operator's input (debug hook)
+  __global__ void __launch_bounds__(256) narrow_kernel(const uint64_t n, const double *__restrict__ in,
+                                                       float *__restrict__ out)
+  {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      out[i] = (float)in[i];
+  }
+
+  // out = (double) in: the FP32 operator's output (debug hook)
+  __global__ void __launch_bounds__(256) widen_kernel(const uint64_t n, const float *__restrict__ in,
+                                                      double *__restrict__ out)
+  {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+      out[i] = (double)in[i];
   }
 
   // inverse diagonal of the scalar GLL(p+1) Laplacian (poisson_operator.h:392-426): one
